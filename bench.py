@@ -1,9 +1,10 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/sec of the fused rollout (+ policy act) hot path, TRPO update ms, roofline.
 
-Contract (see the task statement): `python bench.py --gpus N --steps K --warmup W`; for N > 1 the driver
-launches it under torchrun (one rank per GPU, RANK/LOCAL_RANK/WORLD_SIZE/MASTER_* in the env).  One JSON
-line on stdout from rank 0.
+Usage: `python bench.py --gpus N --steps K --warmup W`; for N > 1 run it under torchrun (one rank per GPU,
+RANK/LOCAL_RANK/WORLD_SIZE/MASTER_* in the env).  One JSON line on stdout from rank 0.  `--dump-outputs DIR`
+also writes the trajectory of the last timed step to DIR (see dump_outputs): the inputs are seeded, so two builds
+run with the same arguments can be compared output for output.
 
 Workload = BASELINE.json configs[1] "cartpole-trpo": CartPole + VisibleStepLimit(500), MLP policy 5->128->2,
 E = 4096 lanes per GPU, T = 256 steps per lane per period (N = 1 048 576 env-steps per GPU per step of this
@@ -47,6 +48,7 @@ FLOP_ISSUED_PER_SAMPLE_CRITIC_TC = 28672
 # period stays in the 126 MB L2 while the kernel runs and drains afterwards, so the in-kernel DRAM traffic
 # is far BELOW the algorithmic 26 B/env-step, not above it.
 K2C_NCU_DRAM_BYTES_PER_LAUNCH = 62208
+DUMP_MAX_BYTES = 64_000_000  # --dump-outputs: beyond this, a fixed sample of lanes is written
 
 
 WORKLOAD = "cartpole-trpo rollout (CartPole+VisibleStepLimit(500), MLP 5-128-2 policy: env step + policy act + sample + trajectory write)"
@@ -341,6 +343,8 @@ def run_ours(args):
     total_ms = max_over_ranks(dist, local, kernel_ms)
     steps_per_period = E * T
     value = world * steps_per_period * args.steps / (total_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, traj.to_host())
 
     # ---- e2e through the C ABI with host buffers: weights H2D (pinned) -> rollout -> summary D2H ----
     w_pinned = ctx.pinned_array((params.size,), np.float32)
@@ -475,6 +479,31 @@ def run_ours(args):
         emit(line)
     if dist is not None:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir: str, host: dict) -> None:
+    """Write a Trajectory.to_host() as DIR/<name>.npy: obs, next_obs [T, E, F], action, reward, succ [T, E] and
+    lane_len [E] in float32, and lane [E] in float64, the trajectory lane of each column.  Slots the rollout leaves
+    undefined are written as 0 (every field but succ at padding steps, succ == RL_PAD; next_obs except at interrupted
+    steps), so two builds that agree compare equal.  When all lanes would exceed DUMP_MAX_BYTES, a fixed seeded
+    sample of lanes is written."""
+    from relearn_b200 import _lib as L
+
+    T, E, F = host["obs"].shape
+    lane_bytes = 4 * T * (2 * F + 3) + 4 + 8
+    keep = min(E, DUMP_MAX_BYTES // lane_bytes)
+    lanes = np.arange(E) if keep == E else np.sort(np.random.default_rng(0).choice(E, keep, replace=False))
+    succ = host["succ"][:, lanes]
+    pad, intr = succ == L.RL_PAD, succ == L.RL_INTERRUPT
+    out = {"obs": np.where(pad[..., None], 0, host["obs"][:, lanes]),
+           "next_obs": np.where(intr[..., None], host["next_obs"][:, lanes], 0),
+           "action": np.where(pad, 0, host["action"][:, lanes]),
+           "reward": np.where(pad, 0, host["reward"][:, lanes]),
+           "succ": succ, "lane_len": host["lane_len"][lanes]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
+    np.save(os.path.join(out_dir, "lane.npy"), lanes.astype(np.float64))
 
 
 def kernel_rooflines(ctx, R, L, hbm_peak):
@@ -874,7 +903,11 @@ def main():
     ap.add_argument("--cpu-update-sample", dest="cpu_update_full", action="store_false",
                     help="time the CPU update baseline on a 65 536-step sample instead of the full batch")
     ap.add_argument("--sweep", action="store_true", help="BASELINE config 5: rollout throughput over E = 2^10 .. 2^24 (see run_sweep)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the trajectory of the last timed step (rank 0's lanes) to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.sweep or args.impl == "reference"):
+        ap.error("--dump-outputs writes the GPU rollout's trajectory: it needs --impl ours and no --sweep")
     if args.sweep:
         run_sweep(args)
     elif args.impl == "reference":
