@@ -283,8 +283,10 @@ typedef enum {
 
 /* rl_actor_cfg.lanes_per_env value selecting the tensor-core rollout kernel (CartPole + 5/4-128-2 ReLU network) */
 #define RL_LANES_TENSOR_CORE 128
-/* rl_actor_cfg.lanes_per_env value selecting the warp-specialised rollout kernel (K2w: policy and dynamics of an env on
- * different warps; CartPole + 5/4-128-2 ReLU network, categorical actor, Philox noise) */
+/* rl_actor_cfg.lanes_per_env value selecting the warp-specialised rollout kernels (policy and dynamics of an env on
+ * different warps; CartPole + 5/4-128-2 ReLU network): K2z up to 16 envs per SM, K2q beyond, at any size.  Their results
+ * are bit-identical to lanes_per_env = 8.  They serve the categorical actor on Philox noise only; any other actor or
+ * replayed noise is refused with RL_ERR_UNSUPPORTED. */
 #define RL_LANES_WARP_SPECIALIZED 160
 typedef struct rl_actor_cfg {
     int32_t kind;                 /* rl_actor_kind */
@@ -293,8 +295,9 @@ typedef struct rl_actor_cfg {
     rl_tabq *table;               /* TABULAR_EPS_GREEDY */
     double exploration_rate;      /* EPS_GREEDY_Q / TABULAR_EPS_GREEDY */
     int32_t training;             /* ActorMode::Training (src/agents/mod.rs:144) */
-    int32_t lanes_per_env;        /* 0 = auto; threads cooperating on one env's MLP (1,2,4,8,16,32), or
-                                   * RL_LANES_TENSOR_CORE: 128-env tiles, hidden layer on tcgen05 (K2t) */
+    int32_t lanes_per_env;        /* 0 = auto; threads cooperating on one env's MLP (1,2,4,8,16,32),
+                                   * RL_LANES_TENSOR_CORE (128): 128-env tiles, hidden layer on tcgen05 (K2t), or
+                                   * RL_LANES_WARP_SPECIALIZED (160): K2z / K2q */
     rl_grunet *seq_net;           /* CATEGORICAL_POLICY with a recurrent module (Chain<Gru, Linear>) instead of `net` */
     rl_ucb1 *ucb;                 /* UCB1 (training: maximise the upper confidence bound; evaluation: the most selected action) */
 } rl_actor_cfg;

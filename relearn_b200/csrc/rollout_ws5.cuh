@@ -1,40 +1,104 @@
-// rollout_ws5.cuh -- K2z: K2v (rollout_ws4.cuh) with the dynamics warp's loop cut down to what only it can do.
-// Per-phase clocks of K2v's loops (scripts/ws_clocks.sh, profiles/r2_summary.md section 5; one CTA per SM) showed a
-// dynamics-warp iteration of ~850 clk = candidate step 480 + select / convert / publish 171 + "off-chain" record 192, the
-// policy warps' row -> action chain (624 clk) running beside it and never waited for: the period is the dynamics warp's own
-// instruction stream.  K2z keeps K2v's operations on the same operands (bit-identical trajectories) and moves work:
-//  * each dynamics lane (env, action) publishes ITS candidate's next row -- observation after the step or, if the step
-//    ends the episode, after the reset; would-be `active` flag; successor code -- BEFORE the action is known, into a
-//    double-buffered mailbox rows[step parity][action][env]; the policy warps pick the row of the action they sampled
-//    themselves, so the select (shuffles) that follows serves only the dynamics warp's own next step;
+// rollout_ws5.cuh -- K2z: the warp-specialised CartPole rollout for few envs (E <= 16 per SM), and what it shares with
+// K2q (rollout_ws6.cuh, included after this file).  Included by rollout.cu inside its anonymous namespace.
+//
+// K2c<8> (rollout.cu) has each warp carry 4 envs x 8 threads and issue BOTH halves of the step chain: the policy
+// (obs -> hidden layer -> logit difference -> compare) and the f64 dynamics, the latter redundantly in all 8 threads of an
+// env.  With few envs the period is that combined instruction stream.  K2z splits it by warp.  A CTA owns 16 envs and has
+// six warps:
+//  * four POLICY warps, 4 envs x 8 threads each, with exactly K2c<8>'s register-resident hidden layer;
+//  * one DYNAMICS warp whose lane (env, a) steps env `env` with action `a` speculatively: both actions of 16 envs fill
+//    the warp, so nothing is computed redundantly;
+//  * one AUX warp that draws every Philox block: the actor's uniform of each step, as its logit-space threshold, and the
+//    would-be reset state of each step.  It fills them WS_CHUNK steps at a time into WS_RING-step shared-memory rings,
+//    up to WS_AHEAD steps ahead of the dynamics warp.  Progress is three counters in shared memory, not a barrier:
+//    `prod` (steps filled, written by the aux warp), `cons` (the dynamics warp's iteration, posted every fourth) and
+//    `done` (the dynamics loop is over).  The dynamics warp waits on `prod` every fourth iteration, the policy warps
+//    before every fourth step's thresholds.
+// Per step, each dynamics lane publishes ITS candidate's next row -- observation after the step or, if the step ends the
+// episode, after the reset; would-be `active` flag; successor code -- BEFORE the action is known, into a double-buffered
+// mailbox rows[step parity][action][env].  The policy warps pick the row of the action they sampled themselves, so the
+// select (shuffles) that follows serves only the dynamics warp's own next step.  Further work leaves the dynamics warp:
 //  * the step record's successor code and reward are stored by two idle threads of the env's policy group one iteration
-//    later (the row carries the previous step's code), the observation / action as before; only the post-step observation
-//    of an Interrupt (once per max_steps) is still stored by the dynamics warp, behind a vote taken at the loop top;
+//    later (the row carries the previous step's code), the observation / action by the others; only the post-step
+//    observation of an Interrupt (once per max_steps) is stored by the dynamics warp, behind a vote taken at the loop top;
 //  * episode statistics are integer counters (exact, converted once); the copies kept for finalize_last_episode are
 //    read back from the trajectory after the CTA-wide barrier that ends the loops;
 //  * the loop condition uses the vote of the PREVIOUS iteration (one idle iteration at the end instead of a vote ->
 //    branch dependency in every iteration); the policy warps stop on a flag in the row.
+// Per-phase clocks (scripts/ws_clocks.sh, profiles/r2_summary.md section 5) put the period on the dynamics warp's own
+// instruction stream; warps map to the four sub-partitions by index, and the dynamics warp sits on warp 2, the aux warp
+// on warp 5 (RolloutArgs::dyn_* / aux_*, set by launch_ws5).
 // Barriers: 1 / 3 = row of an even / odd step published (dynamics arrives, policy syncs), 2 / 4 = action of an even / odd
 // step published (policy arrives, dynamics syncs).  Two ids per direction because the dynamics warp publishes the row of
 // step i + 1 BEFORE it waits for the action of step i: with one id its arrival could land in the phase of step i that a
-// late policy warp has not joined yet (seen as a hang with two CTAs per SM).  Included by rollout.cu after rollout_ws4.cuh.
+// late policy warp has not joined yet (seen as a hang with two CTAs per SM).
+// Same operations on the same operands as K2c<8> (summation order of the logits included): bit-identical trajectories
+// and summaries (tests/test_gpu_envs.py).  Philox noise and the categorical actor only.
 #pragma once
+
+constexpr int ZK_ENVS = 16, ZK_THREADS = 192, ZK_SYNC = 160;  // 160: the policy and dynamics warps meet at the barriers
+constexpr int WS_RING = 16, WS_CHUNK = 4, WS_AHEAD = 11;        // the aux warp's rings (K2z and K2q)
+
+__device__ __forceinline__ void named_bar_sync(int id, int n) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n) : "memory"); }
+__device__ __forceinline__ void named_bar_arrive(int id, int n) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(n) : "memory"); }
+
+// Shared memory through explicit 32-bit shared-window addresses (ld.shared / st.shared): with generic pointers ptxas
+// rematerialises the window base (S2UR SR_CgaCtaId + ULEA) inside the loops.
+__device__ __forceinline__ float4 smem_ld4(uint32_t a) {
+    float4 v;
+    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(a));
+    return v;
+}
+__device__ __forceinline__ void smem_st4(uint32_t a, float4 v) {
+    asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(a), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
+}
+__device__ __forceinline__ double2 smem_ldd2(uint32_t a) {
+    double2 v;
+    asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "r"(a));
+    return v;
+}
+__device__ __forceinline__ void smem_std2(uint32_t a, double2 v) {
+    asm volatile("st.shared.v2.f64 [%0], {%1, %2};" ::"r"(a), "d"(v.x), "d"(v.y) : "memory");
+}
+__device__ __forceinline__ float smem_ldf(uint32_t a) {
+    float v;
+    asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(a));
+    return v;
+}
+__device__ __forceinline__ uint32_t smem_ldu(uint32_t a) {
+    uint32_t v;
+    asm volatile("ld.volatile.shared.u32 %0, [%1];" : "=r"(v) : "r"(a));
+    return v;
+}
+__device__ __forceinline__ void smem_stu(uint32_t a, uint32_t v) { asm volatile("st.volatile.shared.u32 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
+__device__ __forceinline__ void smem_stf(uint32_t a, float v) { asm volatile("st.shared.f32 [%0], %1;" ::"r"(a), "f"(v) : "memory"); }
+
+#ifdef RL_WS_CLOCKS  // measurement build only (scripts/ws_clocks.sh): per-phase clocks of the dynamics / policy loops of two CTAs
+__device__ __forceinline__ long long ws_clk(double dep, uint32_t dep2) {
+    long long c;
+    asm volatile("mov.u64 %0, %%clock64;" : "=l"(c) : "d"(dep), "r"(dep2) : "memory");
+    return c;
+}
+#define WS_CLK(var, dep, dep2) const long long var = ws_clk(dep, dep2)
+#else
+#define WS_CLK(var, dep, dep2)
+#endif
 
 struct ZkShared {
     float4 sw4[4 * GK_PAIRS];
     float tail[4 + GK_REM_TABLE_MAX];
     // rows[step parity][action taken in the previous step][env]: (x, x', theta, theta') | (remaining, flags, -, -)
     // flags: bit 0 this env takes the step, bit 1 stop, bit 2 the env took the previous step, bits 8.. its successor code
-    float4 rows[2][2][VK_ENVS][2];
-    uint32_t act[2][VK_ENVS];          // [step parity][env]
-    float thr[VK_RING][VK_ENVS];       // logit-space thresholds
-    double2 slot[VK_RING][VK_ENVS][2]; // would-be reset states (x, x') | (theta, theta')
+    float4 rows[2][2][ZK_ENVS][2];
+    uint32_t act[2][ZK_ENVS];          // [step parity][env]
+    float thr[WS_RING][ZK_ENVS];       // logit-space thresholds
+    double2 slot[WS_RING][ZK_ENVS][2]; // would-be reset states (x, x') | (theta, theta')
     uint32_t prod, cons, done, pad;
 };
 #define ZK_OFF(member) ((uint32_t)offsetof(ZkShared, member))
 constexpr uint32_t ZK_ACTIVE = 1u, ZK_STOP = 2u, ZK_PREV_ACTIVE = 4u;
 
-__global__ void __launch_bounds__(VK_THREADS, 2) rollout_cartpole_ws5_kernel(CartPoleEnv::Params p, RolloutArgs a) {
+__global__ void __launch_bounds__(ZK_THREADS, 2) rollout_cartpole_ws5_kernel(CartPoleEnv::Params p, RolloutArgs a) {
     using EnvT = CartPoleEnv;
     constexpr int LANES = 8, PPL = GK_PAIRS / LANES;
     constexpr unsigned FULL = 0xffffffffu;
@@ -46,14 +110,14 @@ __global__ void __launch_bounds__(VK_THREADS, 2) rollout_cartpole_ws5_kernel(Car
     stage_pair_weights(a.net, sh.sw4, sh.tail, p, rem_table ? (int)p.max_steps + 1 : 0);
     const uint32_t rem_addr = sb + ZK_OFF(tail) + 8;
     auto remaining_feature = [&](uint32_t r) {
-        return p.max_steps == 0 ? 0.0f : rem_table ? yk_ldf(rem_addr + 4u * r) : (float)__ddiv_rn((double)r, (double)p.max_steps);
+        return p.max_steps == 0 ? 0.0f : rem_table ? smem_ldf(rem_addr + 4u * r) : (float)__ddiv_rn((double)r, (double)p.max_steps);
     };
     const int hw_warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const bool later_cta = (int)blockIdx.x >= a.sm_count;
     const int dyn_warp = later_cta ? a.dyn_second : a.dyn_first, aux_warp = later_cta ? a.aux_second : a.aux_first;
     const bool is_dyn = hw_warp == dyn_warp, is_aux = hw_warp == aux_warp;
     const int warp = hw_warp - (hw_warp > dyn_warp ? 1 : 0) - (hw_warp > aux_warp ? 1 : 0);  // policy warp index 0..3
-    const uint64_t e_base = (uint64_t)blockIdx.x * VK_ENVS;
+    const uint64_t e_base = (uint64_t)blockIdx.x * ZK_ENVS;
     const uint32_t t0 = a.noise.step_counter;
     const uint64_t seed = a.noise.seed;
     const int F = a.F;
@@ -65,14 +129,14 @@ __global__ void __launch_bounds__(VK_THREADS, 2) rollout_cartpole_ws5_kernel(Car
     uint32_t fin_steps = 0;                                      // dynamics lanes: what finalize_last_episode needs after the loops
     int fin_succ_last = RL_TERMINATE, fin_succ_prev = RL_TERMINATE;
 
-    // ---- aux: one chunk = VK_CHUNK steps x 16 envs; lane = (env, half) handles steps k0 + 2 half + {0, 1} ----
+    // ---- aux: one chunk = WS_CHUNK steps x 16 envs; lane = (env, half) handles steps k0 + 2 half + {0, 1} ----
     auto aux_fill = [&](uint32_t k0) {
         const int el = lane & 15, half = lane >> 4;
         const uint64_t eg = e_base + el, lg = a.lane_offset + (eg < a.E ? eg : 0);
 #pragma unroll 1
         for (int j = 0; j < 2; ++j) {
             const uint32_t k = k0 + 2u * (uint32_t)half + (uint32_t)j;
-            const uint32_t ring = k & (VK_RING - 1);
+            const uint32_t ring = k & (WS_RING - 1);
             uint32_t oa[4], o0[4], o1[4];
             // policies/actor.rs:42-55: the actor's uniform of step k as the logit-space threshold (rl_logit_threshold)
             rl_philox4x32_10((uint32_t)lg, (uint32_t)(lg >> 32), t0 + k, (uint32_t)RL_STREAM_ACTOR * 64u, (uint32_t)seed,
@@ -82,43 +146,43 @@ __global__ void __launch_bounds__(VK_THREADS, 2) rollout_cartpole_ws5_kernel(Car
                              (uint32_t)(seed >> 32), o0);
             rl_philox4x32_10((uint32_t)lg, (uint32_t)(lg >> 32), t0 + k, (uint32_t)RL_STREAM_ENV_RESET * 64u + 1u, (uint32_t)seed,
                              (uint32_t)(seed >> 32), o1);
-            yk_stf(sb + ZK_OFF(thr) + 4u * (ring * VK_ENVS + el), rl_logit_threshold(rl_u32_to_f32(oa[0])));
+            smem_stf(sb + ZK_OFF(thr) + 4u * (ring * ZK_ENVS + el), rl_logit_threshold(rl_u32_to_f32(oa[0])));
             const double x = rl_u64_to_uniform((uint64_t)o0[0] | ((uint64_t)o0[1] << 32), p.reset_low, p.reset_scale);
             const double xd = rl_u64_to_uniform((uint64_t)o0[2] | ((uint64_t)o0[3] << 32), p.reset_low, p.reset_scale);
             const double th = rl_u64_to_uniform((uint64_t)o1[0] | ((uint64_t)o1[1] << 32), p.reset_low, p.reset_scale);
             const double thd = rl_u64_to_uniform((uint64_t)o1[2] | ((uint64_t)o1[3] << 32), p.reset_low, p.reset_scale);
-            const uint32_t sa = sb + ZK_OFF(slot) + 32u * (ring * VK_ENVS + el);
-            yk_std2(sa, make_double2(x, xd));
-            yk_std2(sa + 16, make_double2(th, thd));
+            const uint32_t sa = sb + ZK_OFF(slot) + 32u * (ring * ZK_ENVS + el);
+            smem_std2(sa, make_double2(x, xd));
+            smem_std2(sa + 16, make_double2(th, thd));
         }
     };
     if (threadIdx.x == 0) { sh.prod = 0; sh.cons = 0; sh.done = 0; }
     if (is_aux) {
         aux_fill(0);
-        aux_fill(VK_CHUNK);
+        aux_fill(WS_CHUNK);
     }
     __syncthreads();
-    if (is_aux && lane == 0) yk_stu(sb + ZK_OFF(prod), 2 * VK_CHUNK);
+    if (is_aux && lane == 0) smem_stu(sb + ZK_OFF(prod), 2 * WS_CHUNK);
 
     if (is_aux) {
         // ------------------------------ aux warp ------------------------------
-        uint32_t k0 = 2 * VK_CHUNK;
+        uint32_t k0 = 2 * WS_CHUNK;
         while (k0 <= cap + 1) {
             // slots of steps k0 - 16 .. k0 - 13 are reused: their readers (thresholds at iteration k, reset states at
             // k - 1) are done once the dynamics warp is at iteration >= k0 - 12
-            uint32_t c = yk_ldu(sb + ZK_OFF(cons));
+            uint32_t c = smem_ldu(sb + ZK_OFF(cons));
             bool over = false;
-            while (k0 > c + VK_AHEAD) {
-                if (yk_ldu(sb + ZK_OFF(done))) { over = true; break; }
+            while (k0 > c + WS_AHEAD) {
+                if (smem_ldu(sb + ZK_OFF(done))) { over = true; break; }
                 __nanosleep(64);
-                c = yk_ldu(sb + ZK_OFF(cons));
+                c = smem_ldu(sb + ZK_OFF(cons));
             }
             if (over) break;
             aux_fill(k0);
             __threadfence_block();
             __syncwarp();
-            k0 += VK_CHUNK;
-            if (lane == 0) yk_stu(sb + ZK_OFF(prod), k0);
+            k0 += WS_CHUNK;
+            if (lane == 0) smem_stu(sb + ZK_OFF(prod), k0);
         }
     } else if (is_dyn) {
         // ------------------------------ dynamics warp: lane = (env el, action act) ------------------------------
@@ -132,8 +196,8 @@ __global__ void __launch_bounds__(VK_THREADS, 2) rollout_cartpole_ws5_kernel(Car
         const uint32_t act_addr = sb + ZK_OFF(act) + 4u * (uint32_t)el;                          // + 64 * step parity
         // the reset state of noise step t0 + k, from the ring the aux warp keeps ahead
         auto fresh_state = [&](uint32_t k, EnvT::State &f) {
-            const uint32_t sa = slot0 + 512u * (k & (VK_RING - 1));
-            const double2 lo = yk_ldd2(sa), hi = yk_ldd2(sa + 16);
+            const uint32_t sa = slot0 + 512u * (k & (WS_RING - 1));
+            const double2 lo = smem_ldd2(sa), hi = smem_ldd2(sa + 16);
             f.x = lo.x; f.xd = lo.y; f.th = hi.x; f.thd = hi.y;
             f.meta = 0x80000000u | p.max_steps;
         };
@@ -148,10 +212,10 @@ __global__ void __launch_bounds__(VK_THREADS, 2) rollout_cartpole_ws5_kernel(Car
             if (n > 0) { s = f; obs4 = rem_full; }
         }
         bool go = __any_sync(FULL, n > 0);  // loop condition, one iteration behind
-        yk_st4(my_row, make_float4((float)s.x, (float)s.xd, (float)s.th, (float)s.thd));
-        yk_st4(my_row + 16, make_float4(obs4, __uint_as_float((n > 0 ? ZK_ACTIVE : 0u) | (go ? 0u : ZK_STOP)), 0.0f, 0.0f));
+        smem_st4(my_row, make_float4((float)s.x, (float)s.xd, (float)s.th, (float)s.thd));
+        smem_st4(my_row + 16, make_float4(obs4, __uint_as_float((n > 0 ? ZK_ACTIVE : 0u) | (go ? 0u : ZK_STOP)), 0.0f, 0.0f));
         __syncwarp();
-        named_bar_arrive(1, VK_SYNC);                     // row of step 0
+        named_bar_arrive(1, ZK_SYNC);                     // row of step 0
         uint32_t it = 0;                                  // loop counter (= step index of the envs still active)
         uint32_t i = 0, cur_len = 0, n_eps = 0;           // steps stored, length of the running episode, episodes ended
         unsigned long long sum_el = 0ull, sum_el2 = 0ull; // sum of episode lengths and of their squares
@@ -160,14 +224,14 @@ __global__ void __launch_bounds__(VK_THREADS, 2) rollout_cartpole_ws5_kernel(Car
         long long ck[5] = {0, 0, 0, 0, 0};
 #endif
         while (go) {
-            VK_CLK(c0, s.x, it);
+            WS_CLK(c0, s.x, it);
             const bool active = n > 0;
             const uint32_t r_now = s.meta & 0x7FFFFFFFu;
             // an Interrupt can only come from the step limit running out (step_limit.rs:202-223): known before the step
             const bool some_limit = __any_sync(FULL, active && p.max_steps != 0 && r_now == 1);
-            if ((it & 3u) == 0u && lane == 0) yk_stu(sb + ZK_OFF(cons), it);
+            if ((it & 3u) == 0u && lane == 0) smem_stu(sb + ZK_OFF(cons), it);
             if ((it & 3u) == 3u) {  // the reset states of steps it + 1 .. it + 4
-                while (yk_ldu(sb + ZK_OFF(prod)) < it + 5u) { }
+                while (smem_ldu(sb + ZK_OFF(prod)) < it + 5u) { }
                 asm volatile("fence.acq_rel.cta;" ::: "memory");
             }
             // this lane's world: the step with action `act`, then -- if it ends the episode -- the reset (steps.rs:116-124)
@@ -187,16 +251,16 @@ __global__ void __launch_bounds__(VK_THREADS, 2) rollout_cartpole_ws5_kernel(Car
                 if (cand_ended && n_cand <= a.slack) n_cand = 0;  // take_steps.rs:83-88
             }
             const uint32_t row_w = my_row + 1024u * ((it + 1u) & 1u);
-            yk_st4(row_w, make_float4((float)nxt.x, (float)nxt.xd, (float)nxt.th, (float)nxt.thd));
-            yk_st4(row_w + 16, make_float4(cand_ended ? rem_full : rem_cont,
+            smem_st4(row_w, make_float4((float)nxt.x, (float)nxt.xd, (float)nxt.th, (float)nxt.thd));
+            smem_st4(row_w + 16, make_float4(cand_ended ? rem_full : rem_cont,
                                            __uint_as_float((n_cand > 0 ? ZK_ACTIVE : 0u) | (active ? ZK_PREV_ACTIVE : 0u) | ((uint32_t)cand_sc << 8)),
                                            0.0f, 0.0f));
             __syncwarp();
-            named_bar_arrive(1 + 2 * (int)((it + 1u) & 1u), VK_SYNC);
-            VK_CLK(c1, nxt.x + nxt.thd, n_cand);
-            named_bar_sync(2 + 2 * (int)(it & 1u), VK_SYNC);
-            VK_CLK(c2, 0.0, 0u);
-            const uint32_t action = yk_ldu(act_addr + 64u * (it & 1u));
+            named_bar_arrive(1 + 2 * (int)((it + 1u) & 1u), ZK_SYNC);
+            WS_CLK(c1, nxt.x + nxt.thd, n_cand);
+            named_bar_sync(2 + 2 * (int)(it & 1u), ZK_SYNC);
+            WS_CLK(c2, 0.0, 0u);
+            const uint32_t action = smem_ldu(act_addr + 64u * (it & 1u));
             const int src = el + 16 * (int)action;
             s.th = __shfl_sync(FULL, nxt.th, src);
             s.thd = __shfl_sync(FULL, nxt.thd, src);
@@ -205,7 +269,7 @@ __global__ void __launch_bounds__(VK_THREADS, 2) rollout_cartpole_ws5_kernel(Car
             s.meta = __shfl_sync(FULL, nxt.meta, src);
             const int sc = __shfl_sync(FULL, cand_sc, src);
             const uint32_t n_next = __shfl_sync(FULL, n_cand, src);
-            VK_CLK(c3, s.x + s.th, n_next);
+            WS_CLK(c3, s.x + s.th, n_next);
             if (some_limit) {  // rare (once per max_steps): the post-step observation of an Interrupt (remaining == 0)
                 const double px = __shfl_sync(FULL, cand.x, src), pxd = __shfl_sync(FULL, cand.xd, src);
                 const double pth = __shfl_sync(FULL, cand.th, src), pthd = __shfl_sync(FULL, cand.thd, src);
@@ -233,7 +297,7 @@ __global__ void __launch_bounds__(VK_THREADS, 2) rollout_cartpole_ws5_kernel(Car
             go = __any_sync(FULL, active);  // == the vote on n > 0 taken one iteration ago
             it += 1;
 #ifdef RL_WS_CLOCKS
-            const long long c4 = vk_clk((double)sum_el2, i + cur_len);
+            const long long c4 = ws_clk((double)sum_el2, i + cur_len);
             ck[0] += c1 - c0; ck[1] += c2 - c1; ck[2] += c3 - c2; ck[3] += c4 - c3; ck[4] += 1;
 #endif
         }
@@ -241,10 +305,10 @@ __global__ void __launch_bounds__(VK_THREADS, 2) rollout_cartpole_ws5_kernel(Car
             // The policy warps have taken the rows of steps 0 .. it and wait for one more: tell them to stop, and take the
             // action they publish for step `it` (no env is active in steps it - 1 and it).
             const uint32_t row_w = my_row + 1024u * ((it + 1u) & 1u);
-            yk_st4(row_w + 16, make_float4(0.0f, __uint_as_float(ZK_STOP), 0.0f, 0.0f));
+            smem_st4(row_w + 16, make_float4(0.0f, __uint_as_float(ZK_STOP), 0.0f, 0.0f));
             __syncwarp();
-            named_bar_arrive(1 + 2 * (int)((it + 1u) & 1u), VK_SYNC);
-            named_bar_sync(2 + 2 * (int)(it & 1u), VK_SYNC);
+            named_bar_arrive(1 + 2 * (int)((it + 1u) & 1u), ZK_SYNC);
+            named_bar_sync(2 + 2 * (int)(it & 1u), ZK_SYNC);
         }
 #ifdef RL_WS_CLOCKS
         if (lane == 0 && ck[4] > 0 && (blockIdx.x == 0 || blockIdx.x == gridDim.x - 1))
@@ -252,7 +316,7 @@ __global__ void __launch_bounds__(VK_THREADS, 2) rollout_cartpole_ws5_kernel(Car
                    "select %.1f, bookkeeping %.1f\n", (int)blockIdx.x, ck[4], (double)ck[0] / ck[4], (double)ck[1] / ck[4],
                    (double)ck[2] / ck[4], (double)ck[3] / ck[4]);
 #endif
-        if (lane == 0) yk_stu(sb + ZK_OFF(done), 1u);
+        if (lane == 0) smem_stu(sb + ZK_OFF(done), 1u);
         st.v[ST_STEPS] = st.v[ST_R] = st.v[ST_R2] = (double)i;
         st.v[ST_EPS] = (double)n_eps; st.v[ST_ER] = st.v[ST_EL] = (double)sum_el; st.v[ST_ER2] = st.v[ST_EL2] = (double)sum_el2;
         fin_steps = i; fin_succ_last = succ_last; fin_succ_prev = succ_prev;
@@ -286,19 +350,19 @@ __global__ void __launch_bounds__(VK_THREADS, 2) rollout_cartpole_ws5_kernel(Car
         long long pk[4] = {0, 0, 0, 0};
 #endif
         for (uint32_t i = 0;; ++i) {
-            VK_CLK(q0, 0.0, i);
+            WS_CLK(q0, 0.0, i);
             if ((i & 3u) == 0u) {  // thresholds of steps i .. i + 3
                 // (`done`: the dynamics warp has left its loop and the aux warp may have stopped; this iteration only breaks)
-                while (yk_ldu(sb + ZK_OFF(prod)) < i + 4u && !yk_ldu(sb + ZK_OFF(done))) { }
+                while (smem_ldu(sb + ZK_OFF(prod)) < i + 4u && !smem_ldu(sb + ZK_OFF(done))) { }
                 asm volatile("fence.acq_rel.cta;" ::: "memory");
             }
-            const float theta = yk_ldf(thr_addr + 64u * (i & (VK_RING - 1)));
+            const float theta = smem_ldf(thr_addr + 64u * (i & (WS_RING - 1)));
             const uint32_t row = row0 + 1024u * (i & 1u) + 512u * prev_action;
-            named_bar_sync(1 + 2 * (int)(i & 1u), VK_SYNC);
-            VK_CLK(q1, 0.0, 0u);
-            const float4 ov = yk_ld4(row);
-            const float4 tv = yk_ld4(row + 16);
-            const float mine = yk_ldf(row + mine_off);
+            named_bar_sync(1 + 2 * (int)(i & 1u), ZK_SYNC);
+            WS_CLK(q1, 0.0, 0u);
+            const float4 ov = smem_ld4(row);
+            const float4 tv = smem_ld4(row + 16);
+            const float mine = smem_ldf(row + mine_off);
             const float ob4 = tv.x;
             const uint32_t flags = __float_as_uint(tv.y);
             // the previous step's successor code and reward (simulation/mod.rs PartialStep -> buffers/vec.rs)
@@ -339,10 +403,10 @@ __global__ void __launch_bounds__(VK_THREADS, 2) rollout_cartpole_ws5_kernel(Car
             for (int o = LANES / 2; o > 0; o >>= 1) d += __shfl_xor_sync(FULL, d, o);
             d += b2d;
             const uint32_t action = d < theta ? 0u : 1u;  // policies/actor.rs:42-55 (rl_logit_threshold)
-            if (sub == 0) yk_stu(act_addr + 64u * (i & 1u), action);
+            if (sub == 0) smem_stu(act_addr + 64u * (i & 1u), action);
             __syncwarp();
-            named_bar_arrive(2 + 2 * (int)(i & 1u), VK_SYNC);
-            VK_CLK(q2, 0.0, action);
+            named_bar_arrive(2 + 2 * (int)(i & 1u), ZK_SYNC);
+            WS_CLK(q2, 0.0, action);
             // ---- off the chain: the observation and the action of the step record ----
             if (active && stores_obs) *obs_ptr = mine;
             if (active && stores_action) *act_ptr = (uint8_t)action;
@@ -352,7 +416,7 @@ __global__ void __launch_bounds__(VK_THREADS, 2) rollout_cartpole_ws5_kernel(Car
             reward_ptr += a.E;
             prev_action = action;
 #ifdef RL_WS_CLOCKS
-            const long long q3 = vk_clk(0.0, (uint32_t)(uintptr_t)act_ptr);
+            const long long q3 = ws_clk(0.0, (uint32_t)(uintptr_t)act_ptr);
             pk[0] += q1 - q0; pk[1] += q2 - q1; pk[2] += q3 - q2; pk[3] += 1;
 #endif
         }

@@ -1,18 +1,21 @@
-// rollout_ws6.cuh -- K2q: the warp-specialised CartPole rollout with ONE CTA per SM at the bench size.
-// Per-phase clocks of K2v (scripts/ws_clocks.sh, profiles/r2_summary.md section 5): with one 16-env CTA on an SM an
-// iteration of the dynamics warp takes ~850 clk (candidate step 480, select / convert / publish 171, step record 192) and
-// the policy warps are never waited for; with two CTAs on an SM (E = 4096) the same stream takes ~1150 clk because the
-// dynamics warp -- ~75 % issue-busy on its own -- shares its scheduler with policy warps.  K2q therefore
+// rollout_ws6.cuh -- K2q: the warp-specialised CartPole rollout with ONE CTA per SM at the bench size (E > 16 per SM).
+// K2z (rollout_ws5.cuh) puts 16 envs on a six-warp CTA, two of them per SM once E > 16 per SM.  Its per-phase clocks
+// (scripts/ws_clocks.sh, profiles/r2_summary.md section 5): with one CTA on an SM an iteration of the dynamics warp takes
+// ~850 clk (candidate step 480, select / convert / publish 171, step record 192) and the policy warps are never waited
+// for; with two CTAs on an SM (E = 4096) the same stream takes ~1150 clk because the dynamics warp -- ~75 % issue-busy on
+// its own -- shares its scheduler with policy warps.  K2q therefore
 //  * puts 32 envs on ONE dynamics warp, lane = env, which evaluates the step for BOTH actions in the same thread (four
 //    independent chains: 2 actions x 2 friction signs; everything that does not depend on the action -- sin / cos, the
 //    reciprocals, beta -- is computed once), so the select needs no shuffles and E = 4096 fits one CTA per SM (128 CTAs);
 //  * gives that warp a scheduler of its own: twelve warps, the two other warps of the dynamics warp's sub-partition
 //    idle at the final barrier, eight policy warps and the aux (Philox) warp on the other three sub-partitions;
-//  * takes the step record off the dynamics warp (as K2z, rollout_ws5.cuh): successor code and reward are stored one
-//    iteration later by two idle threads of the env's policy group (the row carries the previous step's code), episode
-//    statistics are integer counters, finalize_last_episode reads the dropped observation back from the trajectory.
-// Protocol otherwise K2v's (row -> barrier 1 -> policy -> action -> barrier 2 -> select); same operations on the same
-// operands as K2c<8>: bit-identical trajectories.  Included by rollout.cu after rollout_ws5.cuh.
+//  * takes the step record off the dynamics warp (as K2z): successor code and reward are stored one iteration later by
+//    two idle threads of the env's policy group (the row carries the previous step's code), episode statistics are
+//    integer counters, finalize_last_episode reads the dropped observation back from the trajectory.
+// The aux warp and its rings are K2z's (WS_RING / WS_CHUNK / WS_AHEAD, lane = env).  The hand-off has one row per env:
+// dynamics publishes the row of step i -> barrier 1 -> policy samples -> action -> barrier 2 -> dynamics selects.  The
+// grid is one CTA per 4 x policy_warps envs, so any number of waves runs.  Same operations on the same operands as
+// K2c<8>: bit-identical trajectories.  Included by rollout.cu after rollout_ws5.cuh.
 #pragma once
 
 constexpr int QK_ENVS = 32, QK_THREADS = 384, QK_POLICY_WARPS = 8;  // at most; RolloutArgs::policy_warps x 4 envs are used
@@ -25,8 +28,8 @@ struct QkShared {
     // the CTA does, bit 2 the env took the previous step, bits 8.. that step's successor code
     float4 rows[QK_ENVS][2];
     uint32_t act[QK_ENVS];
-    float thr[VK_RING][QK_ENVS];       // logit-space thresholds
-    double2 slot[VK_RING][QK_ENVS][2]; // would-be reset states (x, x') | (theta, theta')
+    float thr[WS_RING][QK_ENVS];       // logit-space thresholds
+    double2 slot[WS_RING][QK_ENVS][2]; // would-be reset states (x, x') | (theta, theta')
     uint32_t prod, cons, done, pad;
 };
 #define QK_OFF(member) ((uint32_t)offsetof(QkShared, member))
@@ -44,7 +47,7 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
     stage_pair_weights(a.net, sh.sw4, sh.tail, p, rem_table ? (int)p.max_steps + 1 : 0);
     const uint32_t rem_addr = sb + QK_OFF(tail) + 8;
     auto remaining_feature = [&](uint32_t r) {
-        return p.max_steps == 0 ? 0.0f : rem_table ? yk_ldf(rem_addr + 4u * r) : (float)__ddiv_rn((double)r, (double)p.max_steps);
+        return p.max_steps == 0 ? 0.0f : rem_table ? smem_ldf(rem_addr + 4u * r) : (float)__ddiv_rn((double)r, (double)p.max_steps);
     };
     const int hw_warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     // roles by hardware warp (warp w runs on sub-partition w % 4)
@@ -63,14 +66,14 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
     uint32_t fin_steps = 0;                                      // dynamics lanes: what finalize_last_episode needs after the loops
     int fin_succ_last = RL_TERMINATE, fin_succ_prev = RL_TERMINATE;
 
-    // ---- aux: one chunk = VK_CHUNK steps x 32 envs; lane = env ----
+    // ---- aux: one chunk = WS_CHUNK steps x 32 envs; lane = env ----
     auto aux_fill = [&](uint32_t k0) {
         const int el = lane;
         const uint64_t eg = e_base + el, lg = a.lane_offset + (eg < a.E ? eg : 0);  // (lanes past the CTA's envs: unused slots)
 #pragma unroll 1
-        for (int j = 0; j < VK_CHUNK; ++j) {
+        for (int j = 0; j < WS_CHUNK; ++j) {
             const uint32_t k = k0 + (uint32_t)j;
-            const uint32_t ring = k & (VK_RING - 1);
+            const uint32_t ring = k & (WS_RING - 1);
             uint32_t oa[4], o0[4], o1[4];
             // policies/actor.rs:42-55: the actor's uniform of step k as the logit-space threshold (rl_logit_threshold)
             rl_philox4x32_10((uint32_t)lg, (uint32_t)(lg >> 32), t0 + k, (uint32_t)RL_STREAM_ACTOR * 64u, (uint32_t)seed,
@@ -80,45 +83,45 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
                              (uint32_t)(seed >> 32), o0);
             rl_philox4x32_10((uint32_t)lg, (uint32_t)(lg >> 32), t0 + k, (uint32_t)RL_STREAM_ENV_RESET * 64u + 1u, (uint32_t)seed,
                              (uint32_t)(seed >> 32), o1);
-            yk_stf(sb + QK_OFF(thr) + 4u * (ring * QK_ENVS + el), rl_logit_threshold(rl_u32_to_f32(oa[0])));
+            smem_stf(sb + QK_OFF(thr) + 4u * (ring * QK_ENVS + el), rl_logit_threshold(rl_u32_to_f32(oa[0])));
             const double x = rl_u64_to_uniform((uint64_t)o0[0] | ((uint64_t)o0[1] << 32), p.reset_low, p.reset_scale);
             const double xd = rl_u64_to_uniform((uint64_t)o0[2] | ((uint64_t)o0[3] << 32), p.reset_low, p.reset_scale);
             const double th = rl_u64_to_uniform((uint64_t)o1[0] | ((uint64_t)o1[1] << 32), p.reset_low, p.reset_scale);
             const double thd = rl_u64_to_uniform((uint64_t)o1[2] | ((uint64_t)o1[3] << 32), p.reset_low, p.reset_scale);
             const uint32_t sa = sb + QK_OFF(slot) + 32u * (ring * QK_ENVS + el);
-            yk_std2(sa, make_double2(x, xd));
-            yk_std2(sa + 16, make_double2(th, thd));
+            smem_std2(sa, make_double2(x, xd));
+            smem_std2(sa + 16, make_double2(th, thd));
         }
     };
     if (threadIdx.x == 0) { sh.prod = 0; sh.cons = 0; sh.done = 0; }
     if (is_aux) {
         aux_fill(0);
-        aux_fill(VK_CHUNK);
+        aux_fill(WS_CHUNK);
     }
     __syncthreads();
-    if (is_aux && lane == 0) yk_stu(sb + QK_OFF(prod), 2 * VK_CHUNK);
+    if (is_aux && lane == 0) smem_stu(sb + QK_OFF(prod), 2 * WS_CHUNK);
 
     if (is_idle) {
         // (keeps the dynamics warp's scheduler free; waits at the barrier below)
     } else if (is_aux) {
         // ------------------------------ aux warp ------------------------------
-        uint32_t k0 = 2 * VK_CHUNK;
+        uint32_t k0 = 2 * WS_CHUNK;
         while (k0 <= cap + 1) {
             // slots of steps k0 - 16 .. k0 - 13 are reused: their readers (thresholds at iteration k, reset states at
             // k - 1) are done once the dynamics warp is at iteration >= k0 - 12
-            uint32_t c = yk_ldu(sb + QK_OFF(cons));
+            uint32_t c = smem_ldu(sb + QK_OFF(cons));
             bool over = false;
-            while (k0 > c + VK_AHEAD) {
-                if (yk_ldu(sb + QK_OFF(done))) { over = true; break; }
+            while (k0 > c + WS_AHEAD) {
+                if (smem_ldu(sb + QK_OFF(done))) { over = true; break; }
                 __nanosleep(64);
-                c = yk_ldu(sb + QK_OFF(cons));
+                c = smem_ldu(sb + QK_OFF(cons));
             }
             if (over) break;
             aux_fill(k0);
             __threadfence_block();
             __syncwarp();
-            k0 += VK_CHUNK;
-            if (lane == 0) yk_stu(sb + QK_OFF(prod), k0);
+            k0 += WS_CHUNK;
+            if (lane == 0) smem_stu(sb + QK_OFF(prod), k0);
         }
     } else if (is_dyn) {
         // ------------------------------ dynamics warp: lane = env ------------------------------
@@ -131,8 +134,8 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
         const uint32_t act_addr = sb + QK_OFF(act) + 4u * (uint32_t)el;
         // the reset state of noise step t0 + k, from the ring the aux warp keeps ahead
         auto fresh_state = [&](uint32_t k, EnvT::State &f) {
-            const uint32_t sa = slot0 + 32u * QK_ENVS * (k & (VK_RING - 1));
-            const double2 lo = yk_ldd2(sa), hi = yk_ldd2(sa + 16);
+            const uint32_t sa = slot0 + 32u * QK_ENVS * (k & (WS_RING - 1));
+            const double2 lo = smem_ldd2(sa), hi = smem_ldd2(sa + 16);
             f.x = lo.x; f.xd = lo.y; f.th = hi.x; f.thd = hi.y;
             f.meta = 0x80000000u | p.max_steps;
         };
@@ -147,8 +150,8 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
             if (n > 0) { s = f; obs4 = rem_full; }
         }
         bool any = __any_sync(FULL, n > 0);
-        yk_st4(row, make_float4((float)s.x, (float)s.xd, (float)s.th, (float)s.thd));
-        yk_st4(row + 16, make_float4(obs4, __uint_as_float((n > 0 ? QK_ACTIVE : 0u) | (any ? QK_ANY : 0u)), 0.0f, 0.0f));
+        smem_st4(row, make_float4((float)s.x, (float)s.xd, (float)s.th, (float)s.thd));
+        smem_st4(row + 16, make_float4(obs4, __uint_as_float((n > 0 ? QK_ACTIVE : 0u) | (any ? QK_ANY : 0u)), 0.0f, 0.0f));
         __syncwarp();
         named_bar_arrive(1, QK_SYNC);
         uint32_t it = 0;                                  // loop counter (= step index of the envs still active)
@@ -159,11 +162,11 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
         long long ck[5] = {0, 0, 0, 0, 0};
 #endif
         while (any) {
-            VK_CLK(c0, s.x, it);
+            WS_CLK(c0, s.x, it);
             const bool active = n > 0;
-            if ((it & 3u) == 0u && lane == 0) yk_stu(sb + QK_OFF(cons), it);
+            if ((it & 3u) == 0u && lane == 0) smem_stu(sb + QK_OFF(cons), it);
             if ((it & 3u) == 3u) {  // the reset states of steps it + 1 .. it + 4
-                while (yk_ldu(sb + QK_OFF(prod)) < it + 5u) { }
+                while (smem_ldu(sb + QK_OFF(prod)) < it + 5u) { }
                 asm volatile("fence.acq_rel.cta;" ::: "memory");
             }
             // before the action is known: the step for both actions, the would-be reset state, and the `remaining` feature
@@ -175,10 +178,10 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
             fresh_state(it + 1, fresh);
             const uint32_t r_now = s.meta & 0x7FFFFFFFu;
             const float rem_cont = remaining_feature(r_now > 0 ? r_now - 1 : 0);
-            VK_CLK(c1, c0s.x + c1s.x + c0s.thd + c1s.thd + fresh.x, (uint32_t)(sc0 + sc1) + __float_as_uint(rem_cont));
+            WS_CLK(c1, c0s.x + c1s.x + c0s.thd + c1s.thd + fresh.x, (uint32_t)(sc0 + sc1) + __float_as_uint(rem_cont));
             named_bar_sync(2, QK_SYNC);
-            VK_CLK(c2, 0.0, 0u);
-            const bool one = yk_ldu(act_addr) != 0u;
+            WS_CLK(c2, 0.0, 0u);
+            const bool one = smem_ldu(act_addr) != 0u;
             EnvT::State post;
             post.x = one ? c1s.x : c0s.x; post.xd = one ? c1s.xd : c0s.xd;
             post.th = one ? c1s.th : c0s.th; post.thd = one ? c1s.thd : c0s.thd;
@@ -194,14 +197,14 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
                 if (ended && n_next <= a.slack) n_next = 0;  // take_steps.rs:83-88
             }
             const bool any_next = __any_sync(FULL, n_next > 0);
-            yk_st4(row, make_float4((float)s.x, (float)s.xd, (float)s.th, (float)s.thd));
-            yk_st4(row + 16, make_float4(ended ? rem_full : rem_cont,
+            smem_st4(row, make_float4((float)s.x, (float)s.xd, (float)s.th, (float)s.thd));
+            smem_st4(row + 16, make_float4(ended ? rem_full : rem_cont,
                                          __uint_as_float((n_next > 0 ? QK_ACTIVE : 0u) | (any_next ? QK_ANY : 0u) |
                                                          (active ? QK_PREV_ACTIVE : 0u) | ((uint32_t)sc << 8)),
                                          0.0f, 0.0f));
             __syncwarp();
             named_bar_arrive(1, QK_SYNC);
-            VK_CLK(c3, 0.0, 0u);
+            WS_CLK(c3, 0.0, 0u);
             // ---- off the chain ----
             if (active && sc == RL_INTERRUPT) {  // rare: once per max_steps; the post-step observation (remaining == 0)
                 const uint64_t io = (uint64_t)i * FE + e_safe;
@@ -225,7 +228,7 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
             any = any_next;
             it += 1;
 #ifdef RL_WS_CLOCKS
-            const long long c4 = vk_clk((double)sum_el2, i + cur_len);
+            const long long c4 = ws_clk((double)sum_el2, i + cur_len);
             ck[0] += c1 - c0; ck[1] += c2 - c1; ck[2] += c3 - c2; ck[3] += c4 - c3; ck[4] += 1;
 #endif
         }
@@ -235,7 +238,7 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
                    "select + publish %.1f, bookkeeping %.1f\n", (int)blockIdx.x, ck[4], (double)ck[0] / ck[4], (double)ck[1] / ck[4],
                    (double)ck[2] / ck[4], (double)ck[3] / ck[4]);
 #endif
-        if (lane == 0) yk_stu(sb + QK_OFF(done), 1u);
+        if (lane == 0) smem_stu(sb + QK_OFF(done), 1u);
         // (kept for after the barrier that ends the loops)
         st.v[ST_STEPS] = st.v[ST_R] = st.v[ST_R2] = (double)i;
         st.v[ST_EPS] = (double)n_eps; st.v[ST_ER] = st.v[ST_EL] = (double)sum_el; st.v[ST_ER2] = st.v[ST_EL2] = (double)sum_el2;
@@ -272,16 +275,16 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
         long long pk[4] = {0, 0, 0, 0};
 #endif
         for (uint32_t i = 0;; ++i) {
-            VK_CLK(q0, 0.0, i);
+            WS_CLK(q0, 0.0, i);
             // (No poll of `prod` here: the dynamics warp saw the thresholds of steps <= i + 1 published before it arrived
             // at barrier 1 for the row of step i -- it polls every fourth iteration, up to four steps ahead -- and the
             // barrier orders that observation before the load below.)
             named_bar_sync(1, QK_SYNC);
-            VK_CLK(q1, 0.0, 0u);
-            const float4 ov = yk_ld4(row);
-            const float4 tv = yk_ld4(row + 16);
-            const float mine = yk_ldf(mine_addr);
-            const float theta = yk_ldf(thr_addr + 4u * QK_ENVS * (i & (VK_RING - 1)));
+            WS_CLK(q1, 0.0, 0u);
+            const float4 ov = smem_ld4(row);
+            const float4 tv = smem_ld4(row + 16);
+            const float mine = smem_ldf(mine_addr);
+            const float theta = smem_ldf(thr_addr + 4u * QK_ENVS * (i & (WS_RING - 1)));
             const float ob4 = tv.x;
             const uint32_t flags = __float_as_uint(tv.y);
             // this thread's column of the step record (sub >= 6: of the previous step); off the chain except at the end
@@ -326,15 +329,15 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
             for (int o = LANES / 2; o > 0; o >>= 1) d += __shfl_xor_sync(FULL, d, o);
             d += b2d;
             const uint32_t action = d < theta ? 0u : 1u;  // policies/actor.rs:42-55 (rl_logit_threshold)
-            if (sub == 0) yk_stu(act_addr, action);
+            if (sub == 0) smem_stu(act_addr, action);
             __syncwarp();
             named_bar_arrive(2, QK_SYNC);
-            VK_CLK(q2, 0.0, action);
+            WS_CLK(q2, 0.0, action);
             // ---- off the chain: the step record ----
             store_column(action);
             col_ptr += col_stride;
 #ifdef RL_WS_CLOCKS
-            const long long q3 = vk_clk(0.0, (uint32_t)(uintptr_t)col_ptr);
+            const long long q3 = ws_clk(0.0, (uint32_t)(uintptr_t)col_ptr);
             pk[0] += q1 - q0; pk[1] += q2 - q1; pk[2] += q3 - q2; pk[3] += 1;
 #endif
         }

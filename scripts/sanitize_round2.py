@@ -14,8 +14,8 @@ from relearn_b200 import _lib as L
 ctx = R.Context(0)
 rng = np.random.default_rng(0)
 cfg = R.CartPoleConfig().wrap(R.VisibleStepLimit(9))
-for variant, E in (("5", 37), ("6", 45), ("6", 28)):
-    os.environ["RL_WS_VARIANT"] = variant
+# K2z (E <= 16 per SM), K2q with 28-env CTAs and with 32-env CTAs (E > 28 per SM); every last CTA ragged
+for E in (37, 2400, 4700):
     env = R.build_env(ctx, cfg, E, seed=2, lane_offset=3)
     net = R.Mlp(ctx, 5, [128], 2)
     net.set_weights(R.init_params(rng, 5, 128, 2))
@@ -23,7 +23,7 @@ for variant, E in (("5", 37), ("6", 45), ("6", 28)):
     for _ in range(2):
         summ = R.rollout(env, R.ActorSpec(kind=L.RL_ACTOR_CATEGORICAL_POLICY, net=net, lanes_per_env=L.RL_LANES_WARP_SPECIALIZED),
                          R.HistoryDataBound(20, 4), traj)
-    print("variant", variant, "E", E, "steps", summ.step_reward.count, "packed", R.pack_history(traj)["num_episodes"])
+    print("E", E, "steps", summ.step_reward.count, "packed", R.pack_history(traj)["num_episodes"])
 # deep module: rollout + TRPO + critic + PPO
 env = R.build_env(ctx, R.MemoryGame(4, 3), 40, seed=5)
 mc = R.MlpConfig(hidden_sizes=[24, 17], activation="tanh")

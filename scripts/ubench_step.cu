@@ -32,8 +32,7 @@ __global__ void lat_kernel(double a, double b, long long *out, double *sink, int
     sink[blockIdx.x * blockDim.x + threadIdx.x] = x + xf;
 }
 
-// step_fast chained: VARIANT 0 = step_fast, 1 = step_with_head with the head computed in-line (same work, other order)
-template <int VARIANT>
+// step_fast chained
 __global__ void step_kernel(CartPoleEnv::Params p, long long *out, double *sink, int iters, int active_warp_stride) {
     using E = CartPoleEnv;
     E::State s;
@@ -41,20 +40,12 @@ __global__ void step_kernel(CartPoleEnv::Params p, long long *out, double *sink,
     s.meta = 0x80000000u | 500u;
     const int warp = threadIdx.x >> 5;
     if (warp % active_warp_stride != 0) return;
-    const double y_ml = E::rcp_refined(p.mass_length_pole);
     int term = 0;
     const long long t0 = clock64();
 #pragma unroll 1
     for (int i = 0; i < iters; ++i) {
         const uint32_t action = (uint32_t)(__double2loint(s.x) >> 3) & 1u;
-        int sc;
-        if (VARIANT == 0) {
-            sc = E::step_fast(p, s, action);
-        } else {
-            E::Head h;
-            E::head_of(p, s.th, h);
-            sc = E::step_with_head(p, s, h, y_ml, action);
-        }
+        const int sc = E::step_fast(p, s, action);
         if (sc != RL_CONTINUE) {
             term++;
             s.x = 0.01; s.xd = 0.0; s.th = 0.02; s.thd = 0.0; s.meta = 0x80000000u | 500u;
@@ -162,13 +153,11 @@ int main() {
     p.time_step = 0.02; p.action_force = 10.0; p.max_pos = 2.4; p.max_angle = 0.2094;
     p.total_weight = 1.1 * 9.8; p.inv_total_mass = 1.0 / 1.1; p.mass_length_pole = 0.05; p.reset_low = -0.05; p.reset_scale = 0.1;
     p.max_steps = 500; p.visible = 1;
-    for (int variant = 0; variant < 2; ++variant)
-        for (int warps = 1; warps <= 8; warps *= 2) {
-            if (variant == 0) step_kernel<0><<<1, 32 * warps>>>(p, out, sink, 4000, 1);
-            else step_kernel<1><<<1, 32 * warps>>>(p, out, sink, 4000, 1);
-            cudaDeviceSynchronize();
-            printf("step variant %d, %d warps on one SM: %.1f clk per step (warp 0)\n", variant, warps, (double)out[0] / 4000.0);
-        }
+    for (int warps = 1; warps <= 8; warps *= 2) {
+        step_kernel<<<1, 32 * warps>>>(p, out, sink, 4000, 1);
+        cudaDeviceSynchronize();
+        printf("step, %d warps on one SM: %.1f clk per step (warp 0)\n", warps, (double)out[0] / 4000.0);
+    }
     ffma2_kernel<1><<<1, 32>>>(1.0f, 0.5f, out, sink, iters);
     cudaDeviceSynchronize();
     printf("FFMA2 dependent: %.2f clk per op\n", (double)out[0] / (iters * 16.0));

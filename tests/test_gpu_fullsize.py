@@ -265,11 +265,11 @@ def _check_lanes_against_oracle(host, lanes, T, seed, params, what):
 
 
 def test_bench_size_rollout_lanes_against_the_oracle(ctx, trpo_batch):
-    """configs[1] at its full size (E = 4096, T = 256, the kernel `lanes_per_env = 0` picks = K2w): 64 evenly spaced lanes
+    """configs[1] at its full size (E = 4096, T = 256, the kernel `lanes_per_env = 0` picks = K2q): 64 evenly spaced lanes
     replayed through the CPU oracle -- successor codes, lane lengths, rewards exactly, observations to 1e-6, and every
     action the inverse-CDF choice of the oracle's softmax under the step's Philox uniform."""
     env, agent, traj, summ, host, params = trpo_batch
-    _check_lanes_against_oracle(host, np.linspace(0, 4095, 64).astype(int), 256, 77, params, "K2w E=4096")
+    _check_lanes_against_oracle(host, np.linspace(0, 4095, 64).astype(int), 256, 77, params, "K2q E=4096")
 
 
 def test_tensor_core_rollout_lanes_against_the_oracle(ctx):
