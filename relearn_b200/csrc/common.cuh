@@ -51,6 +51,8 @@ struct rl_ctx {
     // pinned host scratch for scalar read-backs
     void *pinned = nullptr;
     size_t pinned_bytes = 0;
+    // K2q's count of finished CTAs (rollout.cu): 0 between launches
+    unsigned *rollout_ticket = nullptr;
     // timing events of the update entry points (created once, destroyed with the context: no leak on an early return)
     cudaEvent_t upd_ev[2] = {nullptr, nullptr};
 };

@@ -79,6 +79,7 @@ rl_status rl_ctx_destroy(rl_ctx *ctx) {
     if (ctx->scratch) cudaFree(ctx->scratch);
     if (ctx->scratch2) cudaFree(ctx->scratch2);
     if (ctx->pinned) cudaFreeHost(ctx->pinned);
+    if (ctx->rollout_ticket) cudaFree(ctx->rollout_ticket);
     for (cudaEvent_t ev : ctx->upd_ev)
         if (ev) cudaEventDestroy(ev);
     if (ctx->owns_stream) cudaStreamDestroy(ctx->stream);

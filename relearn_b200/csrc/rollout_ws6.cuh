@@ -11,7 +11,9 @@
 //    idle at the final barrier, eight policy warps and the aux (Philox) warp on the other three sub-partitions;
 //  * takes the step record off the dynamics warp (as K2z): successor code and reward are stored one iteration later by
 //    two idle threads of the env's policy group (the row carries the previous step's code), episode statistics are
-//    integer counters, finalize_last_episode reads the dropped observation back from the trajectory.
+//    integer counters, finalize_last_episode reads the dropped observation back from the trajectory;
+//  * needs no work around the launch: the dynamics lanes fill `succ` with RL_PAD past their last step, and the last CTA
+//    to finish sums every CTA's statistics (finalize_stat: rollout_finalize_kernel's sum, in its order).
 // The aux warp and its rings are K2z's (WS_RING / WS_CHUNK / WS_AHEAD, lane = env).  The hand-off has one row per env:
 // dynamics publishes the row of step i -> barrier 1 -> policy samples -> action -> barrier 2 -> dynamics selects.  The
 // grid is one CTA per 4 x policy_warps envs, so any number of waves runs.  Same operations on the same operands as
@@ -30,7 +32,7 @@ struct QkShared {
     uint32_t act[QK_ENVS];
     float thr[WS_RING][QK_ENVS];       // logit-space thresholds
     double2 slot[WS_RING][QK_ENVS][2]; // would-be reset states (x, x') | (theta, theta')
-    uint32_t prod, cons, done, pad;
+    uint32_t prod, cons, done, last;
 };
 #define QK_OFF(member) ((uint32_t)offsetof(QkShared, member))
 constexpr uint32_t QK_ACTIVE = 1u, QK_ANY = 2u, QK_PREV_ACTIVE = 4u;
@@ -365,6 +367,8 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
                     eps += 1.0;
                 }
             }
+            // the slots no step was stored in (rl_rollout fills `succ` with RL_PAD before the other kernels)
+            for (uint64_t k = i; k < a.Tcap; ++k) a.succ[k * a.E + e] = RL_PAD;
             a.lane_len[e] = len;
             a.lane_flags[e] = (uint8_t)flags;
             st.v[ST_STORED_STEPS] = (double)len;
@@ -373,4 +377,15 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
         }
     }
     block_reduce_stats(st, contributes, a.partials);
+    // The last CTA to finish publishes the totals (each CTA's partials are visible device-wide before it takes its
+    // ticket; that CTA puts the ticket back to 0 for the next launch).
+    if (threadIdx.x < ST_COUNT) __threadfence();
+    __syncthreads();
+    if (threadIdx.x == 0) sh.last = atomicAdd(a.ticket, 1u) == gridDim.x - 1 ? 1u : 0u;
+    __syncthreads();
+    if (sh.last) {
+        if (hw_warp < ST_COUNT)
+            finalize_stat(a.partials, (int)gridDim.x, hw_warp, lane, a.partials - ST_COUNT, a.traj_counts, a.summary_host);
+        if (threadIdx.x == 0) *a.ticket = 0u;
+    }
 }
