@@ -28,6 +28,7 @@
 
 #include "handles.cuh"
 #include "tcgen05.cuh"
+#include "steps.cuh"
 
 struct rl_grunet {
     rl_ctx *ctx = nullptr;
@@ -93,32 +94,6 @@ __device__ __forceinline__ void grunet_step(const GruView &m, const float *__res
     }
 }
 
-template <int MAXA>
-__device__ __forceinline__ uint32_t categorical_sample_seq(const float *z, int A, float u) {
-    // Categorical::new + sample (categorical.rs:29-33,52-54): inverse CDF over exp(log_softmax(z))
-    float m = z[0];
-#pragma unroll
-    for (int k = 1; k < MAXA; ++k)
-        if (k < A) m = fmaxf(m, z[k]);
-    float sum = 0.0f;
-#pragma unroll
-    for (int k = 0; k < MAXA; ++k)
-        if (k < A) sum += expf(z[k] - m);
-    const float lse = m + logf(sum);
-    float c = 0.0f;
-    uint32_t a = (uint32_t)(A - 1);
-    bool found = false;
-#pragma unroll
-    for (int k = 0; k < MAXA; ++k)
-        if (k < A && !found) {
-            c += expf(z[k] - lse);
-            if (u < c) { a = (uint32_t)k; found = true; }
-        }
-    return a;
-}
-
-enum { SQ_STEPS = 0, SQ_R, SQ_R2, SQ_EPS, SQ_ER, SQ_ER2, SQ_EL, SQ_EL2, SQ_STORED_STEPS, SQ_STORED_EPS, SQ_COUNT };
-
 struct SeqArgs {
     uint64_t E, lane_offset;
     NoiseSource noise;
@@ -130,7 +105,7 @@ struct SeqArgs {
     GruView net;
     int weights_in_smem;
     int F, A;
-    double *partials;  // f64 [gridDim.x][SQ_COUNT]
+    double *partials;  // f64 [gridDim.x][ST_COUNT]
     const float *wt;   // K8h only: Wt[F + H][3H]
     int tile_envs;     // K8h only: envs per CTA (32 or 64)
     int stepped;       // K8s: two launches per step, the cell on the tensor cores (gru_step_tc.cuh)
@@ -154,9 +129,8 @@ __global__ void __launch_bounds__(128) rollout_seq_kernel(typename EnvT::Params 
     const float *w = a.weights_in_smem ? sw : a.net.params;
     const uint64_t e = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const bool valid = e < a.E;
-    double st[SQ_COUNT];
-#pragma unroll
-    for (int i = 0; i < SQ_COUNT; ++i) st[i] = 0.0;
+    LaneStats st;
+    st.init();
     if (valid) {
         const int F = EXACT ? XF : a.F, A = EXACT ? XA : a.A;
         LaneNoise<REPLAY> nz;
@@ -169,8 +143,7 @@ __global__ void __launch_bounds__(128) rollout_seq_kernel(typename EnvT::Params 
 #pragma unroll
         for (int j = 0; j < HMAX; ++j) h[j] = 0.0f;  // SeqIterative::initial_state (gru.rs:23-28)
         uint32_t n = a.min_steps ? a.min_steps + a.slack : 0;  // take_steps.rs:20-31
-        uint32_t i = 0, cur_len = 0;
-        double cur_reward = 0.0;
+        uint32_t i = 0;
         int succ_last = RL_TERMINATE, succ_prev = RL_TERMINATE;
         if (n > 0) {  // train.rs:135: every period starts fresh episodes
             nz.set_step(t0);
@@ -182,7 +155,7 @@ __global__ void __launch_bounds__(128) rollout_seq_kernel(typename EnvT::Params 
             float z[MA];
             grunet_step<HMAX, MF, MA, EXACT>(a.net, w, obs, h, z);
             const float u = rl_u32_to_f32(nz.template next_u32<RL_STREAM_ACTOR>());
-            const uint32_t action = categorical_sample_seq<MA>(z, A, u);
+            const uint32_t action = categorical_sample<MA>(z, A, u);
 #pragma unroll
             for (int f = 0; f < MF; ++f)
                 if (f < F) {
@@ -207,80 +180,28 @@ __global__ void __launch_bounds__(128) rollout_seq_kernel(typename EnvT::Params 
             a.action[(uint64_t)i * a.E + e] = (uint8_t)action;
             a.reward[(uint64_t)i * a.E + e] = r;
             a.succ[(uint64_t)i * a.E + e] = (uint8_t)sc;
-            {  // OnlineStepsSummary::push (summary.rs:198-216)
-                const double rd = (double)r;
-                st[SQ_STEPS] += 1.0; st[SQ_R] += rd; st[SQ_R2] += rd * rd;
-                cur_len += 1;
-                cur_reward += rd;
-                if (sc != RL_CONTINUE) {
-                    const double ld = (double)cur_len;
-                    st[SQ_EPS] += 1.0; st[SQ_ER] += cur_reward; st[SQ_ER2] += cur_reward * cur_reward;
-                    st[SQ_EL] += ld; st[SQ_EL2] += ld * ld;
-                    cur_reward = 0.0;
-                    cur_len = 0;
-                }
-            }
+            st.push(r, sc);
             succ_prev = succ_last;
             succ_last = sc;
             i += 1;
             n -= 1;
             if (sc != RL_CONTINUE && n <= a.slack) n = 0;  // take_steps.rs:83-88
         }
-        // VecBuffer::end_experience -> finalize_last_episode (buffers/mod.rs:237-261)
-        uint32_t len = i, flags = 0;
-        double eps = st[SQ_EPS];
-        if (i > 0 && succ_last == RL_CONTINUE) {
-            len = i - 1;
-            flags = 1;
-            a.succ[(uint64_t)len * a.E + e] = RL_PAD;
-            if (len > 0 && succ_prev == RL_CONTINUE) {
-                flags = 3;
-                a.succ[(uint64_t)(len - 1) * a.E + e] = RL_INTERRUPT;
+        const LaneEnd end = finalize_last_episode(i, succ_last, succ_prev);
+        if (end.flags & 1u) a.succ[(uint64_t)end.len * a.E + e] = RL_PAD;
+        if (end.flags & 2u) {
+            a.succ[(uint64_t)(end.len - 1) * a.E + e] = RL_INTERRUPT;
 #pragma unroll
-                for (int f = 0; f < MF; ++f)
-                    if (f < F) a.next_obs[((uint64_t)(len - 1) * F + f) * a.E + e] = last_obs[f];
-                eps += 1.0;
-            }
+            for (int f = 0; f < MF; ++f)
+                if (f < F) a.next_obs[((uint64_t)(end.len - 1) * F + f) * a.E + e] = last_obs[f];
         }
-        a.lane_len[e] = len;
-        a.lane_flags[e] = (uint8_t)flags;
-        st[SQ_STORED_STEPS] = (double)len;
-        st[SQ_STORED_EPS] = eps;
+        a.lane_len[e] = end.len;
+        a.lane_flags[e] = (uint8_t)end.flags;
+        st.set_stored(end);
         nz.finish(a.noise, e);
     }
-    // deterministic block reduction -> partials[blockIdx.x][*]
-    __shared__ double red[4][SQ_COUNT];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-#pragma unroll
-    for (int k = 0; k < SQ_COUNT; ++k) {
-        double v = valid ? st[k] : 0.0;
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-        if (lane == 0) red[warp][k] = v;
-    }
-    __syncthreads();
-    if (threadIdx.x < SQ_COUNT) {
-        double v = 0.0;
-        for (int wi = 0; wi < (int)(blockDim.x >> 5); ++wi) v += red[wi][threadIdx.x];
-        a.partials[(size_t)blockIdx.x * SQ_COUNT + threadIdx.x] = v;
-    }
-}
-
-__global__ void __launch_bounds__(32 * SQ_COUNT) seq_finalize_kernel(const double *__restrict__ partials, int nblocks,
-                                                                    double *__restrict__ out, double *__restrict__ traj_counts) {
-    // one warp per statistic, fixed summation order (see rollout_finalize_kernel)
-    const int i = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (i >= SQ_COUNT) return;
-    double s = 0.0;
-#pragma unroll 4
-    for (int b = lane; b < nblocks; b += 32) s += partials[(size_t)b * SQ_COUNT + i];
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-    if (lane == 0) {
-        out[i] = s;
-        if (i == SQ_STORED_STEPS) traj_counts[0] = s;
-        if (i == SQ_STORED_EPS) traj_counts[1] = s;
-    }
+    __shared__ double red[4][ST_COUNT];
+    block_reduce_stats(st, valid, red, a.partials);
 }
 
 #include "gru_tile.cuh"
@@ -391,7 +312,7 @@ rl_status launch_seq(rl_ctx *ctx, const typename EnvT::Params &p, SeqArgs &a, bo
 }  // namespace
 
 // Called by rl_rollout (rollout.cu) when the actor carries a sequence network.
-rl_status rl_rollout_seq(rl_env *env, rl_grunet *net, rl_bound bound, rl_traj *traj, double **totals_out) {
+rl_status rl_rollout_seq(rl_env *env, rl_grunet *net, rl_bound bound, rl_traj *traj, double **partials_out, int *nblocks_out) {
     rl_ctx *ctx = env->ctx;
     const rl_env_structure &es = env->structure;
     RL_REQUIRE(ctx, net->ctx == ctx, "rl_rollout: network belongs to another context");
@@ -427,8 +348,8 @@ rl_status rl_rollout_seq(rl_env *env, rl_grunet *net, rl_bound bound, rl_traj *t
         a.wt = net->wt;
     }
     double *partials;
-    RL_TRY(rl_ctx_scratch(ctx, ((size_t)grid + 1) * SQ_COUNT * sizeof(double), (void **)&partials));
-    a.partials = partials + SQ_COUNT;
+    RL_TRY(rl_ctx_scratch(ctx, ((size_t)grid + 1) * ST_COUNT * sizeof(double), (void **)&partials));
+    a.partials = partials + ST_COUNT;
     const bool replay = env->noise.mode == RL_NOISE_REPLAY;
     switch (env->kind) {
     case RL_ENV_BANDIT_META: RL_TRY((launch_seq<BanditMetaEnv>(ctx, env->bandit, a, replay, smem, grid))); break;
@@ -436,8 +357,8 @@ rl_status rl_rollout_seq(rl_env *env, rl_grunet *net, rl_bound bound, rl_traj *t
     case RL_ENV_MEMORY_GAME: RL_TRY((launch_seq<MemoryEnv>(ctx, env->memory, a, replay, smem, grid))); break;
     default: return rl_fail(ctx, RL_ERR_UNSUPPORTED, "rl_rollout: sequence policies are built for the bandit meta-env, MemoryGame and CartPole");
     }
-    RL_LAUNCH(ctx, seq_finalize_kernel, 1, 32 * SQ_COUNT, 0, a.partials, (int)grid, partials, traj->counts_dev);
-    *totals_out = partials;
+    *partials_out = a.partials;
+    *nblocks_out = (int)grid;
     return RL_OK;
 }
 

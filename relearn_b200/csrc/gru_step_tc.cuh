@@ -4,7 +4,7 @@
 // env, that folds relu(h') into the logits, samples, steps the env, stores the step record and writes the next
 // observation.  K8h (gru_tile.cuh) keeps everything of a 64-env tile inside one persistent CTA but runs the cell as an FP32
 // FFMA2 GEMM (56 % of the FMA roof, 338 M env-steps/s); here the cell costs ~10 us per step for 18 944 envs and the env
-// state lives in a global array between launches.  Included by gru.cu after gru_tile.cuh (GtOwner, SeqArgs, SQ_*).
+// state lives in a global array between launches.  Included by gru.cu after gru_tile.cuh (GtOwner, SeqArgs, steps.cuh).
 #pragma once
 
 template <class EnvT, bool REPLAY>
@@ -14,10 +14,8 @@ __global__ void __launch_bounds__(128) seq_owner_init_kernel(typename EnvT::Para
     const uint64_t e = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= a.E) return;
     GtOwner<EnvT, REPLAY> o;
-#pragma unroll
-    for (int k = 0; k < SQ_COUNT; ++k) o.st[k] = 0.0;
-    o.cur_reward = 0.0;
-    o.i = o.cur_len = 0;
+    o.st.init();
+    o.i = 0;
     o.succ_last = o.succ_prev = RL_TERMINATE;
     o.n = a.min_steps ? a.min_steps + a.slack : 0;  // take_steps.rs:20-31
 #pragma unroll
@@ -87,7 +85,7 @@ __global__ void __launch_bounds__(256, 2) seq_owner_step_kernel(typename EnvT::P
     const uint32_t t0 = a.noise.step_counter, i = o.i;
     o.nz.set_step(t0 + i);
     const float u = rl_u32_to_f32(o.nz.template next_u32<RL_STREAM_ACTOR>());
-    const uint32_t action = categorical_sample_seq<MA>(zl, A, u);
+    const uint32_t action = categorical_sample<MA>(zl, A, u);
     {  // the step's observation: loads first, stores after (written pairwise the loads queued behind the stores)
         const float *__restrict__ xin = xplane;
         float *__restrict__ obs_out = a.obs;
@@ -122,19 +120,7 @@ __global__ void __launch_bounds__(256, 2) seq_owner_step_kernel(typename EnvT::P
     a.action[(uint64_t)i * E + e] = (uint8_t)action;
     a.reward[(uint64_t)i * E + e] = r;
     a.succ[(uint64_t)i * E + e] = (uint8_t)sc;
-    {  // OnlineStepsSummary::push (summary.rs:198-216)
-        const double rd = (double)r;
-        o.st[SQ_STEPS] += 1.0; o.st[SQ_R] += rd; o.st[SQ_R2] += rd * rd;
-        o.cur_len += 1;
-        o.cur_reward += rd;
-        if (sc != RL_CONTINUE) {
-            const double ld = (double)o.cur_len;
-            o.st[SQ_EPS] += 1.0; o.st[SQ_ER] += o.cur_reward; o.st[SQ_ER2] += o.cur_reward * o.cur_reward;
-            o.st[SQ_EL] += ld; o.st[SQ_EL2] += ld * ld;
-            o.cur_reward = 0.0;
-            o.cur_len = 0;
-        }
-    }
+    o.st.push(r, sc);
     o.succ_prev = o.succ_last;
     o.succ_last = sc;
     o.i = i + 1;
@@ -150,50 +136,26 @@ __global__ void __launch_bounds__(128) seq_owner_finish_kernel(SeqArgs a, GtOwne
     constexpr int MF = EnvT::MAXF;
     const uint64_t e = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const int F = a.F;
-    double st[SQ_COUNT];
-#pragma unroll
-    for (int k = 0; k < SQ_COUNT; ++k) st[k] = 0.0;
+    LaneStats st;
+    st.init();
     if (e < a.E) {
         GtOwner<EnvT, REPLAY> &o = owners[e];
+        st = o.st;
+        const LaneEnd end = finalize_last_episode(o.i, o.succ_last, o.succ_prev);
+        if (end.flags & 1u) a.succ[(uint64_t)end.len * a.E + e] = RL_PAD;
+        if (end.flags & 2u) {
+            a.succ[(uint64_t)(end.len - 1) * a.E + e] = RL_INTERRUPT;
 #pragma unroll
-        for (int k = 0; k < SQ_COUNT; ++k) st[k] = o.st[k];
-        const uint32_t i = o.i;
-        uint32_t len = i, flags = 0;
-        double eps = st[SQ_EPS];
-        if (i > 0 && o.succ_last == RL_CONTINUE) {
-            len = i - 1;
-            flags = 1;
-            a.succ[(uint64_t)len * a.E + e] = RL_PAD;
-            if (len > 0 && o.succ_prev == RL_CONTINUE) {
-                flags = 3;
-                a.succ[(uint64_t)(len - 1) * a.E + e] = RL_INTERRUPT;
-#pragma unroll
-                for (int f = 0; f < MF; ++f)
-                    if (f < F) a.next_obs[((uint64_t)(len - 1) * F + f) * a.E + e] = o.last_obs[f];
-                eps += 1.0;
-            }
+            for (int f = 0; f < MF; ++f)
+                if (f < F) a.next_obs[((uint64_t)(end.len - 1) * F + f) * a.E + e] = o.last_obs[f];
         }
-        a.lane_len[e] = len;
-        a.lane_flags[e] = (uint8_t)flags;
-        st[SQ_STORED_STEPS] = (double)len;
-        st[SQ_STORED_EPS] = eps;
+        a.lane_len[e] = end.len;
+        a.lane_flags[e] = (uint8_t)end.flags;
+        st.set_stored(end);
         o.nz.finish(a.noise, e);
     }
-    __shared__ double red[4][SQ_COUNT];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-#pragma unroll
-    for (int k = 0; k < SQ_COUNT; ++k) {
-        double v = st[k];
-#pragma unroll
-        for (int s = 16; s > 0; s >>= 1) v += __shfl_xor_sync(0xffffffffu, v, s);
-        if (lane == 0) red[warp][k] = v;
-    }
-    __syncthreads();
-    if (threadIdx.x < SQ_COUNT) {
-        double v = 0.0;
-        for (int w = 0; w < 4; ++w) v += red[w][threadIdx.x];
-        a.partials[(size_t)blockIdx.x * SQ_COUNT + threadIdx.x] = v;
-    }
+    __shared__ double red[4][ST_COUNT];
+    block_reduce_stats(st, e < a.E, red, a.partials);
 }
 
 template <class EnvT, bool REPLAY>

@@ -1,6 +1,6 @@
 // gru_tile.cuh -- K8h: fused rollout with the rl2-sized recurrent policy (Chain<Gru(F -> 128), Linear(128 -> A)>,
 // rl2-bandits.rs:379-393) where the GRU cell of a step is one register-tiled FP32 GEMM over the envs of a CTA.
-// Included by gru.cu inside its anonymous namespace (uses GruView, SeqArgs, SQ_*, categorical_sample_seq).
+// Included by gru.cu inside its anonymous namespace (uses GruView, SeqArgs and steps.cuh).
 //
 // Per step the cell is  [64 envs x (F + 128)] . [(F + 128) x 384]  (gate order r, z, n; libtorch gru_cell, see
 // gru.cu) -- 1.1e5 FLOP per env-step, FP32-FMA bound (SURVEY 8d, K8).  K8a (one thread per env, hidden state in
@@ -67,10 +67,9 @@ template <class EnvT, bool REPLAY>
 struct GtOwner {
     typename EnvT::State s;
     LaneNoise<REPLAY> nz;
-    double st[SQ_COUNT];
-    double cur_reward;
+    LaneStats st;
     float last_obs[EnvT::MAXF];
-    uint32_t n, i, cur_len;
+    uint32_t n, i;
     int succ_last, succ_prev;
 };
 
@@ -152,10 +151,8 @@ __global__ void __launch_bounds__(S::threads, 256 / S::threads) rollout_seq_tile
     };
     __syncthreads();
     if (owner) {
-#pragma unroll
-        for (int k = 0; k < SQ_COUNT; ++k) o.st[k] = 0.0;
-        o.cur_reward = 0.0;
-        o.i = o.cur_len = 0;
+        o.st.init();
+        o.i = 0;
         o.succ_last = o.succ_prev = RL_TERMINATE;
         o.n = (valid && a.min_steps) ? a.min_steps + a.slack : 0;  // take_steps.rs:20-31
 #pragma unroll
@@ -294,7 +291,7 @@ __global__ void __launch_bounds__(S::threads, 256 / S::threads) rollout_seq_tile
             const uint32_t i = o.i;
             o.nz.set_step(t0 + i);
             const float u = rl_u32_to_f32(o.nz.template next_u32<RL_STREAM_ACTOR>());
-            const uint32_t action = categorical_sample_seq<MA>(zl, A, u);
+            const uint32_t action = categorical_sample<MA>(zl, A, u);
 #pragma unroll
             for (int f = 0; f < MF; ++f)
                 if (f < F) {
@@ -320,19 +317,7 @@ __global__ void __launch_bounds__(S::threads, 256 / S::threads) rollout_seq_tile
             a.action[(uint64_t)i * a.E + e] = (uint8_t)action;
             a.reward[(uint64_t)i * a.E + e] = r;
             a.succ[(uint64_t)i * a.E + e] = (uint8_t)sc;
-            {  // OnlineStepsSummary::push (summary.rs:198-216)
-                const double rd = (double)r;
-                o.st[SQ_STEPS] += 1.0; o.st[SQ_R] += rd; o.st[SQ_R2] += rd * rd;
-                o.cur_len += 1;
-                o.cur_reward += rd;
-                if (sc != RL_CONTINUE) {
-                    const double ld = (double)o.cur_len;
-                    o.st[SQ_EPS] += 1.0; o.st[SQ_ER] += o.cur_reward; o.st[SQ_ER2] += o.cur_reward * o.cur_reward;
-                    o.st[SQ_EL] += ld; o.st[SQ_EL2] += ld * ld;
-                    o.cur_reward = 0.0;
-                    o.cur_len = 0;
-                }
-            }
+            o.st.push(r, sc);
             o.succ_prev = o.succ_last;
             o.succ_last = sc;
             o.i = i + 1;
@@ -346,51 +331,25 @@ __global__ void __launch_bounds__(S::threads, 256 / S::threads) rollout_seq_tile
     // chunks already in flight must land before the CTA may exit
     for (; g < issued; ++g) tc::mbar_wait(tc::smem_u32(&bars[g % GT_NBUF]), (g / GT_NBUF) & 1u);
 
-    // VecBuffer::end_experience -> finalize_last_episode (buffers/mod.rs:237-261)
-    double st[SQ_COUNT];
-#pragma unroll
-    for (int k = 0; k < SQ_COUNT; ++k) st[k] = 0.0;
+    LaneStats st;
+    st.init();
     if (owner && valid) {
+        st = o.st;
+        const LaneEnd end = finalize_last_episode(o.i, o.succ_last, o.succ_prev);
+        if (end.flags & 1u) a.succ[(uint64_t)end.len * a.E + e] = RL_PAD;
+        if (end.flags & 2u) {
+            a.succ[(uint64_t)(end.len - 1) * a.E + e] = RL_INTERRUPT;
 #pragma unroll
-        for (int k = 0; k < SQ_COUNT; ++k) st[k] = o.st[k];
-        const uint32_t i = o.i;
-        uint32_t len = i, flags = 0;
-        double eps = st[SQ_EPS];
-        if (i > 0 && o.succ_last == RL_CONTINUE) {
-            len = i - 1;
-            flags = 1;
-            a.succ[(uint64_t)len * a.E + e] = RL_PAD;
-            if (len > 0 && o.succ_prev == RL_CONTINUE) {
-                flags = 3;
-                a.succ[(uint64_t)(len - 1) * a.E + e] = RL_INTERRUPT;
-#pragma unroll
-                for (int f = 0; f < MF; ++f)
-                    if (f < F) a.next_obs[((uint64_t)(len - 1) * F + f) * a.E + e] = o.last_obs[f];
-                eps += 1.0;
-            }
+            for (int f = 0; f < MF; ++f)
+                if (f < F) a.next_obs[((uint64_t)(end.len - 1) * F + f) * a.E + e] = o.last_obs[f];
         }
-        a.lane_len[e] = len;
-        a.lane_flags[e] = (uint8_t)flags;
-        st[SQ_STORED_STEPS] = (double)len;
-        st[SQ_STORED_EPS] = eps;
+        a.lane_len[e] = end.len;
+        a.lane_flags[e] = (uint8_t)end.flags;
+        st.set_stored(end);
         o.nz.finish(a.noise, e);
     }
-    // deterministic block reduction -> partials[blockIdx.x][*] (xs is free now)
-    double *red = reinterpret_cast<double *>(xs);  // [8][SQ_COUNT]
-    __syncthreads();
-#pragma unroll
-    for (int k = 0; k < SQ_COUNT; ++k) {
-        double v = st[k];
-#pragma unroll
-        for (int s = 16; s > 0; s >>= 1) v += __shfl_xor_sync(0xffffffffu, v, s);
-        if (lane == 0) red[warp * SQ_COUNT + k] = v;
-    }
-    __syncthreads();
-    if (tid < SQ_COUNT) {
-        double v = 0.0;
-        for (int wi = 0; wi < GT_THREADS / 32; ++wi) v += red[wi * SQ_COUNT + tid];
-        a.partials[(size_t)blockIdx.x * SQ_COUNT + tid] = v;
-    }
+    __syncthreads();  // xs is free now: it takes the block reduction's per-warp rows
+    block_reduce_stats(st, owner && valid, reinterpret_cast<double (*)[ST_COUNT]>(xs), a.partials);
 }
 
 template <class EnvT, class S>

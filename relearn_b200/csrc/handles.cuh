@@ -124,8 +124,10 @@ struct rl_grunet_view { rl_ctx *ctx; int in_dim, hidden, out_dim, act; uint64_t 
 rl_grunet_view rl_grunet_view_of(rl_grunet *g);
 rl_status rl_grunet_seq_enqueue(rl_grunet *g, rl_traj *traj, float *out_dev, float *out_next_dev);
 
-// gru.cu: fused rollout with a recurrent policy; *totals_out receives the device pointer of the ST_COUNT sums
-rl_status rl_rollout_seq(rl_env *env, rl_grunet *net, rl_bound bound, rl_traj *traj, double **totals_out);
+// gru.cu: fused rollout with a recurrent policy.  *partials_out receives the device pointer of its *nblocks_out rows of
+// per-block statistics (steps.cuh: ST_COUNT sums each), with one more row in front of them for the totals; rl_rollout
+// sums them as it does for every rollout.
+rl_status rl_rollout_seq(rl_env *env, rl_grunet *net, rl_bound bound, rl_traj *traj, double **partials_out, int *nblocks_out);
 
 struct rl_tabq {
     rl_ctx *ctx = nullptr;

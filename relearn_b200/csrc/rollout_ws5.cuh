@@ -426,7 +426,8 @@ __global__ void __launch_bounds__(ZK_THREADS, 2) rollout_cartpole_ws5_kernel(Car
         const int act = lane >> 4;
         const uint64_t e = e_base + (lane & 15);
         if (e < a.E && act == 0) {
-            // VecBuffer::end_experience -> finalize_last_episode (buffers/mod.rs:237-261)
+            // VecBuffer::end_experience -> finalize_last_episode (buffers/mod.rs:237-261), steps.cuh's rule spelled out: with
+            // the helper, ptxas schedules the step loops above differently, and K2q's period was 0.3 % longer (B200, 1000 W)
             const uint32_t i = fin_steps;
             const int succ_last = fin_succ_last, succ_prev = fin_succ_prev;
             uint32_t len = i, flags = 0;
@@ -452,5 +453,6 @@ __global__ void __launch_bounds__(ZK_THREADS, 2) rollout_cartpole_ws5_kernel(Car
             contributes = true;
         }
     }
-    block_reduce_stats(st, contributes, a.partials);
+    __shared__ double red[32][ST_COUNT];
+    block_reduce_stats(st, contributes, red, a.partials);
 }

@@ -348,7 +348,8 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
     if (is_dyn) {
         const uint64_t e = e_base + lane;
         if (lane < cta_envs && e < a.E) {
-            // VecBuffer::end_experience -> finalize_last_episode (buffers/mod.rs:237-261)
+            // VecBuffer::end_experience -> finalize_last_episode (buffers/mod.rs:237-261), steps.cuh's rule spelled out: with
+            // the helper, ptxas schedules the step loops above differently, and K2q's period was 0.3 % longer (B200, 1000 W)
             const uint32_t i = fin_steps;
             const int succ_last = fin_succ_last, succ_prev = fin_succ_prev;
             uint32_t len = i, flags = 0;
@@ -376,7 +377,8 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
             contributes = true;
         }
     }
-    block_reduce_stats(st, contributes, a.partials);
+    __shared__ double red[32][ST_COUNT];
+    block_reduce_stats(st, contributes, red, a.partials);
     // The last CTA to finish publishes the totals (each CTA's partials are visible device-wide before it takes its
     // ticket; that CTA puts the ticket back to 0 for the next launch).
     if (threadIdx.x < ST_COUNT) __threadfence();

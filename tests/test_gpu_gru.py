@@ -23,6 +23,14 @@ def _episodes_of_lane(host, e):
     return [(int(a), int(b) + 1) for a, b in zip(starts, ends)]
 
 
+def _check_stored_counts(host, summ):
+    """The trajectory's step count (rl_traj_view_of) and the summary's stored steps and episodes agree with the stored
+    steps themselves: an episode ends at every stored Terminate or Interrupt."""
+    stored = np.arange(host["succ"].shape[0])[:, None] < host["lane_len"][None, :]
+    assert host["num_steps"] == summ.num_stored_steps == int(host["lane_len"].sum())
+    assert summ.num_stored_episodes == int(((host["succ"] != L.RL_CONTINUE) & stored).sum())
+
+
 def _check_actions(host, logits, awords, atol=2e-6):
     """Every action is the inverse-CDF choice of exp(log_softmax(logits)) for the replayed uniform."""
     T, E, A = logits.shape
@@ -58,11 +66,13 @@ def test_gru_policy_rollout_bandit_meta(ctx, hidden, arms, episodes):
     net.set_weights(params)
     np.testing.assert_array_equal(net.get_weights(), params)
     traj = R.Trajectory(env, T)
-    R.rollout(env, R.ActorSpec(kind=L.RL_ACTOR_CATEGORICAL_POLICY, seq_net=net), R.HistoryDataBound(T, 0), traj)
+    summ = R.rollout(env, R.ActorSpec(kind=L.RL_ACTOR_CATEGORICAL_POLICY, seq_net=net), R.HistoryDataBound(T, 0), traj)
     host = traj.to_host()
-    # (i) the dynamics given the kernel's own actions match the oracle bit for bit
+    # (i) the dynamics given the kernel's own actions match the oracle bit for bit, and so does the summary
     ref = P.oracle_rollout(cfg, E, T, 0, actor_kind=O.ACTOR_REPLAY, actions=host["action"].copy(), env_words=ewords)
     P.compare_traj(host, ref, what="gru bandit meta")
+    P.compare_summary(summ, ref["summary"])
+    _check_stored_counts(host, summ)
     # (ii) logits of the stored episodes: SeqPacked on the device vs SeqIterative in torch
     got = net.seq_packed(traj)
     want = np.zeros_like(got)
@@ -151,7 +161,13 @@ def test_gru128_tiled_rollout_matches_thread_per_env_kernel(ctx, monkeypatch):
     # the tiled kernel's own trajectory is a valid one: the oracle reproduces it from its actions
     ref = P.oracle_rollout(cfg, E, T, slack, actor_kind=O.ACTOR_REPLAY, actions=tile["action"].copy(), env_words=ewords)
     P.compare_traj(tile, ref, what="K8h")
-    assert tile["num_steps"] == st.num_stored_steps == int(tile["lane_len"].sum())
+    P.compare_summary(st, ref["summary"])
+    _check_stored_counts(tile, st)
+    # ... and so is the thread-per-env kernel's, summary included
+    ref1 = P.oracle_rollout(cfg, E, T, slack, actor_kind=O.ACTOR_REPLAY, actions=thread["action"].copy(), env_words=ewords)
+    P.compare_traj(thread, ref1, what="K8a")
+    P.compare_summary(sh, ref1["summary"])
+    _check_stored_counts(thread, sh)
     # K8s (gru_step_tc.cuh): two launches per step, the cell as bf16-piece tcgen05 MMAs over all envs.  Same contract: lanes
     # whose sampled actions agree with the thread-per-env kernel agree in every stored byte, and the oracle reproduces the
     # stepped kernel's own trajectory from its actions.
@@ -162,7 +178,8 @@ def test_gru128_tiled_rollout_matches_thread_per_env_kernel(ctx, monkeypatch):
         np.testing.assert_array_equal(stepped[k][:, same2], thread[k][:, same2], err_msg=f"stepped {k}")
     ref2 = P.oracle_rollout(cfg, E, T, slack, actor_kind=O.ACTOR_REPLAY, actions=stepped["action"].copy(), env_words=ewords)
     P.compare_traj(stepped, ref2, what="K8s")
-    assert stepped["num_steps"] == ss.num_stored_steps == int(stepped["lane_len"].sum())
+    P.compare_summary(ss, ref2["summary"])
+    _check_stored_counts(stepped, ss)
 
 
 def test_gru128_stepped_rollout_logits_match_gru_cell(ctx, monkeypatch):
