@@ -278,8 +278,24 @@ typedef enum {
     RL_ACTOR_CATEGORICAL_POLICY = 2, /* PolicyActor::act (src/torch/agents/policies/actor.rs:42-55) */
     RL_ACTOR_EPS_GREEDY_Q = 3,       /* DqnActor::act (src/torch/agents/dqn.rs:360-379) */
     RL_ACTOR_TABULAR_EPS_GREEDY = 4, /* BaseTabularQLearningActor::act (src/agents/tabular.rs:222-232) */
-    RL_ACTOR_UCB1 = 5                /* BaseUCB1Actor::act (src/agents/bandits/ucb.rs:214-243) */
+    RL_ACTOR_UCB1 = 5,               /* BaseUCB1Actor::act (src/agents/bandits/ucb.rs:214-243) */
+    /* ResettingMetaAgent (src/agents/meta.rs:16-227) over the inner agent rl_actor_cfg.inner_kind, on RL_ENV_BANDIT_META
+     * only (RL_ERR_UNSUPPORTED elsewhere).  Every lane carries its own inner agent, rebuilt at every trial start from the
+     * inner env structure (one observation, num_arms actions, the env's reward range) and updated online from the meta
+     * observation's previous step; it lives one trial inside one launch and never reaches device memory.  The inner actor
+     * always acts in training mode (meta.rs:103-106), so rl_actor_cfg.training is ignored.  lanes_per_env must be 0. */
+    RL_ACTOR_RESETTING_META = 6
 } rl_actor_kind;
+
+/* rl_actor_cfg.inner_kind: the agent RL_ACTOR_RESETTING_META rebuilds at each trial (the rl2-bandits baselines) */
+typedef enum {
+    RL_INNER_RANDOM = 0,    /* RandomAgent (src/agents/random.rs) */
+    RL_INNER_TABULAR_Q = 1, /* BaseTabularQLearningAgent (src/agents/tabular.rs:84-232): values 0, counts 0 (build_agent
+                             * ignores initial_action_count / initial_action_value, tabular.rs:61-77), epsilon-greedy with
+                             * epsilon = exploration_rate */
+    RL_INNER_UCB1 = 2       /* BaseUCB1Agent (src/agents/bandits/ucb.rs:78-243): one success and one failure per arm,
+                             * rewards scaled by the env's reward range, exploration_rate scales the bound */
+} rl_inner_agent_kind;
 
 /* rl_actor_cfg.lanes_per_env value selecting the tensor-core rollout kernel (CartPole + 5/4-128-2 ReLU network) */
 #define RL_LANES_TENSOR_CORE 128
@@ -293,13 +309,15 @@ typedef struct rl_actor_cfg {
     rl_mlp *net;                  /* CATEGORICAL_POLICY / EPS_GREEDY_Q */
     const uint8_t *actions_dev;   /* REPLAY_ACTIONS: u8 [T][E] */
     rl_tabq *table;               /* TABULAR_EPS_GREEDY */
-    double exploration_rate;      /* EPS_GREEDY_Q / TABULAR_EPS_GREEDY */
+    double exploration_rate;      /* EPS_GREEDY_Q / TABULAR_EPS_GREEDY; RESETTING_META: the inner tabular agent's epsilon
+                                   * or the inner UCB1 agent's exploration rate (unused for the random inner agent) */
     int32_t training;             /* ActorMode::Training (src/agents/mod.rs:144) */
     int32_t lanes_per_env;        /* 0 = auto; threads cooperating on one env's MLP (1,2,4,8,16,32),
                                    * RL_LANES_TENSOR_CORE (128): 128-env tiles, hidden layer on tcgen05 (K2t), or
                                    * RL_LANES_WARP_SPECIALIZED (160): K2z / K2q */
     rl_grunet *seq_net;           /* CATEGORICAL_POLICY with a recurrent module (Chain<Gru, Linear>) instead of `net` */
     rl_ucb1 *ucb;                 /* UCB1 (training: maximise the upper confidence bound; evaluation: the most selected action) */
+    int32_t inner_kind;           /* RESETTING_META: rl_inner_agent_kind; read for no other kind */
 } rl_actor_cfg;
 
 /* HistoryDataBound (src/agents/buffers/mod.rs:25-113), per lane */

@@ -3,7 +3,8 @@ in `torch_agents.py`."""
 from __future__ import annotations
 
 import ctypes as C
-from dataclasses import dataclass
+import math
+from dataclasses import dataclass, field
 
 import numpy as np
 
@@ -145,3 +146,78 @@ class UCB1Agent:
         v = np.ascontiguousarray(visits, np.uint64)
         L.check(self._lib.rl_ucb1_set_tables(self.handle, m.ctypes.data_as(C.c_void_p), c.ctypes.data_as(C.c_void_p),
                                              v.ctypes.data_as(C.c_void_p)), self.ctx.handle)
+
+
+@dataclass
+class RandomAgentConfig:
+    """RandomAgentConfig (src/agents/random.rs): acts uniformly at random and never learns.  Here only as the inner agent of
+    `ResettingMetaAgentConfig`."""
+
+
+@dataclass
+class TabularQLearningAgentConfig:
+    """TabularQLearningAgentConfig (src/agents/tabular.rs:43-51).  Here only as the inner agent of
+    `ResettingMetaAgentConfig`; `TabularQ` is the standalone agent.  `build_agent` in the reference ignores
+    `initial_action_count` and `initial_action_value` and starts every table from value 0 and count 0
+    (tabular.rs:61-77,97-111); the fields are kept, with no effect, so that configs read the same as the reference's."""
+
+    exploration_rate: float = 0.2
+    initial_action_count: int = 0
+    initial_action_value: float = 0.0
+
+
+@dataclass
+class ResettingMetaAgentConfig:
+    """ResettingMetaAgentConfig (src/agents/meta.rs:16-70): lifts a bandit agent onto the bandit meta-env.  The inner agent
+    is rebuilt at the start of every trial and learns online within it.  `agent_config` is a `RandomAgentConfig`, a
+    `TabularQLearningAgentConfig` or a `UCB1AgentConfig`."""
+
+    agent_config: object = field(default_factory=UCB1AgentConfig)
+
+    def build_agent(self, env) -> "ResettingMetaAgent":
+        """BuildAgent::build_agent (meta.rs:72-100): checks the inner agent can be built on the inner env structure (one
+        observation, the meta-env's actions, its reward range)."""
+        from .envs import MetaEnv
+
+        if not isinstance(env.config, MetaEnv):
+            raise ValueError("ResettingMetaAgent needs a meta environment (MetaEnv)")
+        c = self.agent_config
+        if isinstance(c, RandomAgentConfig):
+            inner, rate = L.RL_INNER_RANDOM, 0.0
+        elif isinstance(c, TabularQLearningAgentConfig):
+            inner, rate = L.RL_INNER_TABULAR_Q, float(c.exploration_rate)
+        elif isinstance(c, UCB1AgentConfig):
+            st = env.structure
+            width = st.reward_hi - st.reward_lo
+            if not math.isfinite(width) or not width > 0.0:  # BuildAgentError::UnboundedReward (ucb.rs:112-117)
+                raise ValueError("UCB1 needs a bounded reward range")
+            inner, rate = L.RL_INNER_UCB1, float(c.exploration_rate)
+        else:
+            raise ValueError(f"ResettingMetaAgent has no device inner agent for {type(c).__name__}")
+        return ResettingMetaAgent(inner, rate)
+
+
+class ResettingMetaAgent:
+    """ResettingMetaAgent (src/agents/meta.rs:102-227).  All its learning happens inside the rollout: each lane rebuilds the
+    inner agent at every trial start and folds each pull into it as the next meta observation reports it.  There is
+    nothing to update between rollouts."""
+
+    def __init__(self, inner_kind: int, exploration_rate: float):
+        self.inner_kind = inner_kind
+        self.exploration_rate = exploration_rate
+
+    def actor(self, training: bool = True) -> ActorSpec:
+        """Agent::actor (meta.rs:103-106): the mode is ignored; the inner agent always acts in training mode."""
+        return ActorSpec(kind=L.RL_ACTOR_RESETTING_META, inner_kind=self.inner_kind, exploration_rate=self.exploration_rate,
+                         training=training)
+
+    def min_update_size(self):
+        """HistoryDataBound::empty (meta.rs:211-213)."""
+        from .simulation import HistoryDataBound
+
+        return HistoryDataBound(0, 0)
+
+    def batch_update(self, traj: Trajectory, logger=None):
+        """No updates at the meta level (meta.rs:215-226)."""
+
+    update = batch_update

@@ -50,6 +50,7 @@ class ActorSpec:
     lanes_per_env: int = 0
     seq_net: object = None             # modules.GruLinear (recurrent CATEGORICAL_POLICY)
     ucb: object = None                 # agents.UCB1Agent
+    inner_kind: int = L.RL_INNER_RANDOM  # RESETTING_META: the inner agent (L.RL_INNER_*)
 
 
 class Trajectory:
@@ -129,6 +130,7 @@ def rollout(env: BatchedEnv, actor: ActorSpec, bound: HistoryDataBound, traj: Tr
     cfg.lanes_per_env = actor.lanes_per_env
     cfg.seq_net = actor.seq_net.handle if actor.seq_net is not None else None
     cfg.ucb = actor.ucb.handle if actor.ucb is not None else None
+    cfg.inner_kind = actor.inner_kind
     summ = L.StepsSummary() if want_summary else None
     L.check(lib.rl_rollout(env.handle, C.byref(cfg), L.Bound(bound.min_steps, bound.slack_steps), traj.handle,
                            C.byref(summ) if want_summary else None), env.ctx.handle)
