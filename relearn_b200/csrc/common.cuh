@@ -31,6 +31,7 @@ struct rl_ctx {
     int sm_count = 148;
     int cc_major = 0, cc_minor = 0;
     size_t total_mem = 0;
+    size_t smem_optin = 0;  // shared memory one block may opt in to (cudaFuncAttributeMaxDynamicSharedMemorySize + static)
     uint64_t launches = 0;
     std::string last_error;
     // NCCL data-parallel group (nccl.cu)
@@ -70,12 +71,15 @@ inline rl_status rl_fail(rl_ctx *ctx, rl_status st, const char *fmt, ...) {
     return st;
 }
 
+// The thread's last error is cleared on failure, so that a later RL_LAUNCH cannot report this call's error as its own.
 #define RL_CUDA(ctx, expr)                                                                          \
     do {                                                                                            \
         cudaError_t _e = (expr);                                                                    \
-        if (_e != cudaSuccess)                                                                      \
+        if (_e != cudaSuccess) {                                                                    \
+            cudaGetLastError();                                                                     \
             return rl_fail((ctx), _e == cudaErrorMemoryAllocation ? RL_ERR_OOM : RL_ERR_CUDA,       \
                            "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(_e), __FILE__, __LINE__); \
+        }                                                                                           \
     } while (0)
 
 #define RL_REQUIRE(ctx, cond, msg)                                                                  \

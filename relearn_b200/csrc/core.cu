@@ -61,6 +61,7 @@ rl_status rl_ctx_create(int32_t device, void *stream, rl_ctx **out) {
     ctx->cc_major = prop.major;
     ctx->cc_minor = prop.minor;
     ctx->total_mem = prop.totalGlobalMem;
+    ctx->smem_optin = prop.sharedMemPerBlockOptin;
     if (stream) {
         ctx->stream = (cudaStream_t)stream;
     } else {

@@ -170,6 +170,41 @@ def check_policy_consistency(host: dict, params, hidden, A, actor_words, atol=2e
     return checked, near_ties
 
 
+def check_eps_greedy_consistency(host: dict, params, hidden, A, eps, *, actor_words=None, philox=None, activation="relu"):
+    """DqnActor (dqn.rs:360-379) on every stored step: the lane's actor stream is walked in order -- `actor_words[e]` for
+    replayed noise, or `philox = (seed, lane_offset, t0)` with the step index set per step -- and decides with
+    Bernoulli(eps) whether the step explores.  An exploring action must equal the uniform draw over A; any other must be
+    the first argmax of the module's outputs for the recorded observation, unless the two outputs lie within
+    1e-5 * max(1, |z|) of each other (rounding near-tie).  Returns (steps checked, near-ties)."""
+    assert (actor_words is None) != (philox is None)
+    lib = O.lib()
+    T, E, F = host["obs"].shape
+    near_ties = 0
+    checked = 0
+    for e in range(E):
+        n = int(host["lane_len"][e])
+        rng = O.ScriptRng(actor_words[e]) if philox is None else O.PhiloxRng(philox[0], philox[1] + e, philox[2])
+        q = mlp_forward_any(params, F, hidden, A, host["obs"][:n, e], activation) if n else None
+        for i in range(n):
+            if philox is not None:
+                lib.ro_rng_set_step(rng.ref, philox[2] + i)
+            got = int(host["action"][i, e])
+            if lib.ro_gen_bool(rng.ref, O.STREAM_ACTOR, eps):
+                want = int(lib.ro_gen_range(rng.ref, O.STREAM_ACTOR, A))
+                if got != want:
+                    raise AssertionError(f"lane {e} step {i}: exploring action {got} != drawn {want}")
+                continue
+            z = q[i]
+            best = int(np.argmax(z))
+            if got != best:
+                if got < A and abs(float(z[got]) - float(z[best])) < 1e-5 * max(1.0, float(np.abs(z).max())):
+                    near_ties += 1
+                else:
+                    raise AssertionError(f"lane {e} step {i}: greedy action {got} != argmax {best} (q={z})")
+        checked += n
+    return checked, near_ties
+
+
 def smoke_check():
     """Small fused CartPole rollout with replayed actions and noise, compared with the oracle."""
     ctx = R.Context(0)

@@ -177,24 +177,6 @@ def test_fused_rollout_policy_cartpole_consistent(ctx, lanes):
     P.compare_traj(host, ref, obs_rtol=1e-6, obs_atol=1e-7, what=f"policy lanes={lanes}")
 
 
-def test_coop_kernel_matches_single_lane_kernel(ctx):
-    """The cooperative (L threads per env) kernel and the thread-per-env kernel agree on everything but
-    logit rounding; with replayed actions they are identical."""
-    rng = np.random.default_rng(40)
-    E, T = 64, 40
-    actions = rng.integers(0, 2, size=(T, E), dtype=np.uint8)
-    words = P.random_words(rng, E, 8 * T + 64)
-    hosts = []
-    for _ in range(2):
-        env = R.build_env(ctx, CARTPOLE, E, seed=3)
-        env.set_noise_replay(words, None)
-        traj = R.Trajectory(env, T)
-        R.rollout(env, R.ActorSpec(kind=L.RL_ACTOR_REPLAY_ACTIONS, actions=actions), R.HistoryDataBound(T, 0), traj)
-        hosts.append(traj.to_host())
-    for k in ("obs", "action", "reward", "succ", "lane_len"):
-        np.testing.assert_array_equal(hosts[0][k], hosts[1][k])
-
-
 def test_eps_greedy_q_actor_chain(ctx):
     rng = np.random.default_rng(50)
     cfg = R.Chain()
