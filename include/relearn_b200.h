@@ -62,6 +62,7 @@ typedef struct rl_adam rl_adam;
 typedef struct rl_traj rl_traj;
 typedef struct rl_tabq rl_tabq;
 typedef struct rl_ucb1 rl_ucb1;
+typedef struct rl_bts rl_bts;
 typedef struct rl_replay rl_replay;
 typedef struct rl_grunet rl_grunet;
 
@@ -284,7 +285,11 @@ typedef enum {
      * inner env structure (one observation, num_arms actions, the env's reward range) and updated online from the meta
      * observation's previous step; it lives one trial inside one launch and never reaches device memory.  The inner actor
      * always acts in training mode (meta.rs:103-106), so rl_actor_cfg.training is ignored.  lanes_per_env must be 0. */
-    RL_ACTOR_RESETTING_META = 6
+    RL_ACTOR_RESETTING_META = 6,
+    /* BaseBetaThompsonSamplingActor::act (src/agents/bandits/thompson_sampling.rs:192-212) over rl_actor_cfg.bts: training
+     * draws num_samples Beta(high, low) values per action from the device's own Beta sampler (DESIGN section 5) and keeps
+     * the largest sum, evaluation the largest high / (high + low); ties go to the LAST maximal action.  Thread per env. */
+    RL_ACTOR_BETA_THOMPSON = 7
 } rl_actor_kind;
 
 /* rl_actor_cfg.inner_kind: the agent RL_ACTOR_RESETTING_META rebuilds at each trial (the rl2-bandits baselines) */
@@ -293,8 +298,11 @@ typedef enum {
     RL_INNER_TABULAR_Q = 1, /* BaseTabularQLearningAgent (src/agents/tabular.rs:84-232): values 0, counts 0 (build_agent
                              * ignores initial_action_count / initial_action_value, tabular.rs:61-77), epsilon-greedy with
                              * epsilon = exploration_rate */
-    RL_INNER_UCB1 = 2       /* BaseUCB1Agent (src/agents/bandits/ucb.rs:78-243): one success and one failure per arm,
+    RL_INNER_UCB1 = 2,      /* BaseUCB1Agent (src/agents/bandits/ucb.rs:78-243): one success and one failure per arm,
                              * rewards scaled by the env's reward range, exploration_rate scales the bound */
+    RL_INNER_BETA_THOMPSON = 3 /* BaseBetaThompsonSamplingAgent (src/agents/bandits/thompson_sampling.rs:94-212): counts
+                                * (1, 1) per arm, the reward threshold halfway through the env's reward range,
+                                * rl_actor_cfg.num_samples Beta draws per arm */
 } rl_inner_agent_kind;
 
 /* rl_actor_cfg.lanes_per_env value selecting the tensor-core rollout kernel (CartPole + 5/4-128-2 ReLU network) */
@@ -318,6 +326,8 @@ typedef struct rl_actor_cfg {
     rl_grunet *seq_net;           /* CATEGORICAL_POLICY with a recurrent module (Chain<Gru, Linear>) instead of `net` */
     rl_ucb1 *ucb;                 /* UCB1 (training: maximise the upper confidence bound; evaluation: the most selected action) */
     int32_t inner_kind;           /* RESETTING_META: rl_inner_agent_kind; read for no other kind */
+    rl_bts *bts;                  /* BETA_THOMPSON (the draw count comes from the handle) */
+    int32_t num_samples;          /* RESETTING_META with RL_INNER_BETA_THOMPSON: Beta draws summed per arm, 1 .. 1024 */
 } rl_actor_cfg;
 
 /* HistoryDataBound (src/agents/buffers/mod.rs:25-113), per lane */
@@ -492,6 +502,19 @@ rl_status rl_ucb1_update(rl_ucb1 *u, rl_traj *traj);
 rl_status rl_ucb1_get_tables(rl_ucb1 *u, double *mean_host, uint64_t *action_count_host, uint64_t *visit_count_host);
 rl_status rl_ucb1_set_tables(rl_ucb1 *u, const double *mean_host, const uint64_t *action_count_host,
                              const uint64_t *visit_count_host);
+
+/* BetaThompsonSamplingAgent (src/agents/bandits/thompson_sampling.rs:20-212): Beta-Bernoulli Thompson sampling applied
+ * independently to each state of a finite observation space.  Tables per replica: low and high reward counts u64 [S][A],
+ * both starting at 1; a step counts as high when its reward is above (reward_lo + reward_hi) / 2 (f64, strict).  As for
+ * rl_ucb1, num_replicas = 1 is one agent shared by every lane (train_parallel) and num_replicas = num_envs one agent per
+ * lane; the counts are integer increments, so rl_bts_update's result does not depend on the order of the steps.
+ * num_samples (1 .. 1024) is the number of Beta draws summed per action in training mode. */
+rl_status rl_bts_create(rl_ctx *ctx, uint64_t num_replicas, int32_t num_observations, int32_t num_actions, double reward_lo,
+                        double reward_hi, int32_t num_samples, rl_bts **out);
+rl_status rl_bts_destroy(rl_bts *b);
+rl_status rl_bts_update(rl_bts *b, rl_traj *traj);
+rl_status rl_bts_get_counts(rl_bts *b, uint64_t *low_host, uint64_t *high_host);
+rl_status rl_bts_set_counts(rl_bts *b, const uint64_t *low_host, const uint64_t *high_host);
 
 /* ------------------------------------------------------------------------------------------ */
 /* DQN (ReplayBuffer src/agents/buffers/replay.rs:11-126; DqnAgent::batch_update                 */

@@ -13,8 +13,9 @@ from .simulation import (ActorSpec, HistoryDataBound, TrainParallelConfig, Traje
 from .logging import DisplayLogger, HistoryLogger, NullLogger, StatsLogger  # noqa: F401
 
 __version__ = "0.1.0"
-from .agents import (RandomAgentConfig, ResettingMetaAgent, ResettingMetaAgentConfig, TabularQ,  # noqa: F401,E402
-                     TabularQLearningAgentConfig, UCB1Agent, UCB1AgentConfig)
+from .agents import (BetaThompsonSamplingAgent, BetaThompsonSamplingAgentConfig, RandomAgentConfig,  # noqa: F401,E402
+                     ResettingMetaAgent, ResettingMetaAgentConfig, TabularQ, TabularQLearningAgentConfig, UCB1Agent,
+                     UCB1AgentConfig)
 from .torch_agents import (ActorCriticAgent, ActorCriticConfig, Adam, AdamConfig,  # noqa: F401,E402
                            ConjugateGradientOptimizerConfig, DataCollectionSchedule, DqnAgent, DqnConfig,
                            ExplorationRateSchedule, OptimizerStepError, Ppo, PpoConfig, Reinforce, ReinforceConfig,

@@ -23,8 +23,9 @@ RL_NOISE_PHILOX, RL_NOISE_REPLAY = 0, 1
 RL_SPACE_INTERVAL, RL_SPACE_INDEX, RL_SPACE_BOOLEAN, RL_SPACE_OPTION_INDEX = 0, 1, 2, 3
 RL_ACT_IDENTITY, RL_ACT_RELU, RL_ACT_SIGMOID, RL_ACT_TANH = 0, 1, 2, 3
 (RL_ACTOR_REPLAY_ACTIONS, RL_ACTOR_RANDOM, RL_ACTOR_CATEGORICAL_POLICY, RL_ACTOR_EPS_GREEDY_Q,
- RL_ACTOR_TABULAR_EPS_GREEDY, RL_ACTOR_UCB1, RL_ACTOR_RESETTING_META) = range(7)
-RL_INNER_RANDOM, RL_INNER_TABULAR_Q, RL_INNER_UCB1 = 0, 1, 2  # rl_actor_cfg.inner_kind of RL_ACTOR_RESETTING_META
+ RL_ACTOR_TABULAR_EPS_GREEDY, RL_ACTOR_UCB1, RL_ACTOR_RESETTING_META, RL_ACTOR_BETA_THOMPSON) = range(8)
+# rl_actor_cfg.inner_kind of RL_ACTOR_RESETTING_META
+RL_INNER_RANDOM, RL_INNER_TABULAR_Q, RL_INNER_UCB1, RL_INNER_BETA_THOMPSON = 0, 1, 2, 3
 RL_STREAM_ENV_STEP, RL_STREAM_ENV_RESET, RL_STREAM_ACTOR, RL_STREAM_SAMPLER = 0, 1, 2, 3
 RL_NCCL_UNIQUE_ID_BYTES = 128
 RL_PASS_KERNEL_FFMA, RL_PASS_KERNEL_TCGEN05 = 0, 1
@@ -63,7 +64,7 @@ class StepOut(C.Structure):
 class ActorCfg(C.Structure):
     _fields_ = [("kind", C.c_int32), ("net", vp), ("actions_dev", vp), ("table", vp),
                 ("exploration_rate", C.c_double), ("training", C.c_int32), ("lanes_per_env", C.c_int32),
-                ("seq_net", vp), ("ucb", vp), ("inner_kind", C.c_int32)]
+                ("seq_net", vp), ("ucb", vp), ("inner_kind", C.c_int32), ("bts", vp), ("num_samples", C.c_int32)]
 
 
 class PackedInfo(C.Structure):
@@ -231,6 +232,11 @@ SIGNATURES = {
     "rl_ucb1_update": (st, [vp, vp]),
     "rl_ucb1_get_tables": (st, [vp, vp, vp, vp]),
     "rl_ucb1_set_tables": (st, [vp, vp, vp, vp]),
+    "rl_bts_create": (st, [vp, C.c_uint64, C.c_int32, C.c_int32, C.c_double, C.c_double, C.c_int32, P(vp)]),
+    "rl_bts_destroy": (st, [vp]),
+    "rl_bts_update": (st, [vp, vp]),
+    "rl_bts_get_counts": (st, [vp, vp, vp]),
+    "rl_bts_set_counts": (st, [vp, vp, vp]),
     "rl_replay_create": (st, [vp, C.c_uint64, P(vp)]),
     "rl_replay_destroy": (st, [vp]),
     "rl_replay_append": (st, [vp, vp]),

@@ -1,4 +1,4 @@
-"""Finite-space agents (src/agents): tabular Q-learning and UCB1; the neural agents (ActorCritic / TRPO / PPO, DQN) live
+"""Finite-space agents (src/agents): tabular Q-learning, UCB1 and Beta Thompson sampling; the neural agents (ActorCritic / TRPO / PPO, DQN) live
 in `torch_agents.py`."""
 from __future__ import annotations
 
@@ -149,6 +149,81 @@ class UCB1Agent:
 
 
 @dataclass
+class BetaThompsonSamplingAgentConfig:
+    """BetaThompsonSamplingAgentConfig (src/agents/bandits/thompson_sampling.rs:20-39): `num_samples` Beta draws are summed
+    per action (1 is plain Thompson sampling; rl2-bandits' "OTS" row uses 10)."""
+
+    num_samples: int = 1
+
+    def build_agent(self, env, num_replicas: int = 1) -> "BetaThompsonSamplingAgent":
+        """BuildAgent::build_agent (thompson_sampling.rs:41-75): counts sized by the env's finite observation / action
+        spaces, the reward threshold halfway through its feedback range.  `num_replicas`: 1 = one agent shared by every
+        lane (train_parallel), env.num_envs = one independent agent per lane."""
+        st = env.structure
+        if st.num_observations <= 0:
+            raise ValueError("Thompson sampling needs a finite observation space")
+        return BetaThompsonSamplingAgent(env.ctx, num_replicas, st.num_observations, st.num_actions,
+                                         (st.reward_lo, st.reward_hi), self.num_samples)
+
+
+class BetaThompsonSamplingAgent:
+    """BaseBetaThompsonSamplingAgent (src/agents/bandits/thompson_sampling.rs:84-212): a Beta posterior over each state-action
+    pair's chance of a reward above the threshold.  The device draws Beta samples with its own sampler (DESIGN section 5):
+    exact in distribution, not the reference's bit stream."""
+
+    def __init__(self, ctx: Context, num_replicas: int, num_observations: int, num_actions: int, reward_range,
+                 num_samples: int = 1):
+        self.ctx, self._lib = ctx, ctx._lib
+        self.shape = (num_replicas, num_observations, num_actions)
+        self.num_samples = num_samples
+        h = C.c_void_p()
+        L.check(self._lib.rl_bts_create(ctx.handle, num_replicas, num_observations, num_actions, float(reward_range[0]),
+                                        float(reward_range[1]), int(num_samples), C.byref(h)), ctx.handle)
+        self.handle = h
+
+    def close(self):
+        if self.handle and self.ctx.handle:
+            self._lib.rl_bts_destroy(self.handle)
+        self.handle = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def actor(self, training: bool = True) -> ActorSpec:
+        """Agent::actor(mode) (thompson_sampling.rs:139-147): Training samples, Evaluation takes the posterior mean."""
+        return ActorSpec(kind=L.RL_ACTOR_BETA_THOMPSON, bts=self, training=training)
+
+    def update(self, traj: Trajectory, logger=None):
+        """BatchUpdate::batch_update (thompson_sampling.rs:166-177)."""
+        L.check(self._lib.rl_bts_update(self.handle, traj.handle), self.ctx.handle)
+
+    batch_update = update
+
+    def min_update_size(self):
+        """thompson_sampling.rs:159-164."""
+        from .simulation import HistoryDataBound
+
+        return HistoryDataBound(1, 0)
+
+    def get_counts(self):
+        """(low reward count u64 [R, S, A], high reward count u64 [R, S, A])."""
+        lo = np.empty(self.shape, np.uint64)
+        hi = np.empty(self.shape, np.uint64)
+        L.check(self._lib.rl_bts_get_counts(self.handle, lo.ctypes.data_as(C.c_void_p), hi.ctypes.data_as(C.c_void_p)),
+                self.ctx.handle)
+        return lo, hi
+
+    def set_counts(self, low, high):
+        lo = np.ascontiguousarray(low, np.uint64)
+        hi = np.ascontiguousarray(high, np.uint64)
+        L.check(self._lib.rl_bts_set_counts(self.handle, lo.ctypes.data_as(C.c_void_p), hi.ctypes.data_as(C.c_void_p)),
+                self.ctx.handle)
+
+
+@dataclass
 class RandomAgentConfig:
     """RandomAgentConfig (src/agents/random.rs): acts uniformly at random and never learns.  Here only as the inner agent of
     `ResettingMetaAgentConfig`."""
@@ -170,7 +245,7 @@ class TabularQLearningAgentConfig:
 class ResettingMetaAgentConfig:
     """ResettingMetaAgentConfig (src/agents/meta.rs:16-70): lifts a bandit agent onto the bandit meta-env.  The inner agent
     is rebuilt at the start of every trial and learns online within it.  `agent_config` is a `RandomAgentConfig`, a
-    `TabularQLearningAgentConfig` or a `UCB1AgentConfig`."""
+    `TabularQLearningAgentConfig`, a `UCB1AgentConfig` or a `BetaThompsonSamplingAgentConfig`."""
 
     agent_config: object = field(default_factory=UCB1AgentConfig)
 
@@ -192,6 +267,10 @@ class ResettingMetaAgentConfig:
             if not math.isfinite(width) or not width > 0.0:  # BuildAgentError::UnboundedReward (ucb.rs:112-117)
                 raise ValueError("UCB1 needs a bounded reward range")
             inner, rate = L.RL_INNER_UCB1, float(c.exploration_rate)
+        elif isinstance(c, BetaThompsonSamplingAgentConfig):
+            if not 1 <= int(c.num_samples) <= 1024:
+                raise ValueError("Thompson sampling needs num_samples in 1 .. 1024")
+            return ResettingMetaAgent(L.RL_INNER_BETA_THOMPSON, 0.0, int(c.num_samples))
         else:
             raise ValueError(f"ResettingMetaAgent has no device inner agent for {type(c).__name__}")
         return ResettingMetaAgent(inner, rate)
@@ -202,14 +281,15 @@ class ResettingMetaAgent:
     inner agent at every trial start and folds each pull into it as the next meta observation reports it.  There is
     nothing to update between rollouts."""
 
-    def __init__(self, inner_kind: int, exploration_rate: float):
+    def __init__(self, inner_kind: int, exploration_rate: float, num_samples: int = 1):
         self.inner_kind = inner_kind
         self.exploration_rate = exploration_rate
+        self.num_samples = num_samples
 
     def actor(self, training: bool = True) -> ActorSpec:
         """Agent::actor (meta.rs:103-106): the mode is ignored; the inner agent always acts in training mode."""
         return ActorSpec(kind=L.RL_ACTOR_RESETTING_META, inner_kind=self.inner_kind, exploration_rate=self.exploration_rate,
-                         training=training)
+                         training=training, num_samples=self.num_samples)
 
     def min_update_size(self):
         """HistoryDataBound::empty (meta.rs:211-213)."""

@@ -148,6 +148,16 @@ struct rl_ucb1 {
     unsigned long long *visits = nullptr;    // u64 [R][S]
 };
 
+struct rl_bts {
+    rl_ctx *ctx = nullptr;
+    uint64_t R = 0;
+    int S = 0, A = 0;
+    int num_samples = 1;
+    double threshold = 0.0;                  // (reward_min + reward_max) / 2 (thompson_sampling.rs:102-103)
+    unsigned long long *low = nullptr;       // u64 [R][S][A]
+    unsigned long long *high = nullptr;      // u64 [R][S][A]
+};
+
 // Mlp weights passed by value into kernels
 struct MlpView {
     const float *params;

@@ -13,7 +13,7 @@
 //  1. with a previous step (has_prev), fold it into the inner agent at once: observation 0, action prev_action, reward
 //     prev_reward, successor Terminate (every inner bandit episode is one step, so SerialActorAgent's update bound
 //     {1, 0} is met after every step, serial.rs:60-76, buffers/mod.rs:94-101);
-//  2. at the end of an inner episode (inner_done) reset the inner actor state (nothing, for all three agents) and
+//  2. at the end of an inner episode (inner_done) reset the inner actor state (nothing, for all four agents) and
 //     take action 0 (some_element, index.rs:57-60) without a draw;
 //  3. otherwise act with the inner agent in training mode (SerialActorAgent::new, serial.rs:49).
 // The last pull of a trial is never folded in: it ends the trial (Interrupt) and the agent is rebuilt.  Every draw
@@ -21,10 +21,13 @@
 #pragma once
 
 #include "finite_agents.cuh"
+#include "beta.cuh"
 
 struct MetaInnerArgs {
     double rate;          // tabular: epsilon; UCB1: exploration rate
     double shift, scale;  // UCB1: the reward scaling (ucb.rs:112-123)
+    double threshold;     // Thompson sampling: (reward_min + reward_max) / 2 (thompson_sampling.rs:102-103)
+    int num_samples;      // Thompson sampling: Beta draws summed per arm
 };
 
 template <int INNER>
@@ -33,6 +36,7 @@ struct MetaInnerAgent {
     double v[K];      // tabular: action values; UCB1: mean scaled reward
     uint32_t c[K];    // selection counts
     uint32_t visits;  // UCB1: visit count of the single inner observation
+    uint32_t low[K], high[K];  // Thompson sampling: low / high reward counts (thompson_sampling.rs:91-92)
 
     // build_agent over the inner env structure; none of the builders draws (tabular.rs:61-77, ucb.rs:49-74, random.rs)
     __device__ __forceinline__ void build(int k) {
@@ -43,6 +47,9 @@ struct MetaInnerAgent {
 #pragma unroll
             for (int i = 0; i < K; ++i) { v[i] = 0.5; c[i] = 2u; }
             visits = 2u * (uint32_t)k;
+        } else if constexpr (INNER == RL_INNER_BETA_THOMPSON) {  // (1, 1) per arm (thompson_sampling.rs:104-105)
+#pragma unroll
+            for (int i = 0; i < K; ++i) { low[i] = 1u; high[i] = 1u; }
         }
     }
 
@@ -63,6 +70,14 @@ struct MetaInnerAgent {
                     c[i] += 1u;
                     v[i] = ucb1_mean_update(v[i], (double)c[i], scaled);
                 }
+        } else if constexpr (INNER == RL_INNER_BETA_THOMPSON) {  // thompson_sampling.rs:126-136: strictly above, in f64
+            const bool is_high = reward > m.threshold;
+#pragma unroll
+            for (int i = 0; i < K; ++i)
+                if ((uint32_t)i == action) {
+                    if (is_high) high[i] += 1u;
+                    else low[i] += 1u;
+                }
         }
     }
 
@@ -79,6 +94,21 @@ struct MetaInnerAgent {
 #pragma unroll
             for (int i = 1; i < K; ++i)
                 if (i < k && v[i] > bv) { bv = v[i]; best = (uint32_t)i; }
+            return best;
+        } else if constexpr (INNER == RL_INNER_BETA_THOMPSON) {
+            // thompson_sampling.rs:192-205 in training mode: per arm in order, the sum of num_samples Beta(high, low)
+            // draws (beta.cuh); argmax_by keeps the LAST maximal element.  The counts are read by a predicated select so
+            // that the draw loops are not unrolled per arm.
+            uint32_t best = 0;
+            double bv = 0.0;
+            for (int i = 0; i < k; ++i) {
+                uint32_t lo = low[0], hi = high[0];
+#pragma unroll
+                for (int j = 1; j < K; ++j)
+                    if (j == i) { lo = low[j]; hi = high[j]; }
+                const double u = rl_beta_sample_sum<REPLAY>(nz, (double)hi, (double)lo, m.num_samples);
+                if (i == 0 || u >= bv) { bv = u; best = (uint32_t)i; }
+            }
             return best;
         } else {  // ucb.rs:219-231; argmax_by keeps the LAST maximal element (utils/iter/cmp.rs:58-76)
             const double lsv = ucb1_log_squared_visits((double)visits);

@@ -1,4 +1,5 @@
-// tabq.cu -- the finite-space agents: tabular Q-learning (src/agents/tabular.rs:84-232) and UCB1 (src/agents/bandits/ucb.rs).
+// tabq.cu -- the finite-space agents: tabular Q-learning (src/agents/tabular.rs:84-232), UCB1 (src/agents/bandits/ucb.rs) and
+// Beta Thompson sampling (src/agents/bandits/thompson_sampling.rs).
 //
 // The reference update is a strictly sequential fold over the buffer whose bootstrap term reads the
 // live table (tabular.rs:160-178), so a single shared table cannot be updated in parallel and stay
@@ -94,9 +95,97 @@ __global__ void __launch_bounds__(128)
         }
 }
 
+// BaseBetaThompsonSamplingAgent::batch_update (thompson_sampling.rs:166-177) = step_update (:126-136) over every stored
+// step: one thread per lane.  The counts are integer increments, so a shared table (R == 1) takes every lane's steps
+// through atomics and ends bit-identical to the reference's sequential fold in any order.
+__global__ void __launch_bounds__(128)
+    bts_update_kernel(unsigned long long *__restrict__ low, unsigned long long *__restrict__ high, uint64_t R, int S, int A,
+                      double threshold, const float *__restrict__ obs, const uint8_t *__restrict__ action,
+                      const float *__restrict__ reward, const uint8_t *__restrict__ succ, uint64_t T, uint64_t E, int F) {
+    const uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= E) return;
+    const uint64_t base = R == E ? r * (uint64_t)S * A : 0;
+    for (uint64_t t = 0; t < T; ++t) {
+        if (succ[t * E + r] == RL_PAD) break;
+        int o = 0;  // finite observation spaces are stored one-hot (index.rs:97-115)
+        for (int f = 0; f < F; ++f)
+            if (obs[(t * F + f) * E + r] != 0.0f) o = f;
+        const uint64_t idx = base + (uint64_t)o * A + action[t * E + r];
+        atomicAdd((double)reward[t * E + r] > threshold ? &high[idx] : &low[idx], 1ull);
+    }
+}
+
 }  // namespace
 
 extern "C" {
+
+rl_status rl_bts_create(rl_ctx *ctx, uint64_t num_replicas, int32_t num_observations, int32_t num_actions, double reward_lo,
+                        double reward_hi, int32_t num_samples, rl_bts **out) {
+    RL_REQUIRE(ctx, ctx && out, "rl_bts_create: NULL argument");
+    RL_REQUIRE(ctx, num_replicas > 0 && num_observations > 0 && num_actions > 0, "rl_bts_create: empty table");
+    RL_REQUIRE(ctx, num_samples >= 1 && num_samples <= 1024, "rl_bts_create: num_samples must be in 1 .. 1024");
+    RL_CUDA(ctx, cudaSetDevice(ctx->device));
+    rl_bts *b = new (std::nothrow) rl_bts();
+    if (!b) return rl_fail(ctx, RL_ERR_OOM, "rl_bts_create: host allocation failed");
+    b->ctx = ctx; b->R = num_replicas; b->S = num_observations; b->A = num_actions; b->num_samples = num_samples;
+    b->threshold = (reward_lo + reward_hi) / 2.0;  // thompson_sampling.rs:102-103
+    const size_t n = (size_t)num_replicas * num_observations * num_actions;
+    cudaError_t e = cudaMalloc((void **)&b->low, n * sizeof(unsigned long long));
+    if (e == cudaSuccess) e = cudaMalloc((void **)&b->high, n * sizeof(unsigned long long));
+    if (e != cudaSuccess) {
+        rl_bts_destroy(b);
+        return rl_fail(ctx, RL_ERR_OOM, "rl_bts_create: %s", cudaGetErrorString(e));
+    }
+    std::vector<unsigned long long> ones(n, 1ull);  // (1, 1) for every observation-action pair (:104-105)
+    const rl_status st = rl_bts_set_counts(b, (const uint64_t *)ones.data(), (const uint64_t *)ones.data());
+    if (st != RL_OK) {
+        rl_bts_destroy(b);
+        return st;
+    }
+    *out = b;
+    return RL_OK;
+}
+
+rl_status rl_bts_destroy(rl_bts *b) {
+    if (!b) return RL_OK;
+    cudaSetDevice(b->ctx->device);
+    cudaStreamSynchronize(b->ctx->stream);
+    cudaFree(b->low); cudaFree(b->high);
+    delete b;
+    return RL_OK;
+}
+
+rl_status rl_bts_update(rl_bts *b, rl_traj *traj) {
+    if (!b || !traj) return rl_fail(b ? b->ctx : nullptr, RL_ERR_INVALID_ARG, "rl_bts_update: NULL argument");
+    rl_ctx *ctx = b->ctx;
+    RL_REQUIRE(ctx, traj->E == b->R || b->R == 1, "rl_bts_update: one replica per lane, or one shared set of counts (num_replicas = 1)");
+    RL_REQUIRE(ctx, (int)traj->F == b->S, "rl_bts_update: observation space size mismatch");
+    const uint64_t T = traj->used_T ? traj->used_T : traj->T;
+    const unsigned block = 128, grid = rl_grid_for(traj->E, block);
+    RL_LAUNCH(ctx, bts_update_kernel, grid, block, 0, b->low, b->high, b->R, b->S, b->A, b->threshold, traj->obs, traj->action,
+              traj->reward, traj->succ, T, traj->E, (int)traj->F);
+    return RL_OK;
+}
+
+rl_status rl_bts_get_counts(rl_bts *b, uint64_t *low_host, uint64_t *high_host) {
+    if (!b) return rl_fail(nullptr, RL_ERR_INVALID_ARG, "rl_bts_get_counts: NULL argument");
+    rl_ctx *ctx = b->ctx;
+    const size_t n = (size_t)b->R * b->S * b->A;
+    RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    if (low_host) RL_CUDA(ctx, cudaMemcpy(low_host, b->low, n * sizeof(uint64_t), cudaMemcpyDeviceToHost));
+    if (high_host) RL_CUDA(ctx, cudaMemcpy(high_host, b->high, n * sizeof(uint64_t), cudaMemcpyDeviceToHost));
+    return RL_OK;
+}
+
+rl_status rl_bts_set_counts(rl_bts *b, const uint64_t *low_host, const uint64_t *high_host) {
+    if (!b) return rl_fail(nullptr, RL_ERR_INVALID_ARG, "rl_bts_set_counts: NULL argument");
+    rl_ctx *ctx = b->ctx;
+    const size_t n = (size_t)b->R * b->S * b->A;
+    RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    if (low_host) RL_CUDA(ctx, cudaMemcpy(b->low, low_host, n * sizeof(uint64_t), cudaMemcpyHostToDevice));
+    if (high_host) RL_CUDA(ctx, cudaMemcpy(b->high, high_host, n * sizeof(uint64_t), cudaMemcpyHostToDevice));
+    return RL_OK;
+}
 
 rl_status rl_ucb1_create(rl_ctx *ctx, uint64_t num_replicas, int32_t num_observations, int32_t num_actions, double reward_lo,
                          double reward_hi, double exploration_rate, rl_ucb1 **out) {

@@ -51,6 +51,8 @@ class ActorSpec:
     seq_net: object = None             # modules.GruLinear (recurrent CATEGORICAL_POLICY)
     ucb: object = None                 # agents.UCB1Agent
     inner_kind: int = L.RL_INNER_RANDOM  # RESETTING_META: the inner agent (L.RL_INNER_*)
+    bts: object = None                 # agents.BetaThompsonSamplingAgent
+    num_samples: int = 0               # RESETTING_META with the Thompson-sampling inner agent: Beta draws per arm (1 .. 1024)
 
 
 class Trajectory:
@@ -131,6 +133,8 @@ def rollout(env: BatchedEnv, actor: ActorSpec, bound: HistoryDataBound, traj: Tr
     cfg.seq_net = actor.seq_net.handle if actor.seq_net is not None else None
     cfg.ucb = actor.ucb.handle if actor.ucb is not None else None
     cfg.inner_kind = actor.inner_kind
+    cfg.bts = actor.bts.handle if actor.bts is not None else None
+    cfg.num_samples = actor.num_samples
     summ = L.StepsSummary() if want_summary else None
     L.check(lib.rl_rollout(env.handle, C.byref(cfg), L.Bound(bound.min_steps, bound.slack_steps), traj.handle,
                            C.byref(summ) if want_summary else None), env.ctx.handle)

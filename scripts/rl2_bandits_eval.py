@@ -7,9 +7,11 @@ Each lane runs whole trials: a trial is always 2n - 1 meta steps (n pulls, n - 1
 (m (2n - 1), 0) gives exactly m trials per lane and `--num-trials` trials spread over the lanes.  The result is
 EvalResults: the mean trial reward and its population standard deviation (OnlineMeanVariance::stddev, utils/stats.rs).
 
-Agents as at rl2-bandits.rs:197-220: random, eps-greedy (tabular Q, epsilon 0.2), greedy (epsilon 0), UCB1 (exploration
-rate 0.2).  The tabular configs there set initial_action_count 2 / initial_action_value 0.5, which build_agent ignores
-(tabular.rs:61-77): every table starts from zeros, here as in the reference.  Thompson sampling is not available.
+Agents as at rl2-bandits.rs:197-220: random, eps-greedy (tabular Q, epsilon 0.2), greedy (epsilon 0), TS (Beta Thompson
+sampling, one sample), OTS (the same with the mean of 10 samples, as the reference defines it) and UCB1 (exploration rate
+0.2).  The tabular configs there set initial_action_count 2 / initial_action_value 0.5, which build_agent ignores
+(tabular.rs:61-77): every table starts from zeros, here as in the reference.  The Thompson agents draw from the device's
+own Beta sampler (DESIGN section 5): the same distribution as the reference's, not its bit stream.
 
 Noise: the device draws env and agent noise from one Philox key; --env-seed and --agent-seed are combined into it.
 
@@ -36,6 +38,8 @@ AGENTS = {
     "random": R.RandomAgentConfig(),
     "eps-greedy": R.TabularQLearningAgentConfig(exploration_rate=0.2, initial_action_count=2, initial_action_value=0.5),
     "greedy": R.TabularQLearningAgentConfig(exploration_rate=0.0, initial_action_count=2, initial_action_value=0.5),
+    "ts": R.BetaThompsonSamplingAgentConfig(num_samples=1),
+    "ots": R.BetaThompsonSamplingAgentConfig(num_samples=10),
     "ucb1": R.UCB1AgentConfig(exploration_rate=0.2),
 }
 
@@ -78,7 +82,7 @@ def time_rollouts(ctx, lanes: int, num_arms: int, num_episodes: int, warmup: int
     traj = R.Trajectory(env, steps)
     bound = R.HistoryDataBound(steps, 0)
     actors = [("random actor (K2a floor)", R.ActorSpec(kind=L.RL_ACTOR_RANDOM))]
-    for name in ("random", "eps-greedy", "ucb1"):
+    for name in ("random", "eps-greedy", "ucb1", "ts", "ots"):
         actors.append((f"meta {name} (K2m)", R.ResettingMetaAgentConfig(AGENTS[name]).build_agent(env).actor()))
     rows = []
     for name, actor in actors:
