@@ -32,6 +32,33 @@ __host__ __device__ inline void rl_philox4x32_10(uint32_t c0, uint32_t c1, uint3
     out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
 }
 
+// rl_philox4x32_10 with its ten round keys, which depend only on the key, computed once: for a loop that draws many
+// blocks under one seed (the same words).
+struct RlPhiloxKeys {
+    uint32_t k0[10], k1[10];
+};
+__device__ __forceinline__ RlPhiloxKeys rl_philox_keys(uint64_t seed) {
+    RlPhiloxKeys k;
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        k.k0[r] = (uint32_t)seed + (uint32_t)r * 0x9E3779B9u;
+        k.k1[r] = (uint32_t)(seed >> 32) + (uint32_t)r * 0xBB67AE85u;
+    }
+    return k;
+}
+__device__ __forceinline__ void rl_philox4x32_10_keyed(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, const RlPhiloxKeys &k,
+                                                       uint32_t out[4]) {
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        const uint64_t p0 = (uint64_t)0xD2511F53u * c0;
+        const uint64_t p1 = (uint64_t)0xCD9E8D57u * c2;
+        const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c1 ^ k.k0[r];
+        const uint32_t n2 = (uint32_t)(p0 >> 32) ^ c3 ^ k.k1[r];
+        c0 = n0; c1 = (uint32_t)p1; c2 = n2; c3 = (uint32_t)p0;
+    }
+    out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
+}
+
 __host__ __device__ inline uint64_t rl_philox_slot_impl(uint64_t seed, uint64_t lane, uint32_t t, int stream,
                                                         uint32_t draw) {
     uint32_t o[4];

@@ -69,6 +69,7 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
     int fin_succ_last = RL_TERMINATE, fin_succ_prev = RL_TERMINATE;
 
     // ---- aux: one chunk = WS_CHUNK steps x 32 envs; lane = env ----
+    const RlPhiloxKeys keys = rl_philox_keys(seed);
     auto aux_fill = [&](uint32_t k0) {
         const int el = lane;
         const uint64_t eg = e_base + el, lg = a.lane_offset + (eg < a.E ? eg : 0);  // (lanes past the CTA's envs: unused slots)
@@ -78,14 +79,11 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
             const uint32_t ring = k & (WS_RING - 1);
             uint32_t oa[4], o0[4], o1[4];
             // policies/actor.rs:42-55: the actor's uniform of step k as the logit-space threshold (rl_logit_threshold)
-            rl_philox4x32_10((uint32_t)lg, (uint32_t)(lg >> 32), t0 + k, (uint32_t)RL_STREAM_ACTOR * 64u, (uint32_t)seed,
-                             (uint32_t)(seed >> 32), oa);
+            rl_philox4x32_10_keyed((uint32_t)lg, (uint32_t)(lg >> 32), t0 + k, (uint32_t)RL_STREAM_ACTOR * 64u, keys, oa);
             // cartpole.rs:103-115: four uniform draws in field order = blocks 0 (x, x') and 1 (theta, theta')
-            rl_philox4x32_10((uint32_t)lg, (uint32_t)(lg >> 32), t0 + k, (uint32_t)RL_STREAM_ENV_RESET * 64u, (uint32_t)seed,
-                             (uint32_t)(seed >> 32), o0);
-            rl_philox4x32_10((uint32_t)lg, (uint32_t)(lg >> 32), t0 + k, (uint32_t)RL_STREAM_ENV_RESET * 64u + 1u, (uint32_t)seed,
-                             (uint32_t)(seed >> 32), o1);
-            smem_stf(sb + QK_OFF(thr) + 4u * (ring * QK_ENVS + el), rl_logit_threshold(rl_u32_to_f32(oa[0])));
+            rl_philox4x32_10_keyed((uint32_t)lg, (uint32_t)(lg >> 32), t0 + k, (uint32_t)RL_STREAM_ENV_RESET * 64u, keys, o0);
+            rl_philox4x32_10_keyed((uint32_t)lg, (uint32_t)(lg >> 32), t0 + k, (uint32_t)RL_STREAM_ENV_RESET * 64u + 1u, keys, o1);
+            smem_stf(sb + QK_OFF(thr) + 4u * (ring * QK_ENVS + el), rl_logit_threshold_fast(rl_u32_to_f32(oa[0])));
             const double x = rl_u64_to_uniform((uint64_t)o0[0] | ((uint64_t)o0[1] << 32), p.reset_low, p.reset_scale);
             const double xd = rl_u64_to_uniform((uint64_t)o0[2] | ((uint64_t)o0[3] << 32), p.reset_low, p.reset_scale);
             const double th = rl_u64_to_uniform((uint64_t)o1[0] | ((uint64_t)o1[1] << 32), p.reset_low, p.reset_scale);
@@ -141,6 +139,16 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
             f.x = lo.x; f.xd = lo.y; f.th = hi.x; f.thd = hi.y;
             f.meta = 0x80000000u | p.max_steps;
         };
+        // step_fast's parameters and coefficients in registers for the whole loop.  Left to ptxas, they are reloaded from
+        // the constant bank on every step, about twenty loads on the dynamics warp's stream, which is what bounds the
+        // step cycle; ptxas does not rematerialise a shuffle's result.
+        EnvT::Params q = p;
+        for (double *v : {&q.gravity, &q.mass_pole, &q.length_half_pole, &q.friction_cart, &q.friction_pole, &q.time_step,
+                          &q.action_force, &q.max_pos, &q.max_angle, &q.total_weight, &q.inv_total_mass, &q.mass_length_pole})
+            *v = __shfl_sync(FULL, *v, 0);
+        double coef[14];
+#pragma unroll
+        for (int c = 0; c < 14; ++c) coef[c] = __shfl_sync(FULL, rl_cartpole_sincos_coef[c], 0);
         EnvT::State s;
         s.x = s.xd = s.th = s.thd = 0.0;
         s.meta = 0x80000000u | p.max_steps;
@@ -174,8 +182,8 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
             // before the action is known: the step for both actions, the would-be reset state, and the `remaining` feature
             // of the next observation
             EnvT::State c0s = s, c1s = s;
-            const int sc0 = EnvT::step_fast(p, c0s, 0u);
-            const int sc1 = EnvT::step_fast(p, c1s, 1u);
+            const int sc0 = EnvT::step_fast(q, c0s, 0u, coef);
+            const int sc1 = EnvT::step_fast(q, c1s, 1u, coef);
             EnvT::State fresh;
             fresh_state(it + 1, fresh);
             const uint32_t r_now = s.meta & 0x7FFFFFFFu;
