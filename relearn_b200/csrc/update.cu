@@ -7,19 +7,18 @@
 //
 // The reference runs ~29 full-batch libtorch passes with autograd (first and second order) and a
 // host sync per CG iteration and per line-search try.  Here every pass over the batch is one fused
-// kernel (K5/K6, FP32-FMA bound) that computes forward, the per-sample softmax algebra and the
-// analytic backward / Fisher-vector product in registers, and every piece of P-vector algebra (CG
-// recurrences, step size, line-search bookkeeping, Adam) is a single-CTA kernel driven by device-side
-// flags, so the whole update is enqueued without a host round trip.
+// kernel (K5/K6) that computes forward, the per-sample softmax algebra and the analytic backward /
+// Fisher-vector product, and every piece of P-vector algebra (CG recurrences, step size, line-search
+// bookkeeping, Adam) is a single-CTA kernel driven by device-side flags, so the whole update is
+// enqueued without a host round trip.
 //
-// mlp_pass_kernel<F, A, UPL, MODE>: one warp owns a tile of 32 samples; lane l owns hidden units
-// {l + 32u : u < UPL} (H = 32 * UPL) with their weights in registers.  Forward computes each lane's
-// partial logits for 8 samples at a time and combines them with a shuffle reduce-scatter; the lane
-// that loaded sample s does that sample's softmax / loss / KL algebra; the backward sweep re-derives
-// the hidden activations (cheaper than staging them through shared memory) and accumulates this
-// lane's slice of the parameter gradient in f32 registers, flushed to per-warp f64 totals in shared
-// memory every few tiles.  Blocks write f64 partial rows; rows are summed in a fixed order, so the
-// result is deterministic and independent of scheduling.
+// Three kernels run the passes (launch_pass picks one).  Each writes one f64 partial row per CTA; rows
+// are summed in a fixed order, so the result is deterministic and independent of scheduling.
+//   mlp_pass_tc_kernel<A, MODE> (pass_tc.cuh): the reference's default networks, the 5 -> 128 -> 1
+//     critic and the 5 -> 128 -> 2 policy / action-value network, on the tensor cores;
+//   mlp_pass_kernel: the same networks on the FP32 pipe, the cross-check of the tensor-core kernel
+//     (RL_PASS_KERNEL=ffma or rl_pass_kernel_select(RL_PASS_KERNEL_FFMA));
+//   mlp_pass_any_kernel<MODE>: every other supported module, on the FP32 pipe.
 //
 // Exactness: the Hessian of mean KL(p0 || p_theta) at theta0 equals the Fisher matrix
 // mean J^T (diag p - p p^T) J (the first-order term vanishes because p = p0 there), so the analytic
@@ -113,6 +112,17 @@ __device__ __forceinline__ double warp_sum_f64(double x) {
 __device__ __forceinline__ float2 f2(float a, float b) { return make_float2(a, b); }
 __device__ __forceinline__ float2 dup2(float a) { return make_float2(a, a); }
 
+// mlp_pass_kernel<F, A, UPL, MODE, CH, MINB>: one warp owns a tile of 32 samples; lane l owns hidden units
+// {l + 32u : u < UPL} (H = 32 * UPL) with their weights in registers.  Forward computes each lane's
+// partial logits for 8 samples at a time and combines them with a shuffle reduce-scatter; the lane
+// that loaded sample s does that sample's softmax / loss / KL algebra; the backward sweep re-derives
+// the hidden activations (cheaper than staging them through shared memory) and accumulates this
+// lane's slice of the parameter gradient in f32 registers, flushed to per-warp f64 totals in shared
+// memory every few tiles.
+//
+// It stays as the FP32 cross-check of the default networks because mlp_pass_any_kernel is not accurate enough
+// there: on the saturated two-action policy (logits up to |z| ~ 270) its gradient is 1.1e-4 from f64, against
+// 4e-5 for this kernel and a 1e-4 bound (tests/test_gpu_update.py, test_policy_pass_large_logits_and_padding).
 template <int F, int A, int UPL, int MODE, int CH, int MINB>
 __global__ void __launch_bounds__(PASS_THREADS, MINB) mlp_pass_kernel(PassArgs a) {
     static_assert(UPL % 2 == 0, "hidden units are processed in pairs (FFMA2)");
@@ -1350,8 +1360,15 @@ rl_status reduce_over_group(rl_ctx *ctx, const PassPlan &plan, int rows, const i
     return RL_OK;
 }
 
-template <int F, int A, int UPL, int MODE, int CH, int MINB>
-rl_status launch_pass_variant(rl_ctx *ctx, const PassPlan &plan, PassArgs args, bool reduce = true) {
+// The default networks' passes on the FP32 pipe (mlp_pass_kernel): the cross-check of the tensor-core kernel, selected by
+// RL_PASS_KERNEL=ffma or rl_pass_kernel_select(RL_PASS_KERNEL_FFMA).  Tile-chunk size and CTAs per SM per mode:
+// forward-only passes fit 2 CTAs/SM at CH = 8; the critic and Q-loss passes run at CH = 4 with 2 CTAs/SM; the
+// gradient / Fisher-vector passes need the registers of 1 CTA/SM.
+template <int A, int MODE>
+rl_status launch_pass_ffma(rl_ctx *ctx, const PassPlan &plan, PassArgs args, bool reduce) {
+    constexpr int F = 5, UPL = 4;
+    constexpr bool MSE = MODE == PASS_VALUE || MODE == PASS_QLOSS, FWD = MODE == PASS_STATS || MODE == PASS_EVAL;
+    constexpr int CH = MSE ? 4 : 8, MINB = MSE || FWD ? 2 : 1;
     const size_t smem = pass_smem_bytes<F, A, UPL>();
     static bool configured = false;
     if (!configured) {
@@ -1365,9 +1382,8 @@ rl_status launch_pass_variant(rl_ctx *ctx, const PassPlan &plan, PassArgs args, 
     return reduce_over_group(ctx, plan, plan.grid, args.skip_flag);
 }
 
-// Passes of the reference's default networks (5 -> 128 -> 1 critic, 5 -> 128 -> 2 policy) run on the tensor cores
-// (pass_tc.cuh); the Q-loss pass and RL_PASS_KERNEL=ffma / rl_pass_kernel_select(RL_PASS_KERNEL_FFMA) use the FP32-pipe
-// kernel above.
+// Which kernel runs the default networks' passes (RL_PASS_KERNEL_*): RL_PASS_KERNEL from the environment until
+// rl_pass_kernel_select sets it.
 int g_pass_kernel = -1;
 int pass_kernel() {
     if (g_pass_kernel < 0) {
@@ -1376,30 +1392,11 @@ int pass_kernel() {
     }
     return g_pass_kernel;
 }
-template <int F, int A, int UPL, int MODE>
-constexpr bool tc_built() {
-    return F == 5 && UPL == 4 &&
-           ((A == 1 && MODE == PASS_VALUE) ||
-            (A == 2 && (MODE == PASS_STATS || MODE == PASS_EVAL || MODE == PASS_GRAD || MODE == PASS_FVP || MODE == PASS_PPO ||
-                        MODE == PASS_REINFORCE || MODE == PASS_QLOSS)));
-}
-template <int F, int A, int UPL, int MODE>
-bool pass_on_tensor_cores() {
-    return tc_built<F, A, UPL, MODE>() && pass_kernel() == RL_PASS_KERNEL_TCGEN05;
-}
 // CTAs of a tensor-core pass: the plan's count (3 per SM) capped at what the mode keeps resident per SM
 template <int A, int MODE>
 int tc_grid(const rl_ctx *ctx, const PassPlan &plan) {
     const int cap = ctx->sm_count * TcPass<A, MODE>::CTAS_PER_SM;
     return plan.grid_tc < cap ? plan.grid_tc : cap;
-}
-// rows of plan.partials the pass writes
-template <int F, int A, int UPL, int MODE>
-int pass_rows(const rl_ctx *ctx, const PassPlan &plan) {
-    if constexpr (tc_built<F, A, UPL, MODE>()) {
-        if (pass_on_tensor_cores<F, A, UPL, MODE>()) return tc_grid<A, MODE>(ctx, plan);
-    }
-    return plan.grid;
 }
 
 template <int A, int MODE>
@@ -1415,60 +1412,6 @@ rl_status launch_pass_tc(rl_ctx *ctx, const PassPlan &plan, PassArgs args, bool 
     RL_LAUNCH(ctx, (mlp_pass_tc_kernel<A, MODE>), grid, tc::TC_THREADS, smem, args);
     if (!reduce) return RL_OK;
     return reduce_over_group(ctx, plan, grid, args.skip_flag);
-}
-
-int pass_variant() {
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("RL_PASS_VARIANT");
-        v = e ? atoi(e) : 0;
-    }
-    return v;
-}
-
-// Tile-chunk size and CTAs/SM per mode, chosen from B200 timings (profiles/r1_update_variants.md):
-// forward-only passes fit 2 CTAs/SM at CH=8; the critic pass is fastest at CH=4 with 2 CTAs/SM; the
-// gradient / Fisher-vector passes need the registers of 1 CTA/SM.  RL_PASS_VARIANT overrides (experiments).
-template <int F, int A, int UPL, int MODE>
-rl_status launch_pass(rl_ctx *ctx, const PassPlan &plan, PassArgs args, bool reduce = true) {
-    if constexpr (tc_built<F, A, UPL, MODE>()) {
-        if (pass_on_tensor_cores<F, A, UPL, MODE>()) return launch_pass_tc<A, MODE>(ctx, plan, args, reduce);
-    }
-    switch (pass_variant()) {
-    case 1: return launch_pass_variant<F, A, UPL, MODE, 8, 1>(ctx, plan, args, reduce);
-    case 2: return launch_pass_variant<F, A, UPL, MODE, 4, 2>(ctx, plan, args, reduce);
-    case 3: return launch_pass_variant<F, A, UPL, MODE, 4, 1>(ctx, plan, args, reduce);
-    case 4: return launch_pass_variant<F, A, UPL, MODE, 4, 3>(ctx, plan, args, reduce);
-    default:
-        if (MODE == PASS_VALUE || MODE == PASS_QLOSS) return launch_pass_variant<F, A, UPL, MODE, 4, 2>(ctx, plan, args, reduce);
-        if (MODE == PASS_STATS || MODE == PASS_EVAL) return launch_pass_variant<F, A, UPL, MODE, 8, 2>(ctx, plan, args, reduce);
-        return launch_pass_variant<F, A, UPL, MODE, 8, 1>(ctx, plan, args, reduce);
-    }
-}
-
-// One optimizer step on the sums of the pass just launched: pass -> [reduce -> all-reduce] -> Adam
-// (n_backward_steps: zero_grad, backward, step; torch/agents/mod.rs:50-55, coptimizer.rs:13-27).
-template <int F, int A, int UPL, int MODE>
-rl_status pass_and_adam(rl_ctx *ctx, const PassPlan &plan, const PassArgs &pa, rl_mlp *net, rl_adam *adam, const AdamArgs &ac,
-                        double *loss_out) {
-    adam->step += 1;
-    if (ctx->world > 1 && ctx->x_ok && rl_div_up(plan.W, 32) <= RL_X_BLOCKS) {
-        // pass -> ONE kernel: row reduction + peer exchange + Adam
-        RL_TRY((launch_pass<F, A, UPL, MODE>(ctx, plan, pa, false)));
-        ctx->x_seq += 1;
-        RL_LAUNCH(ctx, reduce_rows_x_kernel<true>, rl_div_up(plan.W, 32), 256, 0, plan.partials, (pass_rows<F, A, UPL, MODE>(ctx, plan)),
-                  plan.W, plan.P, plan.sums, ctx->x, ctx->x_seq, (const int *)nullptr,
-                  (XAdam{net->params, adam->m, adam->v, ac, adam->step, loss_out, plan.P}));
-    } else if (ctx->world > 1) {
-        RL_TRY((launch_pass<F, A, UPL, MODE>(ctx, plan, pa)));
-        RL_LAUNCH(ctx, adam_step_kernel, 1, VEC_THREADS, 0, plan.sums, plan.P, net->params, adam->m, adam->v, ac, adam->step,
-                  loss_out);
-    } else {
-        RL_TRY((launch_pass<F, A, UPL, MODE>(ctx, plan, pa, false)));
-        RL_LAUNCH(ctx, reduce_rows_adam_kernel, rl_div_up(plan.W, 32), 256, 0, plan.partials, (pass_rows<F, A, UPL, MODE>(ctx, plan)),
-                  plan.W, plan.P, plan.sums, net->params, adam->m, adam->v, ac, adam->step, loss_out);
-    }
-    return RL_OK;
 }
 
 rl_status make_plan(rl_ctx *ctx, int P, uint64_t TE, PassPlan *plan, size_t extra_bytes, void **extra) {
@@ -1492,8 +1435,8 @@ rl_status make_plan(rl_ctx *ctx, int P, uint64_t TE, PassPlan *plan, size_t extr
 
 // ------------------------------------------------------------------------------------------------
 // Run-time dispatch over module shapes: the reference's default networks (5 -> 128 -> 1 critic, 5 -> 128 -> 2 policy /
-// action-value network, ReLU) take the compile-time kernels above (tensor cores or FP32 pipe); every other
-// one-hidden-layer module takes mlp_pass_any_kernel.
+// action-value network, ReLU) take the kernels above (tensor cores, or the FP32 pipe when selected); every other
+// module takes mlp_pass_any_kernel.
 // ------------------------------------------------------------------------------------------------
 struct PassNet {
     bool deflt;
@@ -1541,48 +1484,40 @@ rl_status launch_pass_any_mode(rl_ctx *ctx, const PassPlan &plan, PassArgs args,
     return reduce_over_group(ctx, plan, plan.grid, args.skip_flag);
 }
 
-// One full-batch pass of `pn` in `mode` by whichever kernel serves its shape; *rows = partial rows it wrote.
-rl_status launch_pass_rt(rl_ctx *ctx, const PassPlan &plan, const PassArgs &pa, int mode, const PassNet &pn, bool reduce = true,
-                         int *rows = nullptr) {
-    constexpr int F = 5, UPL = 4;
-    if (pn.deflt && pn.sh.A == 1 && mode == PASS_VALUE) {
-        if (rows) *rows = pass_rows<F, 1, UPL, PASS_VALUE>(ctx, plan);
-        return launch_pass<F, 1, UPL, PASS_VALUE>(ctx, plan, pa, reduce);
-    }
-    if (pn.deflt && pn.sh.A == 2 && mode != PASS_VALUE) {
-#define RL_DEFAULT_CASE(M)                                          \
-    case M:                                                         \
-        if (rows) *rows = pass_rows<F, 2, UPL, M>(ctx, plan);       \
-        return launch_pass<F, 2, UPL, M>(ctx, plan, pa, reduce);
-        switch (mode) {
-            RL_DEFAULT_CASE(PASS_STATS)
-            RL_DEFAULT_CASE(PASS_EVAL)
-            RL_DEFAULT_CASE(PASS_GRAD)
-            RL_DEFAULT_CASE(PASS_FVP)
-            RL_DEFAULT_CASE(PASS_PPO)
-            RL_DEFAULT_CASE(PASS_REINFORCE)
-            RL_DEFAULT_CASE(PASS_QLOSS)
-        default: return rl_fail(ctx, RL_ERR_INVALID_ARG, "unknown pass mode %d", mode);
-        }
-#undef RL_DEFAULT_CASE
+// One full-batch pass of `pn` in MODE; *rows = partial rows it wrote.  The critic pass of the default 5 -> 128 -> 1
+// network and every other pass of the default 5 -> 128 -> 2 network run on the tensor cores, or on the FP32 pipe when
+// that is selected; every other module runs on mlp_pass_any_kernel.
+template <int MODE>
+rl_status launch_pass(rl_ctx *ctx, const PassPlan &plan, const PassArgs &pa, const PassNet &pn, bool reduce, int *rows) {
+    constexpr int A = MODE == PASS_VALUE ? 1 : 2;
+    if (pn.deflt && pn.sh.A == A && pass_kernel() == RL_PASS_KERNEL_TCGEN05) {
+        if (rows) *rows = tc_grid<A, MODE>(ctx, plan);
+        return launch_pass_tc<A, MODE>(ctx, plan, pa, reduce);
     }
     if (rows) *rows = plan.grid;
+    if (pn.deflt && pn.sh.A == A) return launch_pass_ffma<A, MODE>(ctx, plan, pa, reduce);
+    return launch_pass_any_mode<MODE>(ctx, plan, pa, pn.sh, reduce);
+}
+
+rl_status launch_pass_rt(rl_ctx *ctx, const PassPlan &plan, const PassArgs &pa, int mode, const PassNet &pn, bool reduce = true,
+                         int *rows = nullptr) {
     switch (mode) {
-    case PASS_STATS: return launch_pass_any_mode<PASS_STATS>(ctx, plan, pa, pn.sh, reduce);
-    case PASS_EVAL: return launch_pass_any_mode<PASS_EVAL>(ctx, plan, pa, pn.sh, reduce);
-    case PASS_GRAD: return launch_pass_any_mode<PASS_GRAD>(ctx, plan, pa, pn.sh, reduce);
-    case PASS_FVP: return launch_pass_any_mode<PASS_FVP>(ctx, plan, pa, pn.sh, reduce);
-    case PASS_PPO: return launch_pass_any_mode<PASS_PPO>(ctx, plan, pa, pn.sh, reduce);
-    case PASS_REINFORCE: return launch_pass_any_mode<PASS_REINFORCE>(ctx, plan, pa, pn.sh, reduce);
-    case PASS_QLOSS: return launch_pass_any_mode<PASS_QLOSS>(ctx, plan, pa, pn.sh, reduce);
-    case PASS_VALUE: return launch_pass_any_mode<PASS_VALUE>(ctx, plan, pa, pn.sh, reduce);
+    case PASS_STATS: return launch_pass<PASS_STATS>(ctx, plan, pa, pn, reduce, rows);
+    case PASS_EVAL: return launch_pass<PASS_EVAL>(ctx, plan, pa, pn, reduce, rows);
+    case PASS_GRAD: return launch_pass<PASS_GRAD>(ctx, plan, pa, pn, reduce, rows);
+    case PASS_FVP: return launch_pass<PASS_FVP>(ctx, plan, pa, pn, reduce, rows);
+    case PASS_PPO: return launch_pass<PASS_PPO>(ctx, plan, pa, pn, reduce, rows);
+    case PASS_REINFORCE: return launch_pass<PASS_REINFORCE>(ctx, plan, pa, pn, reduce, rows);
+    case PASS_QLOSS: return launch_pass<PASS_QLOSS>(ctx, plan, pa, pn, reduce, rows);
+    case PASS_VALUE: return launch_pass<PASS_VALUE>(ctx, plan, pa, pn, reduce, rows);
     default: return rl_fail(ctx, RL_ERR_INVALID_ARG, "unknown pass mode %d", mode);
     }
 }
 
-// pass_and_adam over launch_pass_rt
-rl_status pass_and_adam_rt(rl_ctx *ctx, const PassPlan &plan, const PassArgs &pa, int mode, const PassNet &pn, rl_mlp *net,
-                           rl_adam *adam, const AdamArgs &ac, double *loss_out) {
+// One optimizer step on the sums of the pass just launched: pass -> [reduce -> all-reduce] -> Adam
+// (n_backward_steps: zero_grad, backward, step; torch/agents/mod.rs:50-55, coptimizer.rs:13-27).
+rl_status pass_and_adam(rl_ctx *ctx, const PassPlan &plan, const PassArgs &pa, int mode, const PassNet &pn, rl_mlp *net,
+                        rl_adam *adam, const AdamArgs &ac, double *loss_out) {
     adam->step += 1;
     int rows = plan.grid;
     if (ctx->world > 1 && ctx->x_ok && rl_div_up(plan.W, 32) <= RL_X_BLOCKS) {
@@ -1606,7 +1541,7 @@ rl_status pass_and_adam_rt(rl_ctx *ctx, const PassPlan &plan, const PassArgs &pa
 
 // ------------------------------------------------------------------------------------------------
 // Trust-region step, network-agnostic: `pass(mode, vec, skip_flag)` runs one full-batch pass of the policy
-// module (MLP: mlp_pass_kernel; GRU: gru_pass_kernel) and leaves the all-reduced f64 sums in plan.sums.
+// module (MLP: launch_pass_rt; GRU: gru_pass_kernel) and leaves the all-reduced f64 sums in plan.sums.
 // ------------------------------------------------------------------------------------------------
 using PassFn = std::function<rl_status(int mode, const float *vec, const int *skip_flag)>;
 
@@ -1867,7 +1802,7 @@ rl_status rl_value_update(rl_traj *traj, const float *targets_dev, rl_mlp *value
     AdamArgs ac{adam->cfg.learning_rate, adam->cfg.beta1, adam->cfg.beta2, adam->cfg.weight_decay, adam->cfg.eps};
     for (int s = 0; s < n_steps; ++s) {
         // n_backward_steps: loss -> zero_grad -> backward -> step (torch/agents/mod.rs:50-55, coptimizer.rs:13-27)
-        RL_TRY(pass_and_adam_rt(ctx, plan, pa, PASS_VALUE, pn, value_fn, adam, ac, losses + s));
+        RL_TRY(pass_and_adam(ctx, plan, pa, PASS_VALUE, pn, value_fn, adam, ac, losses + s));
     }
     if (stats) {
         RL_CUDA(ctx, cudaEventRecord(ev1, ctx->stream));
@@ -1961,10 +1896,10 @@ static rl_status policy_adam_update(rl_traj *traj, const float *adv_dev, rl_mlp 
         RL_TRY(launch_pass_rt(ctx, plan, pa, PASS_STATS, pn));
         RL_CUDA(ctx, cudaMemcpyAsync(entropy_sum, plan.sums + P + SC_ENTROPY, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
         RL_CUDA(ctx, cudaMemcpyAsync(entropy_sum + 1, plan.sums + P + SC_COUNT, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
-        for (int s = 0; s < n_steps; ++s) RL_TRY(pass_and_adam_rt(ctx, plan, pa, PASS_PPO, pn, policy, adam, ac, losses + s));
+        for (int s = 0; s < n_steps; ++s) RL_TRY(pass_and_adam(ctx, plan, pa, PASS_PPO, pn, policy, adam, ac, losses + s));
     } else {
         for (int s = 0; s < n_steps; ++s) {
-            RL_TRY(pass_and_adam_rt(ctx, plan, pa, PASS_REINFORCE, pn, policy, adam, ac, losses + s));
+            RL_TRY(pass_and_adam(ctx, plan, pa, PASS_REINFORCE, pn, policy, adam, ac, losses + s));
             if (s == 0) {  // entropies.get_or_insert_with: the distribution of the first loss evaluation (reinforce.rs:76)
                 RL_CUDA(ctx, cudaMemcpyAsync(entropy_sum, plan.sums + P + SC_ENTROPY, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
                 RL_CUDA(ctx, cudaMemcpyAsync(entropy_sum + 1, plan.sums + P + SC_COUNT, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
@@ -2186,7 +2121,7 @@ rl_status rl_dqn_update(rl_replay *rb, rl_mlp *q, rl_adam *adam, const rl_dqn_cf
         pa.T = 1; pa.E = mb.capacity;
         pa.theta = q->params; pa.target = mb.target + set * mb.capacity;
         // loss_fn + backward_step (dqn.rs:316-336, coptimizer.rs:13-27)
-        RL_TRY(pass_and_adam_rt(ctx, plan, pa, PASS_QLOSS, pn, q, adam, ac, losses + s));
+        RL_TRY(pass_and_adam(ctx, plan, pa, PASS_QLOSS, pn, q, adam, ac, losses + s));
     }
     uint64_t m_last = 0;
     if (n_steps > 0) RL_TRY(rl_replay_sample_finish(rb, &m_last, nullptr));

@@ -26,4 +26,4 @@ for it in range(4):
     st = agent.policy.update(traj, adv, log)
     cs = agent.critic.update(traj, log)
     res.append((e0.elapsed_ms(e1), log["policy/update_time"] * 1e3, cs.update_ms, st, log["num_backtracks"], log["cg_iterations"]))
-print("variant", os.environ.get("RL_PASS_VARIANT", "0"), "adv/policy/critic ms, status, backtracks, cg:", [tuple(round(x, 3) if isinstance(x, float) else x for x in r) for r in res[1:]])
+print("adv/policy/critic ms, status, backtracks, cg:", [tuple(round(x, 3) if isinstance(x, float) else x for x in r) for r in res[1:]])
