@@ -314,7 +314,7 @@ typedef enum {
 #define RL_LANES_WARP_SPECIALIZED 160
 typedef struct rl_actor_cfg {
     int32_t kind;                 /* rl_actor_kind */
-    rl_mlp *net;                  /* CATEGORICAL_POLICY / EPS_GREEDY_Q */
+    rl_mlp *net;                  /* CATEGORICAL_POLICY / EPS_GREEDY_Q with a feed-forward module */
     const uint8_t *actions_dev;   /* REPLAY_ACTIONS: u8 [T][E] */
     rl_tabq *table;               /* TABULAR_EPS_GREEDY */
     double exploration_rate;      /* EPS_GREEDY_Q / TABULAR_EPS_GREEDY; RESETTING_META: the inner tabular agent's epsilon
@@ -323,7 +323,10 @@ typedef struct rl_actor_cfg {
     int32_t lanes_per_env;        /* 0 = auto; threads cooperating on one env's MLP (1,2,4,8,16,32),
                                    * RL_LANES_TENSOR_CORE (128): 128-env tiles, hidden layer on tcgen05 (K2t), or
                                    * RL_LANES_WARP_SPECIALIZED (160): K2z / K2q */
-    rl_grunet *seq_net;           /* CATEGORICAL_POLICY with a recurrent module (Chain<Gru, Linear>) instead of `net` */
+    rl_grunet *seq_net;           /* CATEGORICAL_POLICY / EPS_GREEDY_Q with a recurrent module (Chain<Gru, Linear>) instead of
+                                   * `net`; hidden state zero at every episode start.  EPS_GREEDY_Q keeps the reference's order:
+                                   * gen_bool(eps), then gen_range(A) on an explored step WITHOUT stepping the module (its hidden
+                                   * state does not advance), else the module step and the first maximal Q-value */
     rl_ucb1 *ucb;                 /* UCB1 (training: maximise the upper confidence bound; evaluation: the most selected action) */
     int32_t inner_kind;           /* RESETTING_META: rl_inner_agent_kind; read for no other kind */
     rl_bts *bts;                  /* BETA_THOMPSON (the draw count comes from the handle) */
@@ -555,6 +558,24 @@ rl_status rl_replay_read_lane(rl_replay *rb, uint64_t lane, uint64_t max_steps, 
  * (dqn.rs:263-337); with a data-parallel group every rank samples its own minibatch_steps and the
  * gradient sums are all-reduced. */
 rl_status rl_dqn_update(rl_replay *rb, rl_mlp *q, rl_adam *adam, const rl_dqn_cfg *cfg, rl_opt_stats *stats);
+/* The same update with a recurrent action-value module (Chain<Gru, Linear>; DqnAgent over SeqPacked + SeqIterative modules,
+ * dqn.rs:75-83,190-197,341-352).  Every optimizer step draws the episodes rl_dqn_update would draw (same sample_seed and draw
+ * index) and lays them out as padded sequences, one episode per lane from a zero hidden state; the Q-loss is averaged over the
+ * valid steps and back-propagated through time (hidden <= 8: one thread per episode; up to 128: GEMMs over the episodes of a
+ * step).  OneStepTd targets come from a SeqPacked forward with the current parameters; an interrupted episode's successor
+ * observation continues that episode's hidden state.  Synchronises once per optimizer step (the sampled sizes are read back). */
+rl_status rl_dqn_update_seq(rl_replay *rb, rl_grunet *q, rl_adam *adam, const rl_dqn_cfg *cfg, rl_opt_stats *stats);
+/* Diagnostic read of one sequence minibatch of rl_dqn_update_seq (synchronises): out->num_lanes = B episodes taken (in draw
+ * order), out->step_capacity = L = the longest, out->lane_len = episode lengths, out->num_steps = M; planes in the device layouts
+ * above with B lanes and L steps: succ is RL_CONTINUE inside an episode, its stored code on its last step and RL_PAD beyond;
+ * next_obs is valid where succ == RL_INTERRUPT.  *target_dev: f32 [L][B] targets per cfg (q is needed for OneStepTd only).
+ * Device pointers are valid until the next sample or update on this buffer. */
+rl_status rl_replay_sample_seq(rl_replay *rb, const rl_dqn_cfg *cfg, rl_grunet *q, uint32_t draw_index, rl_traj_view *out,
+                               const float **target_dev);
+/* The Q-loss pass of rl_dqn_update_seq on the sequence minibatch of `draw_index`, for diagnostics and parity checks: the
+ * mean loss (dqn.rs:316-326) and its flat gradient at the current parameters, no optimizer step.  grad_host: f32 [num_params];
+ * either output may be NULL. */
+rl_status rl_dqn_probe_seq(rl_replay *rb, const rl_dqn_cfg *cfg, rl_grunet *q, uint32_t draw_index, double *loss, float *grad_host);
 /* ExplorationRateSchedule::LinearAnnealed (schedules.rs:35-45) */
 double rl_exploration_rate(double start, double end, uint64_t period, uint64_t global_steps, int32_t training);
 

@@ -244,6 +244,9 @@ SIGNATURES = {
     "rl_replay_sample": (st, [vp, P(DqnCfg), vp, C.c_uint32, P(MinibatchView)]),
     "rl_replay_read_lane": (st, [vp, C.c_uint64, C.c_uint64, vp, vp, vp, vp, vp, vp, P(ReplayStats)]),
     "rl_dqn_update": (st, [vp, vp, vp, P(DqnCfg), P(OptStats)]),
+    "rl_dqn_update_seq": (st, [vp, vp, vp, P(DqnCfg), P(OptStats)]),
+    "rl_replay_sample_seq": (st, [vp, P(DqnCfg), vp, C.c_uint32, P(TrajView), P(vp)]),
+    "rl_dqn_probe_seq": (st, [vp, P(DqnCfg), vp, C.c_uint32, P(C.c_double), P(C.c_float)]),
     "rl_exploration_rate": (C.c_double, [C.c_double, C.c_double, C.c_uint64, C.c_uint64, C.c_int32]),
 }
 

@@ -10,6 +10,9 @@
 //   r = sigmoid(W_ir x + b_ir + W_hr h + b_hr)      z = sigmoid(W_iz x + b_iz + W_hz h + b_hz)
 //   n = tanh(W_in x + b_in + r * (W_hn h + b_hn))   h' = (h - n) * z + n
 //
+// The same kernels run DqnActor::act (dqn.rs:360-379) for a recurrent Q-network (SeqArgs::eps_greedy): epsilon-greedy on the
+// module's outputs, the hidden state held where the actor explores.
+//
 //  K8a rollout_seq_kernel<EnvT, HMAX>   one thread per env; hidden state in registers (hidden <= 8) or
 //                                       thread-local memory (hidden <= 128); weights read as warp-wide
 //                                       broadcasts from shared memory when they fit, else through L1.
@@ -109,10 +112,22 @@ struct SeqArgs {
     const float *wt;   // K8h only: Wt[F + H][3H]
     int tile_envs;     // K8h only: envs per CTA (32 or 64)
     int stepped;       // K8s: two launches per step, the cell on the tensor cores (gru_step_tc.cuh)
+    int eps_greedy;    // the actor: 0 = PolicyActor (categorical on the logits), 1 = DqnActor (epsilon-greedy on the Q-values)
+    double eps;        // DqnActor's exploration rate
 };
 
-// XF / XA > 0: features / actions (and hidden = HMAX) fixed at compile time, see grunet_step<EXACT>.
-template <class EnvT, bool REPLAY, int HMAX, int XF = 0, int XA = 0>
+// DqnActor::act (dqn.rs:360-379): gen_bool(eps) on the actor stream, then gen_range(A) when it explores.  The reference returns
+// before action_value_fn.step on an explored step, so the caller leaves the episode's hidden state where it was.
+template <bool REPLAY>
+__device__ __forceinline__ bool dqn_explore(const SeqArgs &a, LaneNoise<REPLAY> &nz, int A, uint32_t &action) {
+    if (!rl_gen_bool<REPLAY, RL_STREAM_ACTOR>(nz, a.eps)) return false;
+    action = rl_gen_range<REPLAY, RL_STREAM_ACTOR>(nz, (uint32_t)A);
+    return true;
+}
+
+// XF / XA > 0: features / actions (and hidden = HMAX) fixed at compile time, see grunet_step<EXACT>.  EPS: the epsilon-greedy
+// actor of a recurrent Q-network instead of the categorical policy.
+template <class EnvT, bool REPLAY, int HMAX, bool EPS, int XF = 0, int XA = 0>
 __global__ void __launch_bounds__(128) rollout_seq_kernel(typename EnvT::Params p, SeqArgs a) {
     constexpr bool EXACT = XF > 0;
     constexpr int MF = EXACT ? XF : EnvT::MAXF, MA = EXACT ? XA : EnvT::MAXA;
@@ -153,9 +168,17 @@ __global__ void __launch_bounds__(128) rollout_seq_kernel(typename EnvT::Params 
         while (n > 0) {
             nz.set_step(t0 + i);
             float z[MA];
-            grunet_step<HMAX, MF, MA, EXACT>(a.net, w, obs, h, z);
-            const float u = rl_u32_to_f32(nz.template next_u32<RL_STREAM_ACTOR>());
-            const uint32_t action = categorical_sample<MA>(z, A, u);
+            uint32_t action;
+            if (EPS) {
+                if (!dqn_explore<REPLAY>(a, nz, A, action)) {
+                    grunet_step<HMAX, MF, MA, EXACT>(a.net, w, obs, h, z);
+                    action = argmax_first<MA>(z, A);
+                }
+            } else {
+                grunet_step<HMAX, MF, MA, EXACT>(a.net, w, obs, h, z);
+                const float u = rl_u32_to_f32(nz.template next_u32<RL_STREAM_ACTOR>());
+                action = categorical_sample<MA>(z, A, u);
+            }
 #pragma unroll
             for (int f = 0; f < MF; ++f)
                 if (f < F) {
@@ -271,35 +294,29 @@ GruView view_of(const rl_grunet *g) {
 
 constexpr size_t SEQ_SMEM_LIMIT = 160 * 1024;
 
-template <class EnvT, int HMAX>
-rl_status launch_seq_h(rl_ctx *ctx, const typename EnvT::Params &p, SeqArgs &a, bool replay, size_t smem, unsigned grid) {
-    if (replay) {
-        RL_CUDA(ctx, cudaFuncSetAttribute(rollout_seq_kernel<EnvT, true, HMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        RL_LAUNCH(ctx, (rollout_seq_kernel<EnvT, true, HMAX>), grid, 128, smem, p, a);
-    } else {
-        RL_CUDA(ctx, cudaFuncSetAttribute(rollout_seq_kernel<EnvT, false, HMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        RL_LAUNCH(ctx, (rollout_seq_kernel<EnvT, false, HMAX>), grid, 128, smem, p, a);
-    }
+template <class EnvT, bool REPLAY, int HMAX, bool EPS, int XF = 0, int XA = 0>
+rl_status launch_seq_k8a(rl_ctx *ctx, const typename EnvT::Params &p, SeqArgs &a, size_t smem, unsigned grid) {
+    RL_CUDA(ctx, cudaFuncSetAttribute(rollout_seq_kernel<EnvT, REPLAY, HMAX, EPS, XF, XA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    RL_LAUNCH(ctx, (rollout_seq_kernel<EnvT, REPLAY, HMAX, EPS, XF, XA>), grid, 128, smem, p, a);
     return RL_OK;
 }
 
-// BASELINE config 4: 2-armed bandit meta-env (6 features) with the rnn.rs-sized GRU (hidden 4)
-rl_status launch_seq_bandit_6_4_2(rl_ctx *ctx, const BanditMetaEnv::Params &p, SeqArgs &a, bool replay, size_t smem, unsigned grid) {
-    if (replay) {
-        RL_CUDA(ctx, cudaFuncSetAttribute(rollout_seq_kernel<BanditMetaEnv, true, 4, 6, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        RL_LAUNCH(ctx, (rollout_seq_kernel<BanditMetaEnv, true, 4, 6, 2>), grid, 128, smem, p, a);
-    } else {
-        RL_CUDA(ctx, cudaFuncSetAttribute(rollout_seq_kernel<BanditMetaEnv, false, 4, 6, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        RL_LAUNCH(ctx, (rollout_seq_kernel<BanditMetaEnv, false, 4, 6, 2>), grid, 128, smem, p, a);
+template <class EnvT, int HMAX, int XF = 0, int XA = 0>
+rl_status launch_seq_h(rl_ctx *ctx, const typename EnvT::Params &p, SeqArgs &a, bool replay, size_t smem, unsigned grid) {
+    if (a.eps_greedy) {
+        if (replay) return launch_seq_k8a<EnvT, true, HMAX, true, XF, XA>(ctx, p, a, smem, grid);
+        return launch_seq_k8a<EnvT, false, HMAX, true, XF, XA>(ctx, p, a, smem, grid);
     }
-    return RL_OK;
+    if (replay) return launch_seq_k8a<EnvT, true, HMAX, false, XF, XA>(ctx, p, a, smem, grid);
+    return launch_seq_k8a<EnvT, false, HMAX, false, XF, XA>(ctx, p, a, smem, grid);
 }
 
 template <class EnvT>
 rl_status launch_seq(rl_ctx *ctx, const typename EnvT::Params &p, SeqArgs &a, bool replay, size_t smem, unsigned grid) {
     const int H = a.net.H;
     if constexpr (std::is_same<EnvT, BanditMetaEnv>::value) {
-        if (H == 4 && a.F == 6 && a.A == 2 && p.num_arms == 2) return launch_seq_bandit_6_4_2(ctx, p, a, replay, smem, grid);
+        // BASELINE config 4: 2-armed bandit meta-env (6 features) with the rnn.rs-sized GRU (hidden 4)
+        if (H == 4 && a.F == 6 && a.A == 2 && p.num_arms == 2) return launch_seq_h<BanditMetaEnv, 4, 6, 2>(ctx, p, a, replay, smem, grid);
     }
     if (H <= 8) return launch_seq_h<EnvT, 8>(ctx, p, a, replay, smem, grid);
     if constexpr (EnvT::MAXA <= GT_LW) {
@@ -312,7 +329,8 @@ rl_status launch_seq(rl_ctx *ctx, const typename EnvT::Params &p, SeqArgs &a, bo
 }  // namespace
 
 // Called by rl_rollout (rollout.cu) when the actor carries a sequence network.
-rl_status rl_rollout_seq(rl_env *env, rl_grunet *net, rl_bound bound, rl_traj *traj, double **partials_out, int *nblocks_out) {
+rl_status rl_rollout_seq(rl_env *env, rl_grunet *net, bool eps_greedy, double eps, rl_bound bound, rl_traj *traj, double **partials_out,
+                         int *nblocks_out) {
     rl_ctx *ctx = env->ctx;
     const rl_env_structure &es = env->structure;
     RL_REQUIRE(ctx, net->ctx == ctx, "rl_rollout: network belongs to another context");
@@ -325,6 +343,8 @@ rl_status rl_rollout_seq(rl_env *env, rl_grunet *net, rl_bound bound, rl_traj *t
     a.lane_len = traj->lane_len; a.lane_flags = traj->lane_flags;
     a.net = view_of(net);
     a.F = es.num_features; a.A = es.num_actions;
+    a.eps_greedy = eps_greedy ? 1 : 0;
+    a.eps = eps;
     const size_t wbytes = net->n_params * sizeof(float);
     a.weights_in_smem = wbytes <= SEQ_SMEM_LIMIT;
     const size_t smem = a.weights_in_smem ? wbytes : 16;
@@ -334,8 +354,9 @@ rl_status rl_rollout_seq(rl_env *env, rl_grunet *net, rl_bound bound, rl_traj *t
                        env->kind != RL_ENV_MEMORY_GAME && !(pick && strcmp(pick, "thread") == 0);
     a.tile_envs = (pick && strcmp(pick, "tile32") == 0) ? 32 : 64;
     // K8s (gru_step_tc.cuh): the cell of all envs as one tensor-core launch per step.  Picked above 4 096 envs (below, the
-    // persistent K8h tile kernel has the shorter step); RL_GRU_KERNEL=stepped / tile / tile32 / thread force a kernel.
-    a.stepped = tiled && rl_seq_big_cell_supports(net->in_dim, net->hidden) &&
+    // persistent K8h tile kernel has the shorter step); RL_GRU_KERNEL=stepped / tile / tile32 / thread force a kernel.  K8s
+    // serves the categorical policy only: the epsilon-greedy actor takes K8h (tile) wherever K8s would run.
+    a.stepped = tiled && !eps_greedy && rl_seq_big_cell_supports(net->in_dim, net->hidden) &&
                 ((pick && strcmp(pick, "stepped") == 0) || (!pick && a.E >= 4096));
     const unsigned grid = a.stepped ? rl_grid_for(a.E, 128) : tiled ? (unsigned)((a.E + a.tile_envs - 1) / a.tile_envs) : rl_grid_for(a.E, 128);
     if (tiled && !a.stepped) {

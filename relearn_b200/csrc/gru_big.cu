@@ -318,8 +318,8 @@ template <int MODE, int HEAD_MAXA>
 __global__ void __launch_bounds__(HEAD_THREADS) big_head_kernel(rl_seq_pass_args a, const float *__restrict__ HNEW,
                                                                 const float *__restrict__ THNEW, double *__restrict__ scal_part) {
     constexpr bool BACKWARD = MODE == RL_PASS_GRAD || MODE == RL_PASS_FVP || MODE == RL_PASS_VALUE || MODE == RL_PASS_PPO ||
-                              MODE == RL_PASS_REINFORCE;
-    constexpr bool IS_POLICY = MODE != RL_PASS_VALUE;
+                              MODE == RL_PASS_REINFORCE || MODE == RL_PASS_QLOSS;
+    constexpr bool IS_POLICY = MODE != RL_PASS_VALUE && MODE != RL_PASS_QLOSS;
     constexpr bool FVP = MODE == RL_PASS_FVP;
     constexpr bool USES_ADV = MODE == RL_PASS_EVAL || MODE == RL_PASS_GRAD || MODE == RL_PASS_PPO || MODE == RL_PASS_REINFORCE;
     constexpr bool USES_LP0 = MODE == RL_PASS_EVAL || MODE == RL_PASS_GRAD || MODE == RL_PASS_PPO;
@@ -432,6 +432,17 @@ __global__ void __launch_bounds__(HEAD_THREADS) big_head_kernel(rl_seq_pass_args
                     for (int k = 0; k < HEAD_MAXA; ++k)
                         if (k < A) dz[k] = p[k] * (zd[k] - pd);
                 }
+            } else if (MODE == RL_PASS_QLOSS) {  // mse(Q(obs).gather(action), targets)  (dqn.rs:316-326)
+                const int act_s = (int)a.action[idx];
+                float q = z[0];
+#pragma unroll
+                for (int k = 1; k < HEAD_MAXA; ++k)
+                    if (k == act_s) q = z[k];
+                const float diff = q - a.target[idx];
+                loss_s = diff * diff;
+#pragma unroll
+                for (int k = 0; k < HEAD_MAXA; ++k)
+                    if (k == act_s) dz[k] = 2.0f * diff;
             } else {  // VALUE: mse(V(obs), targets)  (opt.rs:109-115)
                 const float diff = z[0] - a.target[idx];
                 loss_s = diff * diff;
@@ -640,7 +651,7 @@ rl_status rl_seq_big_pass_launch(rl_ctx *ctx, int mode, const rl_seq_pass_args &
     const uint64_t T = a.T, E = a.E, HE = (uint64_t)H * E, TE = T * E;
     const bool fvp = mode == RL_PASS_FVP;
     const bool backward = mode == RL_PASS_GRAD || mode == RL_PASS_FVP || mode == RL_PASS_VALUE || mode == RL_PASS_PPO ||
-                          mode == RL_PASS_REINFORCE;
+                          mode == RL_PASS_REINFORCE || mode == RL_PASS_QLOSS;
     const int *skip = a.skip_flag;
     // ---- scratch (second context scratch: the plan and hbuf / dzbuf / logp0 live in the first) ----
     const int splits = 32;
@@ -736,6 +747,7 @@ rl_status rl_seq_big_pass_launch(rl_ctx *ctx, int mode, const rl_seq_pass_args &
     case RL_PASS_VALUE: RL_TRY(launch_head<RL_PASS_VALUE>(ctx, a, pl, scal_part, head_blocks)); break;
     case RL_PASS_PPO: RL_TRY(launch_head<RL_PASS_PPO>(ctx, a, pl, scal_part, head_blocks)); break;
     case RL_PASS_REINFORCE: RL_TRY(launch_head<RL_PASS_REINFORCE>(ctx, a, pl, scal_part, head_blocks)); break;
+    case RL_PASS_QLOSS: RL_TRY(launch_head<RL_PASS_QLOSS>(ctx, a, pl, scal_part, head_blocks)); break;
     default: return rl_fail(ctx, RL_ERR_INVALID_ARG, "rl_seq_big_pass_launch: bad mode %d", mode);
     }
     // ---- backward through time, then the weight gradients as two split-K GEMMs over all (t, e) ----

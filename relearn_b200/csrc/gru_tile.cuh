@@ -81,7 +81,9 @@ constexpr size_t gt_smem_bytes() {
            (size_t)GT_LW * GT_H * 4 + 4 * GT_H * 4 + 64 + S::envs * sizeof(GtOwner<EnvT, REPLAY>) + 64;
 }
 
-template <class EnvT, bool REPLAY, class S>
+// EPS: the epsilon-greedy actor of a recurrent Q-network.  The cell runs for every env of the tile before the actor draws; an env
+// whose actor explores copies its old state over the new one, so its hidden state does not advance (DqnActor::act, gru.cu).
+template <class EnvT, bool REPLAY, class S, bool EPS>
 __global__ void __launch_bounds__(S::threads, 256 / S::threads) rollout_seq_tile_kernel(typename EnvT::Params p, SeqArgs a) {
     constexpr int GT_ENVS = S::envs, GT_THREADS = S::threads, GT_ROWS = S::rows, GT_NBUF = S::nbuf, GT_HLD = S::hld;
     constexpr int MF = EnvT::MAXF, MA = EnvT::MAXA;
@@ -290,8 +292,17 @@ __global__ void __launch_bounds__(S::threads, 256 / S::threads) rollout_seq_tile
         if (owner && o.n > 0) {
             const uint32_t i = o.i;
             o.nz.set_step(t0 + i);
-            const float u = rl_u32_to_f32(o.nz.template next_u32<RL_STREAM_ACTOR>());
-            const uint32_t action = categorical_sample<MA>(zl, A, u);
+            uint32_t action;
+            if (EPS) {
+                if (dqn_explore<REPLAY>(a, o.nz, A, action)) {
+                    for (int j = 0; j < GT_H; ++j) hn[(size_t)j * GT_HLD + oe] = hc[(size_t)j * GT_HLD + oe];
+                } else {
+                    action = argmax_first<MA>(zl, A);
+                }
+            } else {
+                const float u = rl_u32_to_f32(o.nz.template next_u32<RL_STREAM_ACTOR>());
+                action = categorical_sample<MA>(zl, A, u);
+            }
 #pragma unroll
             for (int f = 0; f < MF; ++f)
                 if (f < F) {
@@ -352,19 +363,23 @@ __global__ void __launch_bounds__(S::threads, 256 / S::threads) rollout_seq_tile
     block_reduce_stats(st, owner && valid, reinterpret_cast<double (*)[ST_COUNT]>(xs), a.partials);
 }
 
+template <class EnvT, bool REPLAY, class S, bool EPS>
+rl_status launch_seq_tile_k8h(rl_ctx *ctx, const typename EnvT::Params &p, SeqArgs &a) {
+    const unsigned grid = (unsigned)((a.E + S::envs - 1) / S::envs);
+    constexpr size_t smem = gt_smem_bytes<EnvT, REPLAY, S>();
+    RL_CUDA(ctx, cudaFuncSetAttribute(rollout_seq_tile_kernel<EnvT, REPLAY, S, EPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    RL_LAUNCH(ctx, (rollout_seq_tile_kernel<EnvT, REPLAY, S, EPS>), grid, S::threads, smem, p, a);
+    return RL_OK;
+}
+
 template <class EnvT, class S>
 rl_status launch_seq_tile_shape(rl_ctx *ctx, const typename EnvT::Params &p, SeqArgs &a, bool replay) {
-    const unsigned grid = (unsigned)((a.E + S::envs - 1) / S::envs);
-    if (replay) {
-        constexpr size_t smem = gt_smem_bytes<EnvT, true, S>();
-        RL_CUDA(ctx, cudaFuncSetAttribute(rollout_seq_tile_kernel<EnvT, true, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        RL_LAUNCH(ctx, (rollout_seq_tile_kernel<EnvT, true, S>), grid, S::threads, smem, p, a);
-    } else {
-        constexpr size_t smem = gt_smem_bytes<EnvT, false, S>();
-        RL_CUDA(ctx, cudaFuncSetAttribute(rollout_seq_tile_kernel<EnvT, false, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        RL_LAUNCH(ctx, (rollout_seq_tile_kernel<EnvT, false, S>), grid, S::threads, smem, p, a);
+    if (a.eps_greedy) {
+        if (replay) return launch_seq_tile_k8h<EnvT, true, S, true>(ctx, p, a);
+        return launch_seq_tile_k8h<EnvT, false, S, true>(ctx, p, a);
     }
-    return RL_OK;
+    if (replay) return launch_seq_tile_k8h<EnvT, true, S, false>(ctx, p, a);
+    return launch_seq_tile_k8h<EnvT, false, S, false>(ctx, p, a);
 }
 
 using GtWide = GtShape<64, 16, 3>;

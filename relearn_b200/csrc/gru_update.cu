@@ -1,5 +1,5 @@
-// gru_update.cu -- full-batch passes over trajectories for a recurrent policy / critic (Chain<Gru, Linear>):
-// what autograd does for the reference when the module of Trpo / Ppo / Reinforce / ValuesOpt is a GRU
+// gru_update.cu -- full-batch passes over trajectories for a recurrent policy / critic / Q-network (Chain<Gru, Linear>):
+// what autograd does for the reference when the module of Trpo / Ppo / Reinforce / ValuesOpt / DqnAgent is a GRU
 // (src/torch/agents/policies/trpo.rs:97-164 with cuDNN disabled :104-108, critics/opt.rs:100-127,
 // modules/seq/rnn/gru.rs:72-102, modules/chain.rs:157-168).
 //
@@ -83,8 +83,9 @@ __global__ void __launch_bounds__(RL_SEQ_BLOCK) gru_pass_kernel(rl_seq_pass_args
     constexpr int GH = TH ? TH : GH_MAX, GF = TF ? TF : GF_MAX, GA = TA ? TA : GA_MAX;
     constexpr int GP_MAX = 3 * GH * GF + 3 * GH * GH + 6 * GH + GA * GH + GA;
     constexpr bool BACKWARD = MODE == RL_PASS_GRAD || MODE == RL_PASS_FVP || MODE == RL_PASS_VALUE || MODE == RL_PASS_PPO ||
-                              MODE == RL_PASS_REINFORCE;
-    constexpr bool IS_POLICY = MODE != RL_PASS_VALUE;
+                              MODE == RL_PASS_REINFORCE || MODE == RL_PASS_QLOSS;
+    constexpr bool IS_POLICY = MODE != RL_PASS_VALUE && MODE != RL_PASS_QLOSS;
+    constexpr bool USES_TARGET = MODE == RL_PASS_VALUE || MODE == RL_PASS_QLOSS;
     constexpr bool FVP = MODE == RL_PASS_FVP;
     constexpr bool USES_ADV = MODE == RL_PASS_EVAL || MODE == RL_PASS_GRAD || MODE == RL_PASS_PPO || MODE == RL_PASS_REINFORCE;
     constexpr bool USES_LP0 = MODE == RL_PASS_EVAL || MODE == RL_PASS_GRAD || MODE == RL_PASS_PPO;
@@ -120,7 +121,7 @@ __global__ void __launch_bounds__(RL_SEQ_BLOCK) gru_pass_kernel(rl_seq_pass_args
         float x_next[GF], tgt_next = 0.0f;
 #pragma unroll
         for (int f = 0; f < F; ++f) x_next[f] = a.T ? a.obs[(uint64_t)f * E + e] : 0.0f;
-        if (MODE == RL_PASS_VALUE && a.T) tgt_next = a.target[e];
+        if (USES_TARGET && a.T) tgt_next = a.target[e];
         for (uint64_t t = 0; t < a.T; ++t) {
             const uint8_t sc = sc_next;
             if (sc == RL_PAD) break;
@@ -133,7 +134,7 @@ __global__ void __launch_bounds__(RL_SEQ_BLOCK) gru_pass_kernel(rl_seq_pass_args
                 sc_next = a.succ[(t + 1) * E + e];
 #pragma unroll
                 for (int f = 0; f < F; ++f) x_next[f] = a.obs[((t + 1) * F + f) * E + e];
-                if (MODE == RL_PASS_VALUE) tgt_next = a.target[(t + 1) * E + e];
+                if (USES_TARGET) tgt_next = a.target[(t + 1) * E + e];
             } else {
                 sc_next = RL_PAD;
             }
@@ -248,6 +249,17 @@ __global__ void __launch_bounds__(RL_SEQ_BLOCK) gru_pass_kernel(rl_seq_pass_args
 #pragma unroll
                     for (int k = 0; k < A; ++k) dz[k] = p[k] * (zd[k] - pd);
                 }
+            } else if (MODE == RL_PASS_QLOSS) {  // mse(Q(obs).gather(action), targets)  (dqn.rs:316-326)
+                const int act_s = (int)a.action[n_idx];
+                float q = z[0];
+#pragma unroll
+                for (int k = 1; k < A; ++k)
+                    if (k == act_s) q = z[k];
+                const float diff = q - tgt_cur;
+                loss_s = diff * diff;
+#pragma unroll
+                for (int k = 0; k < A; ++k)
+                    if (k == act_s) dz[k] = 2.0f * diff;
             } else {  // VALUE: mse(V(obs), targets)  (opt.rs:109-115)
                 const float diff = z[0] - tgt_cur;
                 loss_s = diff * diff;
@@ -388,7 +400,7 @@ rl_status launch_sized(rl_ctx *ctx, const rl_seq_pass_args &a, int grid, size_t 
 // BASELINE config 4 (2-armed bandit meta-env, rnn.rs-sized GRU): features 6, hidden 4, 2 logits (policy) or 1 (critic)
 template <int MODE>
 rl_status launch_mode(rl_ctx *ctx, const rl_seq_pass_args &a, int grid, size_t smem) {
-    constexpr bool POLICY = MODE != RL_PASS_VALUE;
+    constexpr bool POLICY = MODE != RL_PASS_VALUE;  // the Q-loss pass has one output per action, like a policy
     if (a.F == 6 && a.H == 4 && a.A == (POLICY ? 2 : 1)) return launch_sized<MODE, 6, 4, POLICY ? 2 : 1>(ctx, a, grid, smem);
     return launch_sized<MODE, 0, 0, 0>(ctx, a, grid, smem);
 }
@@ -412,6 +424,7 @@ rl_status rl_seq_pass_launch(rl_ctx *ctx, int mode, const rl_seq_pass_args &a, i
     case RL_PASS_VALUE: return launch_mode<RL_PASS_VALUE>(ctx, a, grid, smem);
     case RL_PASS_PPO: return launch_mode<RL_PASS_PPO>(ctx, a, grid, smem);
     case RL_PASS_REINFORCE: return launch_mode<RL_PASS_REINFORCE>(ctx, a, grid, smem);
+    case RL_PASS_QLOSS: return launch_mode<RL_PASS_QLOSS>(ctx, a, grid, smem);
     default: return rl_fail(ctx, RL_ERR_INVALID_ARG, "rl_seq_pass_launch: bad mode %d", mode);
     }
 }

@@ -87,6 +87,14 @@ rl_status rl_replay_sample_finish(rl_replay *rb, uint64_t *num_steps, uint64_t *
 uint32_t rl_replay_next_draw_index(rl_replay *rb);
 rl_ctx *rl_replay_ctx(rl_replay *rb);
 int rl_replay_num_features(rl_replay *rb);
+// The same draws as sequences for a recurrent Q-network (replay.cu K4g / K4h): *out_traj views B = episodes taken lanes of
+// L = the longest episode's steps (valid until the next sequence sample on this buffer), *out_target f32 [L][B].  Synchronises.
+rl_status rl_replay_sample_seq_dev(rl_replay *rb, uint64_t minibatch_steps, uint64_t seed, uint32_t draw_index, int one_step_td,
+                                   float discount, rl_grunet *q, rl_traj **out_traj, const float **out_target);
+
+struct rl_grunet_view { rl_ctx *ctx; int in_dim, hidden, out_dim, act; uint64_t n_params; float *params; };
+rl_grunet_view rl_grunet_view_of(rl_grunet *g);
+rl_status rl_grunet_seq_enqueue(rl_grunet *g, rl_traj *traj, float *out_dev, float *out_next_dev);
 
 // Full-batch pass modes shared by the MLP passes (update.cu) and the recurrent passes (gru_update.cu)
 enum { RL_PASS_STATS = 0, RL_PASS_EVAL = 1, RL_PASS_GRAD = 2, RL_PASS_FVP = 3, RL_PASS_VALUE = 4, RL_PASS_QLOSS = 5,
@@ -120,14 +128,13 @@ rl_status rl_seq_big_prepare(rl_ctx *ctx, const float *params, int F, int H, voi
 rl_status rl_seq_big_cell(rl_ctx *ctx, const void *prepared, int F, int H, const float *x, const float *h, uint64_t E, float *hnew);
 rl_status rl_seq_big_forward(rl_ctx *ctx, const float *params, int F, int H, int A, int act, const float *obs, const float *next_obs,
                              const uint8_t *succ, uint64_t T, uint64_t E, float *out, float *out_next);
-struct rl_grunet_view { rl_ctx *ctx; int in_dim, hidden, out_dim, act; uint64_t n_params; float *params; };
-rl_grunet_view rl_grunet_view_of(rl_grunet *g);
-rl_status rl_grunet_seq_enqueue(rl_grunet *g, rl_traj *traj, float *out_dev, float *out_next_dev);
 
 // gru.cu: fused rollout with a recurrent policy.  *partials_out receives the device pointer of its *nblocks_out rows of
 // per-block statistics (steps.cuh: ST_COUNT sums each), with one more row in front of them for the totals; rl_rollout
 // sums them as it does for every rollout.
-rl_status rl_rollout_seq(rl_env *env, rl_grunet *net, rl_bound bound, rl_traj *traj, double **partials_out, int *nblocks_out);
+// eps_greedy selects DqnActor (epsilon-greedy on the Q-values, exploration rate eps) instead of PolicyActor.
+rl_status rl_rollout_seq(rl_env *env, rl_grunet *net, bool eps_greedy, double eps, rl_bound bound, rl_traj *traj, double **partials_out,
+                         int *nblocks_out);
 
 struct rl_tabq {
     rl_ctx *ctx = nullptr;

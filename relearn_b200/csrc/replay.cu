@@ -21,6 +21,10 @@
 //  K4e sample_gather_kernel warp per sampled episode: ring -> minibatch planes [F][M] + reward-to-go
 //                           targets (sequential f32 recurrence, bit-identical to packed.rs:312-342).
 //  K4f q_values_kernel / td_target_kernel   OneStepTd: r + gamma * max_a Q(next) (critics/mod.rs:139-151).
+//  K4g seq_gather_kernel    the same taken episodes as SEQUENCES for a recurrent Q-network: warp per episode, ring ->
+//                           column b of [Lmax][.][B] planes in the trajectory layout (rows past the episode are RL_PAD),
+//                           reward-to-go targets by K4e's recurrence.
+//  K4h seq_td_target_kernel OneStepTd on the sequence planes from a SeqPacked forward over them.
 #include "handles.cuh"
 
 namespace {
@@ -177,6 +181,7 @@ struct SampleMeta {
     unsigned long long num_steps;   // M: steps in the minibatch
     unsigned int num_episodes;      // episodes taken
     int error;
+    unsigned int max_len;           // longest episode taken (sizes the sequence planes of rl_replay_sample_seq_dev)
 };
 
 // Draw j picks buffer j mod E (iter::repeat(buffers).flatten()) and a uniformly random stored episode
@@ -239,7 +244,7 @@ __global__ void __launch_bounds__(1024)
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     if (tid == 0) carry_s = 0;
     __syncthreads();
-    unsigned int taken = 0;
+    unsigned int taken = 0, longest = 0;
     unsigned long long last_end = 0;
     for (uint64_t base = 0; base < J; base += 4096) {
         const unsigned long long carry = carry_s;
@@ -277,6 +282,7 @@ __global__ void __launch_bounds__(1024)
                 if (run < minibatch_steps) {
                     taken += 1;
                     last_end = run + l[k];
+                    longest = l[k] > longest ? l[k] : longest;
                 }
                 run += l[k];
             }
@@ -287,6 +293,7 @@ __global__ void __launch_bounds__(1024)
     if (taken) {
         atomicAdd(&meta->num_episodes, taken);
         atomicMax(&meta->num_steps, last_end);
+        atomicMax(&meta->max_len, longest);
     }
 }
 
@@ -422,6 +429,79 @@ __global__ void __launch_bounds__(256)
     mb.target[col] = __fadd_rn(mb.reward[col], __fmul_rn(discount, next));
 }
 
+// Sequence planes of one sample: B = episodes taken (one column each, in draw order), L = the longest of them.
+struct SeqPlanes {
+    uint64_t B, L;
+    float *obs, *nobs, *reward, *target, *qout, *qout_next;  // obs / nobs f32 [L][F][B]; reward, target [L][B]; q* [L][A][B]
+    uint8_t *action, *succ;                                  // u8 [L][B]
+    uint32_t *len;                                           // u32 [B] episode lengths
+};
+
+// One warp per taken episode, walking it from the end in 32-step chunks like sample_gather_kernel: step idx of draw j goes to
+// row idx of column j.  The reward-to-go carry is the same sequential f32 recurrence, so the targets are bit-identical to the
+// flat minibatch's.  Column j's successor codes are RL_CONTINUE up to the last step, which keeps the stored code.
+__global__ void __launch_bounds__(256)
+    seq_gather_kernel(ReplayPtrs rb, const uint32_t *__restrict__ sel_lane, const uint32_t *__restrict__ sel_start,
+                      const uint32_t *__restrict__ sel_len, SeqPlanes sp, float discount, int rtg) {
+    const int lane_id = threadIdx.x & 31;
+    const uint64_t warp_global = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const uint64_t total_warps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
+    const uint32_t C = (uint32_t)rb.C;
+    const int F = rb.F;
+    const uint64_t B = sp.B;
+    for (uint64_t j = warp_global; j < B; j += total_warps) {
+        const uint64_t lane = sel_lane[j];
+        const uint32_t start = sel_start[j], len = sel_len[j];
+        if (lane_id == 0) sp.len[j] = len;
+        float carry = 0.0f;
+        for (int c = (int)((len + 31) / 32) - 1; c >= 0; --c) {
+            const uint32_t idx = (uint32_t)c * 32 + lane_id;
+            const bool valid = idx < len;
+            const uint64_t base = lane * rb.C + (valid ? wrap_add(start, idx, C) : 0);
+            const uint64_t cell = (uint64_t)idx * B + j;
+            float r = 0.0f;
+            if (valid) {
+                r = rb.reward[base];
+                const uint8_t code = idx + 1 < len ? (uint8_t)RL_CONTINUE : rb.succ[base];
+                sp.reward[cell] = r;
+                sp.action[cell] = rb.action[base];
+                sp.succ[cell] = code;
+                for (int f = 0; f < F; ++f) sp.obs[((uint64_t)idx * F + f) * B + j] = rb.obs[base * F + f];
+                if (code == RL_INTERRUPT)
+                    for (int f = 0; f < F; ++f) sp.nobs[((uint64_t)idx * F + f) * B + j] = rb.next_obs[base * F + f];
+            }
+            if (rtg) {  // packed.rs:336, as in sample_gather_kernel
+                const int n_here = (int)(len - (uint32_t)c * 32 < 32u ? len - (uint32_t)c * 32 : 32u);
+                float y = 0.0f;
+                for (int i = n_here - 1; i >= 0; --i) {
+                    const float xi = __shfl_sync(0xffffffffu, r, i);
+                    carry = __fadd_rn(xi, __fmul_rn(carry, discount));
+                    if (lane_id == i) y = carry;
+                }
+                if (valid) sp.target[cell] = y;
+            }
+        }
+    }
+}
+
+// one_step_values on the sequence planes (critics/mod.rs:139-151) from Q = seq_packed over them (qout) and Q on the successor
+// observation of the interrupted last steps (qout_next, one more step of the same sequence): the operations of q_values_kernel's
+// max and td_target_kernel's sum, in the same order.
+__global__ void __launch_bounds__(256) seq_td_target_kernel(SeqPlanes sp, int A, float discount) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x, B = sp.B;
+    if (i >= sp.L * B) return;
+    const uint64_t t = i / B, b = i - t * B;
+    const uint8_t code = sp.succ[i];
+    if (code == RL_PAD) return;
+    auto qmax = [&](const float *q, uint64_t row) {
+        float best = q[(row * A) * B + b];
+        for (int k = 1; k < A; ++k) best = fmaxf(best, q[(row * A + k) * B + b]);
+        return best;
+    };
+    const float next = code == RL_CONTINUE ? qmax(sp.qout, t + 1) : code == RL_INTERRUPT ? qmax(sp.qout_next, t) : 0.0f;
+    sp.target[i] = __fadd_rn(sp.reward[i], __fmul_rn(discount, next));
+}
+
 }  // namespace
 
 struct rl_replay {
@@ -441,9 +521,57 @@ struct rl_replay {
     SampleMeta *meta_sets = nullptr;   // [mb_sets] for batched samples
     uint32_t last_sets = 1;            // minibatches of the last enqueue (rl_replay_sample_finish reads the last one)
     uint32_t draw_counter = 0;
+    // sequence sampler (rl_replay_sample_seq_dev): planes grown to the largest B * L seen, and the rl_traj that views them
+    SeqPlanes seq{};
+    uint64_t seq_cells = 0, seq_cols = 0;
+    int seq_A = 0;
+    rl_traj seq_traj{};
 };
 
 namespace {
+
+void free_seq(rl_replay *rb) {
+    SeqPlanes &q = rb->seq;
+    cudaFree(q.obs); cudaFree(q.nobs); cudaFree(q.reward); cudaFree(q.target); cudaFree(q.qout); cudaFree(q.qout_next);
+    cudaFree(q.action); cudaFree(q.succ); cudaFree(q.len);
+    q = SeqPlanes{};
+    rb->seq_cells = rb->seq_cols = 0;
+    rb->seq_A = 0;
+}
+
+// Planes for `cells` = B * L steps and B columns (A outputs of the Q-network for OneStepTd targets, 0 = none), grown only.
+rl_status ensure_seq(rl_replay *rb, uint64_t cells, uint64_t cols, int A) {
+    rl_ctx *ctx = rb->ctx;
+    if (cells <= rb->seq_cells && cols <= rb->seq_cols && A <= rb->seq_A) return RL_OK;
+    RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    cells = cells > rb->seq_cells ? cells : rb->seq_cells;
+    cols = cols > rb->seq_cols ? cols : rb->seq_cols;
+    A = A > rb->seq_A ? A : rb->seq_A;
+    free_seq(rb);
+    const size_t F = (size_t)rb->p.F;
+    SeqPlanes &q = rb->seq;
+    cudaError_t e = cudaSuccess;
+    auto alloc = [&](void **p, size_t bytes) {
+        if (e == cudaSuccess && bytes) e = cudaMalloc(p, bytes);
+    };
+    alloc((void **)&q.obs, cells * F * sizeof(float));
+    alloc((void **)&q.nobs, cells * F * sizeof(float));
+    alloc((void **)&q.reward, cells * sizeof(float));
+    alloc((void **)&q.target, cells * sizeof(float));
+    alloc((void **)&q.qout, cells * (size_t)A * sizeof(float));
+    alloc((void **)&q.qout_next, cells * (size_t)A * sizeof(float));
+    alloc((void **)&q.action, cells);
+    alloc((void **)&q.succ, cells);
+    alloc((void **)&q.len, cols * sizeof(uint32_t));
+    if (e != cudaSuccess) {
+        free_seq(rb);
+        return rl_fail(ctx, RL_ERR_OOM, "replay sequence sampler: %s", cudaGetErrorString(e));
+    }
+    rb->seq_cells = cells;
+    rb->seq_cols = cols;
+    rb->seq_A = A;
+    return RL_OK;
+}
 
 void free_sampler(rl_replay *rb) {
     cudaFree(rb->mb.obs); cudaFree(rb->mb.nobs); cudaFree(rb->mb.reward); cudaFree(rb->mb.target);
@@ -569,6 +697,63 @@ rl_status rl_replay_sample_finish(rl_replay *rb, uint64_t *num_steps, uint64_t *
     return RL_OK;
 }
 
+// sample_minibatch (dqn.rs:280-314) for a recurrent Q-network: K4c / K4d exactly as rl_replay_sample_enqueue draws and cuts
+// them (same episodes), then the taken episodes as padded sequences in an rl_traj of B lanes and L steps that the recurrent
+// passes and forwards read like a rollout's trajectory.  B and L are known only on the device: one host read of the sample's
+// SampleMeta sizes the planes, so this call synchronises.  OneStepTd targets need `q` (a SeqPacked forward with the current
+// parameters); reward-to-go targets do not.
+rl_status rl_replay_sample_seq_dev(rl_replay *rb, uint64_t minibatch_steps, uint64_t seed, uint32_t draw_index, int one_step_td,
+                                   float discount, rl_grunet *q, rl_traj **out_traj, const float **out_target) {
+    rl_ctx *ctx = rb->ctx;
+    RL_REQUIRE(ctx, minibatch_steps > 0 && minibatch_steps < (1ull << 31), "replay sample: minibatch_steps out of range");
+    rl_grunet_view qv{};
+    if (one_step_td) {
+        RL_REQUIRE(ctx, q != nullptr, "replay sample: OneStepTd targets need the action-value network");
+        qv = rl_grunet_view_of(q);
+        RL_REQUIRE(ctx, qv.ctx == ctx, "replay sample: network belongs to another context");
+        RL_REQUIRE(ctx, qv.in_dim == rb->p.F, "replay sample: network input does not match the observation features");
+    }
+    RL_TRY(ensure_sampler(rb, minibatch_steps, 1, false));
+    SampleMeta *meta = rb->meta_sets;
+    const uint64_t J = minibatch_steps;
+    RL_CUDA(ctx, cudaMemsetAsync(meta, 0, sizeof(SampleMeta), ctx->stream));
+    RL_LAUNCH(ctx, sample_draw_kernel, dim3(rl_grid_for(J, 256), 1), 256, 0, rb->p, J, seed, draw_index, rb->sel_lane, rb->sel_start,
+              rb->sel_len, meta);
+    RL_LAUNCH(ctx, sample_scan_kernel, 1, 1024, 0, rb->sel_len, J, minibatch_steps, rb->sel_off, meta);
+    rb->last_sets = 1;
+    SampleMeta *host;
+    RL_TRY(rl_ctx_pinned(ctx, sizeof(SampleMeta), (void **)&host));
+    RL_CUDA(ctx, cudaMemcpyAsync(host, meta, sizeof(SampleMeta), cudaMemcpyDeviceToHost, ctx->stream));
+    RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    if (host->error == RB_ERR_NO_EPISODES)
+        return rl_fail(ctx, RL_ERR_INVALID_ARG, "replay sample: a lane has no stored episode (Uniform::new(0, 0))");
+    const uint64_t B = host->num_episodes, L = host->max_len, M = host->num_steps;
+    RL_TRY(ensure_seq(rb, B * L, B, one_step_td ? qv.out_dim : 0));
+    SeqPlanes sp = rb->seq;
+    sp.B = B;
+    sp.L = L;
+    rb->seq.B = B;
+    rb->seq.L = L;
+    RL_CUDA(ctx, cudaMemsetAsync(sp.succ, RL_PAD, B * L, ctx->stream));
+    // padded rows are read by the GEMM form of the passes (multiplied by zero cotangents): keep them finite
+    RL_CUDA(ctx, cudaMemsetAsync(sp.obs, 0, B * L * (size_t)rb->p.F * sizeof(float), ctx->stream));
+    RL_LAUNCH(ctx, seq_gather_kernel, (unsigned)ctx->sm_count * 4, 256, 0, rb->p, rb->sel_lane, rb->sel_start, rb->sel_len, sp, discount,
+              one_step_td ? 0 : 1);
+    rl_traj &t = rb->seq_traj;
+    t.ctx = ctx; t.env = rb->env;
+    t.E = B; t.T = L; t.used_T = L; t.F = (uint64_t)rb->p.F;
+    t.obs = sp.obs; t.reward = sp.reward; t.next_obs = sp.nobs; t.action = sp.action; t.succ = sp.succ;
+    t.lane_len = sp.len; t.lane_flags = nullptr; t.counts_dev = nullptr;
+    t.num_steps = M; t.num_episodes = B;
+    if (one_step_td) {
+        RL_TRY(rl_grunet_seq_enqueue(q, &t, sp.qout, sp.qout_next));
+        RL_LAUNCH(ctx, seq_td_target_kernel, rl_grid_for(B * L, 256), 256, 0, sp, qv.out_dim, discount);
+    }
+    *out_traj = &t;
+    *out_target = sp.target;
+    return RL_OK;
+}
+
 uint32_t rl_replay_next_draw_index(rl_replay *rb) { return rb->draw_counter++; }
 uint32_t rl_replay_take_draw_indices(rl_replay *rb, uint32_t n) {
     const uint32_t first = rb->draw_counter;
@@ -635,6 +820,7 @@ rl_status rl_replay_destroy(rl_replay *rb) {
     cudaFree(p.ep_end); cudaFree(p.total); cudaFree(p.index_offset); cudaFree(p.ep_head); cudaFree(p.ep_count);
     cudaFree(rb->write_start); cudaFree(rb->error); cudaFree(rb->stats); cudaFree(rb->meta);
     free_sampler(rb);
+    free_seq(rb);
     delete rb;
     return RL_OK;
 }
@@ -762,6 +948,21 @@ rl_status rl_replay_sample(rl_replay *rb, const rl_dqn_cfg *cfg, rl_mlp *q, uint
     out->action = dev.action;
     out->target = dev.target;
     out->succ = dev.succ;
+    return RL_OK;
+}
+
+rl_status rl_replay_sample_seq(rl_replay *rb, const rl_dqn_cfg *cfg, rl_grunet *q, uint32_t draw_index, rl_traj_view *out,
+                               const float **target_dev) {
+    if (!rb || !cfg || !out || !target_dev)
+        return rl_fail(rb ? rb->ctx : nullptr, RL_ERR_INVALID_ARG, "rl_replay_sample_seq: NULL argument");
+    rl_traj *t = nullptr;
+    RL_TRY(rl_replay_sample_seq_dev(rb, cfg->minibatch_steps, cfg->sample_seed, draw_index, cfg->target_one_step_td,
+                                    cfg->discount_factor, q, &t, target_dev));
+    RL_CUDA(rb->ctx, cudaStreamSynchronize(rb->ctx->stream));
+    out->num_lanes = t->E; out->step_capacity = t->T; out->num_features = t->F;
+    out->obs = t->obs; out->action = t->action; out->reward = t->reward; out->succ = t->succ; out->next_obs = t->next_obs;
+    out->lane_len = t->lane_len;
+    out->num_steps = t->num_steps;
     return RL_OK;
 }
 

@@ -2140,4 +2140,98 @@ rl_status rl_dqn_update(rl_replay *rb, rl_mlp *q, rl_adam *adam, const rl_dqn_cf
     return x_error_check(ctx, "rl_dqn_update");
 }
 
+// DqnAgent::batch_update (dqn.rs:263-337) with a recurrent action-value module: every optimizer step samples its episodes as
+// sequences (rl_replay_sample_seq_dev: the draws of rl_dqn_update, one host read to size the planes), runs the Q-loss pass with
+// back-propagation through time over them (K9 / K10), reduces over the data-parallel group and takes the Adam step.  One sample
+// per optimizer step: the padded planes of a batched update could be opt_steps times B * L, far beyond the flat minibatches.
+rl_status rl_dqn_update_seq(rl_replay *rb, rl_grunet *q, rl_adam *adam, const rl_dqn_cfg *cfg, rl_opt_stats *stats) {
+    if (!rb || !q || !adam || !cfg)
+        return rl_fail(rb ? rl_replay_ctx(rb) : nullptr, RL_ERR_INVALID_ARG, "rl_dqn_update_seq: NULL argument");
+    rl_ctx *ctx = rl_replay_ctx(rb);
+    const rl_grunet_view net = rl_grunet_view_of(q);
+    RL_REQUIRE(ctx, net.ctx == ctx, "rl_dqn_update_seq: network belongs to another context");
+    RL_REQUIRE(ctx, adam->owner == (void *)q, "rl_dqn_update_seq: optimizer belongs to another module");
+    RL_REQUIRE(ctx, cfg->opt_steps_per_update >= 0 && cfg->opt_steps_per_update <= 100000,
+               "rl_dqn_update_seq: opt_steps_per_update out of range");
+    const int F = rl_replay_num_features(rb);
+    if (net.in_dim != F || !(rl_seq_pass_supports(net.in_dim, net.hidden, net.out_dim) || rl_seq_big_supports(net.in_dim, net.hidden, net.out_dim)))
+        return rl_fail(ctx, RL_ERR_UNSUPPORTED, "rl_dqn_update_seq: recurrent passes are built for hidden <= 128, features <= 64, outputs <= 32 "
+                       "(got %d -> %d -> %d on %d features)", net.in_dim, net.hidden, net.out_dim, F);
+    const int P = (int)net.n_params;
+    const int n_steps = cfg->opt_steps_per_update;
+    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+    if (stats) {
+        RL_TRY(update_events(ctx, &ev0, &ev1));
+        RL_CUDA(ctx, cudaEventRecord(ev0, ctx->stream));
+    }
+    AdamArgs ac{adam->cfg.learning_rate, adam->cfg.beta1, adam->cfg.beta2, adam->cfg.weight_decay, adam->cfg.eps};
+    std::vector<double> losses((size_t)n_steps, 0.0);
+    uint64_t m_last = 0;
+    for (int s = 0; s < n_steps; ++s) {
+        rl_traj *mb = nullptr;
+        const float *target = nullptr;
+        // sample_minibatch (dqn.rs:280-314); OneStepTd targets from the parameters of this step
+        RL_TRY(rl_replay_sample_seq_dev(rb, cfg->minibatch_steps, cfg->sample_seed, rl_replay_next_draw_index(rb), cfg->target_one_step_td,
+                                        cfg->discount_factor, q, &mb, &target));
+        m_last = mb->num_steps;
+        PassPlan plan;
+        SeqScratch sc;
+        RL_TRY(make_seq_plan(ctx, net, mb->T, mb->E, 256, &plan, &sc));
+        double *loss_dev = (double *)sc.extra;
+        rl_seq_pass_args a = seq_base_args(mb, net, mb->T, sc, plan);
+        a.target = target;
+        // loss_fn + backward_step (dqn.rs:316-336, coptimizer.rs:13-27)
+        RL_TRY(seq_pass(ctx, plan, PASS_QLOSS, a));
+        adam->step += 1;
+        RL_LAUNCH(ctx, adam_step_kernel, 1, VEC_THREADS, 0, plan.sums, P, net.params, adam->m, adam->v, ac, adam->step, loss_dev);
+        // the next sample synchronises anyway; the plan's scratch may move with the next sample's size
+        if (stats) {
+            RL_CUDA(ctx, cudaMemcpyAsync(&losses[(size_t)s], loss_dev, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+            RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        }
+    }
+    if (stats) {
+        RL_CUDA(ctx, cudaEventRecord(ev1, ctx->stream));
+        RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        stats->loss_first = n_steps > 0 ? losses[0] : 0.0;
+        stats->loss_last = n_steps > 0 ? losses[(size_t)n_steps - 1] : 0.0;
+        stats->num_steps = m_last;
+        stats->opt_steps = (uint64_t)n_steps;
+        cudaEventElapsedTime(&stats->update_ms, ev0, ev1);
+    }
+    return x_error_check(ctx, "rl_dqn_update_seq");
+}
+
+// One Q-loss pass of rl_dqn_update_seq for diagnostics and parity checks: the mean loss of the sequence minibatch of
+// `draw_index` and its flat gradient at the current parameters (no Adam step).
+rl_status rl_dqn_probe_seq(rl_replay *rb, const rl_dqn_cfg *cfg, rl_grunet *q, uint32_t draw_index, double *loss, float *grad_host) {
+    if (!rb || !q || !cfg) return rl_fail(rb ? rl_replay_ctx(rb) : nullptr, RL_ERR_INVALID_ARG, "rl_dqn_probe_seq: NULL argument");
+    rl_ctx *ctx = rl_replay_ctx(rb);
+    const rl_grunet_view net = rl_grunet_view_of(q);
+    RL_REQUIRE(ctx, net.ctx == ctx, "rl_dqn_probe_seq: network belongs to another context");
+    const int F = rl_replay_num_features(rb);
+    if (net.in_dim != F || !(rl_seq_pass_supports(net.in_dim, net.hidden, net.out_dim) || rl_seq_big_supports(net.in_dim, net.hidden, net.out_dim)))
+        return rl_fail(ctx, RL_ERR_UNSUPPORTED, "rl_dqn_probe_seq: recurrent passes are built for hidden <= 128, features <= 64, outputs <= 32 "
+                       "(got %d -> %d -> %d on %d features)", net.in_dim, net.hidden, net.out_dim, F);
+    const int P = (int)net.n_params;
+    rl_traj *mb = nullptr;
+    const float *target = nullptr;
+    RL_TRY(rl_replay_sample_seq_dev(rb, cfg->minibatch_steps, cfg->sample_seed, draw_index, cfg->target_one_step_td, cfg->discount_factor,
+                                    q, &mb, &target));
+    PassPlan plan;
+    SeqScratch sc;
+    RL_TRY(make_seq_plan(ctx, net, mb->T, mb->E, 0, &plan, &sc));
+    rl_seq_pass_args a = seq_base_args(mb, net, mb->T, sc, plan);
+    a.target = target;
+    RL_TRY(seq_pass(ctx, plan, PASS_QLOSS, a));
+    std::vector<double> host((size_t)plan.W);
+    RL_CUDA(ctx, cudaMemcpyAsync(host.data(), plan.sums, (size_t)plan.W * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    const double N = host[P + SC_COUNT];
+    if (loss) *loss = host[P + SC_LOSS] / N;
+    if (grad_host)
+        for (int i = 0; i < P; ++i) grad_host[i] = (float)(host[i] / N);
+    return RL_OK;
+}
+
 }  // extern "C"

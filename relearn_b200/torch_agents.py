@@ -360,6 +360,21 @@ class ReplayBuffer:
         return {"obs": obs[:k], "next_obs": nobs[:k], "action": act[:k], "reward": rew[:k], "succ": succ[:k],
                 "episode_len": eps[:int(s.num_episodes)].astype(np.int64), "total_step_count": int(s.total_step_count)}
 
+    def sample_seq(self, cfg: "L.DqnCfg", q: GruLinear | None, draw_index: int) -> dict:
+        """The same sample_minibatch as padded sequences for a recurrent Q-network, read back to the host: planes
+        [L][.][B] with one episode per column (draw order), succ RL_PAD past each episode, targets [L][B]."""
+        v, tgt = L.TrajView(), C.c_void_p()
+        L.check(self._lib.rl_replay_sample_seq(self.handle, C.byref(cfg), q.handle if q is not None else None, draw_index,
+                                               C.byref(v), C.byref(tgt)), self.ctx.handle)
+        B, T, F = int(v.num_lanes), int(v.step_capacity), int(v.num_features)
+        rd = self.ctx.read
+        return {"num_steps": int(v.num_steps), "num_episodes": B, "max_len": T,
+                "lane_len": rd(v.lane_len, (B,), np.uint32).astype(np.int64),
+                "obs": rd(v.obs, (T, F, B), np.float32).transpose(0, 2, 1).copy(),
+                "next_obs": rd(v.next_obs, (T, F, B), np.float32).transpose(0, 2, 1).copy(),
+                "action": rd(v.action, (T, B), np.uint8), "reward": rd(v.reward, (T, B), np.float32),
+                "succ": rd(v.succ, (T, B), np.uint8), "target": rd(tgt.value, (T, B), np.float32)}
+
     def sample(self, cfg: "L.DqnCfg", q: Mlp | None, draw_index: int) -> dict:
         """One sample_minibatch (dqn.rs:280-314), read back to the host."""
         v = L.MinibatchView()
@@ -399,7 +414,7 @@ class DataCollectionSchedule:
 class DqnConfig:
     """dqn.rs:26-72"""
 
-    action_value_fn_config: MlpConfig = field(default_factory=MlpConfig)
+    action_value_fn_config: MlpConfig | GruLinearConfig = field(default_factory=MlpConfig)
     optimizer_config: AdamConfig = field(default_factory=AdamConfig)
     target_one_step_td: bool = False          # StepValueTarget::RewardToGo is the default
     exploration_rate: ExplorationRateSchedule = field(default_factory=ExplorationRateSchedule)
@@ -426,9 +441,15 @@ class DqnAgent:
         self.discount_factor = np.float32(env.discount_factor)  # dqn.rs:178
         self.global_steps = 0
 
+    @property
+    def recurrent(self) -> bool:
+        return isinstance(self.action_value_fn, GruLinear)
+
     def actor(self, training: bool = True) -> ActorSpec:
         """Agent::actor(mode): epsilon is fixed from global_steps at actor creation (dqn.rs:202-212)."""
         eps = self.cfg.exploration_rate.exploration_rate(self.global_steps, training)
+        if self.recurrent:
+            return ActorSpec(kind=L.RL_ACTOR_EPS_GREEDY_Q, seq_net=self.action_value_fn, exploration_rate=eps, training=training)
         return ActorSpec(kind=L.RL_ACTOR_EPS_GREEDY_Q, net=self.action_value_fn, exploration_rate=eps, training=training)
 
     def buffer(self) -> ReplayBuffer:
@@ -450,8 +471,9 @@ class DqnAgent:
         self.global_steps = buffer.total_step_count()
         stats = L.OptStats()
         cfg = self.c_cfg()
-        L.check(self._lib.rl_dqn_update(buffer.handle, self.action_value_fn.handle, self.optimizer.handle, C.byref(cfg),
-                                        C.byref(stats)), self.ctx.handle)
+        update = self._lib.rl_dqn_update_seq if self.recurrent else self._lib.rl_dqn_update
+        L.check(update(buffer.handle, self.action_value_fn.handle, self.optimizer.handle, C.byref(cfg), C.byref(stats)),
+                self.ctx.handle)
         if logger is not None:
             logger.update({"loss": stats.loss_last, "loss_first": stats.loss_first, "minibatch_steps": stats.num_steps,
                            "agent_update/time": stats.update_ms * 1e-3})
