@@ -48,8 +48,7 @@ struct rl_mlp {
 };
 
 struct rl_adam {
-    rl_mlp *mlp = nullptr;      // owning module when it is an Mlp
-    void *owner = nullptr;      // the module handle this optimizer was built for (rl_mlp* or rl_grunet*)
+    const void *owner = nullptr;  // the module handle this optimizer was built for (rl_mlp* or rl_grunet*)
     rl_ctx *ctx = nullptr;
     rl_adam_cfg cfg{};
     float *m = nullptr, *v = nullptr;  // device, n_params each

@@ -27,7 +27,6 @@
 
 #include <cmath>
 #include <cstdlib>
-#include <functional>
 #include <vector>
 
 namespace {
@@ -1323,15 +1322,6 @@ size_t pass_smem_bytes() {
     return (size_t)nwarps * P * sizeof(double) + (size_t)nwarps * 32 * 12 * sizeof(float);
 }
 
-// The two timing events of an update entry point: per context, created on first use (rl_ctx_destroy frees them).
-rl_status update_events(rl_ctx *ctx, cudaEvent_t *ev0, cudaEvent_t *ev1) {
-    for (int k = 0; k < 2; ++k)
-        if (!ctx->upd_ev[k]) RL_CUDA(ctx, cudaEventCreate(&ctx->upd_ev[k]));
-    *ev0 = ctx->upd_ev[0];
-    *ev1 = ctx->upd_ev[1];
-    return RL_OK;
-}
-
 // Data-parallel group: did a peer-mailbox wait time out (reduce_rows_x_kernel)?  From the failing reduction on every
 // launch of that kernel leaves sums and parameters untouched; the update entry points end with this check and report it.
 rl_status x_error_check(rl_ctx *ctx, const char *what) {
@@ -1383,7 +1373,7 @@ rl_status launch_pass_ffma(rl_ctx *ctx, const PassPlan &plan, PassArgs args, boo
 }
 
 // Which kernel runs the default networks' passes (RL_PASS_KERNEL_*): RL_PASS_KERNEL from the environment until
-// rl_pass_kernel_select sets it.
+// rl_pass_kernel_select sets it.  pass_net_for reads it into the PassNet of an update.
 int g_pass_kernel = -1;
 int pass_kernel() {
     if (g_pass_kernel < 0) {
@@ -1441,6 +1431,7 @@ rl_status make_plan(rl_ctx *ctx, int P, uint64_t TE, PassPlan *plan, size_t extr
 struct PassNet {
     bool deflt;
     AnyShape sh;
+    int kernel;  // RL_PASS_KERNEL_* of a default network
 };
 
 rl_status pass_net_for(rl_ctx *ctx, const rl_mlp *m, int F_data, const char *what, PassNet *out) {
@@ -1449,6 +1440,7 @@ rl_status pass_net_for(rl_ctx *ctx, const rl_mlp *m, int F_data, const char *wha
                        m->in_dim, m->hidden, m->out_dim, F_data);
     out->sh = AnyShape{m->in_dim, m->hidden, m->out_dim, (int)m->act, m->n_hidden, {m->hid[0], m->hid[1], m->hid[2]}};
     out->deflt = m->n_hidden == 1 && F_data == 5 && m->hidden == 128 && m->act == RL_ACT_RELU && (m->out_dim == 1 || m->out_dim == 2);
+    out->kernel = pass_kernel();
     if (m->n_hidden > 1) {
         bool ok = m->in_dim >= 1 && m->in_dim <= ANY_MAXF && m->out_dim >= 1 && m->out_dim <= ANY_MAXA;
         for (int l = 0; l < m->n_hidden; ++l) ok = ok && m->hid[l] >= 1 && m->hid[l] <= ANY_DEEP_MAXH;
@@ -1486,11 +1478,11 @@ rl_status launch_pass_any_mode(rl_ctx *ctx, const PassPlan &plan, PassArgs args,
 
 // One full-batch pass of `pn` in MODE; *rows = partial rows it wrote.  The critic pass of the default 5 -> 128 -> 1
 // network and every other pass of the default 5 -> 128 -> 2 network run on the tensor cores, or on the FP32 pipe when
-// that is selected; every other module runs on mlp_pass_any_kernel.
+// pn.kernel selects it; every other module runs on mlp_pass_any_kernel.
 template <int MODE>
 rl_status launch_pass(rl_ctx *ctx, const PassPlan &plan, const PassArgs &pa, const PassNet &pn, bool reduce, int *rows) {
     constexpr int A = MODE == PASS_VALUE ? 1 : 2;
-    if (pn.deflt && pn.sh.A == A && pass_kernel() == RL_PASS_KERNEL_TCGEN05) {
+    if (pn.deflt && pn.sh.A == A && pn.kernel == RL_PASS_KERNEL_TCGEN05) {
         if (rows) *rows = tc_grid<A, MODE>(ctx, plan);
         return launch_pass_tc<A, MODE>(ctx, plan, pa, reduce);
     }
@@ -1514,123 +1506,9 @@ rl_status launch_pass_rt(rl_ctx *ctx, const PassPlan &plan, const PassArgs &pa, 
     }
 }
 
-// One optimizer step on the sums of the pass just launched: pass -> [reduce -> all-reduce] -> Adam
-// (n_backward_steps: zero_grad, backward, step; torch/agents/mod.rs:50-55, coptimizer.rs:13-27).
-rl_status pass_and_adam(rl_ctx *ctx, const PassPlan &plan, const PassArgs &pa, int mode, const PassNet &pn, rl_mlp *net,
-                        rl_adam *adam, const AdamArgs &ac, double *loss_out) {
-    adam->step += 1;
-    int rows = plan.grid;
-    if (ctx->world > 1 && ctx->x_ok && rl_div_up(plan.W, 32) <= RL_X_BLOCKS) {
-        RL_TRY(launch_pass_rt(ctx, plan, pa, mode, pn, false, &rows));
-        ctx->x_seq += 1;
-        RL_LAUNCH(ctx, reduce_rows_x_kernel<true>, rl_div_up(plan.W, 32), 256, 0, plan.partials, rows, plan.W, plan.P, plan.sums,
-                  ctx->x, ctx->x_seq, (const int *)nullptr, (XAdam{net->params, adam->m, adam->v, ac, adam->step, loss_out, plan.P}));
-    } else if (ctx->world > 1) {
-        RL_TRY(launch_pass_rt(ctx, plan, pa, mode, pn));
-        RL_LAUNCH(ctx, adam_step_kernel, 1, VEC_THREADS, 0, plan.sums, plan.P, net->params, adam->m, adam->v, ac, adam->step,
-                  loss_out);
-    } else {
-        RL_TRY(launch_pass_rt(ctx, plan, pa, mode, pn, false, &rows));
-        RL_LAUNCH(ctx, reduce_rows_adam_kernel, rl_div_up(plan.W, 32), 256, 0, plan.partials, rows, plan.W, plan.P, plan.sums,
-                  net->params, adam->m, adam->v, ac, adam->step, loss_out);
-    }
-    return RL_OK;
-}
-
-
-
 // ------------------------------------------------------------------------------------------------
-// Trust-region step, network-agnostic: `pass(mode, vec, skip_flag)` runs one full-batch pass of the policy
-// module (MLP: launch_pass_rt; GRU: gru_pass_kernel) and leaves the all-reduced f64 sums in plan.sums.
+// Recurrent modules (Chain<Gru, Linear>)
 // ------------------------------------------------------------------------------------------------
-using PassFn = std::function<rl_status(int mode, const float *vec, const int *skip_flag)>;
-
-size_t trpo_vector_bytes(int P) {
-    const size_t vec_bytes = ((size_t)P * sizeof(float) + 255) / 256 * 256;
-    return 256 + 6 * vec_bytes;  // TrpoState + theta0, g, x, r, p, descent
-}
-
-rl_status trpo_update_generic(rl_ctx *ctx, int P, float *theta, const PassPlan &plan, char *ex, const PassFn &pass,
-                              const rl_trpo_cfg *cfg, rl_trpo_stats *stats) {
-    const size_t vec_bytes = ((size_t)P * sizeof(float) + 255) / 256 * 256;
-    TrpoState *st = (TrpoState *)ex;
-    float *theta0 = (float *)(ex + 256), *g = (float *)(ex + 256 + vec_bytes), *x = (float *)(ex + 256 + 2 * vec_bytes);
-    float *r = (float *)(ex + 256 + 3 * vec_bytes), *p = (float *)(ex + 256 + 4 * vec_bytes);
-    float *descent = (float *)(ex + 256 + 5 * vec_bytes);
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    if (stats) {
-        RL_TRY(update_events(ctx, &ev0, &ev1));
-        RL_CUDA(ctx, cudaEventRecord(ev0, ctx->stream));
-    }
-    const float reg = (float)cfg->hpv_reg_coeff;
-    // behaviour-policy statistics (no_grad block, trpo.rs:112-122)
-    RL_TRY(pass(PASS_STATS, nullptr, nullptr));
-    RL_LAUNCH(ctx, trpo_begin_kernel, 1, 32, 0, st, plan.sums, P);
-    // loss gradient at theta0 (conjugate_gradient.rs:121-143)
-    RL_TRY(pass(PASS_GRAD, nullptr, nullptr));
-    RL_LAUNCH(ctx, trpo_cg_init_kernel, 1, VEC_THREADS, 0, st, plan.sums, P, g, x, r, p, theta, theta0);
-    // conjugate gradient on the Fisher matrix (conjugate_gradient.rs:371-403)
-    for (uint64_t it = 0; it < cfg->cg_iterations; ++it) {
-        RL_TRY(pass(PASS_FVP, p, &st->cg_done));
-        RL_LAUNCH(ctx, trpo_cg_step_kernel, 1, VEC_THREADS, 0, st, plan.sums, P, x, r, p, reg, 1e-10);
-    }
-    RL_LAUNCH(ctx, trpo_nan_to_num_kernel, 1, VEC_THREADS, 0, st, x, P);
-    RL_TRY(pass(PASS_FVP, x, nullptr));
-    RL_LAUNCH(ctx, trpo_step_size_kernel, 1, VEC_THREADS, 0, st, plan.sums, P, x, descent, reg, cfg->max_policy_step_kl);
-    // backtracking line search (conjugate_gradient.rs:183-254)
-    for (uint64_t i = 0; i < cfg->max_backtracks; ++i) {
-        const double ratio = std::pow(cfg->backtrack_ratio, (double)i);
-        RL_LAUNCH(ctx, trpo_ls_candidate_kernel, 1, VEC_THREADS, 0, st, theta, theta0, descent, (float)ratio, P);
-        RL_TRY(pass(PASS_EVAL, nullptr, &st->accepted));
-        RL_LAUNCH(ctx, trpo_ls_check_kernel, 1, 32, 0, st, plan.sums, P, cfg->max_policy_step_kl, (int)i, ratio);
-    }
-    RL_LAUNCH(ctx, trpo_ls_finish_kernel, 1, VEC_THREADS, 0, st, theta, theta0, P, cfg->max_policy_step_kl,
-              cfg->accept_violation);
-    TrpoState *host;
-    RL_TRY(rl_ctx_pinned(ctx, sizeof(TrpoState), (void **)&host));
-    RL_CUDA(ctx, cudaMemcpyAsync(host, st, sizeof(TrpoState), cudaMemcpyDeviceToHost, ctx->stream));
-    if (stats) RL_CUDA(ctx, cudaEventRecord(ev1, ctx->stream));
-    RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    if (stats) {
-        stats->entropy = host->entropy; stats->step_size = host->step_size; stats->loss_initial = host->loss0;
-        stats->loss_final = host->loss_final; stats->constraint_val_final = host->kl_final;
-        stats->step_scale = host->step_scale; stats->num_backtracks = host->num_backtracks;
-        stats->cg_iterations = host->cg_iters; stats->num_steps = (uint64_t)host->N;
-        cudaEventElapsedTime(&stats->policy_update_ms, ev0, ev1);
-    }
-    const rl_status trpo_status = (rl_status)host->status;  // (x_error_check reuses the pinned scratch)
-    RL_TRY(x_error_check(ctx, "TRPO update"));
-    return trpo_status;
-}
-
-// Recurrent module: plan with one block of RL_SEQ_BLOCK lanes per partial row, scratch for hbuf / dzbuf / logp0.
-struct SeqScratch {
-    float *logp0, *hbuf, *dzbuf;
-    char *extra;
-};
-
-rl_status make_seq_plan(rl_ctx *ctx, const rl_grunet_view &net, uint64_t T, uint64_t E, size_t extra_bytes, PassPlan *plan,
-                        SeqScratch *sc) {
-    const int P = (int)net.n_params;
-    plan->P = P;
-    plan->W = P + NSCALAR;
-    plan->grid = (int)rl_div_up(E, RL_SEQ_BLOCK);
-    const size_t rows = (size_t)plan->grid * plan->W * sizeof(double), sums = ((size_t)plan->W * sizeof(double) + 255) / 256 * 256;
-    const size_t TE = (size_t)T * E;
-    const size_t lp = (TE * net.out_dim * sizeof(float) + 255) / 256 * 256, hb = (TE * net.hidden * sizeof(float) + 255) / 256 * 256;
-    extra_bytes = (extra_bytes + 255) / 256 * 256;
-    char *buf;
-    RL_TRY(rl_ctx_scratch(ctx, ((rows + 255) / 256 * 256) + sums + extra_bytes + 2 * lp + hb + 256, (void **)&buf));
-    plan->partials = (double *)buf;
-    plan->sums = (double *)(buf + (rows + 255) / 256 * 256);
-    char *q = (char *)plan->sums + sums;
-    sc->extra = q;
-    sc->logp0 = (float *)(q + extra_bytes);
-    sc->dzbuf = (float *)(q + extra_bytes + lp);
-    sc->hbuf = (float *)(q + extra_bytes + 2 * lp);
-    return RL_OK;
-}
-
 // RL_SEQ_FORCE_BIG=1 sends every size through the GEMM formulation (tests: K10 against K9 on the same small module)
 bool seq_force_big() {
     static int v = -1;
@@ -1641,29 +1519,353 @@ bool seq_force_big() {
     return v == 1;
 }
 
-rl_status seq_pass(rl_ctx *ctx, const PassPlan &plan, int mode, const rl_seq_pass_args &a) {
-    if (!rl_seq_pass_supports(a.F, a.H, a.A) || seq_force_big()) {
-        // K10 (gru_big.cu): tiled GEMMs over the lanes of a step; one partial row
-        RL_TRY(rl_seq_big_pass_launch(ctx, mode, a));
-        RL_TRY(reduce_over_group(ctx, plan, 1, a.skip_flag));
-        return RL_OK;
-    }
-    RL_TRY(rl_seq_pass_launch(ctx, mode, a, plan.grid));
-    RL_TRY(reduce_over_group(ctx, plan, plan.grid, a.skip_flag));
+// The shapes the recurrent passes are built for, on batches of F features (out_dim_expected > 0: that many outputs).
+rl_status seq_check(rl_ctx *ctx, const rl_grunet_view &net, int F, int out_dim_expected, const char *what) {
+    if (net.in_dim != F || (out_dim_expected > 0 && net.out_dim != out_dim_expected) ||
+        !(rl_seq_pass_supports(net.in_dim, net.hidden, net.out_dim) || rl_seq_big_supports(net.in_dim, net.hidden, net.out_dim)))
+        return rl_fail(ctx, RL_ERR_UNSUPPORTED, "%s: recurrent passes are built for hidden <= 128, features <= 64, outputs <= 32 "
+                       "(got %d -> %d -> %d on %d features)", what, net.in_dim, net.hidden, net.out_dim, F);
     return RL_OK;
 }
 
-rl_status seq_check(rl_ctx *ctx, rl_traj *traj, const rl_grunet_view &net, int out_dim_expected, const char *what) {
-    RL_REQUIRE(ctx, net.ctx == ctx, "recurrent update: module belongs to another context");
-    if ((int)traj->F != net.in_dim || (out_dim_expected > 0 && net.out_dim != out_dim_expected) ||
-        !(rl_seq_pass_supports(net.in_dim, net.hidden, net.out_dim) || rl_seq_big_supports(net.in_dim, net.hidden, net.out_dim)))
-        return rl_fail(ctx, RL_ERR_UNSUPPORTED, "%s: recurrent passes are built for hidden <= 128, features <= 64, outputs <= 32 "
-                       "(got %d -> %d -> %d on %d features)", what, net.in_dim, net.hidden, net.out_dim, (int)traj->F);
+// ------------------------------------------------------------------------------------------------
+// The module under update: an Mlp or a recurrent module, planned over one batch.  The algorithm drivers below see only
+// its passes and its Adam step; which kind of module it is matters in init, pass and adam_step alone.
+// ------------------------------------------------------------------------------------------------
+// The batch of a trajectory: its planes over the time slots in use.
+PassArgs traj_args(const rl_traj *traj) {
+    PassArgs a{};
+    a.obs = traj->obs; a.action = traj->action; a.succ = traj->succ;
+    a.T = traj->used_T ? traj->used_T : traj->T;
+    a.E = traj->E;
+    return a;
+}
+
+struct UpdateNet {
+    rl_ctx *ctx = nullptr;
+    int P = 0;
+    float *theta = nullptr;
+    PassPlan plan{};
+    char *extra = nullptr;  // the caller's extra_bytes of scratch
+    PassArgs args{};        // batch, parameters and the update's inputs (adv, target, logp0, clip); vec and skip_flag per pass
+    bool recurrent = false;
+    PassNet pn{};            // an Mlp: which pass kernels
+    rl_seq_pass_args seq{};  // a recurrent module: its shape and the scratch of back-propagation through time
+
+    // An Mlp over `batch`; `logp0` reserves the behaviour log-probabilities of the batch after the caller's scratch.
+    rl_status init(rl_ctx *c, rl_mlp *m, const PassNet &net, const PassArgs &batch, size_t extra_bytes, bool logp0) {
+        ctx = c; P = (int)m->n_params; theta = m->params; pn = net;
+        args = batch;
+        args.theta = theta;
+        const uint64_t TE = batch.T * batch.E;
+        RL_TRY(make_plan(ctx, P, TE, &plan, extra_bytes + (logp0 ? TE * (size_t)pn.sh.A * sizeof(float) : 0), (void **)&extra));
+        if (logp0) args.logp0 = (float *)(extra + extra_bytes);
+        return RL_OK;
+    }
+    // A recurrent module over `batch`: one block of RL_SEQ_BLOCK lanes per partial row; after the caller's scratch, the
+    // log-probabilities, the output cotangents and the hidden states of the batch.
+    rl_status init(rl_ctx *c, const rl_grunet_view &net, const PassArgs &batch, size_t extra_bytes) {
+        ctx = c; P = (int)net.n_params; theta = net.params; recurrent = true;
+        plan.P = P;
+        plan.W = P + NSCALAR;
+        plan.grid = (int)rl_div_up(batch.E, RL_SEQ_BLOCK);
+        const size_t rows = (size_t)plan.grid * plan.W * sizeof(double), sums = ((size_t)plan.W * sizeof(double) + 255) / 256 * 256;
+        const size_t TE = (size_t)batch.T * batch.E;
+        const size_t lp = (TE * net.out_dim * sizeof(float) + 255) / 256 * 256, hb = (TE * net.hidden * sizeof(float) + 255) / 256 * 256;
+        extra_bytes = (extra_bytes + 255) / 256 * 256;
+        char *buf;
+        RL_TRY(rl_ctx_scratch(ctx, ((rows + 255) / 256 * 256) + sums + extra_bytes + 2 * lp + hb + 256, (void **)&buf));
+        plan.partials = (double *)buf;
+        plan.sums = (double *)(buf + (rows + 255) / 256 * 256);
+        extra = (char *)plan.sums + sums;
+        args = batch;
+        args.theta = theta;
+        args.logp0 = (float *)(extra + extra_bytes);
+        seq.F = net.in_dim; seq.H = net.hidden; seq.A = net.out_dim; seq.act = net.act;
+        seq.dzbuf = (float *)(extra + extra_bytes + lp);
+        seq.hbuf = (float *)(extra + extra_bytes + 2 * lp);
+        seq.partials = plan.partials;
+        return RL_OK;
+    }
+
+    // One full-batch pass in `mode`; leaves the all-reduced f64 sums in plan.sums.  A recurrent module's pass runs
+    // gru_pass_kernel (K9), or K10's tiled GEMMs above its sizes.
+    rl_status pass(int mode, const float *vec = nullptr, const int *skip_flag = nullptr) const {
+        PassArgs a = args;
+        a.vec = vec;
+        a.skip_flag = skip_flag;
+        if (!recurrent) return launch_pass_rt(ctx, plan, a, mode, pn);
+        rl_seq_pass_args s = seq;
+        s.obs = a.obs; s.action = a.action; s.succ = a.succ; s.T = a.T; s.E = a.E; s.theta = a.theta; s.vec = a.vec;
+        s.adv = a.adv; s.target = a.target; s.logp0 = a.logp0; s.skip_flag = a.skip_flag; s.clip_lo = a.clip_lo;
+        s.clip_hi = a.clip_hi;
+        if (!rl_seq_pass_supports(s.F, s.H, s.A) || seq_force_big()) {
+            // K10 (gru_big.cu): tiled GEMMs over the lanes of a step; one partial row
+            RL_TRY(rl_seq_big_pass_launch(ctx, mode, s));
+            return reduce_over_group(ctx, plan, 1, s.skip_flag);
+        }
+        RL_TRY(rl_seq_pass_launch(ctx, mode, s, plan.grid));
+        return reduce_over_group(ctx, plan, plan.grid, s.skip_flag);
+    }
+
+    // One optimizer step on a pass in `mode`, its mean loss to *loss_out (n_backward_steps: zero_grad, backward, step;
+    // torch/agents/mod.rs:50-55, coptimizer.rs:13-27).  An Mlp's pass leaves its rows to a kernel that reduces them (over
+    // the peer mailboxes of the data-parallel group when they are mapped) and takes the step; a recurrent module's pass
+    // is reduced as every pass is, then adam_step_kernel steps.
+    rl_status adam_step(int mode, rl_adam *adam, const AdamArgs &ac, double *loss_out) const {
+        if (recurrent) {
+            RL_TRY(pass(mode));
+            adam->step += 1;
+            RL_LAUNCH(ctx, adam_step_kernel, 1, VEC_THREADS, 0, plan.sums, P, theta, adam->m, adam->v, ac, adam->step, loss_out);
+            return RL_OK;
+        }
+        adam->step += 1;
+        int rows = plan.grid;
+        if (ctx->world > 1 && ctx->x_ok && rl_div_up(plan.W, 32) <= RL_X_BLOCKS) {
+            RL_TRY(launch_pass_rt(ctx, plan, args, mode, pn, false, &rows));
+            ctx->x_seq += 1;
+            RL_LAUNCH(ctx, reduce_rows_x_kernel<true>, rl_div_up(plan.W, 32), 256, 0, plan.partials, rows, plan.W, plan.P, plan.sums,
+                      ctx->x, ctx->x_seq, (const int *)nullptr, (XAdam{theta, adam->m, adam->v, ac, adam->step, loss_out, plan.P}));
+        } else if (ctx->world > 1) {
+            RL_TRY(launch_pass_rt(ctx, plan, args, mode, pn));
+            RL_LAUNCH(ctx, adam_step_kernel, 1, VEC_THREADS, 0, plan.sums, plan.P, theta, adam->m, adam->v, ac, adam->step, loss_out);
+        } else {
+            RL_TRY(launch_pass_rt(ctx, plan, args, mode, pn, false, &rows));
+            RL_LAUNCH(ctx, reduce_rows_adam_kernel, rl_div_up(plan.W, 32), 256, 0, plan.partials, rows, plan.W, plan.P, plan.sums,
+                      theta, adam->m, adam->v, ac, adam->step, loss_out);
+        }
+        return RL_OK;
+    }
+};
+
+// ------------------------------------------------------------------------------------------------
+// The algorithm drivers and what they share
+// ------------------------------------------------------------------------------------------------
+// Device time of an update when the caller asked for statistics, on the context's two timing events (created on first
+// use, freed by rl_ctx_destroy).
+struct UpdateTimer {
+    rl_ctx *ctx;
+    bool on;
+    rl_status start() {
+        if (!on) return RL_OK;
+        for (int k = 0; k < 2; ++k)
+            if (!ctx->upd_ev[k]) RL_CUDA(ctx, cudaEventCreate(&ctx->upd_ev[k]));
+        RL_CUDA(ctx, cudaEventRecord(ctx->upd_ev[0], ctx->stream));
+        return RL_OK;
+    }
+    rl_status stop() {
+        if (on) RL_CUDA(ctx, cudaEventRecord(ctx->upd_ev[1], ctx->stream));
+        return RL_OK;
+    }
+    void elapsed(float *ms) const { cudaEventElapsedTime(ms, ctx->upd_ev[0], ctx->upd_ev[1]); }  // after a synchronisation
+};
+
+AdamArgs adam_args(const rl_adam *a) {
+    return AdamArgs{a->cfg.learning_rate, a->cfg.beta1, a->cfg.beta2, a->cfg.weight_decay, a->cfg.eps};
+}
+
+// An optimizer for the n_params parameters of `owner` (the module's handle), moments at zero.
+rl_status adam_create(rl_ctx *ctx, const void *owner, uint64_t n_params, const rl_adam_cfg *cfg, rl_adam **out, const char *what) {
+    RL_CUDA(ctx, cudaSetDevice(ctx->device));
+    rl_adam *a = new (std::nothrow) rl_adam();
+    if (!a) return rl_fail(ctx, RL_ERR_OOM, "%s: host allocation failed", what);
+    a->owner = owner;
+    a->ctx = ctx;
+    a->cfg = *cfg;
+    cudaError_t e = cudaMalloc((void **)&a->m, n_params * sizeof(float));
+    if (e == cudaSuccess) e = cudaMalloc((void **)&a->v, n_params * sizeof(float));
+    if (e != cudaSuccess) {
+        rl_adam_destroy(a);
+        return rl_fail(ctx, RL_ERR_OOM, "%s: %s", what, cudaGetErrorString(e));
+    }
+    cudaMemsetAsync(a->m, 0, n_params * sizeof(float), ctx->stream);
+    cudaMemsetAsync(a->v, 0, n_params * sizeof(float), ctx->stream);
+    *out = a;
     return RL_OK;
+}
+
+// The checks of every Adam update: the optimizer was built for `module`, and the step count is in range.
+rl_status adam_check(rl_ctx *ctx, const rl_adam *adam, const void *module, int n_steps, const char *what) {
+    if (adam->owner != module) return rl_fail(ctx, RL_ERR_INVALID_ARG, "%s: optimizer belongs to another module", what);
+    if (n_steps < 0 || n_steps > 100000) return rl_fail(ctx, RL_ERR_INVALID_ARG, "%s: optimizer steps out of range", what);
+    return RL_OK;
+}
+
+// loss_first / loss_last of the n_steps losses (host), the sample count, the step count and the device time.
+template <class Stats>
+void fill_opt_stats(Stats *st, const double *losses, int n_steps, uint64_t num_steps, const UpdateTimer &timer) {
+    st->loss_first = n_steps > 0 ? losses[0] : 0.0;
+    st->loss_last = n_steps > 0 ? losses[n_steps - 1] : 0.0;
+    st->num_steps = num_steps;
+    st->opt_steps = (uint64_t)n_steps;
+    timer.elapsed(&st->update_ms);
+}
+
+// One pass of `u` in `mode`, its sums read back to `host` (P parameter sums, then the SC_* scalars); with `loss` /
+// `grad_host`, the mean loss and the flat gradient of the mean (sums over the pass's sample count).
+rl_status probe_pass(const UpdateNet &u, int mode, const float *vec, std::vector<double> &host, double *loss, float *grad_host) {
+    rl_ctx *ctx = u.ctx;
+    RL_TRY(u.pass(mode, vec));
+    host.resize((size_t)u.plan.W);
+    RL_CUDA(ctx, cudaMemcpyAsync(host.data(), u.plan.sums, (size_t)u.plan.W * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    const double N = host[u.P + SC_COUNT];
+    if (loss) *loss = host[u.P + SC_LOSS] / N;
+    if (grad_host)
+        for (int i = 0; i < u.P; ++i) grad_host[i] = (float)(host[i] / N);
+    return RL_OK;
+}
+
+// A P-vector of f32 in scratch, 256-byte aligned
+size_t vec_bytes(int P) { return ((size_t)P * sizeof(float) + 255) / 256 * 256; }
+size_t trpo_vector_bytes(int P) { return 256 + 6 * vec_bytes(P); }  // TrpoState + theta0, g, x, r, p, descent
+
+// Trpo::update (trpo.rs:97-164) on the policy `u` (inputs: adv); u.extra holds trpo_vector_bytes.
+rl_status trpo_update(const UpdateNet &u, const rl_trpo_cfg *cfg, rl_trpo_stats *stats, const char *what) {
+    rl_ctx *ctx = u.ctx;
+    const int P = u.P;
+    const size_t vb = vec_bytes(P);
+    const double *sums = u.plan.sums;
+    float *theta = u.theta;
+    char *ex = u.extra;
+    TrpoState *st = (TrpoState *)ex;
+    float *theta0 = (float *)(ex + 256), *g = (float *)(ex + 256 + vb), *x = (float *)(ex + 256 + 2 * vb);
+    float *r = (float *)(ex + 256 + 3 * vb), *p = (float *)(ex + 256 + 4 * vb);
+    float *descent = (float *)(ex + 256 + 5 * vb);
+    UpdateTimer timer{ctx, stats != nullptr};
+    RL_TRY(timer.start());
+    const float reg = (float)cfg->hpv_reg_coeff;
+    // behaviour-policy statistics (no_grad block, trpo.rs:112-122)
+    RL_TRY(u.pass(PASS_STATS));
+    RL_LAUNCH(ctx, trpo_begin_kernel, 1, 32, 0, st, sums, P);
+    // loss gradient at theta0 (conjugate_gradient.rs:121-143)
+    RL_TRY(u.pass(PASS_GRAD));
+    RL_LAUNCH(ctx, trpo_cg_init_kernel, 1, VEC_THREADS, 0, st, sums, P, g, x, r, p, theta, theta0);
+    // conjugate gradient on the Fisher matrix (conjugate_gradient.rs:371-403)
+    for (uint64_t it = 0; it < cfg->cg_iterations; ++it) {
+        RL_TRY(u.pass(PASS_FVP, p, &st->cg_done));
+        RL_LAUNCH(ctx, trpo_cg_step_kernel, 1, VEC_THREADS, 0, st, sums, P, x, r, p, reg, 1e-10);
+    }
+    RL_LAUNCH(ctx, trpo_nan_to_num_kernel, 1, VEC_THREADS, 0, st, x, P);
+    RL_TRY(u.pass(PASS_FVP, x));
+    RL_LAUNCH(ctx, trpo_step_size_kernel, 1, VEC_THREADS, 0, st, sums, P, x, descent, reg, cfg->max_policy_step_kl);
+    // backtracking line search (conjugate_gradient.rs:183-254)
+    for (uint64_t i = 0; i < cfg->max_backtracks; ++i) {
+        const double ratio = std::pow(cfg->backtrack_ratio, (double)i);
+        RL_LAUNCH(ctx, trpo_ls_candidate_kernel, 1, VEC_THREADS, 0, st, theta, theta0, descent, (float)ratio, P);
+        RL_TRY(u.pass(PASS_EVAL, nullptr, &st->accepted));
+        RL_LAUNCH(ctx, trpo_ls_check_kernel, 1, 32, 0, st, sums, P, cfg->max_policy_step_kl, (int)i, ratio);
+    }
+    RL_LAUNCH(ctx, trpo_ls_finish_kernel, 1, VEC_THREADS, 0, st, theta, theta0, P, cfg->max_policy_step_kl,
+              cfg->accept_violation);
+    TrpoState *host;
+    RL_TRY(rl_ctx_pinned(ctx, sizeof(TrpoState), (void **)&host));
+    RL_CUDA(ctx, cudaMemcpyAsync(host, st, sizeof(TrpoState), cudaMemcpyDeviceToHost, ctx->stream));
+    RL_TRY(timer.stop());
+    RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    if (stats) {
+        stats->entropy = host->entropy; stats->step_size = host->step_size; stats->loss_initial = host->loss0;
+        stats->loss_final = host->loss_final; stats->constraint_val_final = host->kl_final;
+        stats->step_scale = host->step_scale; stats->num_backtracks = host->num_backtracks;
+        stats->cg_iterations = host->cg_iters; stats->num_steps = (uint64_t)host->N;
+        timer.elapsed(&stats->policy_update_ms);
+    }
+    const rl_status trpo_status = (rl_status)host->status;  // (x_error_check reuses the pinned scratch)
+    RL_TRY(x_error_check(ctx, what));
+    return trpo_status;
+}
+
+// Loss, KL and entropy of the policy `u` (inputs: adv) at its parameters, the flat gradient, and with a vector its
+// Fisher-vector product plus hpv_reg_coeff times the vector; u.extra holds vec_bytes.
+rl_status trpo_probe(const UpdateNet &u, const float *vec_host, double hpv_reg_coeff, double *loss, double *kl, double *entropy,
+                     float *grad_host, float *fvp_host) {
+    rl_ctx *ctx = u.ctx;
+    const int P = u.P;
+    std::vector<double> host;
+    RL_TRY(probe_pass(u, PASS_STATS, nullptr, host, nullptr, nullptr));
+    const double N = host[P + SC_COUNT];
+    if (entropy) *entropy = host[P + SC_ENTROPY] / N;
+    RL_TRY(probe_pass(u, PASS_GRAD, nullptr, host, loss, grad_host));
+    if (kl) *kl = host[P + SC_KL] / N;
+    if (vec_host && fvp_host) {
+        float *vec = (float *)u.extra;
+        RL_CUDA(ctx, cudaMemcpyAsync(vec, vec_host, (size_t)P * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+        RL_TRY(probe_pass(u, PASS_FVP, vec, host, nullptr, nullptr));
+        for (int i = 0; i < P; ++i) fvp_host[i] = (float)(host[i] / N) + vec_host[i] * (float)hpv_reg_coeff;
+    }
+    return RL_OK;
+}
+
+// ValuesOpt::update (opt.rs:100-127): n_steps Adam steps of the state-value module `u` (inputs: target) on the mean
+// squared error; u.extra holds n_steps + 1 losses.
+rl_status value_update(const UpdateNet &u, rl_adam *adam, int n_steps, rl_opt_stats *stats, const char *what) {
+    rl_ctx *ctx = u.ctx;
+    double *losses = (double *)u.extra;
+    UpdateTimer timer{ctx, stats != nullptr};
+    RL_TRY(timer.start());
+    const AdamArgs ac = adam_args(adam);
+    for (int s = 0; s < n_steps; ++s) RL_TRY(u.adam_step(PASS_VALUE, adam, ac, losses + s));
+    if (stats) {
+        RL_TRY(timer.stop());
+        double *host;
+        RL_TRY(rl_ctx_pinned(ctx, (size_t)(n_steps + 4) * sizeof(double), (void **)&host));
+        if (n_steps > 0) RL_CUDA(ctx, cudaMemcpyAsync(host, losses, (size_t)n_steps * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        RL_CUDA(ctx, cudaMemcpyAsync(host + n_steps, u.plan.sums + u.P + SC_COUNT, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        fill_opt_stats(stats, host, n_steps, n_steps > 0 ? (uint64_t)host[n_steps] : 0, timer);
+    }
+    return x_error_check(ctx, what);
+}
+
+// The losses of n_steps policy steps and [sum of entropies, N], 256-byte aligned
+size_t policy_loss_bytes(int n_steps) { return ((size_t)(n_steps + 2) * sizeof(double) + 255) / 256 * 256; }
+
+// Ppo::update (ppo.rs:97-147) with `ppo`, Reinforce::update (reinforce.rs:64-89) without, on the policy `u` (inputs: adv,
+// logp0); u.extra holds policy_loss_bytes.
+rl_status policy_adam_update(UpdateNet &u, rl_adam *adam, int n_steps, double clip_distance, bool ppo, rl_policy_opt_stats *stats,
+                             const char *what) {
+    rl_ctx *ctx = u.ctx;
+    const double *sums = u.plan.sums;
+    const int P = u.P;
+    double *losses = (double *)u.extra;
+    UpdateTimer timer{ctx, stats != nullptr};
+    RL_TRY(timer.start());
+    u.args.clip_lo = (float)(1.0 - clip_distance); u.args.clip_hi = (float)(1.0 + clip_distance);
+    const AdamArgs ac = adam_args(adam);
+    double *entropy_sum = losses + n_steps;  // [sum of entropies, N]
+    if (ppo) {
+        // initial log-probs and entropy under no_grad (ppo.rs:108-119)
+        RL_TRY(u.pass(PASS_STATS));
+        RL_CUDA(ctx, cudaMemcpyAsync(entropy_sum, sums + P + SC_ENTROPY, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+        RL_CUDA(ctx, cudaMemcpyAsync(entropy_sum + 1, sums + P + SC_COUNT, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+        for (int s = 0; s < n_steps; ++s) RL_TRY(u.adam_step(PASS_PPO, adam, ac, losses + s));
+    } else {
+        for (int s = 0; s < n_steps; ++s) {
+            RL_TRY(u.adam_step(PASS_REINFORCE, adam, ac, losses + s));
+            if (s == 0) {  // entropies.get_or_insert_with: the distribution of the first loss evaluation (reinforce.rs:76)
+                RL_CUDA(ctx, cudaMemcpyAsync(entropy_sum, sums + P + SC_ENTROPY, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+                RL_CUDA(ctx, cudaMemcpyAsync(entropy_sum + 1, sums + P + SC_COUNT, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+            }
+        }
+    }
+    if (stats) {
+        RL_TRY(timer.stop());
+        double *host;
+        RL_TRY(rl_ctx_pinned(ctx, (size_t)(n_steps + 4) * sizeof(double), (void **)&host));
+        RL_CUDA(ctx, cudaMemcpyAsync(host, losses, (size_t)(n_steps + 2) * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        const bool have = ppo || n_steps > 0;
+        fill_opt_stats(stats, host, n_steps, have ? (uint64_t)host[n_steps + 1] : 0, timer);
+        stats->entropy = have && host[n_steps + 1] > 0 ? host[n_steps] / host[n_steps + 1] : 0.0;
+    }
+    return x_error_check(ctx, what);
 }
 
 }  // namespace
 
+// ------------------------------------------------------------------------------------------------
+// C entry points: each checks its arguments, builds the UpdateNet of its module and runs the driver
+// ------------------------------------------------------------------------------------------------
 extern "C" {
 
 void rl_trpo_cfg_default(rl_trpo_cfg *c) {
@@ -1677,94 +1879,27 @@ void rl_adam_cfg_default(rl_adam_cfg *c) {
     c->learning_rate = 1e-3; c->beta1 = 0.9; c->beta2 = 0.999; c->weight_decay = 0.0; c->eps = 1e-8;
 }
 
-rl_status rl_trpo_update(rl_traj *traj, const float *adv_dev, rl_mlp *policy, const rl_trpo_cfg *cfg,
-                         rl_trpo_stats *stats) {
-    if (!traj || !adv_dev || !policy || !cfg)
-        return rl_fail(traj ? traj->ctx : nullptr, RL_ERR_INVALID_ARG, "rl_trpo_update: NULL argument");
-    rl_ctx *ctx = traj->ctx;
-    PassNet pn;
-    RL_TRY(pass_net_for(ctx, policy, (int)traj->F, "rl_trpo_update", &pn));
-    const int P = (int)policy->n_params;
-    const uint64_t T = traj->used_T ? traj->used_T : traj->T, TE = T * traj->E;
-    PassPlan plan;
-    const size_t extra = trpo_vector_bytes(P) + TE * (size_t)pn.sh.A * sizeof(float);
-    char *ex;
-    RL_TRY(make_plan(ctx, P, TE, &plan, extra, (void **)&ex));
-    float *logp0 = (float *)(ex + trpo_vector_bytes(P));
-    PassArgs base{};
-    base.obs = traj->obs; base.action = traj->action; base.succ = traj->succ; base.T = T; base.E = traj->E;
-    base.theta = policy->params; base.adv = adv_dev; base.logp0 = logp0;
-    PassFn pass = [&](int mode, const float *vec, const int *skip_flag) -> rl_status {
-        PassArgs pa = base;
-        pa.vec = vec;
-        pa.skip_flag = skip_flag;
-        return launch_pass_rt(ctx, plan, pa, mode == PASS_STATS || mode == PASS_GRAD || mode == PASS_FVP ? mode : PASS_EVAL, pn);
-    };
-    return trpo_update_generic(ctx, P, policy->params, plan, ex, pass, cfg, stats);
+void rl_ppo_cfg_default(rl_ppo_cfg *c) {
+    // ppo.rs:33-41
+    c->opt_steps_per_update = 10;
+    c->clip_distance = 0.2;
 }
 
-rl_status rl_trpo_probe(rl_traj *traj, const float *adv_dev, rl_mlp *policy, const float *vec_host, double hpv_reg_coeff,
-                        double *loss, double *kl, double *entropy, float *grad_host, float *fvp_host) {
-    if (!traj || !adv_dev || !policy) return rl_fail(traj ? traj->ctx : nullptr, RL_ERR_INVALID_ARG, "rl_trpo_probe: NULL argument");
-    rl_ctx *ctx = traj->ctx;
-    PassNet pn;
-    RL_TRY(pass_net_for(ctx, policy, (int)traj->F, "rl_trpo_probe", &pn));
-    const int P = (int)policy->n_params;
-    const uint64_t T = traj->used_T ? traj->used_T : traj->T, TE = T * traj->E;
-    PassPlan plan;
-    const size_t vec_bytes = ((size_t)P * sizeof(float) + 255) / 256 * 256;
-    char *ex;
-    RL_TRY(make_plan(ctx, P, TE, &plan, vec_bytes + TE * (size_t)pn.sh.A * sizeof(float), (void **)&ex));
-    float *vec = (float *)ex, *logp0 = (float *)(ex + vec_bytes);
-    std::vector<double> host((size_t)plan.W);
-    PassArgs pa{};
-    pa.obs = traj->obs; pa.action = traj->action; pa.succ = traj->succ; pa.T = T; pa.E = traj->E;
-    pa.theta = policy->params; pa.adv = adv_dev; pa.logp0 = logp0;
-    auto fetch = [&]() -> rl_status {
-        RL_CUDA(ctx, cudaMemcpyAsync(host.data(), plan.sums, (size_t)plan.W * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        return RL_OK;
-    };
-    RL_TRY(launch_pass_rt(ctx, plan, pa, PASS_STATS, pn));
-    RL_TRY(fetch());
-    const double N = host[P + SC_COUNT];
-    if (entropy) *entropy = host[P + SC_ENTROPY] / N;
-    RL_TRY(launch_pass_rt(ctx, plan, pa, PASS_GRAD, pn));
-    RL_TRY(fetch());
-    if (loss) *loss = host[P + SC_LOSS] / N;
-    if (kl) *kl = host[P + SC_KL] / N;
-    if (grad_host)
-        for (int i = 0; i < P; ++i) grad_host[i] = (float)(host[i] / N);
-    if (vec_host && fvp_host) {
-        RL_CUDA(ctx, cudaMemcpyAsync(vec, vec_host, (size_t)P * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-        pa.vec = vec;
-        RL_TRY(launch_pass_rt(ctx, plan, pa, PASS_FVP, pn));
-        RL_TRY(fetch());
-        for (int i = 0; i < P; ++i) fvp_host[i] = (float)(host[i] / N) + vec_host[i] * (float)hpv_reg_coeff;
-    }
+rl_status rl_pass_kernel_select(int32_t kernel) {
+    if (kernel != RL_PASS_KERNEL_FFMA && kernel != RL_PASS_KERNEL_TCGEN05) return RL_ERR_INVALID_ARG;
+    g_pass_kernel = kernel;
     return RL_OK;
 }
 
 rl_status rl_adam_create(rl_mlp *mlp, const rl_adam_cfg *cfg, rl_adam **out) {
     if (!mlp || !cfg || !out) return rl_fail(mlp ? mlp->ctx : nullptr, RL_ERR_INVALID_ARG, "rl_adam_create: NULL argument");
-    rl_ctx *ctx = mlp->ctx;
-    RL_CUDA(ctx, cudaSetDevice(ctx->device));
-    rl_adam *a = new (std::nothrow) rl_adam();
-    if (!a) return rl_fail(ctx, RL_ERR_OOM, "rl_adam_create: host allocation failed");
-    a->mlp = mlp;
-    a->owner = mlp;
-    a->ctx = ctx;
-    a->cfg = *cfg;
-    cudaError_t e = cudaMalloc((void **)&a->m, mlp->n_params * sizeof(float));
-    if (e == cudaSuccess) e = cudaMalloc((void **)&a->v, mlp->n_params * sizeof(float));
-    if (e != cudaSuccess) {
-        rl_adam_destroy(a);
-        return rl_fail(ctx, RL_ERR_OOM, "rl_adam_create: %s", cudaGetErrorString(e));
-    }
-    cudaMemsetAsync(a->m, 0, mlp->n_params * sizeof(float), ctx->stream);
-    cudaMemsetAsync(a->v, 0, mlp->n_params * sizeof(float), ctx->stream);
-    *out = a;
-    return RL_OK;
+    return adam_create(mlp->ctx, mlp, mlp->n_params, cfg, out, "rl_adam_create");
+}
+
+rl_status rl_adam_create_seq(rl_grunet *net_h, const rl_adam_cfg *cfg, rl_adam **out) {
+    if (!net_h || !cfg || !out) return rl_fail(nullptr, RL_ERR_INVALID_ARG, "rl_adam_create_seq: NULL argument");
+    const rl_grunet_view net = rl_grunet_view_of(net_h);
+    return adam_create(net.ctx, net_h, net.n_params, cfg, out, "rl_adam_create_seq");
 }
 
 rl_status rl_adam_destroy(rl_adam *a) {
@@ -1776,48 +1911,87 @@ rl_status rl_adam_destroy(rl_adam *a) {
     return RL_OK;
 }
 
+rl_status rl_trpo_update(rl_traj *traj, const float *adv_dev, rl_mlp *policy, const rl_trpo_cfg *cfg,
+                         rl_trpo_stats *stats) {
+    if (!traj || !adv_dev || !policy || !cfg)
+        return rl_fail(traj ? traj->ctx : nullptr, RL_ERR_INVALID_ARG, "rl_trpo_update: NULL argument");
+    rl_ctx *ctx = traj->ctx;
+    PassNet pn;
+    RL_TRY(pass_net_for(ctx, policy, (int)traj->F, "rl_trpo_update", &pn));
+    UpdateNet u;
+    RL_TRY(u.init(ctx, policy, pn, traj_args(traj), trpo_vector_bytes((int)policy->n_params), true));
+    u.args.adv = adv_dev;
+    return trpo_update(u, cfg, stats, "rl_trpo_update");
+}
+
+rl_status rl_trpo_update_seq(rl_traj *traj, const float *adv_dev, rl_grunet *policy, const rl_trpo_cfg *cfg,
+                             rl_trpo_stats *stats) {
+    if (!traj || !adv_dev || !policy || !cfg)
+        return rl_fail(traj ? traj->ctx : nullptr, RL_ERR_INVALID_ARG, "rl_trpo_update_seq: NULL argument");
+    rl_ctx *ctx = traj->ctx;
+    const rl_grunet_view net = rl_grunet_view_of(policy);
+    RL_REQUIRE(ctx, net.ctx == ctx, "rl_trpo_update_seq: module belongs to another context");
+    RL_TRY(seq_check(ctx, net, (int)traj->F, 0, "rl_trpo_update_seq"));
+    UpdateNet u;
+    RL_TRY(u.init(ctx, net, traj_args(traj), trpo_vector_bytes((int)net.n_params)));
+    u.args.adv = adv_dev;
+    return trpo_update(u, cfg, stats, "rl_trpo_update_seq");
+}
+
+rl_status rl_trpo_probe(rl_traj *traj, const float *adv_dev, rl_mlp *policy, const float *vec_host, double hpv_reg_coeff,
+                        double *loss, double *kl, double *entropy, float *grad_host, float *fvp_host) {
+    if (!traj || !adv_dev || !policy) return rl_fail(traj ? traj->ctx : nullptr, RL_ERR_INVALID_ARG, "rl_trpo_probe: NULL argument");
+    rl_ctx *ctx = traj->ctx;
+    PassNet pn;
+    RL_TRY(pass_net_for(ctx, policy, (int)traj->F, "rl_trpo_probe", &pn));
+    UpdateNet u;
+    RL_TRY(u.init(ctx, policy, pn, traj_args(traj), vec_bytes((int)policy->n_params), true));
+    u.args.adv = adv_dev;
+    return trpo_probe(u, vec_host, hpv_reg_coeff, loss, kl, entropy, grad_host, fvp_host);
+}
+
+rl_status rl_trpo_probe_seq(rl_traj *traj, const float *adv_dev, rl_grunet *policy, const float *vec_host,
+                            double hpv_reg_coeff, double *loss, double *kl, double *entropy, float *grad_host,
+                            float *fvp_host) {
+    if (!traj || !adv_dev || !policy) return rl_fail(traj ? traj->ctx : nullptr, RL_ERR_INVALID_ARG, "rl_trpo_probe_seq: NULL argument");
+    rl_ctx *ctx = traj->ctx;
+    const rl_grunet_view net = rl_grunet_view_of(policy);
+    RL_REQUIRE(ctx, net.ctx == ctx, "rl_trpo_probe_seq: module belongs to another context");
+    RL_TRY(seq_check(ctx, net, (int)traj->F, 0, "rl_trpo_probe_seq"));
+    UpdateNet u;
+    RL_TRY(u.init(ctx, net, traj_args(traj), vec_bytes((int)net.n_params)));
+    u.args.adv = adv_dev;
+    return trpo_probe(u, vec_host, hpv_reg_coeff, loss, kl, entropy, grad_host, fvp_host);
+}
+
 rl_status rl_value_update(rl_traj *traj, const float *targets_dev, rl_mlp *value_fn, rl_adam *adam, int32_t n_steps,
                           rl_opt_stats *stats) {
     if (!traj || !targets_dev || !value_fn || !adam)
         return rl_fail(traj ? traj->ctx : nullptr, RL_ERR_INVALID_ARG, "rl_value_update: NULL argument");
     rl_ctx *ctx = traj->ctx;
-    RL_REQUIRE(ctx, adam->mlp == value_fn, "rl_value_update: optimizer belongs to another module");
-    RL_REQUIRE(ctx, n_steps >= 0 && n_steps <= 100000, "rl_value_update: n_steps out of range");
+    RL_TRY(adam_check(ctx, adam, value_fn, n_steps, "rl_value_update"));
     RL_REQUIRE(ctx, value_fn->out_dim == 1, "rl_value_update: a state-value module has one output");
     PassNet pn;
     RL_TRY(pass_net_for(ctx, value_fn, (int)traj->F, "rl_value_update", &pn));
-    const int P = (int)value_fn->n_params;
-    const uint64_t T = traj->used_T ? traj->used_T : traj->T, TE = T * traj->E;
-    PassPlan plan;
-    double *losses;
-    RL_TRY(make_plan(ctx, P, TE, &plan, (size_t)(n_steps + 1) * sizeof(double), (void **)&losses));
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    if (stats) {
-        RL_TRY(update_events(ctx, &ev0, &ev1));
-        RL_CUDA(ctx, cudaEventRecord(ev0, ctx->stream));
-    }
-    PassArgs pa{};
-    pa.obs = traj->obs; pa.action = traj->action; pa.succ = traj->succ; pa.T = T; pa.E = traj->E;
-    pa.theta = value_fn->params; pa.target = targets_dev;
-    AdamArgs ac{adam->cfg.learning_rate, adam->cfg.beta1, adam->cfg.beta2, adam->cfg.weight_decay, adam->cfg.eps};
-    for (int s = 0; s < n_steps; ++s) {
-        // n_backward_steps: loss -> zero_grad -> backward -> step (torch/agents/mod.rs:50-55, coptimizer.rs:13-27)
-        RL_TRY(pass_and_adam(ctx, plan, pa, PASS_VALUE, pn, value_fn, adam, ac, losses + s));
-    }
-    if (stats) {
-        RL_CUDA(ctx, cudaEventRecord(ev1, ctx->stream));
-        double *host;
-        RL_TRY(rl_ctx_pinned(ctx, (size_t)(n_steps + 4) * sizeof(double), (void **)&host));
-        if (n_steps > 0) RL_CUDA(ctx, cudaMemcpyAsync(host, losses, (size_t)n_steps * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        RL_CUDA(ctx, cudaMemcpyAsync(host + n_steps, plan.sums + P + SC_COUNT, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        stats->loss_first = n_steps > 0 ? host[0] : 0.0;
-        stats->loss_last = n_steps > 0 ? host[n_steps - 1] : 0.0;
-        stats->num_steps = n_steps > 0 ? (uint64_t)host[n_steps] : 0;
-        stats->opt_steps = (uint64_t)n_steps;
-        cudaEventElapsedTime(&stats->update_ms, ev0, ev1);
-    }
-    return x_error_check(ctx, "rl_value_update");
+    UpdateNet u;
+    RL_TRY(u.init(ctx, value_fn, pn, traj_args(traj), (size_t)(n_steps + 1) * sizeof(double), false));
+    u.args.target = targets_dev;
+    return value_update(u, adam, n_steps, stats, "rl_value_update");
+}
+
+rl_status rl_value_update_seq(rl_traj *traj, const float *targets_dev, rl_grunet *value_fn, rl_adam *adam, int32_t n_steps,
+                              rl_opt_stats *stats) {
+    if (!traj || !targets_dev || !value_fn || !adam)
+        return rl_fail(traj ? traj->ctx : nullptr, RL_ERR_INVALID_ARG, "rl_value_update_seq: NULL argument");
+    rl_ctx *ctx = traj->ctx;
+    const rl_grunet_view net = rl_grunet_view_of(value_fn);
+    RL_REQUIRE(ctx, net.ctx == ctx, "rl_value_update_seq: module belongs to another context");
+    RL_TRY(seq_check(ctx, net, (int)traj->F, 1, "rl_value_update_seq"));
+    RL_TRY(adam_check(ctx, adam, value_fn, n_steps, "rl_value_update_seq"));
+    UpdateNet u;
+    RL_TRY(u.init(ctx, net, traj_args(traj), (size_t)(n_steps + 1) * sizeof(double)));
+    u.args.target = targets_dev;
+    return value_update(u, adam, n_steps, stats, "rl_value_update_seq");
 }
 
 rl_status rl_value_probe(rl_traj *traj, const float *targets_dev, rl_mlp *value_fn, int32_t kernel, double *loss,
@@ -1828,279 +2002,58 @@ rl_status rl_value_probe(rl_traj *traj, const float *targets_dev, rl_mlp *value_
     PassNet pn;
     RL_TRY(pass_net_for(ctx, value_fn, (int)traj->F, "rl_value_probe", &pn));
     RL_REQUIRE(ctx, kernel == RL_PASS_KERNEL_FFMA || kernel == RL_PASS_KERNEL_TCGEN05, "rl_value_probe: unknown kernel");
-    const int P = (int)value_fn->n_params;
-    const uint64_t T = traj->used_T ? traj->used_T : traj->T, TE = T * traj->E;
-    PassPlan plan;
-    RL_TRY(make_plan(ctx, P, TE, &plan, 0, nullptr));
-    PassArgs pa{};
-    pa.obs = traj->obs; pa.action = traj->action; pa.succ = traj->succ; pa.T = T; pa.E = traj->E;
-    pa.theta = value_fn->params; pa.target = targets_dev;
-    const int selected = pass_kernel();
-    g_pass_kernel = kernel;
-    const rl_status launched = launch_pass_rt(ctx, plan, pa, PASS_VALUE, pn);
-    g_pass_kernel = selected;
-    RL_TRY(launched);
-    std::vector<double> host((size_t)plan.W);
-    RL_CUDA(ctx, cudaMemcpyAsync(host.data(), plan.sums, (size_t)plan.W * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    const double N = host[P + SC_COUNT];
-    if (loss) *loss = host[P + SC_LOSS] / N;
-    if (grad_host)
-        for (int i = 0; i < P; ++i) grad_host[i] = (float)(host[i] / N);
-    return RL_OK;
-}
-
-rl_status rl_pass_kernel_select(int32_t kernel) {
-    if (kernel != RL_PASS_KERNEL_FFMA && kernel != RL_PASS_KERNEL_TCGEN05) return RL_ERR_INVALID_ARG;
-    g_pass_kernel = kernel;
-    return RL_OK;
-}
-
-void rl_ppo_cfg_default(rl_ppo_cfg *c) {
-    // ppo.rs:33-41
-    c->opt_steps_per_update = 10;
-    c->clip_distance = 0.2;
-}
-
-// Ppo::update (ppo.rs:97-147) with opt_steps > 0 and a clip, Reinforce::update (reinforce.rs:64-89) with clip < 0.
-static rl_status policy_adam_update(rl_traj *traj, const float *adv_dev, rl_mlp *policy, rl_adam *adam, int n_steps,
-                                    double clip_distance, bool ppo, rl_policy_opt_stats *stats, const char *what) {
-    if (!traj || !adv_dev || !policy || !adam)
-        return rl_fail(traj ? traj->ctx : nullptr, RL_ERR_INVALID_ARG, "%s: NULL argument", what);
-    rl_ctx *ctx = traj->ctx;
-    RL_REQUIRE(ctx, adam->mlp == policy, "policy update: optimizer belongs to another module");
-    RL_REQUIRE(ctx, n_steps >= 0 && n_steps <= 100000, "policy update: opt_steps_per_update out of range");
-    PassNet pn;
-    RL_TRY(pass_net_for(ctx, policy, (int)traj->F, what, &pn));
-    const int P = (int)policy->n_params;
-    const uint64_t T = traj->used_T ? traj->used_T : traj->T, TE = T * traj->E;
-    PassPlan plan;
-    const size_t loss_bytes = ((size_t)(n_steps + 2) * sizeof(double) + 255) / 256 * 256;
-    char *ex;
-    RL_TRY(make_plan(ctx, P, TE, &plan, loss_bytes + TE * (size_t)pn.sh.A * sizeof(float), (void **)&ex));
-    double *losses = (double *)ex;
-    float *logp0 = (float *)(ex + loss_bytes);
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    if (stats) {
-        RL_TRY(update_events(ctx, &ev0, &ev1));
-        RL_CUDA(ctx, cudaEventRecord(ev0, ctx->stream));
-    }
-    PassArgs pa{};
-    pa.obs = traj->obs; pa.action = traj->action; pa.succ = traj->succ; pa.T = T; pa.E = traj->E;
-    pa.theta = policy->params; pa.adv = adv_dev; pa.logp0 = logp0;
-    pa.clip_lo = (float)(1.0 - clip_distance); pa.clip_hi = (float)(1.0 + clip_distance);
-    AdamArgs ac{adam->cfg.learning_rate, adam->cfg.beta1, adam->cfg.beta2, adam->cfg.weight_decay, adam->cfg.eps};
-    double *entropy_sum = losses + n_steps;  // [sum of entropies, N]
-    if (ppo) {
-        // initial log-probs and entropy under no_grad (ppo.rs:108-119)
-        RL_TRY(launch_pass_rt(ctx, plan, pa, PASS_STATS, pn));
-        RL_CUDA(ctx, cudaMemcpyAsync(entropy_sum, plan.sums + P + SC_ENTROPY, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
-        RL_CUDA(ctx, cudaMemcpyAsync(entropy_sum + 1, plan.sums + P + SC_COUNT, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
-        for (int s = 0; s < n_steps; ++s) RL_TRY(pass_and_adam(ctx, plan, pa, PASS_PPO, pn, policy, adam, ac, losses + s));
-    } else {
-        for (int s = 0; s < n_steps; ++s) {
-            RL_TRY(pass_and_adam(ctx, plan, pa, PASS_REINFORCE, pn, policy, adam, ac, losses + s));
-            if (s == 0) {  // entropies.get_or_insert_with: the distribution of the first loss evaluation (reinforce.rs:76)
-                RL_CUDA(ctx, cudaMemcpyAsync(entropy_sum, plan.sums + P + SC_ENTROPY, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
-                RL_CUDA(ctx, cudaMemcpyAsync(entropy_sum + 1, plan.sums + P + SC_COUNT, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
-            }
-        }
-    }
-    if (stats) {
-        RL_CUDA(ctx, cudaEventRecord(ev1, ctx->stream));
-        double *host;
-        RL_TRY(rl_ctx_pinned(ctx, (size_t)(n_steps + 4) * sizeof(double), (void **)&host));
-        RL_CUDA(ctx, cudaMemcpyAsync(host, losses, (size_t)(n_steps + 2) * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        const bool have = ppo || n_steps > 0;
-        stats->loss_first = n_steps > 0 ? host[0] : 0.0;
-        stats->loss_last = n_steps > 0 ? host[n_steps - 1] : 0.0;
-        stats->num_steps = have ? (uint64_t)host[n_steps + 1] : 0;
-        stats->entropy = have && host[n_steps + 1] > 0 ? host[n_steps] / host[n_steps + 1] : 0.0;
-        stats->opt_steps = (uint64_t)n_steps;
-        cudaEventElapsedTime(&stats->update_ms, ev0, ev1);
-    }
-    return x_error_check(ctx, "policy Adam update");
+    pn.kernel = kernel;
+    UpdateNet u;
+    RL_TRY(u.init(ctx, value_fn, pn, traj_args(traj), 0, false));
+    u.args.target = targets_dev;
+    std::vector<double> host;
+    return probe_pass(u, PASS_VALUE, nullptr, host, loss, grad_host);
 }
 
 rl_status rl_ppo_update(rl_traj *traj, const float *adv_dev, rl_mlp *policy, rl_adam *adam, const rl_ppo_cfg *cfg,
                         rl_policy_opt_stats *stats) {
-    if (!cfg) return rl_fail(traj ? traj->ctx : nullptr, RL_ERR_INVALID_ARG, "rl_ppo_update: NULL argument");
-    return policy_adam_update(traj, adv_dev, policy, adam, (int)cfg->opt_steps_per_update, cfg->clip_distance, true, stats,
-                              "rl_ppo_update");
+    if (!traj || !adv_dev || !policy || !adam || !cfg)
+        return rl_fail(traj ? traj->ctx : nullptr, RL_ERR_INVALID_ARG, "rl_ppo_update: NULL argument");
+    rl_ctx *ctx = traj->ctx;
+    const int n_steps = (int)cfg->opt_steps_per_update;
+    RL_TRY(adam_check(ctx, adam, policy, n_steps, "rl_ppo_update"));
+    PassNet pn;
+    RL_TRY(pass_net_for(ctx, policy, (int)traj->F, "rl_ppo_update", &pn));
+    UpdateNet u;
+    RL_TRY(u.init(ctx, policy, pn, traj_args(traj), policy_loss_bytes(n_steps), true));
+    u.args.adv = adv_dev;
+    return policy_adam_update(u, adam, n_steps, cfg->clip_distance, true, stats, "rl_ppo_update");
 }
 
 rl_status rl_reinforce_update(rl_traj *traj, const float *adv_dev, rl_mlp *policy, rl_adam *adam, rl_policy_opt_stats *stats) {
-    return policy_adam_update(traj, adv_dev, policy, adam, 1, 0.0, false, stats, "rl_reinforce_update");
-}
-
-
-// ------------------------------------------------------------------------------------------------
-// Recurrent modules (Chain<Gru, Linear>): the same updates with gru_pass_kernel as the full-batch pass
-// ------------------------------------------------------------------------------------------------
-static rl_seq_pass_args seq_base_args(rl_traj *traj, const rl_grunet_view &net, uint64_t T, const SeqScratch &sc,
-                                      const PassPlan &plan) {
-    rl_seq_pass_args a{};
-    a.obs = traj->obs; a.action = traj->action; a.succ = traj->succ; a.T = T; a.E = traj->E;
-    a.F = net.in_dim; a.H = net.hidden; a.A = net.out_dim; a.act = net.act;
-    a.theta = net.params; a.logp0 = sc.logp0; a.hbuf = sc.hbuf; a.dzbuf = sc.dzbuf; a.partials = plan.partials;
-    return a;
-}
-
-rl_status rl_trpo_update_seq(rl_traj *traj, const float *adv_dev, rl_grunet *policy, const rl_trpo_cfg *cfg,
-                             rl_trpo_stats *stats) {
-    if (!traj || !adv_dev || !policy || !cfg)
-        return rl_fail(traj ? traj->ctx : nullptr, RL_ERR_INVALID_ARG, "rl_trpo_update_seq: NULL argument");
+    if (!traj || !adv_dev || !policy || !adam)
+        return rl_fail(traj ? traj->ctx : nullptr, RL_ERR_INVALID_ARG, "rl_reinforce_update: NULL argument");
     rl_ctx *ctx = traj->ctx;
-    const rl_grunet_view net = rl_grunet_view_of(policy);
-    RL_TRY(seq_check(ctx, traj, net, 0, "rl_trpo_update_seq"));
-    const int P = (int)net.n_params;
-    const uint64_t T = traj->used_T ? traj->used_T : traj->T;
-    PassPlan plan;
-    SeqScratch sc;
-    RL_TRY(make_seq_plan(ctx, net, T, traj->E, trpo_vector_bytes(P), &plan, &sc));
-    rl_seq_pass_args base = seq_base_args(traj, net, T, sc, plan);
-    base.adv = adv_dev;
-    PassFn pass = [&](int mode, const float *vec, const int *skip_flag) -> rl_status {
-        rl_seq_pass_args a = base;
-        a.vec = vec;
-        a.skip_flag = skip_flag;
-        return seq_pass(ctx, plan, mode, a);
-    };
-    return trpo_update_generic(ctx, P, net.params, plan, sc.extra, pass, cfg, stats);
+    RL_TRY(adam_check(ctx, adam, policy, 1, "rl_reinforce_update"));
+    PassNet pn;
+    RL_TRY(pass_net_for(ctx, policy, (int)traj->F, "rl_reinforce_update", &pn));
+    UpdateNet u;
+    RL_TRY(u.init(ctx, policy, pn, traj_args(traj), policy_loss_bytes(1), true));
+    u.args.adv = adv_dev;
+    return policy_adam_update(u, adam, 1, 0.0, false, stats, "rl_reinforce_update");
 }
 
-rl_status rl_trpo_probe_seq(rl_traj *traj, const float *adv_dev, rl_grunet *policy, const float *vec_host,
-                            double hpv_reg_coeff, double *loss, double *kl, double *entropy, float *grad_host,
-                            float *fvp_host) {
-    if (!traj || !adv_dev || !policy) return rl_fail(traj ? traj->ctx : nullptr, RL_ERR_INVALID_ARG, "rl_trpo_probe_seq: NULL argument");
-    rl_ctx *ctx = traj->ctx;
-    const rl_grunet_view net = rl_grunet_view_of(policy);
-    RL_TRY(seq_check(ctx, traj, net, 0, "rl_trpo_probe_seq"));
-    const int P = (int)net.n_params;
-    const uint64_t T = traj->used_T ? traj->used_T : traj->T;
-    PassPlan plan;
-    SeqScratch sc;
-    const size_t vec_bytes = ((size_t)P * sizeof(float) + 255) / 256 * 256;
-    RL_TRY(make_seq_plan(ctx, net, T, traj->E, vec_bytes, &plan, &sc));
-    float *vec = (float *)sc.extra;
-    rl_seq_pass_args a = seq_base_args(traj, net, T, sc, plan);
-    a.adv = adv_dev;
-    std::vector<double> host((size_t)plan.W);
-    auto fetch = [&]() -> rl_status {
-        RL_CUDA(ctx, cudaMemcpyAsync(host.data(), plan.sums, (size_t)plan.W * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        return RL_OK;
-    };
-    RL_TRY(seq_pass(ctx, plan, PASS_STATS, a));
-    RL_TRY(fetch());
-    const double N = host[P + SC_COUNT];
-    if (entropy) *entropy = host[P + SC_ENTROPY] / N;
-    RL_TRY(seq_pass(ctx, plan, PASS_GRAD, a));
-    RL_TRY(fetch());
-    if (loss) *loss = host[P + SC_LOSS] / N;
-    if (kl) *kl = host[P + SC_KL] / N;
-    if (grad_host)
-        for (int i = 0; i < P; ++i) grad_host[i] = (float)(host[i] / N);
-    if (vec_host && fvp_host) {
-        RL_CUDA(ctx, cudaMemcpyAsync(vec, vec_host, (size_t)P * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-        a.vec = vec;
-        RL_TRY(seq_pass(ctx, plan, PASS_FVP, a));
-        RL_TRY(fetch());
-        for (int i = 0; i < P; ++i) fvp_host[i] = (float)(host[i] / N) + vec_host[i] * (float)hpv_reg_coeff;
-    }
-    return RL_OK;
-}
-
-rl_status rl_adam_create_seq(rl_grunet *net_h, const rl_adam_cfg *cfg, rl_adam **out) {
-    if (!net_h || !cfg || !out) return rl_fail(nullptr, RL_ERR_INVALID_ARG, "rl_adam_create_seq: NULL argument");
-    const rl_grunet_view net = rl_grunet_view_of(net_h);
-    rl_ctx *ctx = net.ctx;
-    RL_CUDA(ctx, cudaSetDevice(ctx->device));
-    rl_adam *a = new (std::nothrow) rl_adam();
-    if (!a) return rl_fail(ctx, RL_ERR_OOM, "rl_adam_create_seq: host allocation failed");
-    a->owner = net_h;
-    a->ctx = ctx;
-    a->cfg = *cfg;
-    cudaError_t e = cudaMalloc((void **)&a->m, net.n_params * sizeof(float));
-    if (e == cudaSuccess) e = cudaMalloc((void **)&a->v, net.n_params * sizeof(float));
-    if (e != cudaSuccess) {
-        rl_adam_destroy(a);
-        return rl_fail(ctx, RL_ERR_OOM, "rl_adam_create_seq: %s", cudaGetErrorString(e));
-    }
-    cudaMemsetAsync(a->m, 0, net.n_params * sizeof(float), ctx->stream);
-    cudaMemsetAsync(a->v, 0, net.n_params * sizeof(float), ctx->stream);
-    *out = a;
-    return RL_OK;
-}
-
-rl_status rl_value_update_seq(rl_traj *traj, const float *targets_dev, rl_grunet *value_fn, rl_adam *adam, int32_t n_steps,
-                              rl_opt_stats *stats) {
-    if (!traj || !targets_dev || !value_fn || !adam)
-        return rl_fail(traj ? traj->ctx : nullptr, RL_ERR_INVALID_ARG, "rl_value_update_seq: NULL argument");
-    rl_ctx *ctx = traj->ctx;
-    const rl_grunet_view net = rl_grunet_view_of(value_fn);
-    RL_TRY(seq_check(ctx, traj, net, 1, "rl_value_update_seq"));
-    RL_REQUIRE(ctx, adam->owner == (void *)value_fn, "rl_value_update_seq: optimizer belongs to another module");
-    RL_REQUIRE(ctx, n_steps >= 0 && n_steps <= 100000, "rl_value_update_seq: n_steps out of range");
-    const int P = (int)net.n_params;
-    const uint64_t T = traj->used_T ? traj->used_T : traj->T;
-    PassPlan plan;
-    SeqScratch sc;
-    RL_TRY(make_seq_plan(ctx, net, T, traj->E, (size_t)(n_steps + 1) * sizeof(double), &plan, &sc));
-    double *losses = (double *)sc.extra;
-    rl_seq_pass_args a = seq_base_args(traj, net, T, sc, plan);
-    a.target = targets_dev;
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    if (stats) {
-        RL_TRY(update_events(ctx, &ev0, &ev1));
-        RL_CUDA(ctx, cudaEventRecord(ev0, ctx->stream));
-    }
-    AdamArgs ac{adam->cfg.learning_rate, adam->cfg.beta1, adam->cfg.beta2, adam->cfg.weight_decay, adam->cfg.eps};
-    for (int s = 0; s < n_steps; ++s) {
-        RL_TRY(seq_pass(ctx, plan, PASS_VALUE, a));
-        adam->step += 1;
-        RL_LAUNCH(ctx, adam_step_kernel, 1, VEC_THREADS, 0, plan.sums, P, net.params, adam->m, adam->v, ac, adam->step,
-                  losses + s);
-    }
-    if (stats) {
-        RL_CUDA(ctx, cudaEventRecord(ev1, ctx->stream));
-        double *host;
-        RL_TRY(rl_ctx_pinned(ctx, (size_t)(n_steps + 4) * sizeof(double), (void **)&host));
-        if (n_steps > 0) RL_CUDA(ctx, cudaMemcpyAsync(host, losses, (size_t)n_steps * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        RL_CUDA(ctx, cudaMemcpyAsync(host + n_steps, plan.sums + P + SC_COUNT, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        stats->loss_first = n_steps > 0 ? host[0] : 0.0;
-        stats->loss_last = n_steps > 0 ? host[n_steps - 1] : 0.0;
-        stats->num_steps = n_steps > 0 ? (uint64_t)host[n_steps] : 0;
-        stats->opt_steps = (uint64_t)n_steps;
-        cudaEventElapsedTime(&stats->update_ms, ev0, ev1);
-    }
-    return x_error_check(ctx, "rl_value_update_seq");
-}
-
+// DqnAgent::batch_update (dqn.rs:263-337) with an Mlp action-value module, on flat minibatch planes.
 rl_status rl_dqn_update(rl_replay *rb, rl_mlp *q, rl_adam *adam, const rl_dqn_cfg *cfg, rl_opt_stats *stats) {
     if (!rb || !q || !adam || !cfg)
         return rl_fail(q ? q->ctx : nullptr, RL_ERR_INVALID_ARG, "rl_dqn_update: NULL argument");
     rl_ctx *ctx = rl_replay_ctx(rb);
     RL_REQUIRE(ctx, q->ctx == ctx, "rl_dqn_update: network belongs to another context");
-    RL_REQUIRE(ctx, adam->mlp == q, "rl_dqn_update: optimizer belongs to another module");
-    RL_REQUIRE(ctx, cfg->opt_steps_per_update >= 0 && cfg->opt_steps_per_update <= 100000,
-               "rl_dqn_update: opt_steps_per_update out of range");
+    RL_TRY(adam_check(ctx, adam, q, cfg->opt_steps_per_update, "rl_dqn_update"));
     PassNet pn;
     RL_TRY(pass_net_for(ctx, q, rl_replay_num_features(rb), "rl_dqn_update", &pn));
     const size_t F = (size_t)pn.sh.F;
-    const int P = (int)q->n_params;
     const int n_steps = cfg->opt_steps_per_update;
-    // the minibatch planes hold at most minibatch_steps + one ring of columns; the plan is sized once
+    UpdateTimer timer{ctx, stats != nullptr};
+    RL_TRY(timer.start());
+    const AdamArgs ac = adam_args(adam);
     rl_minibatch_dev mb{};
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    if (stats) {
-        RL_TRY(update_events(ctx, &ev0, &ev1));
-        RL_CUDA(ctx, cudaEventRecord(ev0, ctx->stream));
-    }
-    AdamArgs ac{adam->cfg.learning_rate, adam->cfg.beta1, adam->cfg.beta2, adam->cfg.weight_decay, adam->cfg.eps};
-    PassPlan plan{};
+    UpdateNet u;
     double *losses = nullptr;
     // sample_minibatch (dqn.rs:280-314): episodes, features and targets (no_grad) of every step.  Reward-to-go targets
     // do not depend on the parameters and the ring does not change during the update, so all n_steps minibatches are
@@ -2114,28 +2067,28 @@ rl_status rl_dqn_update(rl_replay *rb, rl_mlp *q, rl_adam *adam, const rl_dqn_cf
         if (!batched)
             RL_TRY(rl_replay_sample_enqueue(rb, cfg->minibatch_steps, cfg->sample_seed, rl_replay_next_draw_index(rb),
                                             cfg->target_one_step_td, cfg->discount_factor, q, 1, &mb));
-        if (s == 0) RL_TRY(make_plan(ctx, P, mb.capacity, &plan, (size_t)(n_steps + 1) * sizeof(double), (void **)&losses));
+        if (s == 0) {  // the minibatch planes hold at most minibatch_steps + one ring of columns: the plan is sized once
+            PassArgs planes{};
+            planes.T = 1;
+            planes.E = mb.capacity;
+            RL_TRY(u.init(ctx, q, pn, planes, (size_t)(n_steps + 1) * sizeof(double), false));
+            losses = (double *)u.extra;
+        }
         const size_t set = batched ? (size_t)s : 0;
-        PassArgs pa{};
-        pa.obs = mb.obs + set * mb.capacity * F; pa.action = mb.action + set * mb.capacity; pa.succ = mb.succ + set * mb.capacity;
-        pa.T = 1; pa.E = mb.capacity;
-        pa.theta = q->params; pa.target = mb.target + set * mb.capacity;
+        u.args.obs = mb.obs + set * mb.capacity * F; u.args.action = mb.action + set * mb.capacity;
+        u.args.succ = mb.succ + set * mb.capacity; u.args.target = mb.target + set * mb.capacity;
         // loss_fn + backward_step (dqn.rs:316-336, coptimizer.rs:13-27)
-        RL_TRY(pass_and_adam(ctx, plan, pa, PASS_QLOSS, pn, q, adam, ac, losses + s));
+        RL_TRY(u.adam_step(PASS_QLOSS, adam, ac, losses + s));
     }
     uint64_t m_last = 0;
     if (n_steps > 0) RL_TRY(rl_replay_sample_finish(rb, &m_last, nullptr));
     if (stats) {
-        RL_CUDA(ctx, cudaEventRecord(ev1, ctx->stream));
+        RL_TRY(timer.stop());
         double *host;
         RL_TRY(rl_ctx_pinned(ctx, (size_t)(n_steps + 4) * sizeof(double), (void **)&host));
         if (n_steps > 0) RL_CUDA(ctx, cudaMemcpyAsync(host, losses, (size_t)n_steps * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
         RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        stats->loss_first = n_steps > 0 ? host[0] : 0.0;
-        stats->loss_last = n_steps > 0 ? host[n_steps - 1] : 0.0;
-        stats->num_steps = m_last;
-        stats->opt_steps = (uint64_t)n_steps;
-        cudaEventElapsedTime(&stats->update_ms, ev0, ev1);
+        fill_opt_stats(stats, host, n_steps, m_last, timer);
     }
     return x_error_check(ctx, "rl_dqn_update");
 }
@@ -2150,21 +2103,12 @@ rl_status rl_dqn_update_seq(rl_replay *rb, rl_grunet *q, rl_adam *adam, const rl
     rl_ctx *ctx = rl_replay_ctx(rb);
     const rl_grunet_view net = rl_grunet_view_of(q);
     RL_REQUIRE(ctx, net.ctx == ctx, "rl_dqn_update_seq: network belongs to another context");
-    RL_REQUIRE(ctx, adam->owner == (void *)q, "rl_dqn_update_seq: optimizer belongs to another module");
-    RL_REQUIRE(ctx, cfg->opt_steps_per_update >= 0 && cfg->opt_steps_per_update <= 100000,
-               "rl_dqn_update_seq: opt_steps_per_update out of range");
-    const int F = rl_replay_num_features(rb);
-    if (net.in_dim != F || !(rl_seq_pass_supports(net.in_dim, net.hidden, net.out_dim) || rl_seq_big_supports(net.in_dim, net.hidden, net.out_dim)))
-        return rl_fail(ctx, RL_ERR_UNSUPPORTED, "rl_dqn_update_seq: recurrent passes are built for hidden <= 128, features <= 64, outputs <= 32 "
-                       "(got %d -> %d -> %d on %d features)", net.in_dim, net.hidden, net.out_dim, F);
-    const int P = (int)net.n_params;
+    RL_TRY(adam_check(ctx, adam, q, cfg->opt_steps_per_update, "rl_dqn_update_seq"));
+    RL_TRY(seq_check(ctx, net, rl_replay_num_features(rb), 0, "rl_dqn_update_seq"));
     const int n_steps = cfg->opt_steps_per_update;
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    if (stats) {
-        RL_TRY(update_events(ctx, &ev0, &ev1));
-        RL_CUDA(ctx, cudaEventRecord(ev0, ctx->stream));
-    }
-    AdamArgs ac{adam->cfg.learning_rate, adam->cfg.beta1, adam->cfg.beta2, adam->cfg.weight_decay, adam->cfg.eps};
+    UpdateTimer timer{ctx, stats != nullptr};
+    RL_TRY(timer.start());
+    const AdamArgs ac = adam_args(adam);
     std::vector<double> losses((size_t)n_steps, 0.0);
     uint64_t m_last = 0;
     for (int s = 0; s < n_steps; ++s) {
@@ -2174,16 +2118,12 @@ rl_status rl_dqn_update_seq(rl_replay *rb, rl_grunet *q, rl_adam *adam, const rl
         RL_TRY(rl_replay_sample_seq_dev(rb, cfg->minibatch_steps, cfg->sample_seed, rl_replay_next_draw_index(rb), cfg->target_one_step_td,
                                         cfg->discount_factor, q, &mb, &target));
         m_last = mb->num_steps;
-        PassPlan plan;
-        SeqScratch sc;
-        RL_TRY(make_seq_plan(ctx, net, mb->T, mb->E, 256, &plan, &sc));
-        double *loss_dev = (double *)sc.extra;
-        rl_seq_pass_args a = seq_base_args(mb, net, mb->T, sc, plan);
-        a.target = target;
+        UpdateNet u;
+        RL_TRY(u.init(ctx, net, traj_args(mb), 256));
+        u.args.target = target;
+        double *loss_dev = (double *)u.extra;
         // loss_fn + backward_step (dqn.rs:316-336, coptimizer.rs:13-27)
-        RL_TRY(seq_pass(ctx, plan, PASS_QLOSS, a));
-        adam->step += 1;
-        RL_LAUNCH(ctx, adam_step_kernel, 1, VEC_THREADS, 0, plan.sums, P, net.params, adam->m, adam->v, ac, adam->step, loss_dev);
+        RL_TRY(u.adam_step(PASS_QLOSS, adam, ac, loss_dev));
         // the next sample synchronises anyway; the plan's scratch may move with the next sample's size
         if (stats) {
             RL_CUDA(ctx, cudaMemcpyAsync(&losses[(size_t)s], loss_dev, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
@@ -2191,13 +2131,9 @@ rl_status rl_dqn_update_seq(rl_replay *rb, rl_grunet *q, rl_adam *adam, const rl
         }
     }
     if (stats) {
-        RL_CUDA(ctx, cudaEventRecord(ev1, ctx->stream));
+        RL_TRY(timer.stop());
         RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        stats->loss_first = n_steps > 0 ? losses[0] : 0.0;
-        stats->loss_last = n_steps > 0 ? losses[(size_t)n_steps - 1] : 0.0;
-        stats->num_steps = m_last;
-        stats->opt_steps = (uint64_t)n_steps;
-        cudaEventElapsedTime(&stats->update_ms, ev0, ev1);
+        fill_opt_stats(stats, losses.data(), n_steps, m_last, timer);
     }
     return x_error_check(ctx, "rl_dqn_update_seq");
 }
@@ -2209,29 +2145,16 @@ rl_status rl_dqn_probe_seq(rl_replay *rb, const rl_dqn_cfg *cfg, rl_grunet *q, u
     rl_ctx *ctx = rl_replay_ctx(rb);
     const rl_grunet_view net = rl_grunet_view_of(q);
     RL_REQUIRE(ctx, net.ctx == ctx, "rl_dqn_probe_seq: network belongs to another context");
-    const int F = rl_replay_num_features(rb);
-    if (net.in_dim != F || !(rl_seq_pass_supports(net.in_dim, net.hidden, net.out_dim) || rl_seq_big_supports(net.in_dim, net.hidden, net.out_dim)))
-        return rl_fail(ctx, RL_ERR_UNSUPPORTED, "rl_dqn_probe_seq: recurrent passes are built for hidden <= 128, features <= 64, outputs <= 32 "
-                       "(got %d -> %d -> %d on %d features)", net.in_dim, net.hidden, net.out_dim, F);
-    const int P = (int)net.n_params;
+    RL_TRY(seq_check(ctx, net, rl_replay_num_features(rb), 0, "rl_dqn_probe_seq"));
     rl_traj *mb = nullptr;
     const float *target = nullptr;
     RL_TRY(rl_replay_sample_seq_dev(rb, cfg->minibatch_steps, cfg->sample_seed, draw_index, cfg->target_one_step_td, cfg->discount_factor,
                                     q, &mb, &target));
-    PassPlan plan;
-    SeqScratch sc;
-    RL_TRY(make_seq_plan(ctx, net, mb->T, mb->E, 0, &plan, &sc));
-    rl_seq_pass_args a = seq_base_args(mb, net, mb->T, sc, plan);
-    a.target = target;
-    RL_TRY(seq_pass(ctx, plan, PASS_QLOSS, a));
-    std::vector<double> host((size_t)plan.W);
-    RL_CUDA(ctx, cudaMemcpyAsync(host.data(), plan.sums, (size_t)plan.W * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    RL_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    const double N = host[P + SC_COUNT];
-    if (loss) *loss = host[P + SC_LOSS] / N;
-    if (grad_host)
-        for (int i = 0; i < P; ++i) grad_host[i] = (float)(host[i] / N);
-    return RL_OK;
+    UpdateNet u;
+    RL_TRY(u.init(ctx, net, traj_args(mb), 0));
+    u.args.target = target;
+    std::vector<double> host;
+    return probe_pass(u, PASS_QLOSS, nullptr, host, loss, grad_host);
 }
 
 }  // extern "C"
