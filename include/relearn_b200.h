@@ -257,6 +257,13 @@ rl_status rl_mlp_forward(rl_mlp *mlp, const float *x_dev, uint64_t n, float *out
 /* ------------------------------------------------------------------------------------------ */
 rl_status rl_grunet_create(rl_ctx *ctx, int32_t in_dim, int32_t hidden, int32_t out_dim, rl_activation activation,
                            rl_grunet **out);
+/* Chain<Lstm, Linear> (seq/rnn/lstm.rs) behind the same handle type, the cell fixed at creation: one LSTM layer in_dim ->
+ * hidden (num_layers 1, biases present), activation, Linear hidden -> out_dim.  Flat parameters w_ih[4H,in], w_hh[4H,H],
+ * b_ih[4H], b_hh[4H] (gate order i, f, g, o as libtorch's lstm_cell), then kernel[out,H], bias[out]: 4H(in+H) + 8H +
+ * out*H + out values.  (h, c) start at zero in every episode.  Same ranges as rl_grunet_create; every function below that
+ * takes an rl_grunet* accepts it, and rl_grunet_destroy frees it. */
+rl_status rl_lstmnet_create(rl_ctx *ctx, int32_t in_dim, int32_t hidden, int32_t out_dim, rl_activation activation,
+                            rl_grunet **out);
 rl_status rl_grunet_destroy(rl_grunet *net);
 rl_status rl_grunet_num_params(rl_grunet *net, uint64_t *n);
 rl_status rl_grunet_set_weights(rl_grunet *net, const float *host, uint64_t n);

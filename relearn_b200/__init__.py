@@ -6,7 +6,8 @@ Host-side mirror of the reference's interfaces for that path over a C-ABI CUDA l
 from . import _lib  # noqa: F401
 from .envs import (BatchedEnv, CartPole, CartPoleConfig, Chain, LatentStepLimit, MemoryGame, MetaEnv, OneHotBandits, PartitionGame, Successor,  # noqa: F401
                    TrialEpisodeLimit, UniformBernoulliBandits, VisibleStepLimit, build_env)
-from .modules import (GruLinear, GruLinearConfig, Mlp, MlpConfig, init_gru_linear_params, init_params, num_params)  # noqa: F401
+from .modules import (GruLinear, GruLinearConfig, LstmLinear, LstmLinearConfig, Mlp, MlpConfig, init_gru_linear_params,  # noqa: F401
+                      init_lstm_linear_params, init_params, lstm_linear_num_params, num_params)
 from .runtime import Context, DeviceBuffer  # noqa: F401
 from .simulation import (ActorSpec, HistoryDataBound, TrainParallelConfig, Trajectory, pack_history, rollout, train_device,  # noqa: F401
                          train_serial)

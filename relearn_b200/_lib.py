@@ -191,6 +191,7 @@ SIGNATURES = {
     "rl_mlp_get_weights": (st, [vp, vp, C.c_uint64]),
     "rl_mlp_forward": (st, [vp, vp, C.c_uint64, vp]),
     "rl_grunet_create": (st, [vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, P(vp)]),
+    "rl_lstmnet_create": (st, [vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, P(vp)]),
     "rl_grunet_destroy": (st, [vp]),
     "rl_grunet_num_params": (st, [vp, P(C.c_uint64)]),
     "rl_grunet_set_weights": (st, [vp, vp, C.c_uint64]),

@@ -37,8 +37,9 @@ struct rl_grunet {
     rl_ctx *ctx = nullptr;
     int in_dim = 0, hidden = 0, out_dim = 0;
     rl_activation act = RL_ACT_RELU;
+    int cell = RL_CELL_GRU;
     uint64_t n_params = 0;
-    float *params = nullptr;  // w_ih[3H,in], w_hh[3H,H], b_ih[3H], b_hh[3H], kernel[out,H], bias[out]
+    float *params = nullptr;  // w_ih[G H,in], w_hh[G H,H], b_ih[G H], b_hh[G H], kernel[out,H], bias[out]; G = 3 (GRU) or 4 (LSTM)
     float *wt = nullptr;      // K8h: k-major copy of w_ih / w_hh, [in + H][3H] (rebuilt before every tiled rollout)
 };
 
@@ -47,7 +48,11 @@ namespace {
 struct GruView {
     const float *params;
     int F, H, A, act;
-    __host__ __device__ uint64_t count() const { return (uint64_t)3 * H * F + (uint64_t)3 * H * H + 6 * (uint64_t)H + (uint64_t)A * H + A; }
+    int cell;
+    __host__ __device__ uint64_t count() const {
+        const uint64_t G = rl_cell_gates(cell);
+        return G * H * F + G * H * H + 2 * G * H + (uint64_t)A * H + A;
+    }
 };
 
 __device__ __forceinline__ float sigmoidf_ref(float v) { return 1.0f / (1.0f + expf(-v)); }
@@ -97,6 +102,56 @@ __device__ __forceinline__ void grunet_step(const GruView &m, const float *__res
     }
 }
 
+// One lstm_cell + activation + Linear for this thread's env (libtorch's lstm_cell, gate order i, f, g, o):
+//   gates = (W_ih x + b_ih) + (W_hh h + b_hh);  c' = f c + i g;  h' = o tanh(c')
+// c[j] is read and written by unit j alone, so it is updated in place; h waits for all units like grunet_step's.
+template <int HMAX, int MAXF, int MAXA>
+__device__ __forceinline__ void lstmnet_step(const GruView &m, const float *__restrict__ w, const float *x, float *h, float *c, float *z) {
+    const int F = m.F, H = m.H, A = m.A;
+    const float *w_ih = w, *w_hh = w_ih + (size_t)4 * H * F, *b_ih = w_hh + (size_t)4 * H * H, *b_hh = b_ih + 4 * H;
+    const float *lin_w = b_hh + 4 * H, *lin_b = lin_w + (size_t)A * H;
+    constexpr bool SMALL = HMAX <= 8;
+    float hn[HMAX];
+#pragma unroll(SMALL ? HMAX : 1)
+    for (int j = 0; j < (SMALL ? HMAX : H); ++j) {
+        if (SMALL && j >= H) break;
+        float s[4];
+#pragma unroll
+        for (int g = 0; g < 4; ++g) {
+            const int row = g * H + j;
+            float a = b_ih[row], b = b_hh[row];
+#pragma unroll
+            for (int f = 0; f < MAXF; ++f)
+                if (f < F) a = fmaf(w_ih[(size_t)row * F + f], x[f], a);
+#pragma unroll(SMALL ? HMAX : 4)
+            for (int k = 0; k < (SMALL ? HMAX : H); ++k)
+                if (!SMALL || k < H) b = fmaf(w_hh[(size_t)row * H + k], h[k], b);
+            s[g] = __fadd_rn(a, b);
+        }
+        const float i = sigmoidf_ref(s[0]), f = sigmoidf_ref(s[1]), g = tanhf(s[2]), o = sigmoidf_ref(s[3]);
+        c[j] = __fadd_rn(__fmul_rn(f, c[j]), __fmul_rn(i, g));
+        hn[j] = __fmul_rn(o, tanhf(c[j]));
+    }
+#pragma unroll
+    for (int k = 0; k < MAXA; ++k) z[k] = k < A ? lin_b[k] : 0.0f;
+#pragma unroll(SMALL ? HMAX : 1)
+    for (int j = 0; j < (SMALL ? HMAX : H); ++j) {
+        if (SMALL && j >= H) break;
+        h[j] = hn[j];
+        const float a = rl_activate(m.act, hn[j]);
+#pragma unroll
+        for (int k = 0; k < MAXA; ++k)
+            if (k < A) z[k] = fmaf(lin_w[(size_t)k * H + j], a, z[k]);
+    }
+}
+
+// The cell step of a CELL module; c (the LSTM's cell state) is unused by the GRU.
+template <int CELL, int HMAX, int MAXF, int MAXA, bool EXACT = false>
+__device__ __forceinline__ void seq_step(const GruView &m, const float *__restrict__ w, const float *x, float *h, float *c, float *z) {
+    if constexpr (CELL == RL_CELL_LSTM) lstmnet_step<HMAX, MAXF, MAXA>(m, w, x, h, c, z);
+    else grunet_step<HMAX, MAXF, MAXA, EXACT>(m, w, x, h, z);
+}
+
 struct SeqArgs {
     uint64_t E, lane_offset;
     NoiseSource noise;
@@ -126,8 +181,8 @@ __device__ __forceinline__ bool dqn_explore(const SeqArgs &a, LaneNoise<REPLAY> 
 }
 
 // XF / XA > 0: features / actions (and hidden = HMAX) fixed at compile time, see grunet_step<EXACT>.  EPS: the epsilon-greedy
-// actor of a recurrent Q-network instead of the categorical policy.
-template <class EnvT, bool REPLAY, int HMAX, bool EPS, int XF = 0, int XA = 0>
+// actor of a recurrent Q-network instead of the categorical policy.  CELL: GRU or LSTM (whose cell state c sits beside h).
+template <class EnvT, bool REPLAY, int HMAX, bool EPS, int XF = 0, int XA = 0, int CELL = RL_CELL_GRU>
 __global__ void __launch_bounds__(128) rollout_seq_kernel(typename EnvT::Params p, SeqArgs a) {
     constexpr bool EXACT = XF > 0;
     constexpr int MF = EXACT ? XF : EnvT::MAXF, MA = EXACT ? XA : EnvT::MAXA;
@@ -152,11 +207,14 @@ __global__ void __launch_bounds__(128) rollout_seq_kernel(typename EnvT::Params 
         nz.init(a.noise, a.lane_offset + e, e);
         const uint32_t t0 = a.noise.step_counter;
         typename EnvT::State s;
-        float obs[MF], last_obs[MF], h[HMAX];
+        constexpr int CMAX = CELL == RL_CELL_LSTM ? HMAX : 1;
+        float obs[MF], last_obs[MF], h[HMAX], c[CMAX];
 #pragma unroll
         for (int f = 0; f < MF; ++f) obs[f] = last_obs[f] = 0.0f;
 #pragma unroll
-        for (int j = 0; j < HMAX; ++j) h[j] = 0.0f;  // SeqIterative::initial_state (gru.rs:23-28)
+        for (int j = 0; j < HMAX; ++j) h[j] = 0.0f;  // SeqIterative::initial_state (gru.rs:23-28, lstm.rs: (h, c) = 0)
+#pragma unroll
+        for (int j = 0; j < CMAX; ++j) c[j] = 0.0f;
         uint32_t n = a.min_steps ? a.min_steps + a.slack : 0;  // take_steps.rs:20-31
         uint32_t i = 0;
         int succ_last = RL_TERMINATE, succ_prev = RL_TERMINATE;
@@ -171,11 +229,11 @@ __global__ void __launch_bounds__(128) rollout_seq_kernel(typename EnvT::Params 
             uint32_t action;
             if (EPS) {
                 if (!dqn_explore<REPLAY>(a, nz, A, action)) {
-                    grunet_step<HMAX, MF, MA, EXACT>(a.net, w, obs, h, z);
+                    seq_step<CELL, HMAX, MF, MA, EXACT>(a.net, w, obs, h, c, z);
                     action = argmax_first<MA>(z, A);
                 }
             } else {
-                grunet_step<HMAX, MF, MA, EXACT>(a.net, w, obs, h, z);
+                seq_step<CELL, HMAX, MF, MA, EXACT>(a.net, w, obs, h, c, z);
                 const float u = rl_u32_to_f32(nz.template next_u32<RL_STREAM_ACTOR>());
                 action = categorical_sample<MA>(z, A, u);
             }
@@ -198,6 +256,8 @@ __global__ void __launch_bounds__(128) rollout_seq_kernel(typename EnvT::Params 
                 EnvT::template reset<REPLAY>(p, s, nz);
 #pragma unroll
                 for (int j = 0; j < HMAX; ++j) h[j] = 0.0f;  // steps.rs:116-124: actor.initial_state for the new episode
+#pragma unroll
+                for (int j = 0; j < CMAX; ++j) c[j] = 0.0f;
             }
             observe(s, obs);
             a.action[(uint64_t)i * a.E + e] = (uint8_t)action;
@@ -232,7 +292,7 @@ __global__ void __launch_bounds__(128) rollout_seq_kernel(typename EnvT::Params 
 
 // SeqPacked::seq_packed (gru.rs:72-102 -> chain.rs:157-168) over a stored trajectory: thread per lane, hidden
 // state zeroed at the first step of every episode.  out f32 [T][A][E]; PAD slots get zeros.
-template <int HMAX, int XF = 0, int XA = 0>
+template <int HMAX, int XF = 0, int XA = 0, int CELL = RL_CELL_GRU>
 __global__ void __launch_bounds__(128) grunet_seq_kernel(GruView m, int weights_in_smem, const float *__restrict__ obs,
                                                         const float *__restrict__ next_obs, const uint8_t *__restrict__ succ,
                                                         uint64_t T, uint64_t E, float *__restrict__ out,
@@ -249,9 +309,12 @@ __global__ void __launch_bounds__(128) grunet_seq_kernel(GruView m, int weights_
     constexpr bool EXACT = XF > 0;  // sizes fixed at compile time (config 4: 6 features, hidden 4, 1 or 2 outputs)
     constexpr int MAXF = EXACT ? XF : 36, MAXA = EXACT ? XA : 32;
     const int nF = EXACT ? XF : m.F, nA = EXACT ? XA : m.A;
-    float h[HMAX];
+    constexpr int CMAX = CELL == RL_CELL_LSTM ? HMAX : 1;
+    float h[HMAX], c[CMAX];
 #pragma unroll
     for (int j = 0; j < HMAX; ++j) h[j] = 0.0f;
+#pragma unroll
+    for (int j = 0; j < CMAX; ++j) c[j] = 0.0f;
     for (uint64_t t = 0; t < T; ++t) {
         const uint8_t sc = succ[t * E + e];
         float z[MAXA];
@@ -262,19 +325,21 @@ __global__ void __launch_bounds__(128) grunet_seq_kernel(GruView m, int weights_
         float x[MAXF];
 #pragma unroll
         for (int f = 0; f < MAXF; ++f) x[f] = f < nF ? obs[(t * nF + f) * E + e] : 0.0f;
-        grunet_step<HMAX, MAXF, MAXA, EXACT>(m, w, x, h, z);
+        seq_step<CELL, HMAX, MAXF, MAXA, EXACT>(m, w, x, h, c, z);
         #pragma unroll
         for (int k = 0; k < MAXA; ++k)
             if (k < nA) out[(t * nA + k) * E + e] = z[k];
         if (sc == RL_INTERRUPT && out_next) {
             // the extended observation of an interrupted episode (features.rs:139-185): one more step of the same
             // sequence on the successor observation
-            float h2[HMAX];
+            float h2[HMAX], c2[CMAX];
 #pragma unroll
             for (int j = 0; j < HMAX; ++j) h2[j] = h[j];
 #pragma unroll
+            for (int j = 0; j < CMAX; ++j) c2[j] = c[j];
+#pragma unroll
             for (int f = 0; f < MAXF; ++f) x[f] = f < nF ? next_obs[(t * nF + f) * E + e] : 0.0f;
-            grunet_step<HMAX, MAXF, MAXA, EXACT>(m, w, x, h2, z);
+            seq_step<CELL, HMAX, MAXF, MAXA, EXACT>(m, w, x, h2, c2, z);
             #pragma unroll
             for (int k = 0; k < MAXA; ++k)
                 if (k < nA) out_next[(t * nA + k) * E + e] = z[k];
@@ -282,38 +347,44 @@ __global__ void __launch_bounds__(128) grunet_seq_kernel(GruView m, int weights_
         if (sc != RL_CONTINUE) {
 #pragma unroll
             for (int j = 0; j < HMAX; ++j) h[j] = 0.0f;
+#pragma unroll
+            for (int j = 0; j < CMAX; ++j) c[j] = 0.0f;
         }
     }
 }
 
 GruView view_of(const rl_grunet *g) {
     GruView v;
-    v.params = g->params; v.F = g->in_dim; v.H = g->hidden; v.A = g->out_dim; v.act = (int)g->act;
+    v.params = g->params; v.F = g->in_dim; v.H = g->hidden; v.A = g->out_dim; v.act = (int)g->act; v.cell = g->cell;
     return v;
 }
 
 constexpr size_t SEQ_SMEM_LIMIT = 160 * 1024;
 
-template <class EnvT, bool REPLAY, int HMAX, bool EPS, int XF = 0, int XA = 0>
+template <class EnvT, bool REPLAY, int HMAX, bool EPS, int XF, int XA, int CELL>
 rl_status launch_seq_k8a(rl_ctx *ctx, const typename EnvT::Params &p, SeqArgs &a, size_t smem, unsigned grid) {
-    RL_CUDA(ctx, cudaFuncSetAttribute(rollout_seq_kernel<EnvT, REPLAY, HMAX, EPS, XF, XA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    RL_LAUNCH(ctx, (rollout_seq_kernel<EnvT, REPLAY, HMAX, EPS, XF, XA>), grid, 128, smem, p, a);
+    RL_CUDA(ctx, cudaFuncSetAttribute(rollout_seq_kernel<EnvT, REPLAY, HMAX, EPS, XF, XA, CELL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    RL_LAUNCH(ctx, (rollout_seq_kernel<EnvT, REPLAY, HMAX, EPS, XF, XA, CELL>), grid, 128, smem, p, a);
     return RL_OK;
 }
 
-template <class EnvT, int HMAX, int XF = 0, int XA = 0>
+template <class EnvT, int HMAX, int XF = 0, int XA = 0, int CELL = RL_CELL_GRU>
 rl_status launch_seq_h(rl_ctx *ctx, const typename EnvT::Params &p, SeqArgs &a, bool replay, size_t smem, unsigned grid) {
     if (a.eps_greedy) {
-        if (replay) return launch_seq_k8a<EnvT, true, HMAX, true, XF, XA>(ctx, p, a, smem, grid);
-        return launch_seq_k8a<EnvT, false, HMAX, true, XF, XA>(ctx, p, a, smem, grid);
+        if (replay) return launch_seq_k8a<EnvT, true, HMAX, true, XF, XA, CELL>(ctx, p, a, smem, grid);
+        return launch_seq_k8a<EnvT, false, HMAX, true, XF, XA, CELL>(ctx, p, a, smem, grid);
     }
-    if (replay) return launch_seq_k8a<EnvT, true, HMAX, false, XF, XA>(ctx, p, a, smem, grid);
-    return launch_seq_k8a<EnvT, false, HMAX, false, XF, XA>(ctx, p, a, smem, grid);
+    if (replay) return launch_seq_k8a<EnvT, true, HMAX, false, XF, XA, CELL>(ctx, p, a, smem, grid);
+    return launch_seq_k8a<EnvT, false, HMAX, false, XF, XA, CELL>(ctx, p, a, smem, grid);
 }
 
 template <class EnvT>
 rl_status launch_seq(rl_ctx *ctx, const typename EnvT::Params &p, SeqArgs &a, bool replay, size_t smem, unsigned grid) {
     const int H = a.net.H;
+    if (a.net.cell == RL_CELL_LSTM) {  // K8a only: the tiled and tensor-core kernels are GRU cells
+        if (H <= 8) return launch_seq_h<EnvT, 8, 0, 0, RL_CELL_LSTM>(ctx, p, a, replay, smem, grid);
+        return launch_seq_h<EnvT, 128, 0, 0, RL_CELL_LSTM>(ctx, p, a, replay, smem, grid);
+    }
     if constexpr (std::is_same<EnvT, BanditMetaEnv>::value) {
         // BASELINE config 4: 2-armed bandit meta-env (6 features) with the rnn.rs-sized GRU (hidden 4)
         if (H == 4 && a.F == 6 && a.A == 2 && p.num_arms == 2) return launch_seq_h<BanditMetaEnv, 4, 6, 2>(ctx, p, a, replay, smem, grid);
@@ -350,7 +421,7 @@ rl_status rl_rollout_seq(rl_env *env, rl_grunet *net, bool eps_greedy, double ep
     const size_t smem = a.weights_in_smem ? wbytes : 16;
     // K8h (gru_tile.cuh) for the rl2-sized module; RL_GRU_KERNEL=thread keeps the thread-per-env kernel (diagnostics)
     const char *pick = getenv("RL_GRU_KERNEL");
-    const bool tiled = net->hidden == GT_H && net->in_dim <= GT_MAXF && net->out_dim <= GT_LW &&
+    const bool tiled = net->cell == RL_CELL_GRU && net->hidden == GT_H && net->in_dim <= GT_MAXF && net->out_dim <= GT_LW &&
                        env->kind != RL_ENV_MEMORY_GAME && !(pick && strcmp(pick, "thread") == 0);
     a.tile_envs = (pick && strcmp(pick, "tile32") == 0) ? 32 : 64;
     // K8s (gru_step_tc.cuh): the cell of all envs as one tensor-core launch per step.  Picked above 4 096 envs (below, the
@@ -395,6 +466,22 @@ rl_status rl_grunet_seq_enqueue(rl_grunet *g, rl_traj *traj, float *out_dev, flo
     const size_t smem = in_smem ? wbytes : 16;
     const unsigned grid = rl_grid_for(E, 128);
     const GruView v = view_of(g);
+    const bool thread = getenv("RL_GRU_KERNEL") && !strcmp(getenv("RL_GRU_KERNEL"), "thread");
+    if (g->cell == RL_CELL_LSTM) {
+        if (g->hidden > 8 && rl_seq_big_supports(g->in_dim, g->hidden, g->out_dim) && !thread)
+            return rl_seq_big_forward(ctx, RL_CELL_LSTM, g->params, g->in_dim, g->hidden, g->out_dim, (int)g->act, traj->obs, traj->next_obs,
+                                      traj->succ, T, E, out_dev, out_next_dev);
+        if (g->hidden <= 8) {
+            RL_CUDA(ctx, cudaFuncSetAttribute(grunet_seq_kernel<8, 0, 0, RL_CELL_LSTM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            RL_LAUNCH(ctx, (grunet_seq_kernel<8, 0, 0, RL_CELL_LSTM>), grid, 128, smem, v, in_smem, traj->obs, traj->next_obs, traj->succ, T, E,
+                      out_dev, out_next_dev);
+        } else {
+            RL_CUDA(ctx, cudaFuncSetAttribute(grunet_seq_kernel<128, 0, 0, RL_CELL_LSTM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            RL_LAUNCH(ctx, (grunet_seq_kernel<128, 0, 0, RL_CELL_LSTM>), grid, 128, smem, v, in_smem, traj->obs, traj->next_obs, traj->succ, T, E,
+                      out_dev, out_next_dev);
+        }
+        return RL_OK;
+    }
     if (g->hidden == 4 && g->in_dim == 6 && (g->out_dim == 1 || g->out_dim == 2)) {
         if (g->out_dim == 1) {
             RL_CUDA(ctx, cudaFuncSetAttribute(grunet_seq_kernel<4, 6, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -409,9 +496,9 @@ rl_status rl_grunet_seq_enqueue(rl_grunet *g, rl_traj *traj, float *out_dev, flo
         RL_CUDA(ctx, cudaFuncSetAttribute(grunet_seq_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         RL_LAUNCH(ctx, grunet_seq_kernel<8>, grid, 128, smem, v, in_smem, traj->obs, traj->next_obs, traj->succ, T, E, out_dev,
                   out_next_dev);
-    } else if (rl_seq_big_supports(g->in_dim, g->hidden, g->out_dim) && !(getenv("RL_GRU_KERNEL") && !strcmp(getenv("RL_GRU_KERNEL"), "thread"))) {
+    } else if (rl_seq_big_supports(g->in_dim, g->hidden, g->out_dim) && !thread) {
         // hidden 9 .. 128: the GEMM form (gru_big.cu); the thread-per-lane kernel below stays as the cross-check
-        return rl_seq_big_forward(ctx, g->params, g->in_dim, g->hidden, g->out_dim, (int)g->act, traj->obs, traj->next_obs, traj->succ, T, E,
+        return rl_seq_big_forward(ctx, RL_CELL_GRU, g->params, g->in_dim, g->hidden, g->out_dim, (int)g->act, traj->obs, traj->next_obs, traj->succ, T, E,
                                   out_dev, out_next_dev);
     } else {
         RL_CUDA(ctx, cudaFuncSetAttribute(grunet_seq_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -422,29 +509,43 @@ rl_status rl_grunet_seq_enqueue(rl_grunet *g, rl_traj *traj, float *out_dev, flo
 }
 
 rl_grunet_view rl_grunet_view_of(rl_grunet *g) {
-    return rl_grunet_view{g->ctx, g->in_dim, g->hidden, g->out_dim, (int)g->act, g->n_params, g->params};
+    return rl_grunet_view{g->ctx, g->in_dim, g->hidden, g->out_dim, (int)g->act, g->n_params, g->params, g->cell};
 }
+
+namespace {
+
+rl_status seqnet_create(rl_ctx *ctx, int cell, int32_t in_dim, int32_t hidden, int32_t out_dim, rl_activation activation, rl_grunet **out,
+                        const char *what) {
+    if (!ctx || !out) return rl_fail(ctx, RL_ERR_INVALID_ARG, "%s: NULL argument", what);
+    if (!(in_dim >= 1 && in_dim <= 36 && out_dim >= 1 && out_dim <= 32)) return rl_fail(ctx, RL_ERR_INVALID_ARG, "%s: dims out of range", what);
+    if (!(hidden >= 1 && hidden <= 128)) return rl_fail(ctx, RL_ERR_INVALID_ARG, "%s: hidden size out of range (1..128)", what);
+    RL_CUDA(ctx, cudaSetDevice(ctx->device));
+    rl_grunet *g = new (std::nothrow) rl_grunet();
+    if (!g) return rl_fail(ctx, RL_ERR_OOM, "%s: host allocation failed", what);
+    g->ctx = ctx; g->in_dim = in_dim; g->hidden = hidden; g->out_dim = out_dim; g->act = activation; g->cell = cell;
+    g->n_params = view_of(g).count();
+    cudaError_t e = cudaMalloc((void **)&g->params, g->n_params * sizeof(float));
+    if (e != cudaSuccess) {
+        delete g;
+        return rl_fail(ctx, RL_ERR_OOM, "%s: %s", what, cudaGetErrorString(e));
+    }
+    cudaMemsetAsync(g->params, 0, g->n_params * sizeof(float), ctx->stream);
+    *out = g;
+    return RL_OK;
+}
+
+}  // namespace
 
 extern "C" {
 
 rl_status rl_grunet_create(rl_ctx *ctx, int32_t in_dim, int32_t hidden, int32_t out_dim, rl_activation activation,
                            rl_grunet **out) {
-    RL_REQUIRE(ctx, ctx && out, "rl_grunet_create: NULL argument");
-    RL_REQUIRE(ctx, in_dim >= 1 && in_dim <= 36 && out_dim >= 1 && out_dim <= 32, "rl_grunet_create: dims out of range");
-    RL_REQUIRE(ctx, hidden >= 1 && hidden <= 128, "rl_grunet_create: hidden size out of range (1..128)");
-    RL_CUDA(ctx, cudaSetDevice(ctx->device));
-    rl_grunet *g = new (std::nothrow) rl_grunet();
-    if (!g) return rl_fail(ctx, RL_ERR_OOM, "rl_grunet_create: host allocation failed");
-    g->ctx = ctx; g->in_dim = in_dim; g->hidden = hidden; g->out_dim = out_dim; g->act = activation;
-    g->n_params = view_of(g).count();
-    cudaError_t e = cudaMalloc((void **)&g->params, g->n_params * sizeof(float));
-    if (e != cudaSuccess) {
-        delete g;
-        return rl_fail(ctx, RL_ERR_OOM, "rl_grunet_create: %s", cudaGetErrorString(e));
-    }
-    cudaMemsetAsync(g->params, 0, g->n_params * sizeof(float), ctx->stream);
-    *out = g;
-    return RL_OK;
+    return seqnet_create(ctx, RL_CELL_GRU, in_dim, hidden, out_dim, activation, out, "rl_grunet_create");
+}
+
+rl_status rl_lstmnet_create(rl_ctx *ctx, int32_t in_dim, int32_t hidden, int32_t out_dim, rl_activation activation,
+                            rl_grunet **out) {
+    return seqnet_create(ctx, RL_CELL_LSTM, in_dim, hidden, out_dim, activation, out, "rl_lstmnet_create");
 }
 
 rl_status rl_grunet_destroy(rl_grunet *g) {

@@ -20,6 +20,11 @@
 //
 // The Hessian of mean KL(p0 || p_theta) at theta0 is J^T (diag p - p p^T) J for any network, so forward tangent +
 // backward is the reference's double-backward Hessian-vector product (gru_update.cu header).
+// Chain<Lstm, Linear> (a.cell = RL_CELL_LSTM) runs the same GEMMs with its own pointwise kernels: Wc [4H x (F + H)] holds the
+// full [W_ih | W_hh] rows of all four gates i, f, g, o and bc = b_ih + b_hh; the gates kernel keeps i, f, g, o, h' per step and
+// the cell state c before each step (plane CP); the backward pointwise carries (dh, dc) and emits D_t = the four gate
+// pre-activation cotangents, after which carry += W_hh^T [H x 4H] . D_t; d b_ih = d b_hh.  The LSTM stays on the FP32 pipe.
+//
 // GEMMs: hand-written FP32 register-tiled kernels (128 x 128 x 8 tiles, 8 x 8 per thread, register-prefetched; the split-K
 // one contracts over lanes with f64 flushes).  FP32, not tensor cores: the parity bar is 1e-5-class against f64 autograd, which bf16/tf32
 // inputs miss; the bf16-piece tcgen05 form used by pass_tc.cuh is the next step (DESIGN.md section 9).
@@ -263,6 +268,23 @@ __global__ void big_comb_kernel(const float *__restrict__ th, int F, int H, floa
         }
 }
 
+// The LSTM's combined weights: Wc [4H x KP] = [W_ih | W_hh], bc = b_ih + b_hh, WhT [H x 4H] = W_hh^T
+__global__ void lstm_comb_kernel(const float *__restrict__ th, int F, int H, float *__restrict__ Wc, float *__restrict__ bc,
+                                 float *__restrict__ WhT) {
+    const int KP = F + H;
+    const float *w_ih = th, *w_hh = th + (size_t)4 * H * F, *b_ih = w_hh + (size_t)4 * H * H, *b_hh = b_ih + 4 * H;
+    for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < 4 * H * KP; idx += gridDim.x * blockDim.x) {
+        const int m = idx / KP, k = idx - m * KP;
+        Wc[idx] = k < F ? w_ih[(size_t)m * F + k] : w_hh[(size_t)m * H + (k - F)];
+    }
+    for (int m = blockIdx.x * blockDim.x + threadIdx.x; m < 4 * H; m += gridDim.x * blockDim.x) bc[m] = __fadd_rn(b_ih[m], b_hh[m]);
+    if (WhT)
+        for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < 4 * H * H; idx += gridDim.x * blockDim.x) {
+            const int k = idx / (4 * H), c = idx - k * 4 * H;  // WhT[k][c] = w_hh[c][k]
+            WhT[idx] = w_hh[(size_t)c * H + k];
+        }
+}
+
 __global__ void big_zero_kernel(float *p, uint64_t n, const int *skip_flag) {
     if (skip_flag && *skip_flag) return;
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) p[i] = 0.0f;
@@ -270,10 +292,12 @@ __global__ void big_zero_kernel(float *p, uint64_t n, const int *skip_flag) {
 
 struct BigPlanes {
     float *G, *tG;                        // [4H][E] of the current step
-    float *R, *U, *N, *HN, *HNEW, *AV;    // [T][H][E]
+    float *R, *U, *N, *HN, *HNEW, *AV;    // [T][H][E]; an LSTM keeps its gates i, f, g, o in R, U, N, HN
     float *THNEW;                         // [T][H][E] (FVP)
     float *thp, *dh;                      // [H][E]
     float *D;                             // [T][4H][E]
+    float *CP;                            // [T][H][E] LSTM: cell state before each step
+    float *tcp, *dc;                      // [H][E] LSTM: tangent of c (FVP), cell-state carry (backward)
 };
 
 // gates of step t from G (biases included) and hprev = hbuf[t]
@@ -290,6 +314,47 @@ __global__ void big_gates_kernel(const float *__restrict__ G, const float *__res
     const float hnew = __fadd_rn(__fmul_rn(__fsub_rn(hp, n), u), n);
     R[i] = r; U[i] = u; Nn[i] = n; HN[i] = hn; HNEW[i] = hnew;
     if (hnext) hnext[i] = succ_t[e] != RL_CONTINUE ? 0.0f : hnew;  // a new episode starts from zeros; padding stays zero too
+}
+
+// lstm_cell of step t from G (biases included) and cprev: gates, h' = o tanh(c'), c' = f cprev + i g (to cout when given); the
+// next step's (h, c) are zero where the episode ended
+__global__ void lstm_gates_kernel(const float *__restrict__ G, const float *__restrict__ cprev, const uint8_t *__restrict__ succ_t,
+                                  float *__restrict__ I, float *__restrict__ Fg, float *__restrict__ Gg, float *__restrict__ O,
+                                  float *__restrict__ HNEW, float *__restrict__ cout, float *__restrict__ hnext, float *__restrict__ cnext,
+                                  int H, uint64_t E, const int *skip_flag) {
+    if (skip_flag && *skip_flag) return;
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (uint64_t)H * E) return;
+    const uint64_t j = i / E, e = i - j * E, HE = (uint64_t)H * E;
+    const float ig = sigm_b(G[i]), fg = sigm_b(G[HE + i]), gg = tanhf(G[2 * HE + i]), og = sigm_b(G[3 * HE + i]);
+    const float c = __fadd_rn(__fmul_rn(fg, cprev[i]), __fmul_rn(ig, gg));
+    const float hnew = __fmul_rn(og, tanhf(c));
+    I[i] = ig; Fg[i] = fg; Gg[i] = gg; O[i] = og; HNEW[i] = hnew;
+    if (cout) cout[i] = c;
+    const bool done = succ_t[e] != RL_CONTINUE;
+    if (hnext) hnext[i] = done ? 0.0f : hnew;
+    if (cnext) cnext[i] = done ? 0.0f : c;
+}
+
+// LSTM tangents along v: tG = V [x; hprev] + vb + W_hh thprev (all four gate blocks); carries (thp, tcp) cut at episode ends
+__global__ void lstm_gates_tan_kernel(const float *__restrict__ tG, const float *__restrict__ I, const float *__restrict__ Fg,
+                                      const float *__restrict__ Gg, const float *__restrict__ O, const float *__restrict__ cprev,
+                                      float *__restrict__ thp, float *__restrict__ tcp, float *__restrict__ THNEW,
+                                      const uint8_t *__restrict__ succ_t, int H, uint64_t E, const int *skip_flag) {
+    if (skip_flag && *skip_flag) return;
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (uint64_t)H * E) return;
+    const uint64_t j = i / E, e = i - j * E, HE = (uint64_t)H * E;
+    const float ig = I[i], fg = Fg[i], gg = Gg[i], og = O[i], cp = cprev[i];
+    const float tc = tanhf(__fadd_rn(__fmul_rn(fg, cp), __fmul_rn(ig, gg)));
+    const float id = ig * (1.0f - ig) * tG[i], fd = fg * (1.0f - fg) * tG[HE + i];
+    const float gd = (1.0f - gg * gg) * tG[2 * HE + i], od = og * (1.0f - og) * tG[3 * HE + i];
+    const float tcn = fd * cp + fg * tcp[i] + id * gg + ig * gd;
+    const float thn = od * tc + og * (1.0f - tc * tc) * tcn;
+    THNEW[i] = thn;
+    const bool done = succ_t[e] != RL_CONTINUE;
+    thp[i] = done ? 0.0f : thn;
+    tcp[i] = done ? 0.0f : tcn;
 }
 
 // tangent of the gates along v (R-operator): tG = V [x; hprev] + vb + W[:, F:] thprev
@@ -325,8 +390,8 @@ __global__ void __launch_bounds__(HEAD_THREADS) big_head_kernel(rl_seq_pass_args
     constexpr bool USES_LP0 = MODE == RL_PASS_EVAL || MODE == RL_PASS_GRAD || MODE == RL_PASS_PPO;
     if (a.skip_flag && *a.skip_flag) return;
     extern __shared__ float hsm[];  // lw [A][H], lb [A], (FVP) vlw, vlb
-    const int H = a.H, A = a.A, F = a.F;
-    const int o_lw = 3 * H * F + 3 * H * H + 6 * H;
+    const int H = a.H, A = a.A, F = a.F, NG = rl_cell_gates(a.cell);
+    const int o_lw = NG * H * F + NG * H * H + 2 * NG * H;
     float *lw = hsm, *lb = lw + A * H, *vlw = lb + A, *vlb = vlw + A * H;
     for (int i = threadIdx.x; i < A * H + A; i += blockDim.x) {
         lw[i] = a.theta[o_lw + i];
@@ -509,15 +574,65 @@ __global__ void big_bwd_kernel(const float *__restrict__ dz_t, const float *__re
     dh[i] = dhn * u;
 }
 
-// the partial row: parameter order w_ih, w_hh, b_ih, b_hh, lw, lb, then loss, kl, entropy, count
-__global__ void big_assemble_kernel(const double *__restrict__ dWc, const double *__restrict__ dHead, const double *__restrict__ scal_part,
-                                    int nscal, int F, int H, int A, int backward, double *__restrict__ row, const int *skip_flag) {
+// LSTM backward pointwise of step t: D_t = (di, df, dg, do), AV_t, the cell-state carry dc := dc' f, and dh := 0 for the GEMM
+// that adds W_hh^T D_t
+__global__ void lstm_bwd_kernel(const float *__restrict__ dz_t, const float *__restrict__ theta, int o_lw, int act,
+                                const float *__restrict__ I, const float *__restrict__ Fg, const float *__restrict__ Gg,
+                                const float *__restrict__ O, const float *__restrict__ HNEW, const float *__restrict__ cprev,
+                                const uint8_t *__restrict__ succ_t, float *__restrict__ dh, float *__restrict__ dc, float *__restrict__ D,
+                                float *__restrict__ AV, int H, int A, uint64_t E, const int *skip_flag) {
+    if (skip_flag && *skip_flag) return;
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (uint64_t)H * E) return;
+    const uint64_t j = i / E, e = i - j * E, HE = (uint64_t)H * E;
+    const uint8_t sc = succ_t[e];
+    if (sc == RL_PAD) {
+        D[i] = 0.0f; D[HE + i] = 0.0f; D[2 * HE + i] = 0.0f; D[3 * HE + i] = 0.0f;
+        AV[i] = 0.0f;
+        dh[i] = 0.0f;
+        dc[i] = 0.0f;
+        return;
+    }
+    const float *lw = theta + o_lw;
+    float da = 0.0f;
+    for (int k = 0; k < A; ++k) da = fmaf(lw[k * H + j], dz_t[(uint64_t)k * E + e], da);
+    const float hnew = HNEW[i], av = rl_activate(act, hnew);
+    AV[i] = av;
+    const bool last = sc != RL_CONTINUE;  // last step of its episode: nothing flows back from t + 1
+    const float dhn = fmaf(act_grad_b(act, hnew, av), da, last ? 0.0f : dh[i]);
+    const float ig = I[i], fg = Fg[i], gg = Gg[i], og = O[i], cp = cprev[i];
+    const float tc = tanhf(__fadd_rn(__fmul_rn(fg, cp), __fmul_rn(ig, gg)));
+    const float dcn = (last ? 0.0f : dc[i]) + dhn * og * (1.0f - tc * tc);
+    D[i] = dcn * gg * ig * (1.0f - ig);
+    D[HE + i] = dcn * cp * fg * (1.0f - fg);
+    D[2 * HE + i] = dcn * ig * (1.0f - gg * gg);
+    D[3 * HE + i] = dhn * tc * og * (1.0f - og);
+    dc[i] = dcn * fg;
+    dh[i] = 0.0f;
+}
+
+// the partial row: parameter order w_ih, w_hh, b_ih, b_hh, lw, lb, then loss, kl, entropy, count.  An LSTM's rows of dWc are
+// its parameter rows in order (Wc = [W_ih | W_hh]), and its two bias gradients are the same column.
+template <int CELL>
+__device__ __forceinline__ void assemble(const double *__restrict__ dWc, const double *__restrict__ dHead, const double *__restrict__ scal_part,
+                                         int nscal, int F, int H, int A, int backward, double *__restrict__ row, const int *skip_flag) {
     if (skip_flag && *skip_flag) return;
     const int KP = F + H, NB = KP + 1, NH = H + 1;
-    const int o_whh = 3 * H * F, o_bih = o_whh + 3 * H * H, o_bhh = o_bih + 3 * H, o_lw = o_bhh + 3 * H, o_lb = o_lw + A * H, P = o_lb + A;
+    constexpr int NG = rl_cell_gates(CELL);
+    const int o_whh = NG * H * F, o_bih = o_whh + NG * H * H, o_bhh = o_bih + NG * H, o_lw = o_bhh + NG * H, o_lb = o_lw + A * H, P = o_lb + A;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < P; i += gridDim.x * blockDim.x) {
         double v = 0.0;
-        if (backward) {
+        if (CELL == RL_CELL_LSTM && backward && i < o_lw) {
+            if (i < o_whh) {
+                const int row_ = i / F, f = i - row_ * F;
+                v = dWc[(size_t)row_ * NB + f];
+            } else if (i < o_bih) {
+                const int q = i - o_whh, row_ = q / H, k = q - row_ * H;
+                v = dWc[(size_t)row_ * NB + F + k];
+            } else {
+                v = dWc[(size_t)((i - o_bih) % (4 * H)) * NB + KP];
+            }
+        } else if (backward) {
             if (i < o_whh) {  // w_ih[g H + j][f]: gates r, u from blocks 0, 1; n from block 3 (input part)
                 const int row_ = i / F, f = i - row_ * F, g = row_ / H, j = row_ - g * H, blk = g < 2 ? g : 3;
                 v = dWc[(size_t)(blk * H + j) * NB + f];
@@ -553,6 +668,16 @@ __global__ void big_assemble_kernel(const double *__restrict__ dWc, const double
         }
         if (ln == 0) row[P + sc] = red[sc][0];
     }
+}
+
+__global__ void big_assemble_kernel(const double *__restrict__ dWc, const double *__restrict__ dHead, const double *__restrict__ scal_part,
+                                    int nscal, int F, int H, int A, int backward, double *__restrict__ row, const int *skip_flag) {
+    assemble<RL_CELL_GRU>(dWc, dHead, scal_part, nscal, F, H, A, backward, row, skip_flag);
+}
+
+__global__ void lstm_assemble_kernel(const double *__restrict__ dWc, const double *__restrict__ dHead, const double *__restrict__ scal_part,
+                                     int nscal, int F, int H, int A, int backward, double *__restrict__ row, const int *skip_flag) {
+    assemble<RL_CELL_LSTM>(dWc, dHead, scal_part, nscal, F, H, A, backward, row, skip_flag);
 }
 
 // outputs of the Linear head for one step: out[k][e] = lb[k] + sum_j lw[k][j] act(hnew[j][e]); zero where `only` is given and
@@ -652,6 +777,8 @@ rl_status rl_seq_big_pass_launch(rl_ctx *ctx, int mode, const rl_seq_pass_args &
     const bool fvp = mode == RL_PASS_FVP;
     const bool backward = mode == RL_PASS_GRAD || mode == RL_PASS_FVP || mode == RL_PASS_VALUE || mode == RL_PASS_PPO ||
                           mode == RL_PASS_REINFORCE || mode == RL_PASS_QLOSS;
+    const bool lstm = a.cell == RL_CELL_LSTM;
+    const int NG = rl_cell_gates(a.cell);
     const int *skip = a.skip_flag;
     // ---- scratch (second context scratch: the plan and hbuf / dzbuf / logp0 live in the first) ----
     const int splits = 32;
@@ -659,7 +786,7 @@ rl_status rl_seq_big_pass_launch(rl_ctx *ctx, int mode, const rl_seq_pass_args &
     auto al = [](size_t b) { return (b + 255) / 256 * 256; };
     size_t off = 0;
     auto take = [&](size_t bytes) { const size_t o = off; off += al(bytes); return o; };
-    const size_t o_Wc = take((size_t)4 * H * KP * 4), o_bc = take((size_t)4 * H * 4), o_WhT = take((size_t)3 * H * H * 4);
+    const size_t o_Wc = take((size_t)4 * H * KP * 4), o_bc = take((size_t)4 * H * 4), o_WhT = take((size_t)NG * H * H * 4);
     const size_t o_Vc = take((size_t)4 * H * KP * 4), o_vbc = take((size_t)4 * H * 4);
     const size_t o_G = take(4 * HE * 4), o_tG = take(fvp ? 4 * HE * 4 : 0), o_thp = take(fvp ? HE * 4 : 0), o_dh = take(backward ? HE * 4 : 0);
     const size_t plane = T * HE * 4;
@@ -667,8 +794,9 @@ rl_status rl_seq_big_pass_launch(rl_ctx *ctx, int mode, const rl_seq_pass_args &
     const size_t o_AV = take(backward ? plane : 0), o_TH = take(fvp ? plane : 0), o_D = take(backward ? 4 * plane : 0);
     const size_t o_partW = take(backward ? (size_t)splits * 4 * H * NB * 8 : 0), o_partH = take(backward ? (size_t)splits * A * NH * 8 : 0);
     const size_t o_dWc = take((size_t)4 * H * NB * 8), o_dHead = take((size_t)A * NH * 8), o_scal = take((size_t)head_blocks * 4 * 8);
-    // tensor-core form of the per-step GEMMs (gru_big_tc.cuh): weight pieces of the three matrices
-    const bool use_tc = H == 128 && seq_tc_enabled();
+    const size_t o_CP = take(lstm ? plane : 0), o_tcp = take(lstm && fvp ? HE * 4 : 0), o_dc = take(lstm && backward ? HE * 4 : 0);
+    // tensor-core form of the per-step GEMMs (gru_big_tc.cuh, GRU cells only): weight pieces of the three matrices
+    const bool use_tc = H == 128 && seq_tc_enabled() && !lstm;
     const int stW = (KP + 15) / 16, stT = (KP + H + 15) / 16, stB = (3 * H + 15) / 16;
     const size_t o_wpW = take(use_tc ? (size_t)stW * bt::bt_b_stage(512) : 0), o_wpT = take(use_tc && fvp ? (size_t)stT * bt::bt_b_stage(512) : 0);
     const size_t o_wpB = take(use_tc && backward ? (size_t)stB * bt::bt_b_stage(128) : 0);
@@ -688,6 +816,7 @@ rl_status rl_seq_big_pass_launch(rl_ctx *ctx, int mode, const rl_seq_pass_args &
     pl.G = (float *)(base + o_G); pl.tG = (float *)(base + o_tG); pl.thp = (float *)(base + o_thp); pl.dh = (float *)(base + o_dh);
     pl.R = (float *)(base + o_R); pl.U = (float *)(base + o_U); pl.N = (float *)(base + o_N); pl.HN = (float *)(base + o_HN);
     pl.HNEW = (float *)(base + o_HNEW); pl.AV = (float *)(base + o_AV); pl.THNEW = (float *)(base + o_TH); pl.D = (float *)(base + o_D);
+    pl.CP = (float *)(base + o_CP); pl.tcp = (float *)(base + o_tcp); pl.dc = (float *)(base + o_dc);
     double *partW = (double *)(base + o_partW), *partH = (double *)(base + o_partH), *dWc = (double *)(base + o_dWc),
            *dHead = (double *)(base + o_dHead), *scal_part = (double *)(base + o_scal);
     const unsigned pw_grid = (unsigned)rl_div_up(HE, 256);
@@ -705,8 +834,9 @@ rl_status rl_seq_big_pass_launch(rl_ctx *ctx, int mode, const rl_seq_pass_args &
     }
 
     // ---- forward (and the tangent along a.vec) ----
-    RL_LAUNCH(ctx, big_comb_kernel, 64, 256, 0, a.theta, F, H, Wc, bc, WhT);
-    if (fvp) RL_LAUNCH(ctx, big_comb_kernel, 64, 256, 0, a.vec, F, H, Vc, vbc, (float *)nullptr);
+    auto comb = lstm ? lstm_comb_kernel : big_comb_kernel;
+    RL_LAUNCH(ctx, comb, 64, 256, 0, a.theta, F, H, Wc, bc, WhT);
+    if (fvp) RL_LAUNCH(ctx, comb, 64, 256, 0, a.vec, F, H, Vc, vbc, (float *)nullptr);
     if (use_tc) {
         RL_LAUNCH(ctx, bt::big_pieces_kernel, 128, 256, 0, Wc, KP, KP, (const float *)nullptr, 0, 0, 4 * H, stW, wpW);
         if (fvp) RL_LAUNCH(ctx, bt::big_pieces_kernel, 128, 256, 0, Vc, KP, KP, Wc + F, KP, H, 4 * H, stT, wpT);
@@ -714,6 +844,8 @@ rl_status rl_seq_big_pass_launch(rl_ctx *ctx, int mode, const rl_seq_pass_args &
     }
     RL_LAUNCH(ctx, big_zero_kernel, 256, 256, 0, a.hbuf, HE, skip);  // SeqIterative::initial_state (gru.rs:23-28)
     if (fvp) RL_LAUNCH(ctx, big_zero_kernel, 256, 256, 0, pl.thp, HE, skip);
+    if (lstm) RL_LAUNCH(ctx, big_zero_kernel, 256, 256, 0, pl.CP, HE, skip);
+    if (lstm && fvp) RL_LAUNCH(ctx, big_zero_kernel, 256, 256, 0, pl.tcp, HE, skip);
     for (uint64_t t = 0; t < T; ++t) {
         const float *x_t = a.obs + t * (uint64_t)F * E, *hp_t = a.hbuf + t * HE;
         const uint8_t *succ_t = a.succ + t * E;
@@ -730,13 +862,22 @@ rl_status rl_seq_big_pass_launch(rl_ctx *ctx, int mode, const rl_seq_pass_args &
             continue;
         }
         RL_TRY(gemm_nn(ctx, Wc, KP, x_t, hp_t, F, E, pl.G, E, bc, 0, 4 * H, E, KP, skip));
-        RL_LAUNCH(ctx, big_gates_kernel, pw_grid, 256, 0, pl.G, hp_t, succ_t, pl.R + t * HE, pl.U + t * HE, pl.N + t * HE, pl.HN + t * HE,
-                  pl.HNEW + t * HE, t + 1 < T ? a.hbuf + (t + 1) * HE : (float *)nullptr, H, E, skip);
+        if (lstm)
+            RL_LAUNCH(ctx, lstm_gates_kernel, pw_grid, 256, 0, pl.G, pl.CP + t * HE, succ_t, pl.R + t * HE, pl.U + t * HE, pl.N + t * HE,
+                      pl.HN + t * HE, pl.HNEW + t * HE, (float *)nullptr, t + 1 < T ? a.hbuf + (t + 1) * HE : (float *)nullptr,
+                      t + 1 < T ? pl.CP + (t + 1) * HE : (float *)nullptr, H, E, skip);
+        else
+            RL_LAUNCH(ctx, big_gates_kernel, pw_grid, 256, 0, pl.G, hp_t, succ_t, pl.R + t * HE, pl.U + t * HE, pl.N + t * HE, pl.HN + t * HE,
+                      pl.HNEW + t * HE, t + 1 < T ? a.hbuf + (t + 1) * HE : (float *)nullptr, H, E, skip);
         if (fvp) {
             RL_TRY(gemm_nn(ctx, Vc, KP, x_t, hp_t, F, E, pl.tG, E, vbc, 0, 4 * H, E, KP, skip));
             RL_TRY(gemm_nn(ctx, Wc + F, KP, pl.thp, pl.thp, H, E, pl.tG, E, nullptr, 1, 4 * H, E, H, skip));
-            RL_LAUNCH(ctx, big_gates_tan_kernel, pw_grid, 256, 0, pl.tG, pl.R + t * HE, pl.U + t * HE, pl.N + t * HE, pl.HN + t * HE, hp_t,
-                      pl.thp, pl.THNEW + t * HE, succ_t, H, E, skip);
+            if (lstm)
+                RL_LAUNCH(ctx, lstm_gates_tan_kernel, pw_grid, 256, 0, pl.tG, pl.R + t * HE, pl.U + t * HE, pl.N + t * HE, pl.HN + t * HE,
+                          pl.CP + t * HE, pl.thp, pl.tcp, pl.THNEW + t * HE, succ_t, H, E, skip);
+            else
+                RL_LAUNCH(ctx, big_gates_tan_kernel, pw_grid, 256, 0, pl.tG, pl.R + t * HE, pl.U + t * HE, pl.N + t * HE, pl.HN + t * HE, hp_t,
+                          pl.thp, pl.THNEW + t * HE, succ_t, H, E, skip);
         }
     }
     switch (mode) {
@@ -752,12 +893,18 @@ rl_status rl_seq_big_pass_launch(rl_ctx *ctx, int mode, const rl_seq_pass_args &
     }
     // ---- backward through time, then the weight gradients as two split-K GEMMs over all (t, e) ----
     if (backward) {
-        const int o_lw = 3 * H * F + 3 * H * H + 6 * H;
+        const int o_lw = NG * H * F + NG * H * H + 2 * NG * H;
         RL_LAUNCH(ctx, big_zero_kernel, 256, 256, 0, pl.dh, HE, skip);
+        if (lstm) RL_LAUNCH(ctx, big_zero_kernel, 256, 256, 0, pl.dc, HE, skip);
         for (int64_t t = (int64_t)T - 1; t >= 0; --t) {
-            RL_LAUNCH(ctx, big_bwd_kernel, pw_grid, 256, 0, a.dzbuf + (uint64_t)t * A * E, a.theta, o_lw, a.act, pl.R + t * HE, pl.U + t * HE,
-                      pl.N + t * HE, pl.HN + t * HE, pl.HNEW + t * HE, a.hbuf + t * HE, a.succ + (uint64_t)t * E, pl.dh, pl.D + (uint64_t)t * 4 * HE,
-                      pl.AV + t * HE, H, A, E, skip);
+            if (lstm)
+                RL_LAUNCH(ctx, lstm_bwd_kernel, pw_grid, 256, 0, a.dzbuf + (uint64_t)t * A * E, a.theta, o_lw, a.act, pl.R + t * HE, pl.U + t * HE,
+                          pl.N + t * HE, pl.HN + t * HE, pl.HNEW + t * HE, pl.CP + t * HE, a.succ + (uint64_t)t * E, pl.dh, pl.dc,
+                          pl.D + (uint64_t)t * 4 * HE, pl.AV + t * HE, H, A, E, skip);
+            else
+                RL_LAUNCH(ctx, big_bwd_kernel, pw_grid, 256, 0, a.dzbuf + (uint64_t)t * A * E, a.theta, o_lw, a.act, pl.R + t * HE, pl.U + t * HE,
+                          pl.N + t * HE, pl.HN + t * HE, pl.HNEW + t * HE, a.hbuf + t * HE, a.succ + (uint64_t)t * E, pl.dh,
+                          pl.D + (uint64_t)t * 4 * HE, pl.AV + t * HE, H, A, E, skip);
             if (t > 0) {
                 const float *D_t = pl.D + (uint64_t)t * 4 * HE;
                 if (use_tc) {
@@ -766,7 +913,7 @@ rl_status rl_seq_big_pass_launch(rl_ctx *ctx, int mode, const rl_seq_pass_args &
                     g.out = pl.dh; g.skip_flag = skip;
                     RL_TRY((launch_tc<128, bt::EPI_ACC>(ctx, g)));
                 } else {
-                    RL_TRY(gemm_nn(ctx, WhT, 3 * H, D_t, D_t, 3 * H, E, pl.dh, E, nullptr, 1, H, E, 3 * H, skip));
+                    RL_TRY(gemm_nn(ctx, WhT, NG * H, D_t, D_t, NG * H, E, pl.dh, E, nullptr, 1, H, E, NG * H, skip));
                 }
             }
         }
@@ -792,23 +939,28 @@ rl_status rl_seq_big_pass_launch(rl_ctx *ctx, int mode, const rl_seq_pass_args &
         RL_LAUNCH(ctx, gemm_nt_splitk_kernel, gH, NT_THREADS, 0, a.dzbuf, A, pl.AV, H, (const float *)nullptr, 0, T, E, partH, NH, splits, skip);
         RL_LAUNCH(ctx, splitk_reduce_kernel, (unsigned)rl_div_up(A * NH, 256), 256, 0, partH, splits, A * NH, dHead, skip);
     }
-    RL_LAUNCH(ctx, big_assemble_kernel, 32, 256, 0, dWc, dHead, scal_part, head_blocks, F, H, A, backward ? 1 : 0, a.partials, skip);
+    if (lstm)
+        RL_LAUNCH(ctx, lstm_assemble_kernel, 32, 256, 0, dWc, dHead, scal_part, head_blocks, F, H, A, backward ? 1 : 0, a.partials, skip);
+    else
+        RL_LAUNCH(ctx, big_assemble_kernel, 32, 256, 0, dWc, dHead, scal_part, head_blocks, F, H, A, backward ? 1 : 0, a.partials, skip);
     return RL_OK;
 }
 
 // SeqPacked::seq_packed over a stored trajectory (gru.rs:72-102 -> chain.rs:157-168) in the GEMM form: out f32 [T][A][E] (zeros
 // on padding) and, when out_next is given, the module's output on the successor observation of every interrupted step
 // (features.rs:139-185: one more step of the same sequence).  What rl_gae_seq needs from a hidden-128 critic.
-rl_status rl_seq_big_forward(rl_ctx *ctx, const float *params, int F, int H, int A, int act, const float *obs, const float *next_obs,
-                             const uint8_t *succ, uint64_t T, uint64_t E, float *out, float *out_next) {
+rl_status rl_seq_big_forward(rl_ctx *ctx, int cell, const float *params, int F, int H, int A, int act, const float *obs,
+                             const float *next_obs, const uint8_t *succ, uint64_t T, uint64_t E, float *out, float *out_next) {
     const int KP = F + H;
+    const bool lstm = cell == RL_CELL_LSTM;
     const uint64_t HE = (uint64_t)H * E;
     auto al = [](size_t b) { return (b + 255) / 256 * 256; };
     size_t off = 0;
     auto take = [&](size_t bytes) { const size_t o = off; off += al(bytes); return o; };
     const size_t o_Wc = take((size_t)4 * H * KP * 4), o_bc = take((size_t)4 * H * 4), o_G = take(4 * HE * 4);
     const size_t o_tmp = take(4 * HE * 4), o_hn = take(HE * 4), o_h2 = take(HE * 4), o_ha = take(HE * 4), o_hb = take(HE * 4);
-    const bool use_tc = H == 128 && seq_tc_enabled();
+    const size_t o_ca = take(lstm ? HE * 4 : 0), o_cb = take(lstm ? HE * 4 : 0), o_c2 = take(lstm ? HE * 4 : 0);
+    const bool use_tc = H == 128 && seq_tc_enabled() && !lstm;
     const int stW = (KP + 15) / 16;
     const size_t o_wpW = take(use_tc ? (size_t)stW * bt::bt_b_stage(512) : 0);
     char *base;
@@ -816,11 +968,27 @@ rl_status rl_seq_big_forward(rl_ctx *ctx, const float *params, int F, int H, int
     uint16_t *wpW = (uint16_t *)(base + o_wpW);
     float *Wc = (float *)(base + o_Wc), *bc = (float *)(base + o_bc), *G = (float *)(base + o_G), *tmp = (float *)(base + o_tmp);
     float *hnew = (float *)(base + o_hn), *h2 = (float *)(base + o_h2), *hcur = (float *)(base + o_ha), *hnxt = (float *)(base + o_hb);
+    float *ccur = (float *)(base + o_ca), *cnxt = (float *)(base + o_cb), *c2 = (float *)(base + o_c2);
     const unsigned pw_grid = (unsigned)rl_div_up(HE, 256), e_grid = (unsigned)rl_div_up(E, 128);
-    const int o_lw = 3 * H * F + 3 * H * H + 6 * H;
+    const int NG = rl_cell_gates(cell), o_lw = NG * H * F + NG * H * H + 2 * NG * H;
     const size_t hsmem = (size_t)(A * H + A) * sizeof(float);
-    RL_LAUNCH(ctx, big_comb_kernel, 64, 256, 0, params, F, H, Wc, bc, (float *)nullptr);
+    auto comb = lstm ? lstm_comb_kernel : big_comb_kernel;
+    RL_LAUNCH(ctx, comb, 64, 256, 0, params, F, H, Wc, bc, (float *)nullptr);
     RL_LAUNCH(ctx, big_zero_kernel, 256, 256, 0, hcur, HE, (const int *)nullptr);
+    if (lstm) RL_LAUNCH(ctx, big_zero_kernel, 256, 256, 0, ccur, HE, (const int *)nullptr);
+    // one cell step over all lanes: gates into tmp, h' into hout (an LSTM's c' into cout), the next step's state (zero after an
+    // episode's end) into hnext / cnext
+    auto cell_fp32 = [&](const float *x, const float *hp, const float *cp, const uint8_t *succ_t, float *hout, float *cout, float *hnext,
+                         float *cnext) -> rl_status {
+        RL_TRY(gemm_nn(ctx, Wc, KP, x, hp, F, E, G, E, bc, 0, 4 * H, E, KP, nullptr));
+        if (lstm)
+            RL_LAUNCH(ctx, lstm_gates_kernel, pw_grid, 256, 0, G, cp, succ_t, tmp, tmp + HE, tmp + 2 * HE, tmp + 3 * HE, hout, cout, hnext,
+                      cnext, H, E, (const int *)nullptr);
+        else
+            RL_LAUNCH(ctx, big_gates_kernel, pw_grid, 256, 0, G, hp, succ_t, tmp, tmp + HE, tmp + 2 * HE, tmp + 3 * HE, hout, hnext, H, E,
+                      (const int *)nullptr);
+        return RL_OK;
+    };
     if (use_tc) RL_LAUNCH(ctx, bt::big_pieces_kernel, 128, 256, 0, Wc, KP, KP, (const float *)nullptr, 0, 0, 4 * H, stW, wpW);
     auto cell_tc = [&](const float *x, const float *hp, const uint8_t *succ_t, float *hout, float *hnext) -> rl_status {
         bt::BtArgs g{};
@@ -841,18 +1009,16 @@ rl_status rl_seq_big_forward(rl_ctx *ctx, const float *params, int F, int H, int
             std::swap(hcur, hnxt);
             continue;
         }
-        RL_TRY(gemm_nn(ctx, Wc, KP, obs + t * (uint64_t)F * E, hcur, F, E, G, E, bc, 0, 4 * H, E, KP, nullptr));
-        RL_LAUNCH(ctx, big_gates_kernel, pw_grid, 256, 0, G, hcur, succ_t, tmp, tmp + HE, tmp + 2 * HE, tmp + 3 * HE, hnew, hnxt, H, E,
-                  (const int *)nullptr);
+        // the successor step of an interrupted episode continues from (h', c') before they are cut at the episode's end
+        RL_TRY(cell_fp32(obs + t * (uint64_t)F * E, hcur, ccur, succ_t, hnew, lstm && out_next ? c2 : (float *)nullptr, hnxt, cnxt));
         RL_LAUNCH(ctx, big_head_out_kernel, e_grid, 128, hsmem, params, o_lw, act, hnew, succ_t, -1, out + t * (uint64_t)A * E, H, A, E);
         if (out_next) {
-            RL_TRY(gemm_nn(ctx, Wc, KP, next_obs + t * (uint64_t)F * E, hnew, F, E, G, E, bc, 0, 4 * H, E, KP, nullptr));
-            RL_LAUNCH(ctx, big_gates_kernel, pw_grid, 256, 0, G, hnew, succ_t, tmp, tmp + HE, tmp + 2 * HE, tmp + 3 * HE, h2, (float *)nullptr, H,
-                      E, (const int *)nullptr);
+            RL_TRY(cell_fp32(next_obs + t * (uint64_t)F * E, hnew, c2, succ_t, h2, (float *)nullptr, (float *)nullptr, (float *)nullptr));
             RL_LAUNCH(ctx, big_head_out_kernel, e_grid, 128, hsmem, params, o_lw, act, h2, succ_t, (int)RL_INTERRUPT,
                       out_next + t * (uint64_t)A * E, H, A, E);
         }
         std::swap(hcur, hnxt);
+        std::swap(ccur, cnxt);
     }
     return RL_OK;
 }

@@ -16,6 +16,11 @@
 // Hessian-vector product.  Per-thread gradients (f32, <= T terms) are summed in f64 in a fixed order into one
 // partial row per block, then reduced like the MLP passes (update.cu).
 //
+// CELL = RL_CELL_LSTM runs the same passes for Chain<Lstm, Linear> (lstm_cell, gate order i, f, g, o): the forward stores
+// (h, c) before each step (hbuf, cbuf), FVP carries the tangents (th, tc), BPTT carries (dh, dc), both cut at episode ends:
+//   dc = dc_carry + dh' o (1 - tanh^2 c'),  D = (dc g i(1-i), dc c_prev f(1-f), dc i (1-g^2), dh' tanh(c') o(1-o)),
+//   dc_carry = dc f,  dh_carry = W_hh^T D.
+//
 // Sizes: hidden <= 8, features <= 20, actions <= 16 (the rnn.rs-sized and small rl2 bandit modules).  The
 // rl2-sized hidden 128 belongs on tensor cores and is not served by this kernel (DESIGN.md section 9).
 #include "handles.cuh"
@@ -32,10 +37,11 @@ __device__ __forceinline__ float sigm(float v) { return __fdividef(1.0f, 1.0f + 
 
 struct Dims {
     int F, H, A, act;
-    __device__ int o_whh() const { return 3 * H * F; }
-    __device__ int o_bih() const { return o_whh() + 3 * H * H; }
-    __device__ int o_bhh() const { return o_bih() + 3 * H; }
-    __device__ int o_lw() const { return o_bhh() + 3 * H; }
+    int NG;  // gates per unit: 3 (GRU) or 4 (LSTM)
+    __device__ int o_whh() const { return NG * H * F; }
+    __device__ int o_bih() const { return o_whh() + NG * H * H; }
+    __device__ int o_bhh() const { return o_bih() + NG * H; }
+    __device__ int o_lw() const { return o_bhh() + NG * H; }
     __device__ int o_lb() const { return o_lw() + A * H; }
     __device__ int P() const { return o_lb() + A; }
 };
@@ -66,6 +72,31 @@ __device__ __forceinline__ void gru_gates(const Dims &d, const float *__restrict
     }
 }
 
+// activated gates of one lstm_cell from (x, h): i, f, o = sigmoid, g = tanh of (W_ih x + b_ih) + (W_hh h + b_hh)
+__device__ __forceinline__ void lstm_gates(const Dims &d, const float *__restrict__ w, const float *x, const float *h, float *ig, float *fg,
+                                           float *gg, float *og) {
+    const int F = d.F, H = d.H;
+    const float *w_ih = w, *w_hh = w + d.o_whh(), *b_ih = w + d.o_bih(), *b_hh = w + d.o_bhh();
+#pragma unroll
+    for (int j = 0; j < H; ++j) {
+        float s[4];
+#pragma unroll
+        for (int g = 0; g < 4; ++g) {
+            const int row = g * H + j;
+            float a = b_ih[row], b = b_hh[row];
+#pragma unroll
+            for (int f = 0; f < F; ++f) a = fmaf(w_ih[row * F + f], x[f], a);
+#pragma unroll
+            for (int k = 0; k < H; ++k) b = fmaf(w_hh[row * H + k], h[k], b);
+            s[g] = __fadd_rn(a, b);
+        }
+        ig[j] = sigm(s[0]);
+        fg[j] = sigm(s[1]);
+        gg[j] = tanhf(s[2]);
+        og[j] = sigm(s[3]);
+    }
+}
+
 __device__ __forceinline__ float act_fwd(int act, float v) { return rl_activate(act, v); }
 __device__ __forceinline__ float act_grad(int act, float pre, float out) {
     switch (act) {
@@ -76,12 +107,74 @@ __device__ __forceinline__ float act_grad(int act, float pre, float out) {
     }
 }
 
+// Back-propagation through time of one lane of an LSTM (len valid steps), accumulating into the per-thread gradient g:
+// gates recomputed from (x_t, h_{t-1}, c_{t-1}) stored by the forward, both carries cut at episode ends.
+template <int GH, int GF, int GA>
+__device__ __forceinline__ void lstm_bptt(const rl_seq_pass_args &a, const Dims &d, const float *__restrict__ sw, float *g, uint64_t len,
+                                          uint64_t e) {
+    const int F = d.F, H = d.H, A = d.A;
+    const uint64_t E = a.E;
+    const float *w_hh = sw + d.o_whh(), *lw = sw + d.o_lw();
+    float *g_ih = g, *g_hh = g + d.o_whh(), *gb_ih = g + d.o_bih(), *gb_hh = g + d.o_bhh(), *g_lw = g + d.o_lw(), *g_lb = g + d.o_lb();
+    float dh[GH], dc[GH];
+    for (int j = 0; j < H; ++j) dh[j] = dc[j] = 0.0f;
+    for (int64_t t = (int64_t)len - 1; t >= 0; --t) {
+        if (a.succ[t * E + e] != RL_CONTINUE)
+            for (int j = 0; j < H; ++j) dh[j] = dc[j] = 0.0f;  // last step of its episode: nothing flows back from t + 1
+        float x[GF], hp[GH], cp[GH], dz[GA];
+        for (int f = 0; f < F; ++f) x[f] = a.obs[(t * F + f) * E + e];
+        for (int j = 0; j < H; ++j) {
+            hp[j] = a.hbuf[(t * H + j) * E + e];
+            cp[j] = a.cbuf[(t * H + j) * E + e];
+        }
+        for (int k = 0; k < A; ++k) dz[k] = a.dzbuf[(t * A + k) * E + e];
+        float ig[GH], fg[GH], gg[GH], og[GH];
+        lstm_gates(d, sw, x, hp, ig, fg, gg, og);
+        float D[4 * GH], dhp[GH];
+        for (int j = 0; j < H; ++j) {
+            const float cn = __fadd_rn(__fmul_rn(fg[j], cp[j]), __fmul_rn(ig[j], gg[j]));
+            const float tc = tanhf(cn);
+            const float hn = __fmul_rn(og[j], tc);
+            const float av = act_fwd(d.act, hn);
+            float da = 0.0f;
+            for (int k = 0; k < A; ++k) {
+                da = fmaf(lw[k * H + j], dz[k], da);
+                g_lw[k * H + j] = fmaf(dz[k], av, g_lw[k * H + j]);
+            }
+            const float dhn = fmaf(act_grad(d.act, hn, av), da, dh[j]);
+            const float dcn = dc[j] + dhn * og[j] * (1.0f - tc * tc);
+            D[j] = dcn * gg[j] * ig[j] * (1.0f - ig[j]);
+            D[H + j] = dcn * cp[j] * fg[j] * (1.0f - fg[j]);
+            D[2 * H + j] = dcn * ig[j] * (1.0f - gg[j] * gg[j]);
+            D[3 * H + j] = dhn * tc * og[j] * (1.0f - og[j]);
+            dc[j] = dcn * fg[j];
+            dhp[j] = 0.0f;
+        }
+        for (int k = 0; k < A; ++k) g_lb[k] += dz[k];
+        for (int row = 0; row < 4 * H; ++row) {
+            const float dg = D[row];
+            gb_ih[row] += dg;
+            gb_hh[row] += dg;
+            for (int f = 0; f < F; ++f) g_ih[row * F + f] = fmaf(dg, x[f], g_ih[row * F + f]);
+            for (int k = 0; k < H; ++k) {
+                g_hh[row * H + k] = fmaf(dg, hp[k], g_hh[row * H + k]);
+                dhp[k] = fmaf(w_hh[row * H + k], dg, dhp[k]);
+            }
+        }
+        for (int j = 0; j < H; ++j) dh[j] = dhp[j];
+    }
+}
+
 // TF / TH / TA > 0 fix the sizes at compile time (every loop unrolls, every per-thread array -- the 150-odd gradient
 // accumulators included -- lives in registers); 0 = sizes from the arguments, arrays of the maximum sizes in local memory.
-template <int MODE, int TF, int TH, int TA>
+// CELL: RL_CELL_GRU, or RL_CELL_LSTM (run-time sizes only).  The body stays in the kernel itself: moved into a device
+// function behind two kernels, the compile-time-sized GRU instances spilled more (ptxas) and the config-4 update ran 8 % slower.
+template <int MODE, int TF, int TH, int TA, int CELL = RL_CELL_GRU>
 __global__ void __launch_bounds__(RL_SEQ_BLOCK) gru_pass_kernel(rl_seq_pass_args a) {
     constexpr int GH = TH ? TH : GH_MAX, GF = TF ? TF : GF_MAX, GA = TA ? TA : GA_MAX;
-    constexpr int GP_MAX = 3 * GH * GF + 3 * GH * GH + 6 * GH + GA * GH + GA;
+    constexpr bool LSTM = CELL == RL_CELL_LSTM;
+    constexpr int NG = rl_cell_gates(CELL), GC = LSTM ? GH : 1;
+    constexpr int GP_MAX = NG * GH * GF + NG * GH * GH + 2 * NG * GH + GA * GH + GA;
     constexpr bool BACKWARD = MODE == RL_PASS_GRAD || MODE == RL_PASS_FVP || MODE == RL_PASS_VALUE || MODE == RL_PASS_PPO ||
                               MODE == RL_PASS_REINFORCE || MODE == RL_PASS_QLOSS;
     constexpr bool IS_POLICY = MODE != RL_PASS_VALUE && MODE != RL_PASS_QLOSS;
@@ -90,7 +183,7 @@ __global__ void __launch_bounds__(RL_SEQ_BLOCK) gru_pass_kernel(rl_seq_pass_args
     constexpr bool USES_ADV = MODE == RL_PASS_EVAL || MODE == RL_PASS_GRAD || MODE == RL_PASS_PPO || MODE == RL_PASS_REINFORCE;
     constexpr bool USES_LP0 = MODE == RL_PASS_EVAL || MODE == RL_PASS_GRAD || MODE == RL_PASS_PPO;
     if (a.skip_flag && *a.skip_flag) return;
-    const Dims d{TF ? TF : a.F, TH ? TH : a.H, TA ? TA : a.A, a.act};
+    const Dims d{TF ? TF : a.F, TH ? TH : a.H, TA ? TA : a.A, a.act, NG};
     const int F = d.F, H = d.H, A = d.A, P = d.P();
     extern __shared__ __align__(16) unsigned char gsm[];
     float *sw = reinterpret_cast<float *>(gsm);      // theta [P]
@@ -114,6 +207,9 @@ __global__ void __launch_bounds__(RL_SEQ_BLOCK) gru_pass_kernel(rl_seq_pass_args
         float h[GH], hd[GH];
 #pragma unroll
         for (int j = 0; j < H; ++j) h[j] = hd[j] = 0.0f;
+        float c[GC], cd[GC];
+        if constexpr (LSTM)
+            for (int j = 0; j < H; ++j) c[j] = cd[j] = 0.0f;
         uint64_t len = 0;
         // software pipeline: the loads of step t + 1 are in flight while step t is computed (a step is ~400 dependent
         // instructions at 2 warps per scheduler: an exposed DRAM latency per step was 35 % of the stall cycles)
@@ -140,9 +236,42 @@ __global__ void __launch_bounds__(RL_SEQ_BLOCK) gru_pass_kernel(rl_seq_pass_args
             }
             if (BACKWARD)
                 for (int j = 0; j < H; ++j) a.hbuf[(t * H + j) * E + e] = h[j];
+            if constexpr (LSTM)
+                if (BACKWARD)
+                    for (int j = 0; j < H; ++j) a.cbuf[(t * H + j) * E + e] = c[j];
+            float hnew[GH], hdnew[GH], cnew[GC], cdnew[GC];
+            if constexpr (LSTM) {
+                float ig[GH], fg[GH], gg[GH], og[GH];
+                lstm_gates(d, sw, x, h, ig, fg, gg, og);
+#pragma unroll
+                for (int j = 0; j < H; ++j) {
+                    cnew[j] = __fadd_rn(__fmul_rn(fg[j], c[j]), __fmul_rn(ig[j], gg[j]));
+                    const float tc = tanhf(cnew[j]);
+                    hnew[j] = __fmul_rn(og[j], tc);
+                    if (FVP) {
+                        // forward-mode tangents along v of the four pre-activations, then of c' and h'
+                        const float *v_ih = sv, *v_hh = sv + d.o_whh(), *vb_ih = sv + d.o_bih(), *vb_hh = sv + d.o_bhh();
+                        const float *w_hh = sw + d.o_whh();
+                        float pd[4];
+#pragma unroll
+                        for (int q = 0; q < 4; ++q) {
+                            const int row = q * H + j;
+                            float p = vb_ih[row] + vb_hh[row];
+#pragma unroll
+                            for (int f = 0; f < F; ++f) p = fmaf(v_ih[row * F + f], x[f], p);
+#pragma unroll
+                            for (int k = 0; k < H; ++k) p = fmaf(v_hh[row * H + k], h[k], fmaf(w_hh[row * H + k], hd[k], p));
+                            pd[q] = p;
+                        }
+                        const float id = ig[j] * (1.0f - ig[j]) * pd[0], fd = fg[j] * (1.0f - fg[j]) * pd[1];
+                        const float gd = (1.0f - gg[j] * gg[j]) * pd[2], od = og[j] * (1.0f - og[j]) * pd[3];
+                        cdnew[j] = fd * c[j] + fg[j] * cd[j] + id * gg[j] + ig[j] * gd;
+                        hdnew[j] = od * tc + og[j] * (1.0f - tc * tc) * cdnew[j];
+                    }
+                }
+            } else {
             float r[GH], u[GH], n[GH], ghn[GH];
             gru_gates(d, sw, x, h, r, u, n, ghn);
-            float hnew[GH], hdnew[GH];
             if (FVP) {
                 // forward-mode tangents along v: gi' = V_ih x + v_bih ; gh' = V_hh h + W_hh h' + v_bhh
                 const float *v_ih = sv, *v_hh = sv + d.o_whh(), *vb_ih = sv + d.o_bih(), *vb_hh = sv + d.o_bhh();
@@ -169,6 +298,7 @@ __global__ void __launch_bounds__(RL_SEQ_BLOCK) gru_pass_kernel(rl_seq_pass_args
             }
 #pragma unroll
             for (int j = 0; j < H; ++j) hnew[j] = __fadd_rn(__fmul_rn(__fsub_rn(h[j], n[j]), u[j]), n[j]);
+            }
             // Chain: activation, Linear
             const float *lw = sw + d.o_lw(), *lb = sw + d.o_lb();
             float z[GA], zd[GA];
@@ -277,10 +407,16 @@ __global__ void __launch_bounds__(RL_SEQ_BLOCK) gru_pass_kernel(rl_seq_pass_args
             for (int j = 0; j < H; ++j) {
                 h[j] = done ? 0.0f : hnew[j];
                 if (FVP) hd[j] = done ? 0.0f : hdnew[j];
+                if constexpr (LSTM) {
+                    c[j] = done ? 0.0f : cnew[j];
+                    if (FVP) cd[j] = done ? 0.0f : cdnew[j];
+                }
             }
         }
         // ---------------- backward (BPTT) ----------------
-        if (BACKWARD) {
+        if constexpr (LSTM) {
+            if (BACKWARD) lstm_bptt<GH, GF, GA>(a, d, sw, g, len, e);
+        } else if (BACKWARD) {
             float dh[GH];
 #pragma unroll
             for (int j = 0; j < H; ++j) dh[j] = 0.0f;
@@ -390,10 +526,10 @@ __global__ void __launch_bounds__(RL_SEQ_BLOCK) gru_pass_kernel(rl_seq_pass_args
     }
 }
 
-template <int MODE, int TF, int TH, int TA>
+template <int MODE, int TF, int TH, int TA, int CELL = RL_CELL_GRU>
 rl_status launch_sized(rl_ctx *ctx, const rl_seq_pass_args &a, int grid, size_t smem) {
-    RL_CUDA(ctx, cudaFuncSetAttribute(gru_pass_kernel<MODE, TF, TH, TA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    RL_LAUNCH(ctx, (gru_pass_kernel<MODE, TF, TH, TA>), grid, RL_SEQ_BLOCK, smem, a);
+    RL_CUDA(ctx, cudaFuncSetAttribute(gru_pass_kernel<MODE, TF, TH, TA, CELL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    RL_LAUNCH(ctx, (gru_pass_kernel<MODE, TF, TH, TA, CELL>), grid, RL_SEQ_BLOCK, smem, a);
     return RL_OK;
 }
 
@@ -401,6 +537,7 @@ rl_status launch_sized(rl_ctx *ctx, const rl_seq_pass_args &a, int grid, size_t 
 template <int MODE>
 rl_status launch_mode(rl_ctx *ctx, const rl_seq_pass_args &a, int grid, size_t smem) {
     constexpr bool POLICY = MODE != RL_PASS_VALUE;  // the Q-loss pass has one output per action, like a policy
+    if (a.cell == RL_CELL_LSTM) return launch_sized<MODE, 0, 0, 0, RL_CELL_LSTM>(ctx, a, grid, smem);
     if (a.F == 6 && a.H == 4 && a.A == (POLICY ? 2 : 1)) return launch_sized<MODE, 6, 4, POLICY ? 2 : 1>(ctx, a, grid, smem);
     return launch_sized<MODE, 0, 0, 0>(ctx, a, grid, smem);
 }
@@ -413,7 +550,7 @@ bool rl_seq_pass_supports(int F, int H, int A) { return F >= 1 && F <= GF_MAX &&
 
 // One pass; writes `grid` partial rows of P + 4 doubles (order: loss, kl, entropy, count as in update.cu).
 rl_status rl_seq_pass_launch(rl_ctx *ctx, int mode, const rl_seq_pass_args &a, int grid) {
-    const int P = 3 * a.H * a.F + 3 * a.H * a.H + 6 * a.H + a.A * a.H + a.A;
+    const int NG = rl_cell_gates(a.cell), P = NG * a.H * a.F + NG * a.H * a.H + 2 * NG * a.H + a.A * a.H + a.A;
     const size_t smem_w = (size_t)2 * P * sizeof(float), smem_r = (size_t)(RL_SEQ_BLOCK / 32) * (P + 4) * sizeof(double);
     const size_t smem = smem_w > smem_r ? smem_w : smem_r;
     switch (mode) {

@@ -91,7 +91,10 @@ int rl_replay_num_features(rl_replay *rb);
 rl_status rl_replay_sample_seq_dev(rl_replay *rb, uint64_t minibatch_steps, uint64_t seed, uint32_t draw_index, int one_step_td,
                                    float discount, rl_grunet *q, rl_traj **out_traj, const float **out_target);
 
-struct rl_grunet_view { rl_ctx *ctx; int in_dim, hidden, out_dim, act; uint64_t n_params; float *params; };
+// The cell of a recurrent module (rl_grunet_create / rl_lstmnet_create); the kernel selectors below read it.
+enum { RL_CELL_GRU = 0, RL_CELL_LSTM = 1 };
+__host__ __device__ constexpr int rl_cell_gates(int cell) { return cell == RL_CELL_LSTM ? 4 : 3; }
+struct rl_grunet_view { rl_ctx *ctx; int in_dim, hidden, out_dim, act; uint64_t n_params; float *params; int cell; };
 rl_grunet_view rl_grunet_view_of(rl_grunet *g);
 rl_status rl_grunet_seq_enqueue(rl_grunet *g, rl_traj *traj, float *out_dev, float *out_next_dev);
 
@@ -112,6 +115,8 @@ struct rl_seq_pass_args {
     double *partials;
     const int *skip_flag;
     float clip_lo, clip_hi;
+    int cell;       // RL_CELL_GRU / RL_CELL_LSTM
+    float *cbuf;    // f32 [T][H][E]  LSTM: cell state before each step (K9)
 };
 // lanes per block (= per partial row) of the recurrent passes: two warps, so that a block's warps finish close together
 constexpr int RL_SEQ_BLOCK = 64;
@@ -125,8 +130,8 @@ bool rl_seq_big_cell_supports(int F, int H);
 size_t rl_seq_big_prepared_bytes(int F, int H);
 rl_status rl_seq_big_prepare(rl_ctx *ctx, const float *params, int F, int H, void *prepared);
 rl_status rl_seq_big_cell(rl_ctx *ctx, const void *prepared, int F, int H, const float *x, const float *h, uint64_t E, float *hnew);
-rl_status rl_seq_big_forward(rl_ctx *ctx, const float *params, int F, int H, int A, int act, const float *obs, const float *next_obs,
-                             const uint8_t *succ, uint64_t T, uint64_t E, float *out, float *out_next);
+rl_status rl_seq_big_forward(rl_ctx *ctx, int cell, const float *params, int F, int H, int A, int act, const float *obs,
+                             const float *next_obs, const uint8_t *succ, uint64_t T, uint64_t E, float *out, float *out_next);
 
 // gru.cu: fused rollout with a recurrent policy.  *partials_out receives the device pointer of its *nblocks_out rows of
 // per-block statistics (steps.cuh: ST_COUNT sums each), with one more row in front of them for the totals; rl_rollout

@@ -1563,7 +1563,7 @@ struct UpdateNet {
         return RL_OK;
     }
     // A recurrent module over `batch`: one block of RL_SEQ_BLOCK lanes per partial row; after the caller's scratch, the
-    // log-probabilities, the output cotangents and the hidden states of the batch.
+    // log-probabilities, the output cotangents and the hidden states of the batch (and an LSTM's cell states).
     rl_status init(rl_ctx *c, const rl_grunet_view &net, const PassArgs &batch, size_t extra_bytes) {
         ctx = c; P = (int)net.n_params; theta = net.params; recurrent = true;
         plan.P = P;
@@ -1572,18 +1572,20 @@ struct UpdateNet {
         const size_t rows = (size_t)plan.grid * plan.W * sizeof(double), sums = ((size_t)plan.W * sizeof(double) + 255) / 256 * 256;
         const size_t TE = (size_t)batch.T * batch.E;
         const size_t lp = (TE * net.out_dim * sizeof(float) + 255) / 256 * 256, hb = (TE * net.hidden * sizeof(float) + 255) / 256 * 256;
+        const size_t cb = net.cell == RL_CELL_LSTM ? hb : 0;
         extra_bytes = (extra_bytes + 255) / 256 * 256;
         char *buf;
-        RL_TRY(rl_ctx_scratch(ctx, ((rows + 255) / 256 * 256) + sums + extra_bytes + 2 * lp + hb + 256, (void **)&buf));
+        RL_TRY(rl_ctx_scratch(ctx, ((rows + 255) / 256 * 256) + sums + extra_bytes + 2 * lp + hb + cb + 256, (void **)&buf));
         plan.partials = (double *)buf;
         plan.sums = (double *)(buf + (rows + 255) / 256 * 256);
         extra = (char *)plan.sums + sums;
         args = batch;
         args.theta = theta;
         args.logp0 = (float *)(extra + extra_bytes);
-        seq.F = net.in_dim; seq.H = net.hidden; seq.A = net.out_dim; seq.act = net.act;
+        seq.F = net.in_dim; seq.H = net.hidden; seq.A = net.out_dim; seq.act = net.act; seq.cell = net.cell;
         seq.dzbuf = (float *)(extra + extra_bytes + lp);
         seq.hbuf = (float *)(extra + extra_bytes + 2 * lp);
+        seq.cbuf = cb ? (float *)(extra + extra_bytes + 2 * lp + hb) : nullptr;
         seq.partials = plan.partials;
         return RL_OK;
     }

@@ -1,4 +1,4 @@
-"""Mlp module (src/torch/modules/ff/mlp.rs) over the C ABI."""
+"""Mlp module (src/torch/modules/ff/mlp.rs) and the recurrent modules (GRU or LSTM, then a Linear) over the C ABI."""
 from __future__ import annotations
 
 import ctypes as C
@@ -129,15 +129,17 @@ def init_gru_linear_params(rng: np.random.Generator, in_dim: int, hidden: int, o
     return np.concatenate([np.asarray(p, np.float32).ravel() for p in parts])
 
 
-class GruLinear:
-    """One GRU layer -> activation -> Linear.  Flat parameters in Module::variables() order:
-    w_ih[3H,in], w_hh[3H,H], b_ih[3H], b_hh[3H] (rnn/mod.rs:223-258), kernel[out,H], bias[out] (linear.rs:108-110)."""
+class SeqLinear:
+    """The handle methods of a recurrent module -> activation -> Linear (one rl_grunet handle, GRU or LSTM cell).
+    Subclasses name the create call."""
+
+    _create = ""
 
     def __init__(self, ctx: Context, in_dim: int, hidden: int, out_dim: int, activation: str = "relu"):
         self.ctx, self._lib = ctx, ctx._lib
         self.in_dim, self.hidden, self.out_dim = in_dim, hidden, out_dim
         h = C.c_void_p()
-        L.check(self._lib.rl_grunet_create(ctx.handle, in_dim, hidden, out_dim, ACTIVATIONS[activation], C.byref(h)),
+        L.check(getattr(self._lib, self._create)(ctx.handle, in_dim, hidden, out_dim, ACTIVATIONS[activation], C.byref(h)),
                 ctx.handle)
         self.handle = h
         n = C.c_uint64()
@@ -173,3 +175,47 @@ class GruLinear:
         res = out.download((T, self.out_dim, E), np.float32).transpose(0, 2, 1).copy()
         out.free()
         return res
+
+
+class GruLinear(SeqLinear):
+    """One GRU layer -> activation -> Linear.  Flat parameters in Module::variables() order:
+    w_ih[3H,in], w_hh[3H,H], b_ih[3H], b_hh[3H] (rnn/mod.rs:223-258), kernel[out,H], bias[out] (linear.rs:108-110)."""
+
+    _create = "rl_grunet_create"
+
+
+# ------------------------------------------------------------------------------------------------
+# Chain<Lstm, Linear> (src/torch/modules/chain.rs, seq/rnn/lstm.rs, ff/linear.rs)
+# ------------------------------------------------------------------------------------------------
+@dataclass
+class LstmLinearConfig:
+    """ChainConfig<LstmConfig, LinearConfig>: one LSTM layer (hidden_dim 128), the activation, then a Linear."""
+
+    hidden_dim: int = 128
+    activation: str = "relu"
+
+    def build_module(self, ctx: Context, in_dim: int, out_dim: int) -> "LstmLinear":
+        return LstmLinear(ctx, in_dim, self.hidden_dim, out_dim, self.activation)
+
+
+def lstm_linear_num_params(in_dim, hidden, out_dim):
+    return 4 * hidden * in_dim + 4 * hidden * hidden + 8 * hidden + out_dim * hidden + out_dim
+
+
+def init_lstm_linear_params(rng: np.random.Generator, in_dim: int, hidden: int, out_dim: int) -> np.ndarray:
+    """RnnBaseConfig::default(): input weights U(+-sqrt(6 / (in + 4H))), hidden weights orthogonal [4H, H], zero biases;
+    the Linear as in `init_params`.  Values come from numpy and are injected."""
+    lim = np.sqrt(6.0 / (in_dim + 4 * hidden))
+    w_ih = rng.uniform(-lim, lim, size=(4 * hidden, in_dim))
+    q, _ = np.linalg.qr(rng.normal(size=(4 * hidden, hidden)))
+    lim2 = np.sqrt(6.0 / (hidden + 1 + out_dim))
+    parts = [w_ih, q, np.zeros(4 * hidden), np.zeros(4 * hidden), rng.uniform(-lim2, lim2, size=(out_dim, hidden)),
+             rng.uniform(-lim2, lim2, size=(out_dim,))]
+    return np.concatenate([np.asarray(p, np.float32).ravel() for p in parts])
+
+
+class LstmLinear(SeqLinear):
+    """One LSTM layer -> activation -> Linear.  Flat parameters in Module::variables() order:
+    w_ih[4H,in], w_hh[4H,H], b_ih[4H], b_hh[4H] (gate order i, f, g, o), kernel[out,H], bias[out]."""
+
+    _create = "rl_lstmnet_create"

@@ -48,7 +48,7 @@ class ActorSpec:
     exploration_rate: float = 0.0
     training: bool = True
     lanes_per_env: int = 0
-    seq_net: object = None             # modules.GruLinear (recurrent CATEGORICAL_POLICY / EPS_GREEDY_Q)
+    seq_net: object = None             # modules.GruLinear / LstmLinear (recurrent CATEGORICAL_POLICY / EPS_GREEDY_Q)
     ucb: object = None                 # agents.UCB1Agent
     inner_kind: int = L.RL_INNER_RANDOM  # RESETTING_META: the inner agent (L.RL_INNER_*)
     bts: object = None                 # agents.BetaThompsonSamplingAgent

@@ -14,7 +14,7 @@ import numpy as np
 
 from . import _lib as L
 from .envs import BatchedEnv
-from .modules import GruLinear, GruLinearConfig, Mlp, MlpConfig
+from .modules import GruLinearConfig, LstmLinearConfig, Mlp, MlpConfig, SeqLinear
 from .runtime import Context, DeviceBuffer
 from .simulation import ActorSpec, HistoryDataBound, Trajectory
 
@@ -58,7 +58,7 @@ class Adam:
         self.ctx, self._lib, self.mlp = mlp.ctx, mlp.ctx._lib, mlp
         c = L.AdamCfg(cfg.learning_rate, cfg.beta1, cfg.beta2, cfg.weight_decay, cfg.eps)
         h = C.c_void_p()
-        create = self._lib.rl_adam_create_seq if isinstance(mlp, GruLinear) else self._lib.rl_adam_create
+        create = self._lib.rl_adam_create_seq if isinstance(mlp, SeqLinear) else self._lib.rl_adam_create
         L.check(create(mlp.handle, C.byref(c), C.byref(h)), self.ctx.handle)
         self.handle = h
 
@@ -78,7 +78,7 @@ class Adam:
 class TrpoConfig:
     """policies/trpo.rs:17-59"""
 
-    policy_fn_config: object = field(default_factory=MlpConfig)  # MlpConfig | GruLinearConfig
+    policy_fn_config: object = field(default_factory=MlpConfig)  # MlpConfig | GruLinearConfig | LstmLinearConfig
     optimizer_config: ConjugateGradientOptimizerConfig = field(default_factory=ConjugateGradientOptimizerConfig)
     max_policy_step_kl: float = 0.01
 
@@ -95,7 +95,7 @@ class Trpo:
 
     @property
     def recurrent(self) -> bool:
-        return isinstance(self.policy_fn, GruLinear)
+        return isinstance(self.policy_fn, SeqLinear)
 
     def actor(self, lanes_per_env: int = 0) -> ActorSpec:
         """Policy::actor -> PolicyActor (policies/actor.rs)."""
@@ -209,7 +209,7 @@ class Reinforce(_AdamPolicy):
 class ValuesOptConfig:
     """critics/opt.rs:14-50: GAE(lambda 0.95) advantages, reward-to-go targets, 80 Adam steps, gamma <= 0.99."""
 
-    state_value_fn_config: object = field(default_factory=MlpConfig)  # MlpConfig | GruLinearConfig
+    state_value_fn_config: object = field(default_factory=MlpConfig)  # MlpConfig | GruLinearConfig | LstmLinearConfig
     optimizer_config: AdamConfig = field(default_factory=AdamConfig)
     gae_lambda: float = 0.95          # AdvantageFn::Gae { lambda } (critics/mod.rs:78)
     opt_steps_per_update: int = 80
@@ -225,7 +225,7 @@ class ValuesOpt:
     def __init__(self, ctx: Context, cfg: ValuesOptConfig, in_dim: int, discount_factor: float):
         self.ctx, self._lib, self.cfg = ctx, ctx._lib, cfg
         self.state_value_fn = cfg.state_value_fn_config.build_module(ctx, in_dim, 1)
-        self.recurrent = isinstance(self.state_value_fn, GruLinear)
+        self.recurrent = isinstance(self.state_value_fn, SeqLinear)
         self.optimizer = Adam(self.state_value_fn, cfg.optimizer_config)
         self.discount_factor = np.float32(min(cfg.max_discount_factor, discount_factor))  # opt.rs:73
         self._adv = self._rtg = None
@@ -360,7 +360,7 @@ class ReplayBuffer:
         return {"obs": obs[:k], "next_obs": nobs[:k], "action": act[:k], "reward": rew[:k], "succ": succ[:k],
                 "episode_len": eps[:int(s.num_episodes)].astype(np.int64), "total_step_count": int(s.total_step_count)}
 
-    def sample_seq(self, cfg: "L.DqnCfg", q: GruLinear | None, draw_index: int) -> dict:
+    def sample_seq(self, cfg: "L.DqnCfg", q: SeqLinear | None, draw_index: int) -> dict:
         """The same sample_minibatch as padded sequences for a recurrent Q-network, read back to the host: planes
         [L][.][B] with one episode per column (draw order), succ RL_PAD past each episode, targets [L][B]."""
         v, tgt = L.TrajView(), C.c_void_p()
@@ -414,7 +414,7 @@ class DataCollectionSchedule:
 class DqnConfig:
     """dqn.rs:26-72"""
 
-    action_value_fn_config: MlpConfig | GruLinearConfig = field(default_factory=MlpConfig)
+    action_value_fn_config: MlpConfig | GruLinearConfig | LstmLinearConfig = field(default_factory=MlpConfig)
     optimizer_config: AdamConfig = field(default_factory=AdamConfig)
     target_one_step_td: bool = False          # StepValueTarget::RewardToGo is the default
     exploration_rate: ExplorationRateSchedule = field(default_factory=ExplorationRateSchedule)
@@ -443,7 +443,7 @@ class DqnAgent:
 
     @property
     def recurrent(self) -> bool:
-        return isinstance(self.action_value_fn, GruLinear)
+        return isinstance(self.action_value_fn, SeqLinear)
 
     def actor(self, training: bool = True) -> ActorSpec:
         """Agent::actor(mode): epsilon is fixed from global_steps at actor creation (dqn.rs:202-212)."""
