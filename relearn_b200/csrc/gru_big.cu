@@ -12,7 +12,7 @@
 //                           pointwise: r, u = sigmoid, n = tanh(in + r hn), h' = (hprev - n) u + n,
 //                           hprev_{t+1} = 0 where the episode ended (gru.rs:23-28); r, u, n, hn, h', hprev are kept per step
 //   FVP tangent (R-operator along v): tG_t = Vc . [x_t ; hprev_t] + vbc + Wc[:, F:] . thprev_t  (two more GEMMs per step)
-//   head + per-step algebra over all (t, e): logits, log-softmax, loss / KL / entropy, output cotangent dz (gru_update.cu's)
+//   head + per-step algebra over all (t, e): logits, log-softmax, loss / KL / entropy, output cotangent dz (passes.cuh)
 //   backward, t = T-1 .. 0  pointwise: dh' = act'(h') lw^T dz_t + carry  ->  D_t [4H x E] = (dpr, dpu, dpn r, dpn), carry = dh' u
 //                           carry += W_hh^T [H x 3H] . D_t[0:3H]                               (one GEMM per step)
 //   weight gradients        dWc [4H x (F + H + 1)] = sum_t D_t . [x_t ; hprev_t ; 1]^T          (ONE split-K GEMM over all (t, e))
@@ -28,24 +28,13 @@
 // GEMMs: hand-written FP32 register-tiled kernels (128 x 128 x 8 tiles, 8 x 8 per thread, register-prefetched; the split-K
 // one contracts over lanes with f64 flushes).  FP32, not tensor cores: the parity bar is 1e-5-class against f64 autograd, which bf16/tf32
 // inputs miss; the bf16-piece tcgen05 form used by pass_tc.cuh is the next step (DESIGN.md section 9).
-#include "handles.cuh"
+#include "passes.cuh"
 
 #include <algorithm>
 
 namespace {
 
 constexpr int BN = 128, GEMM_THREADS = 256;
-constexpr float F32_LOWEST_B = -3.402823466e+38f;
-
-__device__ __forceinline__ float sigm_b(float v) { return __fdividef(1.0f, 1.0f + expf(-v)); }
-__device__ __forceinline__ float act_grad_b(int act, float pre, float out) {
-    switch (act) {
-    case RL_ACT_RELU: return pre > 0.0f ? 1.0f : 0.0f;
-    case RL_ACT_SIGMOID: return out * (1.0f - out);
-    case RL_ACT_TANH: return 1.0f - out * out;
-    default: return 1.0f;
-    }
-}
 
 // ---------------------------------------------------------------------------------------------------------------------
 // C [M x N] (+)= A [M x K] . B [K x N] (+ bias[m]);  A row-major (lda), B rows 0 .. K0-1 from B0 and K0 .. K-1 from B1 (both
@@ -308,7 +297,7 @@ __global__ void big_gates_kernel(const float *__restrict__ G, const float *__res
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= (uint64_t)H * E) return;
     const uint64_t j = i / E, e = i - j * E, HE = (uint64_t)H * E;
-    const float r = sigm_b(G[i]), u = sigm_b(G[HE + i]), hn = G[2 * HE + i], in = G[3 * HE + i];
+    const float r = sigm(G[i]), u = sigm(G[HE + i]), hn = G[2 * HE + i], in = G[3 * HE + i];
     const float n = tanhf(__fadd_rn(in, __fmul_rn(hn, r)));
     const float hp = hprev[i];
     const float hnew = __fadd_rn(__fmul_rn(__fsub_rn(hp, n), u), n);
@@ -326,7 +315,7 @@ __global__ void lstm_gates_kernel(const float *__restrict__ G, const float *__re
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= (uint64_t)H * E) return;
     const uint64_t j = i / E, e = i - j * E, HE = (uint64_t)H * E;
-    const float ig = sigm_b(G[i]), fg = sigm_b(G[HE + i]), gg = tanhf(G[2 * HE + i]), og = sigm_b(G[3 * HE + i]);
+    const float ig = sigm(G[i]), fg = sigm(G[HE + i]), gg = tanhf(G[2 * HE + i]), og = sigm(G[3 * HE + i]);
     const float c = __fadd_rn(__fmul_rn(fg, cprev[i]), __fmul_rn(ig, gg));
     const float hnew = __fmul_rn(og, tanhf(c));
     I[i] = ig; Fg[i] = fg; Gg[i] = gg; O[i] = og; HNEW[i] = hnew;
@@ -375,19 +364,15 @@ __global__ void big_gates_tan_kernel(const float *__restrict__ tG, const float *
     thp[i] = succ_t[e] != RL_CONTINUE ? 0.0f : thnew;
 }
 
-// Linear head + the per-step algebra of gru_pass_kernel over all (t, e); one partial of the four scalar sums per block
+// Linear head + the per-step loss algebra (passes.cuh) over all (t, e); one partial of the four scalar sums per block
 constexpr int HEAD_THREADS = 128, HEAD_MAXA_ALL = 32;
 // HEAD_MAXA = the compile-time bound of the per-thread arrays over the outputs (logits, probabilities, cotangent): 16 keeps
 // them in registers for the module sizes of the experiments (2 .. 10 arms); 32 serves the rest through local memory
 template <int MODE, int HEAD_MAXA>
 __global__ void __launch_bounds__(HEAD_THREADS) big_head_kernel(rl_seq_pass_args a, const float *__restrict__ HNEW,
                                                                 const float *__restrict__ THNEW, double *__restrict__ scal_part) {
-    constexpr bool BACKWARD = MODE == RL_PASS_GRAD || MODE == RL_PASS_FVP || MODE == RL_PASS_VALUE || MODE == RL_PASS_PPO ||
-                              MODE == RL_PASS_REINFORCE || MODE == RL_PASS_QLOSS;
-    constexpr bool IS_POLICY = MODE != RL_PASS_VALUE && MODE != RL_PASS_QLOSS;
-    constexpr bool FVP = MODE == RL_PASS_FVP;
-    constexpr bool USES_ADV = MODE == RL_PASS_EVAL || MODE == RL_PASS_GRAD || MODE == RL_PASS_PPO || MODE == RL_PASS_REINFORCE;
-    constexpr bool USES_LP0 = MODE == RL_PASS_EVAL || MODE == RL_PASS_GRAD || MODE == RL_PASS_PPO;
+    using M = PassMode<MODE>;
+    constexpr bool FVP = M::FVP;
     if (a.skip_flag && *a.skip_flag) return;
     extern __shared__ float hsm[];  // lw [A][H], lb [A], (FVP) vlw, vlb
     const int H = a.H, A = a.A, F = a.F, NG = rl_cell_gates(a.cell);
@@ -417,7 +402,7 @@ __global__ void __launch_bounds__(HEAD_THREADS) big_head_kernel(rl_seq_pass_args
             for (int j = 0; j < H; ++j) {
                 const float hn = HNEW[(t * H + j) * E + e];
                 const float av = rl_activate(a.act, hn);
-                const float gd = FVP ? act_grad_b(a.act, hn, av) * THNEW[(t * H + j) * E + e] : 0.0f;
+                const float gd = FVP ? act_grad(a.act, hn, av) * THNEW[(t * H + j) * E + e] : 0.0f;
 #pragma unroll
                 for (int k = 0; k < HEAD_MAXA; ++k)
                     if (k < A) {
@@ -425,97 +410,18 @@ __global__ void __launch_bounds__(HEAD_THREADS) big_head_kernel(rl_seq_pass_args
                         if (FVP) zd[k] = fmaf(vlw[k * H + j], av, fmaf(lw[k * H + j], gd, zd[k]));
                     }
             }
-            float loss_s = 0.0f, kl_s = 0.0f, ent_s = 0.0f;
-            if (IS_POLICY) {
-                float m = z[0];
-#pragma unroll
-                for (int k = 1; k < HEAD_MAXA; ++k)
-                    if (k < A) m = fmaxf(m, z[k]);
-                float sum = 0.0f;
+            float lp[HEAD_MAXA];
+            const SampleLoss ls = sample_loss<MODE, HEAD_MAXA>(z, zd, A, M::USES_ACT ? (int)a.action[idx] : 0, M::USES_ADV ? a.adv[idx] : 0.0f,
+                                                               M::USES_TARGET ? a.target[idx] : 0.0f, float2{},
+                                                               [&](int k) { return a.logp0[(t * A + k) * E + e]; }, lp, dz);
+            if (MODE == RL_PASS_STATS) {
 #pragma unroll
                 for (int k = 0; k < HEAD_MAXA; ++k)
-                    if (k < A) sum += expf(z[k] - m);
-                const float lse = m + logf(sum);
-                float lp[HEAD_MAXA], p[HEAD_MAXA];
-#pragma unroll
-                for (int k = 0; k < HEAD_MAXA; ++k) {
-                    lp[k] = k < A ? z[k] - lse : 0.0f;
-                    p[k] = k < A ? expf(lp[k]) : 0.0f;
-                }
-                const int act_s = (int)a.action[idx];
-                const float adv_s = USES_ADV ? a.adv[idx] : 0.0f;
-                float lp_act = 0.0f;
-#pragma unroll
-                for (int k = 0; k < HEAD_MAXA; ++k)
-                    if (k == act_s) lp_act = lp[k];
-                if (MODE == RL_PASS_STATS) {
-#pragma unroll
-                    for (int k = 0; k < HEAD_MAXA; ++k)
-                        if (k < A) {
-                            ent_s -= fmaxf(lp[k], F32_LOWEST_B) * p[k];
-                            a.logp0[(t * A + k) * E + e] = lp[k];
-                        }
-                }
-                if (USES_LP0) {
-                    const float lp0a = a.logp0[(t * A + act_s) * E + e];
-                    const float ratio = expf(lp_act - lp0a);
-                    if (MODE == RL_PASS_PPO) {
-                        const float clipped = fminf(fmaxf(ratio, a.clip_lo), a.clip_hi);
-                        const float t1 = ratio * adv_s, t2 = clipped * adv_s;
-                        loss_s = -fminf(t1, t2);
-                        const bool inside = ratio >= a.clip_lo && ratio <= a.clip_hi;
-                        const float gg = (inside || t1 < t2) ? -t1 : 0.0f;
-#pragma unroll
-                        for (int k = 0; k < HEAD_MAXA; ++k)
-                            if (k < A) dz[k] = gg * ((act_s == k ? 1.0f : 0.0f) - p[k]);
-                    } else {
-                        loss_s = -(ratio * adv_s);
-#pragma unroll
-                        for (int k = 0; k < HEAD_MAXA; ++k)
-                            if (k < A) {
-                                const float lp0k = a.logp0[(t * A + k) * E + e];
-                                kl_s += fmaxf(lp0k - lp[k], F32_LOWEST_B) * expf(lp0k);
-                                if (MODE == RL_PASS_GRAD) dz[k] = loss_s * ((act_s == k ? 1.0f : 0.0f) - p[k]);
-                            }
-                    }
-                }
-                if (MODE == RL_PASS_REINFORCE) {
-                    loss_s = -(lp_act * adv_s);
-#pragma unroll
-                    for (int k = 0; k < HEAD_MAXA; ++k)
-                        if (k < A) {
-                            ent_s -= fmaxf(lp[k], F32_LOWEST_B) * p[k];
-                            dz[k] = -adv_s * ((act_s == k ? 1.0f : 0.0f) - p[k]);
-                        }
-                }
-                if (FVP) {
-                    float pd = 0.0f;
-#pragma unroll
-                    for (int k = 0; k < HEAD_MAXA; ++k)
-                        if (k < A) pd = fmaf(p[k], zd[k], pd);
-#pragma unroll
-                    for (int k = 0; k < HEAD_MAXA; ++k)
-                        if (k < A) dz[k] = p[k] * (zd[k] - pd);
-                }
-            } else if (MODE == RL_PASS_QLOSS) {  // mse(Q(obs).gather(action), targets)  (dqn.rs:316-326)
-                const int act_s = (int)a.action[idx];
-                float q = z[0];
-#pragma unroll
-                for (int k = 1; k < HEAD_MAXA; ++k)
-                    if (k == act_s) q = z[k];
-                const float diff = q - a.target[idx];
-                loss_s = diff * diff;
-#pragma unroll
-                for (int k = 0; k < HEAD_MAXA; ++k)
-                    if (k == act_s) dz[k] = 2.0f * diff;
-            } else {  // VALUE: mse(V(obs), targets)  (opt.rs:109-115)
-                const float diff = z[0] - a.target[idx];
-                loss_s = diff * diff;
-                dz[0] = 2.0f * diff;
+                    if (k < A) a.logp0[(t * A + k) * E + e] = lp[k];
             }
-            s_cnt = 1.0; s_loss = (double)loss_s; s_kl = (double)kl_s; s_ent = (double)ent_s;
+            s_cnt = 1.0; s_loss = (double)ls.loss; s_kl = (double)ls.kl; s_ent = (double)ls.entropy;
         }
-        if (BACKWARD) {
+        if (M::BACKWARD) {
 #pragma unroll
             for (int k = 0; k < HEAD_MAXA; ++k)
                 if (k < A) a.dzbuf[(t * A + k) * E + e] = dz[k];  // zero on padding
@@ -562,7 +468,7 @@ __global__ void big_bwd_kernel(const float *__restrict__ dz_t, const float *__re
     const float hnew = HNEW[i], av = rl_activate(act, hnew);
     AV[i] = av;
     const float carry = sc != RL_CONTINUE ? 0.0f : dh[i];  // last step of its episode: nothing flows back from t + 1
-    const float dhn = fmaf(act_grad_b(act, hnew, av), da, carry);
+    const float dhn = fmaf(act_grad(act, hnew, av), da, carry);
     const float r = R[i], u = U[i], n = Nn[i], hn = HN[i], hp = hprev[i];
     // h' = u h + (1 - u) n
     const float du = dhn * (hp - n), dn = dhn * (1.0f - u);
@@ -599,7 +505,7 @@ __global__ void lstm_bwd_kernel(const float *__restrict__ dz_t, const float *__r
     const float hnew = HNEW[i], av = rl_activate(act, hnew);
     AV[i] = av;
     const bool last = sc != RL_CONTINUE;  // last step of its episode: nothing flows back from t + 1
-    const float dhn = fmaf(act_grad_b(act, hnew, av), da, last ? 0.0f : dh[i]);
+    const float dhn = fmaf(act_grad(act, hnew, av), da, last ? 0.0f : dh[i]);
     const float ig = I[i], fg = Fg[i], gg = Gg[i], og = O[i], cp = cprev[i];
     const float tc = tanhf(__fadd_rn(__fmul_rn(fg, cp), __fmul_rn(ig, gg)));
     const float dcn = (last ? 0.0f : dc[i]) + dhn * og * (1.0f - tc * tc);
@@ -775,8 +681,7 @@ rl_status rl_seq_big_pass_launch(rl_ctx *ctx, int mode, const rl_seq_pass_args &
     const int F = a.F, H = a.H, A = a.A, KP = F + H, NB = KP + 1, NH = H + 1;
     const uint64_t T = a.T, E = a.E, HE = (uint64_t)H * E, TE = T * E;
     const bool fvp = mode == RL_PASS_FVP;
-    const bool backward = mode == RL_PASS_GRAD || mode == RL_PASS_FVP || mode == RL_PASS_VALUE || mode == RL_PASS_PPO ||
-                          mode == RL_PASS_REINFORCE || mode == RL_PASS_QLOSS;
+    const bool backward = pass_backward(mode);
     const bool lstm = a.cell == RL_CELL_LSTM;
     const int NG = rl_cell_gates(a.cell);
     const int *skip = a.skip_flag;
@@ -886,8 +791,6 @@ rl_status rl_seq_big_pass_launch(rl_ctx *ctx, int mode, const rl_seq_pass_args &
     case RL_PASS_GRAD: RL_TRY(launch_head<RL_PASS_GRAD>(ctx, a, pl, scal_part, head_blocks)); break;
     case RL_PASS_FVP: RL_TRY(launch_head<RL_PASS_FVP>(ctx, a, pl, scal_part, head_blocks)); break;
     case RL_PASS_VALUE: RL_TRY(launch_head<RL_PASS_VALUE>(ctx, a, pl, scal_part, head_blocks)); break;
-    case RL_PASS_PPO: RL_TRY(launch_head<RL_PASS_PPO>(ctx, a, pl, scal_part, head_blocks)); break;
-    case RL_PASS_REINFORCE: RL_TRY(launch_head<RL_PASS_REINFORCE>(ctx, a, pl, scal_part, head_blocks)); break;
     case RL_PASS_QLOSS: RL_TRY(launch_head<RL_PASS_QLOSS>(ctx, a, pl, scal_part, head_blocks)); break;
     default: return rl_fail(ctx, RL_ERR_INVALID_ARG, "rl_seq_big_pass_launch: bad mode %d", mode);
     }

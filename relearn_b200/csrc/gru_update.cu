@@ -1,5 +1,5 @@
 // gru_update.cu -- full-batch passes over trajectories for a recurrent policy / critic / Q-network (Chain<Gru, Linear>):
-// what autograd does for the reference when the module of Trpo / Ppo / Reinforce / ValuesOpt / DqnAgent is a GRU
+// what autograd does for the reference when the module of Trpo / ValuesOpt / DqnAgent is a GRU
 // (src/torch/agents/policies/trpo.rs:97-164 with cuDNN disabled :104-108, critics/opt.rs:100-127,
 // modules/seq/rnn/gru.rs:72-102, modules/chain.rs:157-168).
 //
@@ -23,17 +23,12 @@
 //
 // Sizes: hidden <= 8, features <= 20, actions <= 16 (the rnn.rs-sized and small rl2 bandit modules).  The
 // rl2-sized hidden 128 belongs on tensor cores and is not served by this kernel (DESIGN.md section 9).
-#include "handles.cuh"
+#include "passes.cuh"
 
 namespace {
 
 constexpr int GH_MAX = 8, GF_MAX = 20, GA_MAX = 16;
 constexpr int GP_MAX_ALL = 3 * GH_MAX * GF_MAX + 3 * GH_MAX * GH_MAX + 6 * GH_MAX + GA_MAX * GH_MAX + GA_MAX;
-constexpr float F32_LOWEST_G = -3.402823466e+38f;
-
-// 1 / (1 + e^-v) with the hardware reciprocal (MUFU.RCP, <= 1 ulp) instead of the ~10-instruction IEEE division:
-// 24 of these per step sit on the recurrence's dependency chain
-__device__ __forceinline__ float sigm(float v) { return __fdividef(1.0f, 1.0f + expf(-v)); }
 
 struct Dims {
     int F, H, A, act;
@@ -98,14 +93,6 @@ __device__ __forceinline__ void lstm_gates(const Dims &d, const float *__restric
 }
 
 __device__ __forceinline__ float act_fwd(int act, float v) { return rl_activate(act, v); }
-__device__ __forceinline__ float act_grad(int act, float pre, float out) {
-    switch (act) {
-    case RL_ACT_RELU: return pre > 0.0f ? 1.0f : 0.0f;
-    case RL_ACT_SIGMOID: return out * (1.0f - out);
-    case RL_ACT_TANH: return 1.0f - out * out;
-    default: return 1.0f;
-    }
-}
 
 // Back-propagation through time of one lane of an LSTM (len valid steps), accumulating into the per-thread gradient g:
 // gates recomputed from (x_t, h_{t-1}, c_{t-1}) stored by the forward, both carries cut at episode ends.
@@ -175,13 +162,8 @@ __global__ void __launch_bounds__(RL_SEQ_BLOCK) gru_pass_kernel(rl_seq_pass_args
     constexpr bool LSTM = CELL == RL_CELL_LSTM;
     constexpr int NG = rl_cell_gates(CELL), GC = LSTM ? GH : 1;
     constexpr int GP_MAX = NG * GH * GF + NG * GH * GH + 2 * NG * GH + GA * GH + GA;
-    constexpr bool BACKWARD = MODE == RL_PASS_GRAD || MODE == RL_PASS_FVP || MODE == RL_PASS_VALUE || MODE == RL_PASS_PPO ||
-                              MODE == RL_PASS_REINFORCE || MODE == RL_PASS_QLOSS;
-    constexpr bool IS_POLICY = MODE != RL_PASS_VALUE && MODE != RL_PASS_QLOSS;
-    constexpr bool USES_TARGET = MODE == RL_PASS_VALUE || MODE == RL_PASS_QLOSS;
-    constexpr bool FVP = MODE == RL_PASS_FVP;
-    constexpr bool USES_ADV = MODE == RL_PASS_EVAL || MODE == RL_PASS_GRAD || MODE == RL_PASS_PPO || MODE == RL_PASS_REINFORCE;
-    constexpr bool USES_LP0 = MODE == RL_PASS_EVAL || MODE == RL_PASS_GRAD || MODE == RL_PASS_PPO;
+    using M = PassMode<MODE>;
+    constexpr bool BACKWARD = M::BACKWARD, FVP = M::FVP;
     if (a.skip_flag && *a.skip_flag) return;
     const Dims d{TF ? TF : a.F, TH ? TH : a.H, TA ? TA : a.A, a.act, NG};
     const int F = d.F, H = d.H, A = d.A, P = d.P();
@@ -217,7 +199,7 @@ __global__ void __launch_bounds__(RL_SEQ_BLOCK) gru_pass_kernel(rl_seq_pass_args
         float x_next[GF], tgt_next = 0.0f;
 #pragma unroll
         for (int f = 0; f < F; ++f) x_next[f] = a.T ? a.obs[(uint64_t)f * E + e] : 0.0f;
-        if (USES_TARGET && a.T) tgt_next = a.target[e];
+        if (M::USES_TARGET && a.T) tgt_next = a.target[e];
         for (uint64_t t = 0; t < a.T; ++t) {
             const uint8_t sc = sc_next;
             if (sc == RL_PAD) break;
@@ -230,7 +212,7 @@ __global__ void __launch_bounds__(RL_SEQ_BLOCK) gru_pass_kernel(rl_seq_pass_args
                 sc_next = a.succ[(t + 1) * E + e];
 #pragma unroll
                 for (int f = 0; f < F; ++f) x_next[f] = a.obs[((t + 1) * F + f) * E + e];
-                if (USES_TARGET) tgt_next = a.target[(t + 1) * E + e];
+                if (M::USES_TARGET) tgt_next = a.target[(t + 1) * E + e];
             } else {
                 sc_next = RL_PAD;
             }
@@ -314,13 +296,16 @@ __global__ void __launch_bounds__(RL_SEQ_BLOCK) gru_pass_kernel(rl_seq_pass_args
                 z[k] = acc;
                 zd[k] = accd;
             }
-            // ---- per-step algebra (same definitions as mlp_pass_kernel, update.cu) ----
+            // ---- per-step loss algebra: the one in passes.cuh, written out over per-thread arrays indexed by run-time values
+            // (they live in local memory when the sizes are run-time values).  Routed through sample_loss, whose loops keep
+            // such arrays in registers, the run-time-sized GRU Fisher-vector pass went from 64 to 96 registers and the
+            // hidden-8 TRPO step ran 30 % slower. ----
             float dz[GA];
 #pragma unroll
             for (int k = 0; k < A; ++k) dz[k] = 0.0f;
             float loss_s = 0.0f, kl_s = 0.0f, ent_s = 0.0f;
             const uint64_t n_idx = t * E + e;
-            if (IS_POLICY) {
+            if (M::IS_POLICY) {
                 float m = z[0];
 #pragma unroll
                 for (int k = 1; k < A; ++k) m = fmaxf(m, z[k]);
@@ -335,41 +320,22 @@ __global__ void __launch_bounds__(RL_SEQ_BLOCK) gru_pass_kernel(rl_seq_pass_args
                     p[k] = expf(lp[k]);
                 }
                 const int act_s = (int)a.action[n_idx];
-                const float adv_s = USES_ADV ? a.adv[n_idx] : 0.0f;
                 if (MODE == RL_PASS_STATS) {
 #pragma unroll
                     for (int k = 0; k < A; ++k) {
-                        ent_s -= fmaxf(lp[k], F32_LOWEST_G) * p[k];
+                        ent_s -= fmaxf(lp[k], F32_LOWEST) * p[k];
                         a.logp0[(t * A + k) * E + e] = lp[k];
                     }
                 }
-                if (USES_LP0) {
+                if (M::USES_LP0) {
                     const float lp0a = a.logp0[(t * A + act_s) * E + e];
                     const float ratio = expf(lp[act_s] - lp0a);
-                    if (MODE == RL_PASS_PPO) {
-                        const float clipped = fminf(fmaxf(ratio, a.clip_lo), a.clip_hi);
-                        const float t1 = ratio * adv_s, t2 = clipped * adv_s;
-                        loss_s = -fminf(t1, t2);
-                        const bool inside = ratio >= a.clip_lo && ratio <= a.clip_hi;
-                        const float gg = (inside || t1 < t2) ? -t1 : 0.0f;
-#pragma unroll
-                        for (int k = 0; k < A; ++k) dz[k] = gg * ((act_s == k ? 1.0f : 0.0f) - p[k]);
-                    } else {
-                        loss_s = -(ratio * adv_s);
-#pragma unroll
-                        for (int k = 0; k < A; ++k) {
-                            const float lp0k = a.logp0[(t * A + k) * E + e];
-                            kl_s += fmaxf(lp0k - lp[k], F32_LOWEST_G) * expf(lp0k);
-                            if (MODE == RL_PASS_GRAD) dz[k] = loss_s * ((act_s == k ? 1.0f : 0.0f) - p[k]);
-                        }
-                    }
-                }
-                if (MODE == RL_PASS_REINFORCE) {
-                    loss_s = -(lp[act_s] * adv_s);
+                    loss_s = -(ratio * a.adv[n_idx]);
 #pragma unroll
                     for (int k = 0; k < A; ++k) {
-                        ent_s -= fmaxf(lp[k], F32_LOWEST_G) * p[k];
-                        dz[k] = -adv_s * ((act_s == k ? 1.0f : 0.0f) - p[k]);
+                        const float lp0k = a.logp0[(t * A + k) * E + e];
+                        kl_s += fmaxf(lp0k - lp[k], F32_LOWEST) * expf(lp0k);
+                        if (MODE == RL_PASS_GRAD) dz[k] = loss_s * ((act_s == k ? 1.0f : 0.0f) - p[k]);
                     }
                 }
                 if (FVP) {
@@ -559,8 +525,6 @@ rl_status rl_seq_pass_launch(rl_ctx *ctx, int mode, const rl_seq_pass_args &a, i
     case RL_PASS_GRAD: return launch_mode<RL_PASS_GRAD>(ctx, a, grid, smem);
     case RL_PASS_FVP: return launch_mode<RL_PASS_FVP>(ctx, a, grid, smem);
     case RL_PASS_VALUE: return launch_mode<RL_PASS_VALUE>(ctx, a, grid, smem);
-    case RL_PASS_PPO: return launch_mode<RL_PASS_PPO>(ctx, a, grid, smem);
-    case RL_PASS_REINFORCE: return launch_mode<RL_PASS_REINFORCE>(ctx, a, grid, smem);
     case RL_PASS_QLOSS: return launch_mode<RL_PASS_QLOSS>(ctx, a, grid, smem);
     default: return rl_fail(ctx, RL_ERR_INVALID_ARG, "rl_seq_pass_launch: bad mode %d", mode);
     }

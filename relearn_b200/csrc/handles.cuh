@@ -114,7 +114,6 @@ struct rl_seq_pass_args {
     float *dzbuf;   // f32 [T][A][E]  output cotangent of each step
     double *partials;
     const int *skip_flag;
-    float clip_lo, clip_hi;
     int cell;       // RL_CELL_GRU / RL_CELL_LSTM
     float *cbuf;    // f32 [T][H][E]  LSTM: cell state before each step (K9)
 };

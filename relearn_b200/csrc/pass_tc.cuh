@@ -48,23 +48,17 @@
 
 // One launch = one full-batch pass; grid <= TC_CTAS_PER_SM * SMs, block = 128, dynamic smem = tc::tc_smem(blocks).
 template <int A, int MODE>
-struct TcPass {
-    static constexpr bool FVP = MODE == PASS_FVP;
-    static constexpr bool BACKWARD = MODE == PASS_GRAD || MODE == PASS_FVP || MODE == PASS_VALUE || MODE == PASS_PPO ||
-                                     MODE == PASS_REINFORCE || MODE == PASS_QLOSS;
-    static constexpr bool IS_POLICY = MODE != PASS_VALUE && MODE != PASS_QLOSS;
+struct TcPass : PassMode<MODE> {
     // Y blocks of MMA2: one, except for the Q-loss, whose logit gradients do not sum to zero (only the taken action's
     // output has one): block k holds y where action == k
-    static constexpr int YBLOCKS = MODE == PASS_QLOSS ? 2 : 1;
+    static constexpr int YBLOCKS = MODE == RL_PASS_QLOSS ? 2 : 1;
     static constexpr int N2 = tc::tc_n2(YBLOCKS);
     static constexpr int D2_COLS = N2 <= 32 ? 32 : 64;
     static constexpr int CTAS_PER_SM = YBLOCKS == 1 ? tc::TC_CTAS_PER_SM : 2;  // 128 + 64 TMEM columns, 80 KB of shared memory
-    static constexpr bool USES_ADV = MODE == PASS_EVAL || MODE == PASS_GRAD || MODE == PASS_PPO || MODE == PASS_REINFORCE;
-    static constexpr bool USES_LP0 = MODE == PASS_EVAL || MODE == PASS_GRAD || MODE == PASS_PPO;
     static constexpr int BLOCKS = A;  // 24-column blocks of MMA3: one per logit; FVP: z_0 - z_1 and its tangent
     static constexpr int N3 = tc::tc_n3(BLOCKS);
     static constexpr int SMEM = tc::tc_smem(BLOCKS, YBLOCKS);
-    static_assert((A == 1 && MODE == PASS_VALUE) || (A == 2 && MODE != PASS_VALUE),
+    static_assert((A == 1 && MODE == RL_PASS_VALUE) || (A == 2 && MODE != RL_PASS_VALUE),
                   "built for the critic and for the two-action policy / action-value network");
 };
 
@@ -198,8 +192,8 @@ __global__ void __launch_bounds__(tc::TC_THREADS, TcPass<A, MODE>::CTAS_PER_SM) 
         st.code = in_range ? __ldg(a.succ + n_next) : (uint8_t)RL_PAD;
 #pragma unroll
         for (int f = 0; f < F; ++f) st.x[f] = in_range ? __ldg(a.obs + (t_next * F + f) * a.E + e_next) : 0.0f;
-        st.tgt = ((MODE == PASS_VALUE || MODE == PASS_QLOSS) && in_range) ? __ldg(a.target + n_next) : 0.0f;
-        st.act = ((IS_POLICY || MODE == PASS_QLOSS) && in_range) ? __ldg(a.action + n_next) : (uint8_t)0;
+        st.tgt = (K::USES_TARGET && in_range) ? __ldg(a.target + n_next) : 0.0f;
+        st.act = (K::USES_ACT && in_range) ? __ldg(a.action + n_next) : (uint8_t)0;
         st.adv = (K::USES_ADV && in_range) ? __ldg(a.adv + n_next) : 0.0f;
         st.lp0 = make_float2(0.0f, 0.0f);
         if (K::USES_LP0 && in_range) st.lp0 = __ldg(reinterpret_cast<const float2 *>(a.logp0) + n_next);
@@ -318,28 +312,28 @@ __global__ void __launch_bounds__(tc::TC_THREADS, TcPass<A, MODE>::CTAS_PER_SM) 
             float loss_s = 0.0f, kl_s = 0.0f, ent_s = 0.0f;
             if (IS_POLICY) {
                 float lp[A], p[A];
-                log_softmax<A>(z, lp);
+                log_softmax<A>(z, A, lp);
 #pragma unroll
                 for (int k = 0; k < A; ++k) p[k] = expf(lp[k]);
                 // onehot_0 - p_0 without the cancellation of 1 - p_0 near saturation: p_0 + p_1 = 1
                 const float d0 = act_s == 0 ? p[A > 1 ? 1 : 0] : -p[0];
-                if (MODE == PASS_STATS) {
+                if (MODE == RL_PASS_STATS) {
                     // trpo.rs:112-122: log-probs of the behaviour policy and its entropy (categorical.rs:62-68)
 #pragma unroll
                     for (int k = 0; k < A; ++k) ent_s -= fmaxf(lp[k], F32_LOWEST) * p[k];
                     reinterpret_cast<float2 *>(a.logp0)[tile * 128 + tid] = make_float2(lp[0], lp[A > 1 ? 1 : 0]);
                 }
-                if (MODE == PASS_EVAL || MODE == PASS_GRAD) {
+                if (MODE == RL_PASS_EVAL || MODE == RL_PASS_GRAD) {
                     // trpo.rs:129-144: ratio = exp(logp - logp0); loss = -mean(ratio * adv); KL(p0 || p)
                     const float lpa = act_s == 0 ? lp[0] : lp[A > 1 ? 1 : 0], lp0a = act_s == 0 ? lp0[0] : lp0[1];
                     const float ratio = expf(lpa - lp0a);
                     loss_s = -(ratio * adv_s);
 #pragma unroll
                     for (int k = 0; k < A; ++k) kl_s += fmaxf(lp0[k] - lp[k], F32_LOWEST) * expf(lp0[k]);
-                    if (MODE == PASS_GRAD) dz0 = loss_s * d0;
+                    if (MODE == RL_PASS_GRAD) dz0 = loss_s * d0;
                 }
-                if (MODE == PASS_PPO) {
-                    // ppo.rs:124-138, backward as libtorch (see mlp_pass_kernel)
+                if (MODE == RL_PASS_PPO) {
+                    // ppo.rs:124-138, backward as libtorch (see sample_loss, passes.cuh)
                     const float lpa = act_s == 0 ? lp[0] : lp[A > 1 ? 1 : 0], lp0a = act_s == 0 ? lp0[0] : lp0[1];
                     const float ratio = expf(lpa - lp0a);
                     const float clipped = fminf(fmaxf(ratio, a.clip_lo), a.clip_hi);
@@ -349,7 +343,7 @@ __global__ void __launch_bounds__(tc::TC_THREADS, TcPass<A, MODE>::CTAS_PER_SM) 
                     const float g = (inside || t1 < t2) ? -t1 : 0.0f;
                     dz0 = g * d0;
                 }
-                if (MODE == PASS_REINFORCE) {
+                if (MODE == RL_PASS_REINFORCE) {
                     // reinforce.rs:72-79
                     const float lpa = act_s == 0 ? lp[0] : lp[A > 1 ? 1 : 0];
                     loss_s = -(lpa * adv_s);
@@ -358,7 +352,7 @@ __global__ void __launch_bounds__(tc::TC_THREADS, TcPass<A, MODE>::CTAS_PER_SM) 
                     dz0 = -adv_s * d0;
                 }
                 if (FVP) dz0 = p[0] * (p[A > 1 ? 1 : 0] * zdd);  // u = (diag p - p p^T) zdot with p_0 + p_1 = 1
-            } else if (MODE == PASS_QLOSS) {
+            } else if (MODE == RL_PASS_QLOSS) {
                 // dqn.rs:316-326: mse(Q(obs).gather(action), targets); dz0 is the gradient w.r.t. the TAKEN action's output
                 const float diff = (act_s == 0 ? z[0] : z[A > 1 ? 1 : 0]) - tgt;
                 loss_s = diff * diff;

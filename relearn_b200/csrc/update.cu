@@ -23,7 +23,7 @@
 // Exactness: the Hessian of mean KL(p0 || p_theta) at theta0 equals the Fisher matrix
 // mean J^T (diag p - p p^T) J (the first-order term vanishes because p = p0 there), so the analytic
 // Fisher-vector product is the reference's double-backward Hessian-vector product.
-#include "handles.cuh"
+#include "passes.cuh"
 
 #include <cmath>
 #include <cstdlib>
@@ -31,10 +31,7 @@
 
 namespace {
 
-enum { PASS_STATS = RL_PASS_STATS, PASS_EVAL = RL_PASS_EVAL, PASS_GRAD = RL_PASS_GRAD, PASS_FVP = RL_PASS_FVP, PASS_VALUE = RL_PASS_VALUE,
-       PASS_QLOSS = RL_PASS_QLOSS, PASS_PPO = RL_PASS_PPO, PASS_REINFORCE = RL_PASS_REINFORCE };
 enum { SC_LOSS = 0, SC_KL = 1, SC_ENTROPY = 2, SC_COUNT = 3, NSCALAR = 4 };
-constexpr float F32_LOWEST = -3.402823466e+38f;
 constexpr int PASS_THREADS = 256;
 constexpr int FLUSH_TILES = 4;
 
@@ -48,25 +45,8 @@ struct PassArgs {
     const float *target;  // f32 [T*E]
     double *partials;     // f64 [gridDim.x][P + NSCALAR]
     const int *skip_flag;
-    float clip_lo, clip_hi;  // PASS_PPO: 1 -+ clip_distance as f32 (ppo.rs:131-132)
+    float clip_lo, clip_hi;  // RL_PASS_PPO: 1 -+ clip_distance as f32 (ppo.rs:131-132)
 };
-
-template <int A>
-__device__ __forceinline__ void log_softmax(const float *z, float *lp) {
-    if (A == 1) {
-        lp[0] = 0.0f;
-        return;
-    }
-    float m = z[0];
-#pragma unroll
-    for (int k = 1; k < A; ++k) m = fmaxf(m, z[k]);
-    float sum = 0.0f;
-#pragma unroll
-    for (int k = 0; k < A; ++k) sum += expf(z[k] - m);
-    const float lse = m + logf(sum);
-#pragma unroll
-    for (int k = 0; k < A; ++k) lp[k] = z[k] - lse;
-}
 
 // Reduce v[0..CH-1] across the 32 lanes (CH = 8 or 4); afterwards every lane of group g holds the
 // complete sum of element g, where groups are 32/CH consecutive lanes.  CH=8: 9 shuffles, CH=4: 6.
@@ -132,13 +112,8 @@ __global__ void __launch_bounds__(PASS_THREADS, MINB) mlp_pass_kernel(PassArgs a
     constexpr int W = P + NSCALAR;
     constexpr int XS = 12;          // floats per staged sample: F duplicated pairs (x, x), padded to 3 x float4
     static_assert(2 * F <= XS, "sample stage too small");
-    constexpr bool BACKWARD = MODE == PASS_GRAD || MODE == PASS_FVP || MODE == PASS_VALUE || MODE == PASS_QLOSS ||
-                              MODE == PASS_PPO || MODE == PASS_REINFORCE;
-    constexpr bool IS_POLICY = MODE == PASS_STATS || MODE == PASS_EVAL || MODE == PASS_GRAD || MODE == PASS_FVP ||
-                               MODE == PASS_PPO || MODE == PASS_REINFORCE;
-    constexpr bool USES_ADV = MODE == PASS_EVAL || MODE == PASS_GRAD || MODE == PASS_PPO || MODE == PASS_REINFORCE;
-    constexpr bool USES_LP0 = MODE == PASS_EVAL || MODE == PASS_GRAD || MODE == PASS_PPO;
-    constexpr bool FVP = MODE == PASS_FVP;
+    using M = PassMode<MODE>;
+    constexpr bool BACKWARD = M::BACKWARD, FVP = M::FVP;
     if (a.skip_flag && *a.skip_flag) return;
 
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -247,11 +222,11 @@ __global__ void __launch_bounds__(PASS_THREADS, MINB) mlp_pass_kernel(PassArgs a
         float x[F];
 #pragma unroll
         for (int f = 0; f < F; ++f) x[f] = in_range ? __ldg(a.obs + (t * F + f) * a.E + e) : 0.0f;
-        const int act = ((IS_POLICY || MODE == PASS_QLOSS) && in_range) ? (int)__ldg(a.action + n) : 0;
-        const float adv = (USES_ADV && in_range) ? __ldg(a.adv + n) : 0.0f;
-        const float tgt = ((MODE == PASS_VALUE || MODE == PASS_QLOSS) && in_range) ? __ldg(a.target + n) : 0.0f;
+        const int act = (M::USES_ACT && in_range) ? (int)__ldg(a.action + n) : 0;
+        const float adv = (M::USES_ADV && in_range) ? __ldg(a.adv + n) : 0.0f;
+        const float tgt = (M::USES_TARGET && in_range) ? __ldg(a.target + n) : 0.0f;
         float2 l = make_float2(0.0f, 0.0f);
-        if (USES_LP0 && in_range) l = __ldg(reinterpret_cast<const float2 *>(a.logp0) + n);
+        if (M::USES_LP0 && in_range) l = __ldg(reinterpret_cast<const float2 *>(a.logp0) + n);
         st.valid = sc_code != RL_PAD;
 #pragma unroll
         for (int f = 0; f < F; ++f) st.x[f] = st.valid ? x[f] : 0.0f;
@@ -335,107 +310,30 @@ __global__ void __launch_bounds__(PASS_THREADS, MINB) mlp_pass_kernel(PassArgs a
             // per-sample scalars of that sample live in lane CH*c + g
             const int owner = c * CH + quad_sample;
             const bool s_valid = (valid_mask >> owner) & 1u;
-            const int act_s = (IS_POLICY || MODE == PASS_QLOSS) ? __shfl_sync(0xffffffffu, my_act, owner) : 0;
+            const int act_s = M::USES_ACT ? __shfl_sync(0xffffffffu, my_act, owner) : 0;
             float adv_s = 0.0f, tgt_s = 0.0f, lp0[2] = {0.0f, 0.0f};
-            if (USES_ADV) adv_s = __shfl_sync(0xffffffffu, my_adv, owner);
-            if (USES_LP0) {
+            if (M::USES_ADV) adv_s = __shfl_sync(0xffffffffu, my_adv, owner);
+            if (M::USES_LP0) {
                 lp0[0] = __shfl_sync(0xffffffffu, my_lp0[0], owner);
                 lp0[1] = __shfl_sync(0xffffffffu, my_lp0[1], owner);
             }
-            if (MODE == PASS_VALUE || MODE == PASS_QLOSS) tgt_s = __shfl_sync(0xffffffffu, my_tgt, owner);
+            if (M::USES_TARGET) tgt_s = __shfl_sync(0xffffffffu, my_tgt, owner);
 
             // ---- per-sample algebra (all lanes of a group compute the same values) ----
             float dz[A];
 #pragma unroll
             for (int k = 0; k < A; ++k) dz[k] = 0.0f;
             if (s_valid) {
-                float loss_s = 0.0f, kl_s = 0.0f, ent_s = 0.0f;
-                if (IS_POLICY) {
-                    float lp[A], p[A];
-                    log_softmax<A>(z, lp);
-#pragma unroll
-                    for (int k = 0; k < A; ++k) p[k] = expf(lp[k]);
-                    if (MODE == PASS_STATS) {
-                        // trpo.rs:112-122: log-probs of the behaviour policy and its entropy (categorical.rs:62-68)
-#pragma unroll
-                        for (int k = 0; k < A; ++k) ent_s -= fmaxf(lp[k], F32_LOWEST) * p[k];
-                        if (quad_leader)
-                            reinterpret_cast<float2 *>(a.logp0)[tile * 32 + owner] = make_float2(lp[0], A > 1 ? lp[A > 1 ? 1 : 0] : 0.0f);
-                    }
-                    if (MODE == PASS_EVAL || MODE == PASS_GRAD) {
-                        // trpo.rs:129-144: ratio = exp(logp - logp0); loss = -mean(ratio * adv); KL(p0 || p)
-                        float lpa = lp[0], lp0a = lp0[0];
-#pragma unroll
-                        for (int k = 1; k < A; ++k)
-                            if (act_s == k) { lpa = lp[k]; lp0a = lp0[k]; }
-                        const float ratio = expf(lpa - lp0a);
-                        loss_s = -(ratio * adv_s);
-#pragma unroll
-                        for (int k = 0; k < A; ++k) kl_s += fmaxf(lp0[k] - lp[k], F32_LOWEST) * expf(lp0[k]);
-                        if (MODE == PASS_GRAD) {
-#pragma unroll
-                            for (int k = 0; k < A; ++k) dz[k] = loss_s * ((act_s == k ? 1.0f : 0.0f) - p[k]);
-                        }
-                    }
-                    if (MODE == PASS_PPO) {
-                        // ppo.rs:124-138: -mean(min(ratio * adv, clip(ratio, 1 - eps, 1 + eps) * adv)).  Backward as
-                        // libtorch: clamp passes the gradient on [lo, hi] (inclusive), minimum splits it on ties, so
-                        // d/d ratio = adv when the ratio is inside the clip range or the unclipped term is the smaller.
-                        float lpa = lp[0], lp0a = lp0[0];
-#pragma unroll
-                        for (int k = 1; k < A; ++k)
-                            if (act_s == k) { lpa = lp[k]; lp0a = lp0[k]; }
-                        const float ratio = expf(lpa - lp0a);
-                        const float clipped = fminf(fmaxf(ratio, a.clip_lo), a.clip_hi);
-                        const float t1 = ratio * adv_s, t2 = clipped * adv_s;
-                        loss_s = -fminf(t1, t2);
-                        const bool inside = ratio >= a.clip_lo && ratio <= a.clip_hi;
-                        const float g = (inside || t1 < t2) ? -t1 : 0.0f;
-#pragma unroll
-                        for (int k = 0; k < A; ++k) dz[k] = g * ((act_s == k ? 1.0f : 0.0f) - p[k]);
-                    }
-                    if (MODE == PASS_REINFORCE) {
-                        // reinforce.rs:72-79: -(log_probs * advantages).mean(); entropy of the current policy is logged
-                        float lpa = lp[0];
-#pragma unroll
-                        for (int k = 1; k < A; ++k)
-                            if (act_s == k) lpa = lp[k];
-                        loss_s = -(lpa * adv_s);
-#pragma unroll
-                        for (int k = 0; k < A; ++k) {
-                            ent_s -= fmaxf(lp[k], F32_LOWEST) * p[k];
-                            dz[k] = -adv_s * ((act_s == k ? 1.0f : 0.0f) - p[k]);
-                        }
-                    }
-                    if (FVP) {
-                        // u = (diag p - p p^T) zdot
-                        float pd = 0.0f;
-#pragma unroll
-                        for (int k = 0; k < A; ++k) pd = fmaf(p[k], zd[k], pd);
-#pragma unroll
-                        for (int k = 0; k < A; ++k) dz[k] = p[k] * (zd[k] - pd);
-                    }
-                } else if (MODE == PASS_VALUE) {
-                    // opt.rs:109-115: mse_loss(V(obs), targets, Mean)
-                    const float diff = z[0] - tgt_s;
-                    loss_s = diff * diff;
-                    dz[0] = 2.0f * diff;
-                } else if (MODE == PASS_QLOSS) {
-                    // dqn.rs:316-326: mse(Q(obs).gather(action), targets)
-                    float qv = z[0];
-#pragma unroll
-                    for (int k = 1; k < A; ++k)
-                        if (act_s == k) qv = z[k];
-                    const float diff = qv - tgt_s;
-                    loss_s = diff * diff;
-#pragma unroll
-                    for (int k = 0; k < A; ++k) dz[k] = act_s == k ? 2.0f * diff : 0.0f;
-                }
+                float lp[A];
+                const SampleLoss s = sample_loss<MODE, A>(z, zd, A, act_s, adv_s, tgt_s, make_float2(a.clip_lo, a.clip_hi),
+                                                          [&](int k) { return k == 1 ? lp0[1] : lp0[0]; }, lp, dz);
+                if (MODE == RL_PASS_STATS && quad_leader)
+                    reinterpret_cast<float2 *>(a.logp0)[tile * 32 + owner] = make_float2(lp[0], A > 1 ? lp[A > 1 ? 1 : 0] : 0.0f);
                 if (quad_leader) {
                     sc[SC_COUNT] += 1.0;
-                    sc[SC_LOSS] += (double)loss_s;
-                    sc[SC_KL] += (double)kl_s;
-                    sc[SC_ENTROPY] += (double)ent_s;
+                    sc[SC_LOSS] += (double)s.loss;
+                    sc[SC_KL] += (double)s.kl;
+                    sc[SC_ENTROPY] += (double)s.entropy;
 #pragma unroll
                     for (int k = 0; k < A; ++k) gb2[k] += (double)dz[k];
                 }
@@ -551,15 +449,6 @@ __host__ __device__ inline size_t any_smem_bytes(const AnyShape &sh, int nwarps,
            (size_t)nwarps * 2 * (2 * sh.L + 2) * any_buf_stride(d) * sizeof(float);
 }
 
-__device__ __forceinline__ float any_act_grad(int act, float pre, float h) {
-    switch (act) {
-    case RL_ACT_RELU: return pre > 0.0f ? 1.0f : 0.0f;  // relu'(0) = 0 as in libtorch
-    case RL_ACT_SIGMOID: return h * (1.0f - h);
-    case RL_ACT_TANH: return 1.0f - h * h;
-    default: return 1.0f;
-    }
-}
-
 __device__ __forceinline__ float warp_allsum_f32(float x) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
@@ -601,13 +490,8 @@ __device__ __forceinline__ void any_axpy2(double *__restrict__ tot, int stride, 
 
 template <int MODE>
 __global__ void __launch_bounds__(ANY_THREADS) mlp_pass_any_kernel(PassArgs a, AnyShape sh) {
-    constexpr bool BACKWARD = MODE == PASS_GRAD || MODE == PASS_FVP || MODE == PASS_VALUE || MODE == PASS_QLOSS ||
-                              MODE == PASS_PPO || MODE == PASS_REINFORCE;
-    constexpr bool IS_POLICY = MODE == PASS_STATS || MODE == PASS_EVAL || MODE == PASS_GRAD || MODE == PASS_FVP ||
-                               MODE == PASS_PPO || MODE == PASS_REINFORCE;
-    constexpr bool USES_ADV = MODE == PASS_EVAL || MODE == PASS_GRAD || MODE == PASS_PPO || MODE == PASS_REINFORCE;
-    constexpr bool USES_LP0 = MODE == PASS_EVAL || MODE == PASS_GRAD || MODE == PASS_PPO;
-    constexpr bool FVP = MODE == PASS_FVP;
+    using M = PassMode<MODE>;
+    constexpr bool BACKWARD = M::BACKWARD, FVP = M::FVP;
     constexpr int SB = 2;  // samples in flight per warp
     if (a.skip_flag && *a.skip_flag) return;
     const int F = sh.F, A = sh.A, act = sh.act, LL = sh.L;
@@ -650,9 +534,9 @@ __global__ void __launch_bounds__(ANY_THREADS) mlp_pass_any_kernel(PassArgs a, A
         const bool valid = in_range && a.succ[n] != RL_PAD;
         __syncwarp();
         for (int f = 0; f < F; ++f) xs[lane * F + f] = valid ? __ldg(a.obs + (t * F + f) * a.E + e) : 0.0f;
-        const int my_act = ((IS_POLICY || MODE == PASS_QLOSS) && valid) ? (int)a.action[n] : 0;
-        const float my_adv = (USES_ADV && valid) ? a.adv[n] : 0.0f;
-        const float my_tgt = ((MODE == PASS_VALUE || MODE == PASS_QLOSS) && valid) ? a.target[n] : 0.0f;
+        const int my_act = (M::USES_ACT && valid) ? (int)a.action[n] : 0;
+        const float my_adv = (M::USES_ADV && valid) ? a.adv[n] : 0.0f;
+        const float my_tgt = (M::USES_TARGET && valid) ? a.target[n] : 0.0f;
         unsigned todo = __ballot_sync(0xffffffffu, valid);
         __syncwarp();
         while (todo) {  // warp-uniform: the next two valid samples of the tile (the last one may be alone)
@@ -680,8 +564,8 @@ __global__ void __launch_bounds__(ANY_THREADS) mlp_pass_any_kernel(PassArgs a, A
                         float q0, q1;
                         any_dot2(vWt + j, ld, vin0, vin1, n_in, vbb[j], vbb[j], q0, q1);
                         if (dvin0) any_dot2(Wt + j, ld, dvin0, dvin1, n_in, q0, q1, q0, q1);
-                        d0[j] = any_act_grad(act, a0, a0) * q0;
-                        d1[j] = any_act_grad(act, a1, a1) * q1;
+                        d0[j] = act_grad(act, a0, a0) * q0;
+                        d1[j] = act_grad(act, a1, a1) * q1;
                     }
                 }
                 __syncwarp();
@@ -733,97 +617,30 @@ __global__ void __launch_bounds__(ANY_THREADS) mlp_pass_any_kernel(PassArgs a, A
                 const uint64_t ns = tile * 32 + sidx[b];
                 const int act_s = __shfl_sync(0xffffffffu, my_act, sidx[b]);
                 const float adv_s = __shfl_sync(0xffffffffu, my_adv, sidx[b]), tgt_s = __shfl_sync(0xffffffffu, my_tgt, sidx[b]);
-                float loss_s = 0.0f, kl_s = 0.0f, ent_s = 0.0f;
-                if (IS_POLICY) {
-                    // log_softmax over the A outputs
-                    float m = zz[b][0];
-    #pragma unroll
-                    for (int k = 1; k < ANY_MAXA; ++k)
-                        if (k < A) m = fmaxf(m, zz[b][k]);
-                    float sum = 0.0f;
-    #pragma unroll
+                // the behaviour log-probabilities in registers, each read once; the taken action's by a search
+                float lp[ANY_MAXA], lp0[M::USES_LP0 ? ANY_MAXA : 1];
+                if (M::USES_LP0) {
+#pragma unroll
+                    for (int k = 0; k < ANY_MAXA; ++k) lp0[k] = k < A ? a.logp0[ns * A + k] : 0.0f;
+                }
+                auto lp0_at = [&](int k) {
+                    float v = 0.0f;
+#pragma unroll
+                    for (int j = 0; j < ANY_MAXA; ++j)
+                        if (j == k) v = lp0[j];
+                    return v;
+                };
+                const SampleLoss s = sample_loss<MODE, ANY_MAXA>(zz[b], zzd[b], A, act_s, adv_s, tgt_s, make_float2(a.clip_lo, a.clip_hi),
+                                                                 lp0_at, lp, dzz[b]);
+                if (MODE == RL_PASS_STATS) {
+#pragma unroll
                     for (int k = 0; k < ANY_MAXA; ++k)
-                        if (k < A) sum += expf(zz[b][k] - m);
-                    const float lse = m + logf(sum);
-                    float lp[ANY_MAXA], pr[ANY_MAXA], lp0[USES_LP0 ? ANY_MAXA : 1];
-                    float lpa = 0.0f, lp0a = 0.0f;
-    #pragma unroll
-                    for (int k = 0; k < ANY_MAXA; ++k) {
-                        lp[k] = k < A ? zz[b][k] - lse : 0.0f;
-                        pr[k] = k < A ? expf(lp[k]) : 0.0f;
-                        if (USES_LP0) lp0[k] = k < A ? a.logp0[ns * A + k] : 0.0f;
-                        if (k == act_s) {
-                            lpa = lp[k];
-                            if (USES_LP0) lp0a = lp0[k];
-                        }
-                    }
-                    if (MODE == PASS_STATS) {  // trpo.rs:112-122, categorical.rs:62-68
-    #pragma unroll
-                        for (int k = 0; k < ANY_MAXA; ++k)
-                            if (k < A) {
-                                ent_s -= fmaxf(lp[k], F32_LOWEST) * pr[k];
-                                if (lane == k) a.logp0[ns * A + k] = lp[k];
-                            }
-                    }
-                    if (MODE == PASS_EVAL || MODE == PASS_GRAD) {  // trpo.rs:129-144
-                        const float ratio = expf(lpa - lp0a);
-                        loss_s = -(ratio * adv_s);
-    #pragma unroll
-                        for (int k = 0; k < ANY_MAXA; ++k)
-                            if (k < A) kl_s += fmaxf(lp0[k] - lp[k], F32_LOWEST) * expf(lp0[k]);
-                        if (MODE == PASS_GRAD) {
-    #pragma unroll
-                            for (int k = 0; k < ANY_MAXA; ++k)
-                                if (k < A) dzz[b][k] = loss_s * ((act_s == k ? 1.0f : 0.0f) - pr[k]);
-                        }
-                    }
-                    if (MODE == PASS_PPO) {  // ppo.rs:124-138 (backward as libtorch, see mlp_pass_kernel)
-                        const float ratio = expf(lpa - lp0a);
-                        const float clipped = fminf(fmaxf(ratio, a.clip_lo), a.clip_hi);
-                        const float t1 = ratio * adv_s, t2 = clipped * adv_s;
-                        loss_s = -fminf(t1, t2);
-                        const bool inside = ratio >= a.clip_lo && ratio <= a.clip_hi;
-                        const float g = (inside || t1 < t2) ? -t1 : 0.0f;
-    #pragma unroll
-                        for (int k = 0; k < ANY_MAXA; ++k)
-                            if (k < A) dzz[b][k] = g * ((act_s == k ? 1.0f : 0.0f) - pr[k]);
-                    }
-                    if (MODE == PASS_REINFORCE) {  // reinforce.rs:72-79
-                        loss_s = -(lpa * adv_s);
-    #pragma unroll
-                        for (int k = 0; k < ANY_MAXA; ++k)
-                            if (k < A) {
-                                ent_s -= fmaxf(lp[k], F32_LOWEST) * pr[k];
-                                dzz[b][k] = -adv_s * ((act_s == k ? 1.0f : 0.0f) - pr[k]);
-                            }
-                    }
-                    if (FVP) {  // u = (diag p - p p^T) zdot
-                        float pd = 0.0f;
-    #pragma unroll
-                        for (int k = 0; k < ANY_MAXA; ++k)
-                            if (k < A) pd = fmaf(pr[k], zzd[b][k], pd);
-    #pragma unroll
-                        for (int k = 0; k < ANY_MAXA; ++k)
-                            if (k < A) dzz[b][k] = pr[k] * (zzd[b][k] - pd);
-                    }
-                } else if (MODE == PASS_VALUE) {  // opt.rs:109-115
-                    const float diff = zz[b][0] - tgt_s;
-                    loss_s = diff * diff;
-                    dzz[b][0] = 2.0f * diff;
-                } else {  // PASS_QLOSS, dqn.rs:316-326
-                    float qv = zz[b][0];
-    #pragma unroll
-                    for (int k = 1; k < ANY_MAXA; ++k)
-                        if (k == act_s) qv = zz[b][k];
-                    const float diff = qv - tgt_s;
-                    loss_s = diff * diff;
-    #pragma unroll
-                    for (int k = 0; k < ANY_MAXA; ++k) dzz[b][k] = (k == act_s && k < A) ? 2.0f * diff : 0.0f;
+                        if (k < A && lane == k) a.logp0[ns * A + k] = lp[k];
                 }
                 sc[SC_COUNT] += 1.0;
-                sc[SC_LOSS] += (double)loss_s;
-                sc[SC_KL] += (double)kl_s;
-                sc[SC_ENTROPY] += (double)ent_s;
+                sc[SC_LOSS] += (double)s.loss;
+                sc[SC_KL] += (double)s.kl;
+                sc[SC_ENTROPY] += (double)s.entropy;
 #pragma unroll
                 for (int k = 0; k < ANY_MAXA; ++k) gb2[k] += (double)dzz[b][k];
             }
@@ -845,8 +662,8 @@ __global__ void __launch_bounds__(ANY_THREADS) mlp_pass_any_kernel(PassArgs a, A
                                 dh1 = fmaf(dzz[1][k], wk, dh1);
                                 tot[dl.off_w[LL] + j * ld + k] += (double)fmaf(dzz[1][k], hv1, dzz[0][k] * hv0);
                             }
-                        delta0[j] = dh0 * any_act_grad(act, hv0, hv0);
-                        delta1[j] = dh1 * any_act_grad(act, hv1, hv1);
+                        delta0[j] = dh0 * act_grad(act, hv0, hv0);
+                        delta1[j] = dh1 * act_grad(act, hv1, hv1);
                     }
                     __syncwarp();
                 }
@@ -863,8 +680,8 @@ __global__ void __launch_bounds__(ANY_THREADS) mlp_pass_any_kernel(PassArgs a, A
                         for (int i2 = lane; i2 < n_in; i2 += 32) {
                             float acc0, acc1;
                             any_dot2(Wt + i2 * ld, 1, delta0, delta1, n_out, 0.0f, 0.0f, acc0, acc1);
-                            next0[i2] = acc0 * any_act_grad(act, in0[i2], in0[i2]);
-                            next1[i2] = acc1 * any_act_grad(act, in1[i2], in1[i2]);
+                            next0[i2] = acc0 * act_grad(act, in0[i2], in0[i2]);
+                            next1[i2] = acc1 * act_grad(act, in1[i2], in1[i2]);
                         }
                         __syncwarp();
                         float *t0 = delta0; delta0 = next0; next0 = t0;
@@ -1357,7 +1174,7 @@ rl_status reduce_over_group(rl_ctx *ctx, const PassPlan &plan, int rows, const i
 template <int A, int MODE>
 rl_status launch_pass_ffma(rl_ctx *ctx, const PassPlan &plan, PassArgs args, bool reduce) {
     constexpr int F = 5, UPL = 4;
-    constexpr bool MSE = MODE == PASS_VALUE || MODE == PASS_QLOSS, FWD = MODE == PASS_STATS || MODE == PASS_EVAL;
+    constexpr bool MSE = MODE == RL_PASS_VALUE || MODE == RL_PASS_QLOSS, FWD = MODE == RL_PASS_STATS || MODE == RL_PASS_EVAL;
     constexpr int CH = MSE ? 4 : 8, MINB = MSE || FWD ? 2 : 1;
     const size_t smem = pass_smem_bytes<F, A, UPL>();
     static bool configured = false;
@@ -1460,11 +1277,9 @@ rl_status pass_net_for(rl_ctx *ctx, const rl_mlp *m, int F_data, const char *wha
 
 template <int MODE>
 rl_status launch_pass_any_mode(rl_ctx *ctx, const PassPlan &plan, PassArgs args, const AnyShape &sh, bool reduce) {
-    constexpr bool BACKWARD = MODE == PASS_GRAD || MODE == PASS_FVP || MODE == PASS_VALUE || MODE == PASS_QLOSS ||
-                              MODE == PASS_PPO || MODE == PASS_REINFORCE;
     int nwarps = ANY_THREADS / 32;
-    while (nwarps > 1 && any_smem_bytes(sh, nwarps, BACKWARD, MODE == PASS_FVP) > ANY_SMEM_CAP) nwarps >>= 1;
-    const size_t smem = any_smem_bytes(sh, nwarps, BACKWARD, MODE == PASS_FVP);
+    while (nwarps > 1 && any_smem_bytes(sh, nwarps, pass_backward(MODE), MODE == RL_PASS_FVP) > ANY_SMEM_CAP) nwarps >>= 1;
+    const size_t smem = any_smem_bytes(sh, nwarps, pass_backward(MODE), MODE == RL_PASS_FVP);
     static bool configured = false;
     if (!configured) {
         RL_CUDA(ctx, cudaFuncSetAttribute(mlp_pass_any_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ANY_SMEM_CAP));
@@ -1481,7 +1296,7 @@ rl_status launch_pass_any_mode(rl_ctx *ctx, const PassPlan &plan, PassArgs args,
 // pn.kernel selects it; every other module runs on mlp_pass_any_kernel.
 template <int MODE>
 rl_status launch_pass(rl_ctx *ctx, const PassPlan &plan, const PassArgs &pa, const PassNet &pn, bool reduce, int *rows) {
-    constexpr int A = MODE == PASS_VALUE ? 1 : 2;
+    constexpr int A = MODE == RL_PASS_VALUE ? 1 : 2;
     if (pn.deflt && pn.sh.A == A && pn.kernel == RL_PASS_KERNEL_TCGEN05) {
         if (rows) *rows = tc_grid<A, MODE>(ctx, plan);
         return launch_pass_tc<A, MODE>(ctx, plan, pa, reduce);
@@ -1494,14 +1309,14 @@ rl_status launch_pass(rl_ctx *ctx, const PassPlan &plan, const PassArgs &pa, con
 rl_status launch_pass_rt(rl_ctx *ctx, const PassPlan &plan, const PassArgs &pa, int mode, const PassNet &pn, bool reduce = true,
                          int *rows = nullptr) {
     switch (mode) {
-    case PASS_STATS: return launch_pass<PASS_STATS>(ctx, plan, pa, pn, reduce, rows);
-    case PASS_EVAL: return launch_pass<PASS_EVAL>(ctx, plan, pa, pn, reduce, rows);
-    case PASS_GRAD: return launch_pass<PASS_GRAD>(ctx, plan, pa, pn, reduce, rows);
-    case PASS_FVP: return launch_pass<PASS_FVP>(ctx, plan, pa, pn, reduce, rows);
-    case PASS_PPO: return launch_pass<PASS_PPO>(ctx, plan, pa, pn, reduce, rows);
-    case PASS_REINFORCE: return launch_pass<PASS_REINFORCE>(ctx, plan, pa, pn, reduce, rows);
-    case PASS_QLOSS: return launch_pass<PASS_QLOSS>(ctx, plan, pa, pn, reduce, rows);
-    case PASS_VALUE: return launch_pass<PASS_VALUE>(ctx, plan, pa, pn, reduce, rows);
+    case RL_PASS_STATS: return launch_pass<RL_PASS_STATS>(ctx, plan, pa, pn, reduce, rows);
+    case RL_PASS_EVAL: return launch_pass<RL_PASS_EVAL>(ctx, plan, pa, pn, reduce, rows);
+    case RL_PASS_GRAD: return launch_pass<RL_PASS_GRAD>(ctx, plan, pa, pn, reduce, rows);
+    case RL_PASS_FVP: return launch_pass<RL_PASS_FVP>(ctx, plan, pa, pn, reduce, rows);
+    case RL_PASS_PPO: return launch_pass<RL_PASS_PPO>(ctx, plan, pa, pn, reduce, rows);
+    case RL_PASS_REINFORCE: return launch_pass<RL_PASS_REINFORCE>(ctx, plan, pa, pn, reduce, rows);
+    case RL_PASS_QLOSS: return launch_pass<RL_PASS_QLOSS>(ctx, plan, pa, pn, reduce, rows);
+    case RL_PASS_VALUE: return launch_pass<RL_PASS_VALUE>(ctx, plan, pa, pn, reduce, rows);
     default: return rl_fail(ctx, RL_ERR_INVALID_ARG, "unknown pass mode %d", mode);
     }
 }
@@ -1599,8 +1414,7 @@ struct UpdateNet {
         if (!recurrent) return launch_pass_rt(ctx, plan, a, mode, pn);
         rl_seq_pass_args s = seq;
         s.obs = a.obs; s.action = a.action; s.succ = a.succ; s.T = a.T; s.E = a.E; s.theta = a.theta; s.vec = a.vec;
-        s.adv = a.adv; s.target = a.target; s.logp0 = a.logp0; s.skip_flag = a.skip_flag; s.clip_lo = a.clip_lo;
-        s.clip_hi = a.clip_hi;
+        s.adv = a.adv; s.target = a.target; s.logp0 = a.logp0; s.skip_flag = a.skip_flag;
         if (!rl_seq_pass_supports(s.F, s.H, s.A) || seq_force_big()) {
             // K10 (gru_big.cu): tiled GEMMs over the lanes of a step; one partial row
             RL_TRY(rl_seq_big_pass_launch(ctx, mode, s));
@@ -1738,24 +1552,24 @@ rl_status trpo_update(const UpdateNet &u, const rl_trpo_cfg *cfg, rl_trpo_stats 
     RL_TRY(timer.start());
     const float reg = (float)cfg->hpv_reg_coeff;
     // behaviour-policy statistics (no_grad block, trpo.rs:112-122)
-    RL_TRY(u.pass(PASS_STATS));
+    RL_TRY(u.pass(RL_PASS_STATS));
     RL_LAUNCH(ctx, trpo_begin_kernel, 1, 32, 0, st, sums, P);
     // loss gradient at theta0 (conjugate_gradient.rs:121-143)
-    RL_TRY(u.pass(PASS_GRAD));
+    RL_TRY(u.pass(RL_PASS_GRAD));
     RL_LAUNCH(ctx, trpo_cg_init_kernel, 1, VEC_THREADS, 0, st, sums, P, g, x, r, p, theta, theta0);
     // conjugate gradient on the Fisher matrix (conjugate_gradient.rs:371-403)
     for (uint64_t it = 0; it < cfg->cg_iterations; ++it) {
-        RL_TRY(u.pass(PASS_FVP, p, &st->cg_done));
+        RL_TRY(u.pass(RL_PASS_FVP, p, &st->cg_done));
         RL_LAUNCH(ctx, trpo_cg_step_kernel, 1, VEC_THREADS, 0, st, sums, P, x, r, p, reg, 1e-10);
     }
     RL_LAUNCH(ctx, trpo_nan_to_num_kernel, 1, VEC_THREADS, 0, st, x, P);
-    RL_TRY(u.pass(PASS_FVP, x));
+    RL_TRY(u.pass(RL_PASS_FVP, x));
     RL_LAUNCH(ctx, trpo_step_size_kernel, 1, VEC_THREADS, 0, st, sums, P, x, descent, reg, cfg->max_policy_step_kl);
     // backtracking line search (conjugate_gradient.rs:183-254)
     for (uint64_t i = 0; i < cfg->max_backtracks; ++i) {
         const double ratio = std::pow(cfg->backtrack_ratio, (double)i);
         RL_LAUNCH(ctx, trpo_ls_candidate_kernel, 1, VEC_THREADS, 0, st, theta, theta0, descent, (float)ratio, P);
-        RL_TRY(u.pass(PASS_EVAL, nullptr, &st->accepted));
+        RL_TRY(u.pass(RL_PASS_EVAL, nullptr, &st->accepted));
         RL_LAUNCH(ctx, trpo_ls_check_kernel, 1, 32, 0, st, sums, P, cfg->max_policy_step_kl, (int)i, ratio);
     }
     RL_LAUNCH(ctx, trpo_ls_finish_kernel, 1, VEC_THREADS, 0, st, theta, theta0, P, cfg->max_policy_step_kl,
@@ -1784,15 +1598,15 @@ rl_status trpo_probe(const UpdateNet &u, const float *vec_host, double hpv_reg_c
     rl_ctx *ctx = u.ctx;
     const int P = u.P;
     std::vector<double> host;
-    RL_TRY(probe_pass(u, PASS_STATS, nullptr, host, nullptr, nullptr));
+    RL_TRY(probe_pass(u, RL_PASS_STATS, nullptr, host, nullptr, nullptr));
     const double N = host[P + SC_COUNT];
     if (entropy) *entropy = host[P + SC_ENTROPY] / N;
-    RL_TRY(probe_pass(u, PASS_GRAD, nullptr, host, loss, grad_host));
+    RL_TRY(probe_pass(u, RL_PASS_GRAD, nullptr, host, loss, grad_host));
     if (kl) *kl = host[P + SC_KL] / N;
     if (vec_host && fvp_host) {
         float *vec = (float *)u.extra;
         RL_CUDA(ctx, cudaMemcpyAsync(vec, vec_host, (size_t)P * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-        RL_TRY(probe_pass(u, PASS_FVP, vec, host, nullptr, nullptr));
+        RL_TRY(probe_pass(u, RL_PASS_FVP, vec, host, nullptr, nullptr));
         for (int i = 0; i < P; ++i) fvp_host[i] = (float)(host[i] / N) + vec_host[i] * (float)hpv_reg_coeff;
     }
     return RL_OK;
@@ -1806,7 +1620,7 @@ rl_status value_update(const UpdateNet &u, rl_adam *adam, int n_steps, rl_opt_st
     UpdateTimer timer{ctx, stats != nullptr};
     RL_TRY(timer.start());
     const AdamArgs ac = adam_args(adam);
-    for (int s = 0; s < n_steps; ++s) RL_TRY(u.adam_step(PASS_VALUE, adam, ac, losses + s));
+    for (int s = 0; s < n_steps; ++s) RL_TRY(u.adam_step(RL_PASS_VALUE, adam, ac, losses + s));
     if (stats) {
         RL_TRY(timer.stop());
         double *host;
@@ -1837,13 +1651,13 @@ rl_status policy_adam_update(UpdateNet &u, rl_adam *adam, int n_steps, double cl
     double *entropy_sum = losses + n_steps;  // [sum of entropies, N]
     if (ppo) {
         // initial log-probs and entropy under no_grad (ppo.rs:108-119)
-        RL_TRY(u.pass(PASS_STATS));
+        RL_TRY(u.pass(RL_PASS_STATS));
         RL_CUDA(ctx, cudaMemcpyAsync(entropy_sum, sums + P + SC_ENTROPY, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
         RL_CUDA(ctx, cudaMemcpyAsync(entropy_sum + 1, sums + P + SC_COUNT, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
-        for (int s = 0; s < n_steps; ++s) RL_TRY(u.adam_step(PASS_PPO, adam, ac, losses + s));
+        for (int s = 0; s < n_steps; ++s) RL_TRY(u.adam_step(RL_PASS_PPO, adam, ac, losses + s));
     } else {
         for (int s = 0; s < n_steps; ++s) {
-            RL_TRY(u.adam_step(PASS_REINFORCE, adam, ac, losses + s));
+            RL_TRY(u.adam_step(RL_PASS_REINFORCE, adam, ac, losses + s));
             if (s == 0) {  // entropies.get_or_insert_with: the distribution of the first loss evaluation (reinforce.rs:76)
                 RL_CUDA(ctx, cudaMemcpyAsync(entropy_sum, sums + P + SC_ENTROPY, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
                 RL_CUDA(ctx, cudaMemcpyAsync(entropy_sum + 1, sums + P + SC_COUNT, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
@@ -2009,7 +1823,7 @@ rl_status rl_value_probe(rl_traj *traj, const float *targets_dev, rl_mlp *value_
     RL_TRY(u.init(ctx, value_fn, pn, traj_args(traj), 0, false));
     u.args.target = targets_dev;
     std::vector<double> host;
-    return probe_pass(u, PASS_VALUE, nullptr, host, loss, grad_host);
+    return probe_pass(u, RL_PASS_VALUE, nullptr, host, loss, grad_host);
 }
 
 rl_status rl_ppo_update(rl_traj *traj, const float *adv_dev, rl_mlp *policy, rl_adam *adam, const rl_ppo_cfg *cfg,
@@ -2080,7 +1894,7 @@ rl_status rl_dqn_update(rl_replay *rb, rl_mlp *q, rl_adam *adam, const rl_dqn_cf
         u.args.obs = mb.obs + set * mb.capacity * F; u.args.action = mb.action + set * mb.capacity;
         u.args.succ = mb.succ + set * mb.capacity; u.args.target = mb.target + set * mb.capacity;
         // loss_fn + backward_step (dqn.rs:316-336, coptimizer.rs:13-27)
-        RL_TRY(u.adam_step(PASS_QLOSS, adam, ac, losses + s));
+        RL_TRY(u.adam_step(RL_PASS_QLOSS, adam, ac, losses + s));
     }
     uint64_t m_last = 0;
     if (n_steps > 0) RL_TRY(rl_replay_sample_finish(rb, &m_last, nullptr));
@@ -2125,7 +1939,7 @@ rl_status rl_dqn_update_seq(rl_replay *rb, rl_grunet *q, rl_adam *adam, const rl
         u.args.target = target;
         double *loss_dev = (double *)u.extra;
         // loss_fn + backward_step (dqn.rs:316-336, coptimizer.rs:13-27)
-        RL_TRY(u.adam_step(PASS_QLOSS, adam, ac, loss_dev));
+        RL_TRY(u.adam_step(RL_PASS_QLOSS, adam, ac, loss_dev));
         // the next sample synchronises anyway; the plan's scratch may move with the next sample's size
         if (stats) {
             RL_CUDA(ctx, cudaMemcpyAsync(&losses[(size_t)s], loss_dev, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
@@ -2156,7 +1970,7 @@ rl_status rl_dqn_probe_seq(rl_replay *rb, const rl_dqn_cfg *cfg, rl_grunet *q, u
     RL_TRY(u.init(ctx, net, traj_args(mb), 0));
     u.args.target = target;
     std::vector<double> host;
-    return probe_pass(u, PASS_QLOSS, nullptr, host, loss, grad_host);
+    return probe_pass(u, RL_PASS_QLOSS, nullptr, host, loss, grad_host);
 }
 
 }  // extern "C"

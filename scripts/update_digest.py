@@ -7,8 +7,9 @@ launch the same kernels print the same text, so a change to the host code around
 neither a bit nor a launch: run the script on both builds and diff the outputs.
 
 Covered: TRPO update and probe, critic update, critic probe on both pass kernels, PPO, REINFORCE, DQN with reward-to-go
-and one-step TD targets, on the default 5-128 modules and on a two-hidden-layer tanh Mlp; TRPO update and probe, critic
-update, DQN update and probe on recurrent modules of hidden 8 and 128.
+and one-step TD targets, on the default 5-128 modules (once on the tensor-core pass kernel and once on its FP32-pipe twin,
+rl_pass_kernel_select(RL_PASS_KERNEL_FFMA)) and on a two-hidden-layer tanh Mlp; TRPO update and probe, critic update,
+DQN update and probe on GRU and LSTM modules of hidden 8 and 128.
 
 usage: python scripts/update_digest.py > digest.txt
 """
@@ -184,16 +185,16 @@ def mlp_runs(d, ctx, lib, env, traj, hidden, act, tag):
     d.run(f"{tag} rl_dqn_update one-step-td", dqn(True))
 
 
-def gru_runs(d, ctx, lib, env, traj, hidden):
+def seq_runs(d, ctx, lib, env, traj, hidden, cls, init, tag):
     rng = np.random.default_rng(23)
     F, A = 5, 2
     adv = ctx.to_device(rng.normal(size=(T, E)).astype(np.float32))
     tgt = ctx.to_device((rng.normal(size=(T, E)) * 3.0).astype(np.float32))
-    tag = f"gru-{hidden}"
+    tag = f"{tag}-{hidden}"
 
     def module(out_dim, seed):
-        g = R.GruLinear(ctx, F, hidden, out_dim)
-        g.set_weights(R.init_gru_linear_params(np.random.default_rng(seed), F, hidden, out_dim).astype(np.float32))
+        g = cls(ctx, F, hidden, out_dim)
+        g.set_weights(init(np.random.default_rng(seed), F, hidden, out_dim).astype(np.float32))
         return g
 
     def trpo_update():
@@ -261,9 +262,14 @@ def main():
     R.rollout(env, R.ActorSpec(kind=L.RL_ACTOR_RANDOM), R.HistoryDataBound(T, 0), traj)
     d = Digest(ctx)
     mlp_runs(d, ctx, lib, env, traj, [128], "relu", "mlp-5-128")
+    L.check(lib.rl_pass_kernel_select(L.RL_PASS_KERNEL_FFMA))
+    mlp_runs(d, ctx, lib, env, traj, [128], "relu", "mlp-5-128-ffma")
+    L.check(lib.rl_pass_kernel_select(L.RL_PASS_KERNEL_TCGEN05))
     mlp_runs(d, ctx, lib, env, traj, [32, 32], "tanh", "mlp-5-32x32-tanh")
     for hidden in (8, 128):
-        gru_runs(d, ctx, lib, env, traj, hidden)
+        seq_runs(d, ctx, lib, env, traj, hidden, R.GruLinear, R.init_gru_linear_params, "gru")
+    for hidden in (8, 128):
+        seq_runs(d, ctx, lib, env, traj, hidden, R.LstmLinear, R.init_lstm_linear_params, "lstm")
     print("\n".join(d.lines))
 
 
