@@ -482,6 +482,12 @@ rl_status rl_ppo_update(rl_traj *traj, const float *adv_dev, rl_mlp *policy, rl_
 /* one backward_step on -(log_probs * advantages).mean() */
 rl_status rl_reinforce_update(rl_traj *traj, const float *adv_dev, rl_mlp *policy, rl_adam *adam,
                               rl_policy_opt_stats *stats);
+/* The same two updates for a recurrent policy (Chain<Gru, Linear> or Chain<Lstm, Linear>, the shapes of
+ * rl_trpo_update_seq) with back-propagation through time; `adam` from rl_adam_create_seq on that policy. */
+rl_status rl_ppo_update_seq(rl_traj *traj, const float *adv_dev, rl_grunet *policy, rl_adam *adam, const rl_ppo_cfg *cfg,
+                            rl_policy_opt_stats *stats);
+rl_status rl_reinforce_update_seq(rl_traj *traj, const float *adv_dev, rl_grunet *policy, rl_adam *adam,
+                                  rl_policy_opt_stats *stats);
 
 /* ------------------------------------------------------------------------------------------ */
 /* Tabular Q (BaseTabularQLearningAgent src/agents/tabular.rs:84-232)                           */

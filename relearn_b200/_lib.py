@@ -222,6 +222,8 @@ SIGNATURES = {
     "rl_ppo_cfg_default": (None, [P(PpoCfg)]),
     "rl_ppo_update": (st, [vp, vp, vp, vp, P(PpoCfg), P(PolicyOptStats)]),
     "rl_reinforce_update": (st, [vp, vp, vp, vp, P(PolicyOptStats)]),
+    "rl_ppo_update_seq": (st, [vp, vp, vp, vp, P(PpoCfg), P(PolicyOptStats)]),
+    "rl_reinforce_update_seq": (st, [vp, vp, vp, vp, P(PolicyOptStats)]),
     "rl_pack_history": (st, [vp, vp, vp, vp, vp, vp, vp, vp, P(PackedInfo)]),
     "rl_tabq_create": (st, [vp, C.c_uint64, C.c_int32, C.c_int32, C.c_double, P(vp)]),
     "rl_tabq_destroy": (st, [vp]),

@@ -412,7 +412,7 @@ __global__ void __launch_bounds__(HEAD_THREADS) big_head_kernel(rl_seq_pass_args
             }
             float lp[HEAD_MAXA];
             const SampleLoss ls = sample_loss<MODE, HEAD_MAXA>(z, zd, A, M::USES_ACT ? (int)a.action[idx] : 0, M::USES_ADV ? a.adv[idx] : 0.0f,
-                                                               M::USES_TARGET ? a.target[idx] : 0.0f, float2{},
+                                                               M::USES_TARGET ? a.target[idx] : 0.0f, make_float2(a.clip_lo, a.clip_hi),
                                                                [&](int k) { return a.logp0[(t * A + k) * E + e]; }, lp, dz);
             if (MODE == RL_PASS_STATS) {
 #pragma unroll
@@ -792,6 +792,8 @@ rl_status rl_seq_big_pass_launch(rl_ctx *ctx, int mode, const rl_seq_pass_args &
     case RL_PASS_FVP: RL_TRY(launch_head<RL_PASS_FVP>(ctx, a, pl, scal_part, head_blocks)); break;
     case RL_PASS_VALUE: RL_TRY(launch_head<RL_PASS_VALUE>(ctx, a, pl, scal_part, head_blocks)); break;
     case RL_PASS_QLOSS: RL_TRY(launch_head<RL_PASS_QLOSS>(ctx, a, pl, scal_part, head_blocks)); break;
+    case RL_PASS_PPO: RL_TRY(launch_head<RL_PASS_PPO>(ctx, a, pl, scal_part, head_blocks)); break;
+    case RL_PASS_REINFORCE: RL_TRY(launch_head<RL_PASS_REINFORCE>(ctx, a, pl, scal_part, head_blocks)); break;
     default: return rl_fail(ctx, RL_ERR_INVALID_ARG, "rl_seq_big_pass_launch: bad mode %d", mode);
     }
     // ---- backward through time, then the weight gradients as two split-K GEMMs over all (t, e) ----

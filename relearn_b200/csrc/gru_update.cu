@@ -1,6 +1,6 @@
 // gru_update.cu -- full-batch passes over trajectories for a recurrent policy / critic / Q-network (Chain<Gru, Linear>):
-// what autograd does for the reference when the module of Trpo / ValuesOpt / DqnAgent is a GRU
-// (src/torch/agents/policies/trpo.rs:97-164 with cuDNN disabled :104-108, critics/opt.rs:100-127,
+// what autograd does for the reference when the module of Trpo / Ppo / Reinforce / ValuesOpt / DqnAgent is a GRU
+// (src/torch/agents/policies/trpo.rs:97-164 with cuDNN disabled :104-108, ppo.rs:97-147, reinforce.rs:64-89, critics/opt.rs:100-127,
 // modules/seq/rnn/gru.rs:72-102, modules/chain.rs:157-168).
 //
 // K9 gru_pass_kernel<MODE>: one thread per lane.  Episodes never cross lanes and a lane's steps are a
@@ -330,12 +330,34 @@ __global__ void __launch_bounds__(RL_SEQ_BLOCK) gru_pass_kernel(rl_seq_pass_args
                 if (M::USES_LP0) {
                     const float lp0a = a.logp0[(t * A + act_s) * E + e];
                     const float ratio = expf(lp[act_s] - lp0a);
-                    loss_s = -(ratio * a.adv[n_idx]);
+                    if (MODE == RL_PASS_PPO) {
+                        // -min(ratio adv, clip(ratio) adv); d/d ratio = adv inside [lo, hi] or where the unclipped term is the smaller
+                        const float adv_s = a.adv[n_idx];
+                        const float clipped = fminf(fmaxf(ratio, a.clip_lo), a.clip_hi);
+                        const float t1 = ratio * adv_s, t2 = clipped * adv_s;
+                        loss_s = -fminf(t1, t2);
+                        const bool inside = ratio >= a.clip_lo && ratio <= a.clip_hi;
+                        const float gr = (inside || t1 < t2) ? -t1 : 0.0f;
+#pragma unroll
+                        for (int k = 0; k < A; ++k) dz[k] = gr * ((act_s == k ? 1.0f : 0.0f) - p[k]);
+                    } else {
+                        loss_s = -(ratio * a.adv[n_idx]);
+#pragma unroll
+                        for (int k = 0; k < A; ++k) {
+                            const float lp0k = a.logp0[(t * A + k) * E + e];
+                            kl_s += fmaxf(lp0k - lp[k], F32_LOWEST) * expf(lp0k);
+                            if (MODE == RL_PASS_GRAD) dz[k] = loss_s * ((act_s == k ? 1.0f : 0.0f) - p[k]);
+                        }
+                    }
+                }
+                if (MODE == RL_PASS_REINFORCE) {
+                    // -(log p(a) adv); the entropy of this evaluation is the one logged (reinforce.rs:72-79)
+                    const float adv_s = a.adv[n_idx];
+                    loss_s = -(lp[act_s] * adv_s);
 #pragma unroll
                     for (int k = 0; k < A; ++k) {
-                        const float lp0k = a.logp0[(t * A + k) * E + e];
-                        kl_s += fmaxf(lp0k - lp[k], F32_LOWEST) * expf(lp0k);
-                        if (MODE == RL_PASS_GRAD) dz[k] = loss_s * ((act_s == k ? 1.0f : 0.0f) - p[k]);
+                        ent_s -= fmaxf(lp[k], F32_LOWEST) * p[k];
+                        dz[k] = -adv_s * ((act_s == k ? 1.0f : 0.0f) - p[k]);
                     }
                 }
                 if (FVP) {
@@ -526,6 +548,8 @@ rl_status rl_seq_pass_launch(rl_ctx *ctx, int mode, const rl_seq_pass_args &a, i
     case RL_PASS_FVP: return launch_mode<RL_PASS_FVP>(ctx, a, grid, smem);
     case RL_PASS_VALUE: return launch_mode<RL_PASS_VALUE>(ctx, a, grid, smem);
     case RL_PASS_QLOSS: return launch_mode<RL_PASS_QLOSS>(ctx, a, grid, smem);
+    case RL_PASS_PPO: return launch_mode<RL_PASS_PPO>(ctx, a, grid, smem);
+    case RL_PASS_REINFORCE: return launch_mode<RL_PASS_REINFORCE>(ctx, a, grid, smem);
     default: return rl_fail(ctx, RL_ERR_INVALID_ARG, "rl_seq_pass_launch: bad mode %d", mode);
     }
 }

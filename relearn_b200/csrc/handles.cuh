@@ -116,6 +116,7 @@ struct rl_seq_pass_args {
     const int *skip_flag;
     int cell;       // RL_CELL_GRU / RL_CELL_LSTM
     float *cbuf;    // f32 [T][H][E]  LSTM: cell state before each step (K9)
+    float clip_lo, clip_hi;  // RL_PASS_PPO: 1 -+ clip_distance as f32 (ppo.rs:131-132)
 };
 // lanes per block (= per partial row) of the recurrent passes: two warps, so that a block's warps finish close together
 constexpr int RL_SEQ_BLOCK = 64;

@@ -1415,6 +1415,7 @@ struct UpdateNet {
         rl_seq_pass_args s = seq;
         s.obs = a.obs; s.action = a.action; s.succ = a.succ; s.T = a.T; s.E = a.E; s.theta = a.theta; s.vec = a.vec;
         s.adv = a.adv; s.target = a.target; s.logp0 = a.logp0; s.skip_flag = a.skip_flag;
+        s.clip_lo = a.clip_lo; s.clip_hi = a.clip_hi;
         if (!rl_seq_pass_supports(s.F, s.H, s.A) || seq_force_big()) {
             // K10 (gru_big.cu): tiled GEMMs over the lanes of a step; one partial row
             RL_TRY(rl_seq_big_pass_launch(ctx, mode, s));
@@ -1852,6 +1853,36 @@ rl_status rl_reinforce_update(rl_traj *traj, const float *adv_dev, rl_mlp *polic
     RL_TRY(u.init(ctx, policy, pn, traj_args(traj), policy_loss_bytes(1), true));
     u.args.adv = adv_dev;
     return policy_adam_update(u, adam, 1, 0.0, false, stats, "rl_reinforce_update");
+}
+
+rl_status rl_ppo_update_seq(rl_traj *traj, const float *adv_dev, rl_grunet *policy, rl_adam *adam, const rl_ppo_cfg *cfg,
+                            rl_policy_opt_stats *stats) {
+    if (!traj || !adv_dev || !policy || !adam || !cfg)
+        return rl_fail(traj ? traj->ctx : nullptr, RL_ERR_INVALID_ARG, "rl_ppo_update_seq: NULL argument");
+    rl_ctx *ctx = traj->ctx;
+    const rl_grunet_view net = rl_grunet_view_of(policy);
+    RL_REQUIRE(ctx, net.ctx == ctx, "rl_ppo_update_seq: module belongs to another context");
+    RL_TRY(seq_check(ctx, net, (int)traj->F, 0, "rl_ppo_update_seq"));
+    const uint64_t n_steps = cfg->opt_steps_per_update;
+    RL_TRY(adam_check(ctx, adam, policy, n_steps > 100000 ? -1 : (int)n_steps, "rl_ppo_update_seq"));
+    UpdateNet u;
+    RL_TRY(u.init(ctx, net, traj_args(traj), policy_loss_bytes((int)n_steps)));
+    u.args.adv = adv_dev;
+    return policy_adam_update(u, adam, (int)n_steps, cfg->clip_distance, true, stats, "rl_ppo_update_seq");
+}
+
+rl_status rl_reinforce_update_seq(rl_traj *traj, const float *adv_dev, rl_grunet *policy, rl_adam *adam, rl_policy_opt_stats *stats) {
+    if (!traj || !adv_dev || !policy || !adam)
+        return rl_fail(traj ? traj->ctx : nullptr, RL_ERR_INVALID_ARG, "rl_reinforce_update_seq: NULL argument");
+    rl_ctx *ctx = traj->ctx;
+    const rl_grunet_view net = rl_grunet_view_of(policy);
+    RL_REQUIRE(ctx, net.ctx == ctx, "rl_reinforce_update_seq: module belongs to another context");
+    RL_TRY(seq_check(ctx, net, (int)traj->F, 0, "rl_reinforce_update_seq"));
+    RL_TRY(adam_check(ctx, adam, policy, 1, "rl_reinforce_update_seq"));
+    UpdateNet u;
+    RL_TRY(u.init(ctx, net, traj_args(traj), policy_loss_bytes(1)));
+    u.args.adv = adv_dev;
+    return policy_adam_update(u, adam, 1, 0.0, false, stats, "rl_reinforce_update_seq");
 }
 
 // DqnAgent::batch_update (dqn.rs:263-337) with an Mlp action-value module, on flat minibatch planes.

@@ -147,7 +147,7 @@ class Trpo:
 class PpoConfig:
     """policies/ppo.rs:14-41"""
 
-    policy_fn_config: MlpConfig = field(default_factory=MlpConfig)
+    policy_fn_config: object = field(default_factory=MlpConfig)  # MlpConfig | GruLinearConfig | LstmLinearConfig
     optimizer_config: AdamConfig = field(default_factory=AdamConfig)
     opt_steps_per_update: int = 10
     clip_distance: float = 0.2
@@ -162,7 +162,13 @@ class _AdamPolicy:
         self.ctx, self._lib = policy_fn.ctx, policy_fn.ctx._lib
         self.optimizer = Adam(policy_fn, cfg.optimizer_config)
 
+    @property
+    def recurrent(self) -> bool:
+        return isinstance(self.policy_fn, SeqLinear)
+
     def actor(self, lanes_per_env: int = 0) -> ActorSpec:
+        if self.recurrent:
+            return ActorSpec(kind=L.RL_ACTOR_CATEGORICAL_POLICY, seq_net=self.policy_fn)
         return ActorSpec(kind=L.RL_ACTOR_CATEGORICAL_POLICY, net=self.policy_fn, lanes_per_env=lanes_per_env)
 
     def _log(self, stats, logger):
@@ -177,8 +183,9 @@ class Ppo(_AdamPolicy):
     def update(self, traj: Trajectory, advantages: DeviceBuffer, logger: dict | None = None) -> int:
         stats = L.PolicyOptStats()
         cfg = L.PpoCfg(self.cfg.opt_steps_per_update, self.cfg.clip_distance)
-        L.check(self._lib.rl_ppo_update(traj.handle, advantages.c, self.policy_fn.handle, self.optimizer.handle, C.byref(cfg),
-                                        C.byref(stats)), self.ctx.handle)
+        fn = self._lib.rl_ppo_update_seq if self.recurrent else self._lib.rl_ppo_update
+        L.check(fn(traj.handle, advantages.c, self.policy_fn.handle, self.optimizer.handle, C.byref(cfg), C.byref(stats)),
+                self.ctx.handle)
         self._log(stats, logger)
         return L.RL_OK
 
@@ -187,7 +194,7 @@ class Ppo(_AdamPolicy):
 class ReinforceConfig:
     """policies/reinforce.rs:10-16"""
 
-    policy_fn_config: MlpConfig = field(default_factory=MlpConfig)
+    policy_fn_config: object = field(default_factory=MlpConfig)  # MlpConfig | GruLinearConfig | LstmLinearConfig
     optimizer_config: AdamConfig = field(default_factory=AdamConfig)
 
     def build_policy(self, ctx: Context, in_dim: int, out_dim: int) -> "Reinforce":
@@ -199,8 +206,8 @@ class Reinforce(_AdamPolicy):
 
     def update(self, traj: Trajectory, advantages: DeviceBuffer, logger: dict | None = None) -> int:
         stats = L.PolicyOptStats()
-        L.check(self._lib.rl_reinforce_update(traj.handle, advantages.c, self.policy_fn.handle, self.optimizer.handle,
-                                              C.byref(stats)), self.ctx.handle)
+        fn = self._lib.rl_reinforce_update_seq if self.recurrent else self._lib.rl_reinforce_update
+        L.check(fn(traj.handle, advantages.c, self.policy_fn.handle, self.optimizer.handle, C.byref(stats)), self.ctx.handle)
         self._log(stats, logger)
         return L.RL_OK
 
