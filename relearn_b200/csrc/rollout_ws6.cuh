@@ -149,6 +149,10 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
         double coef[14];
 #pragma unroll
         for (int c = 0; c < 14; ++c) coef[c] = __shfl_sync(FULL, rl_cartpole_sincos_coef[c], 0);
+        // beta's divisor is the constant mass_length_pole: its reciprocal (MUFU.RCP64H and the Newton steps, which ptxas left
+        // inside the loop) once, and the slack bound of the step loop, which it otherwise reloads from the constant bank
+        const double rcp_ml = __shfl_sync(FULL, EnvT::rcp_fast(q.mass_length_pole), 0);
+        const uint32_t slack = __shfl_sync(FULL, a.slack, 0);
         EnvT::State s;
         s.x = s.xd = s.th = s.thd = 0.0;
         s.meta = 0x80000000u | p.max_steps;
@@ -182,8 +186,9 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
             // before the action is known: the step for both actions, the would-be reset state, and the `remaining` feature
             // of the next observation
             EnvT::State c0s = s, c1s = s;
-            const int sc0 = EnvT::step_fast(q, c0s, 0u, coef);
-            const int sc1 = EnvT::step_fast(q, c1s, 1u, coef);
+            // (a state that terminates is replaced by `fresh` below: step_fast need not keep it)
+            const int sc0 = EnvT::step_fast<false>(q, c0s, 0u, coef, rcp_ml);
+            const int sc1 = EnvT::step_fast<false>(q, c1s, 1u, coef, rcp_ml);
             EnvT::State fresh;
             fresh_state(it + 1, fresh);
             const uint32_t r_now = s.meta & 0x7FFFFFFFu;
@@ -204,7 +209,7 @@ __global__ void __launch_bounds__(QK_THREADS, 1) rollout_cartpole_ws6_kernel(Car
             uint32_t n_next = n;
             if (active) {
                 n_next = n - 1;
-                if (ended && n_next <= a.slack) n_next = 0;  // take_steps.rs:83-88
+                if (ended && n_next <= slack) n_next = 0;  // take_steps.rs:83-88
             }
             const bool any_next = __any_sync(FULL, n_next > 0);
             smem_st4(row, make_float4((float)s.x, (float)s.xd, (float)s.th, (float)s.thd));
