@@ -314,10 +314,10 @@ typedef enum {
 
 /* rl_actor_cfg.lanes_per_env value selecting the tensor-core rollout kernel (CartPole + 5/4-128-2 ReLU network) */
 #define RL_LANES_TENSOR_CORE 128
-/* rl_actor_cfg.lanes_per_env value selecting the warp-specialised rollout kernels (policy and dynamics of an env on
- * different warps; CartPole + 5/4-128-2 ReLU network): K2z up to 16 envs per SM, K2q beyond, at any size.  Their results
- * are bit-identical to lanes_per_env = 8.  They serve the categorical actor on Philox noise only; any other actor or
- * replayed noise is refused with RL_ERR_UNSUPPORTED. */
+/* rl_actor_cfg.lanes_per_env value selecting the warp-specialised rollout kernel K2q (policy and dynamics of an env on
+ * different warps; CartPole + 5/4-128-2 ReLU network) at any size.  Its results are bit-identical to lanes_per_env = 8.
+ * It serves the categorical actor on Philox noise only; any other actor or replayed noise is refused with
+ * RL_ERR_UNSUPPORTED. */
 #define RL_LANES_WARP_SPECIALIZED 160
 typedef struct rl_actor_cfg {
     int32_t kind;                 /* rl_actor_kind */
@@ -329,7 +329,7 @@ typedef struct rl_actor_cfg {
     int32_t training;             /* ActorMode::Training (src/agents/mod.rs:144) */
     int32_t lanes_per_env;        /* 0 = auto; threads cooperating on one env's MLP (1,2,4,8,16,32),
                                    * RL_LANES_TENSOR_CORE (128): 128-env tiles, hidden layer on tcgen05 (K2t), or
-                                   * RL_LANES_WARP_SPECIALIZED (160): K2z / K2q */
+                                   * RL_LANES_WARP_SPECIALIZED (160): K2q */
     rl_grunet *seq_net;           /* CATEGORICAL_POLICY / EPS_GREEDY_Q with a recurrent module (Chain<Gru, Linear>) instead of
                                    * `net`; hidden state zero at every episode start.  EPS_GREEDY_Q keeps the reference's order:
                                    * gen_bool(eps), then gen_range(A) on an explored step WITHOUT stepping the module (its hidden

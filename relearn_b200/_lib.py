@@ -17,7 +17,7 @@ RL_ERR_INVALID_ARG, RL_ERR_CUDA, RL_ERR_UNSUPPORTED, RL_ERR_OOM, RL_ERR_NCCL, RL
 RL_STEP_NAN_LOSS, RL_STEP_NAN_CONSTRAINT, RL_STEP_LOSS_NOT_IMPROVING, RL_STEP_CONSTRAINT_VIOLATED = 16, 17, 18, 19
 RL_CONTINUE, RL_TERMINATE, RL_INTERRUPT, RL_PAD = 0, 1, 2, 255
 RL_LANES_TENSOR_CORE = 128  # rl_actor_cfg.lanes_per_env: the tensor-core rollout kernel (K2t)
-RL_LANES_WARP_SPECIALIZED = 160  # the warp-specialised rollout kernels (K2z / K2q by size; bit-identical to lanes_per_env 8)
+RL_LANES_WARP_SPECIALIZED = 160  # the warp-specialised rollout kernel K2q (bit-identical to lanes_per_env 8)
 RL_ENV_CARTPOLE, RL_ENV_CHAIN, RL_ENV_MEMORY_GAME, RL_ENV_BANDIT_META, RL_ENV_PARTITION_GAME = 0, 1, 2, 3, 4
 RL_NOISE_PHILOX, RL_NOISE_REPLAY = 0, 1
 RL_SPACE_INTERVAL, RL_SPACE_INDEX, RL_SPACE_BOOLEAN, RL_SPACE_OPTION_INDEX = 0, 1, 2, 3

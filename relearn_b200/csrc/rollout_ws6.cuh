@@ -1,24 +1,83 @@
-// rollout_ws6.cuh -- K2q: the warp-specialised CartPole rollout with ONE CTA per SM at the bench size (E > 16 per SM).
-// K2z (rollout_ws5.cuh) puts 16 envs on a six-warp CTA, two of them per SM once E > 16 per SM.  Its per-phase clocks
-// (scripts/ws_clocks.sh, profiles/r2_summary.md section 5): with one CTA on an SM an iteration of the dynamics warp takes
-// ~850 clk (candidate step 480, select / convert / publish 171, step record 192) and the policy warps are never waited
-// for; with two CTAs on an SM (E = 4096) the same stream takes ~1150 clk because the dynamics warp -- ~75 % issue-busy on
-// its own -- shares its scheduler with policy warps.  K2q therefore
-//  * puts 32 envs on ONE dynamics warp, lane = env, which evaluates the step for BOTH actions in the same thread (four
-//    independent chains: 2 actions x 2 friction signs; everything that does not depend on the action -- sin / cos, the
-//    reciprocals, beta -- is computed once), so the select needs no shuffles and E = 4096 fits one CTA per SM (128 CTAs);
-//  * gives that warp a scheduler of its own: twelve warps, the two other warps of the dynamics warp's sub-partition
-//    idle at the final barrier, eight policy warps and the aux (Philox) warp on the other three sub-partitions;
-//  * takes the step record off the dynamics warp (as K2z): successor code and reward are stored one iteration later by
-//    two idle threads of the env's policy group (the row carries the previous step's code), episode statistics are
-//    integer counters, finalize_last_episode reads the dropped observation back from the trajectory;
-//  * needs no work around the launch: the dynamics lanes fill `succ` with RL_PAD past their last step, and the last CTA
-//    to finish sums every CTA's statistics (finalize_stat: rollout_finalize_kernel's sum, in its order).
-// The aux warp and its rings are K2z's (WS_RING / WS_CHUNK / WS_AHEAD, lane = env).  The hand-off has one row per env:
-// dynamics publishes the row of step i -> barrier 1 -> policy samples -> action -> barrier 2 -> dynamics selects.  The
-// grid is one CTA per 4 x policy_warps envs, so any number of waves runs.  Same operations on the same operands as
-// K2c<8>: bit-identical trajectories.  Included by rollout.cu after rollout_ws5.cuh.
+// rollout_ws6.cuh -- K2q: the warp-specialised CartPole rollout (RL_LANES_WARP_SPECIALIZED at any size, `lanes_per_env = 0`
+// for the categorical actor on Philox noise up to 64 envs per SM).  Included by rollout.cu inside its anonymous namespace.
+//
+// K2c<8> (rollout.cu) has each warp carry 4 envs x 8 threads and issue BOTH halves of the step chain: the policy
+// (obs -> hidden layer -> logit difference -> compare) and the f64 dynamics, the latter redundantly in all 8 threads of an
+// env.  K2q splits the chain by warp.  A CTA owns 4 x policy_warps envs (1 .. 8 policy warps, launch_ws6's shape rule) and
+// has twelve warps:
+//  * the POLICY warps, 4 envs x 8 threads each, with exactly K2c<8>'s register-resident hidden layer;
+//  * one DYNAMICS warp, lane = env, which evaluates the step for BOTH actions in the same thread (four independent chains:
+//    2 actions x 2 friction signs; everything that does not depend on the action -- sin / cos, the reciprocals, beta -- is
+//    computed once), so the select after the action needs no shuffles;
+//  * one AUX warp that draws every Philox block: the actor's uniform of each step, as its logit-space threshold, and the
+//    would-be reset state of each step.  It fills them WS_CHUNK steps at a time into WS_RING-step shared-memory rings, up
+//    to WS_AHEAD steps ahead of the dynamics warp.  Progress is three counters in shared memory, not a barrier: `prod`
+//    (steps filled, written by the aux warp), `cons` (the dynamics warp's iteration, posted every fourth) and `done` (the
+//    dynamics loop is over);
+//  * warps without a role (QK_ROLE_IDLE), which wait at the final barrier.
+// Warp w runs on sub-partition w % 4, and the dynamics warp has its sub-partition's scheduler to itself: per-phase clocks
+// (scripts/ws_clocks.sh, profiles/r2_summary.md section 5) put the step cycle on the dynamics warp's own instruction
+// stream, ~75 % issue-busy, and a dynamics stream that shared its scheduler with policy warps took ~1150 clk per step
+// instead of ~850.  Further work therefore leaves the dynamics warp: the step record's successor code and reward are
+// stored one iteration later by two idle threads of the env's policy group (the row carries the previous step's code),
+// episode statistics are integer counters, and finalize_last_episode reads the dropped observation back from the
+// trajectory.
+// No work around the launch: the dynamics lanes fill `succ` with RL_PAD past their last step, and the last CTA to finish
+// sums every CTA's statistics (finalize_stat: rollout_finalize_kernel's sum, in its order).
+// The hand-off has one row per env: dynamics publishes the row of step i -> barrier 1 -> policy samples -> action ->
+// barrier 2 -> dynamics selects.  The grid is one CTA per 4 x policy_warps envs, so any number of waves runs.  Same
+// operations on the same operands as K2c<8> (summation order of the logits included): bit-identical trajectories and
+// summaries (tests/test_gpu_envs.py).  Philox noise and the categorical actor only.
+// The earlier six-warp, 16-env kernel for up to 16 envs per SM was measured against K2q and retired
+// (profiles/r2_summary.md section 5, profiles/r4_k2q_small_e.md, git history).
 #pragma once
+
+constexpr int WS_RING = 16, WS_CHUNK = 4, WS_AHEAD = 11;  // the aux warp's rings
+
+__device__ __forceinline__ void named_bar_sync(int id, int n) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n) : "memory"); }
+__device__ __forceinline__ void named_bar_arrive(int id, int n) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(n) : "memory"); }
+
+// Shared memory through explicit 32-bit shared-window addresses (ld.shared / st.shared): with generic pointers ptxas
+// rematerialises the window base (S2UR SR_CgaCtaId + ULEA) inside the loops.
+__device__ __forceinline__ float4 smem_ld4(uint32_t a) {
+    float4 v;
+    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(a));
+    return v;
+}
+__device__ __forceinline__ void smem_st4(uint32_t a, float4 v) {
+    asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(a), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
+}
+__device__ __forceinline__ double2 smem_ldd2(uint32_t a) {
+    double2 v;
+    asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "r"(a));
+    return v;
+}
+__device__ __forceinline__ void smem_std2(uint32_t a, double2 v) {
+    asm volatile("st.shared.v2.f64 [%0], {%1, %2};" ::"r"(a), "d"(v.x), "d"(v.y) : "memory");
+}
+__device__ __forceinline__ float smem_ldf(uint32_t a) {
+    float v;
+    asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(a));
+    return v;
+}
+__device__ __forceinline__ uint32_t smem_ldu(uint32_t a) {
+    uint32_t v;
+    asm volatile("ld.volatile.shared.u32 %0, [%1];" : "=r"(v) : "r"(a));
+    return v;
+}
+__device__ __forceinline__ void smem_stu(uint32_t a, uint32_t v) { asm volatile("st.volatile.shared.u32 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
+__device__ __forceinline__ void smem_stf(uint32_t a, float v) { asm volatile("st.shared.f32 [%0], %1;" ::"r"(a), "f"(v) : "memory"); }
+
+#ifdef RL_WS_CLOCKS  // measurement build only (scripts/ws_clocks.sh): per-phase clocks of the dynamics / policy loops of two CTAs
+__device__ __forceinline__ long long ws_clk(double dep, uint32_t dep2) {
+    long long c;
+    asm volatile("mov.u64 %0, %%clock64;" : "=l"(c) : "d"(dep), "r"(dep2) : "memory");
+    return c;
+}
+#define WS_CLK(var, dep, dep2) const long long var = ws_clk(dep, dep2)
+#else
+#define WS_CLK(var, dep, dep2)
+#endif
 
 constexpr int QK_ENVS = 32, QK_THREADS = 384, QK_POLICY_WARPS = 8;  // at most; RolloutArgs::policy_warps x 4 envs are used
 constexpr int QK_ROLE_DYN = 8, QK_ROLE_AUX = 9, QK_ROLE_IDLE = 15;

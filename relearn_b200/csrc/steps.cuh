@@ -2,8 +2,8 @@
 // OnlineStepsSummary sums (simulation/summary.rs:198-216), VecBuffer::end_experience -> finalize_last_episode
 // (agents/buffers/mod.rs:237-261), the deterministic reduction of the sums into the caller's summary, and the actor's
 // categorical / greedy action choice.  Each kernel keeps its own step loop and stores; the rules and the data format
-// live here.  K2z / K2q (rollout_ws5.cuh, rollout_ws6.cuh) spell finalize_last_episode out themselves: with the helper,
-// ptxas schedules their step loops differently.
+// live here.  K2q (rollout_ws6.cuh) spells finalize_last_episode out itself: with the helper, ptxas schedules its
+// step loops differently.
 #pragma once
 
 #include <cstdint>

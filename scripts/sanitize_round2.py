@@ -1,6 +1,6 @@
 """Small runs of the kernels added in round 2 for compute-sanitizer
 (`compute-sanitizer --tool memcheck|racecheck|synccheck python scripts/sanitize_round2.py`): the warp-specialised
-rollouts K2z / K2q (ragged last CTA, slack, step-limit Interrupts), a rollout and the update passes through a module with
+rollout K2q (ragged last CTA, slack, step-limit Interrupts), a rollout and the update passes through a module with
 two hidden layers, the UCB1 actor / fold, rl_pack_history."""
 import os
 import sys
@@ -14,8 +14,8 @@ from relearn_b200 import _lib as L
 ctx = R.Context(0)
 rng = np.random.default_rng(0)
 cfg = R.CartPoleConfig().wrap(R.VisibleStepLimit(9))
-# K2z (E <= 16 per SM), K2q with 28-env CTAs and with 32-env CTAs (E > 28 per SM); every last CTA ragged
-for E in (37, 2400, 4700):
+# K2q with one policy warp (4-env CTAs), five (20-env CTAs) and eight (32-env CTAs); every last CTA ragged
+for E in (37, 2401, 4700):
     env = R.build_env(ctx, cfg, E, seed=2, lane_offset=3)
     net = R.Mlp(ctx, 5, [128], 2)
     net.set_weights(R.init_params(rng, 5, 128, 2))

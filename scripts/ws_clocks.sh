@@ -1,7 +1,7 @@
 #!/bin/bash
-# Per-phase clocks of the K2z / K2q dynamics and policy loops (measurement build: rollout.cu compiled with -DRL_WS_CLOCKS into
-# build/clk/librelearn_b200.so, swapped in for the duration of this script).  The env count picks the kernel: K2z up to 16
-# envs per SM (E = 1024), K2q beyond (E = 4096).  usage: bash scripts/ws_clocks.sh <tag> [env counts]
+# Per-phase clocks of the K2q dynamics and policy loops (measurement build: rollout.cu compiled with -DRL_WS_CLOCKS into
+# build/clk/librelearn_b200.so, swapped in for the duration of this script).  The env count sets K2q's shape: 2 policy
+# warps per CTA at E = 1024, 7 at E = 4096.  usage: bash scripts/ws_clocks.sh <tag> [env counts]
 # Build it first (here, after __graft_entry__.build()):
 #   mkdir -p build/clk && nvcc -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -Xcompiler -fPIC -DRL_WS_CLOCKS \
 #       -c relearn_b200/csrc/rollout.cu -o build/clk/rollout.o

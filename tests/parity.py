@@ -216,7 +216,9 @@ def smoke_check():
     env.set_noise_replay(words, None)
     actions = rng.integers(0, 2, size=(T, E), dtype=np.uint8)
     traj = R.Trajectory(env, T)
+    n0 = ctx.launch_count
     summ = R.rollout(env, R.ActorSpec(kind=L.RL_ACTOR_REPLAY_ACTIONS, actions=actions), R.HistoryDataBound(T, 0), traj)
+    assert ctx.launch_count - n0 >= 2  # the rollout kernel and rollout_finalize_kernel
     host = traj.to_host()
     ref = oracle_rollout(cfg, E, T, 0, actor_kind=O.ACTOR_REPLAY, actions=actions, env_words=words)
     compare_traj(host, ref, obs_rtol=1e-6, obs_atol=1e-7, what="smoke")
@@ -226,7 +228,8 @@ def smoke_check():
     net = R.Mlp(ctx, 5, [128], 2)
     net.set_weights(params)
     env.set_noise_philox(7, 0)
+    n1 = ctx.launch_count
     summ = R.rollout(env, R.ActorSpec(kind=L.RL_ACTOR_CATEGORICAL_POLICY, net=net), R.HistoryDataBound(T, 0), traj)
     assert summ.step_reward.count == E * T
-    assert ctx.launch_count >= 4
+    assert ctx.launch_count - n1 >= 1  # K2q, which sums the statistics itself
     ctx.close()

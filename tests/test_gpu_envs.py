@@ -403,13 +403,16 @@ def test_fused_rollout_policy_other_envs_consistent(ctx, cfg):
 
 @pytest.mark.parametrize("E,T,slack,limit,visible", [(4096, 64, 0, 500, True), (1000, 70, 9, 20, True), (37, 45, 3, 15, False),
                                                      (16, 33, 0, 500, True), (300, 50, 2, 0, False),
-                                                     # K2q (E > 2368): 28-env CTAs with a ragged last one, 32-env CTAs
+                                                     # a ragged last CTA with each count of policy warps (148 SMs: 1 at
+                                                     # E = 37, 2 .. 6 at 1001 .. 3401, 7 at 4096, 8 at 4700)
+                                                     (1001, 36, 4, 11, True), (1501, 40, 0, 13, False), (2367, 30, 6, 9, True),
+                                                     (2901, 34, 2, 0, False), (3401, 28, 3, 17, False),
                                                      (2400, 40, 5, 20, True), (4700, 33, 0, 15, False), (4736, 21, 2, 9, True),
-                                                     (5000, 20, 3, 9, True), (9472, 12, 0, 500, True),  # two waves of K2q
+                                                     (5000, 20, 3, 9, True), (9472, 12, 0, 500, True),  # two waves
                                                      (12000, 12, 2, 9, True)])  # past two waves, ragged last CTA
 def test_warp_specialized_rollout_is_bit_identical_to_k2c(ctx, E, T, slack, limit, visible):
-    """The warp-specialised kernels `RL_LANES_WARP_SPECIALIZED` picks by size (K2z up to 2368 envs, K2q beyond: policy and
-    dynamics of an env on different warps, hand-off through named barriers) perform the same
+    """K2q, the warp-specialised kernel `RL_LANES_WARP_SPECIALIZED` runs (policy and dynamics of an env on different warps,
+    hand-off through named barriers; 1 to 8 policy warps per CTA by size), performs the same
     operations on the same operands as K2c with 8 threads per env: under Philox noise every stored byte, the lane
     lengths and the summary must be identical -- ragged last CTA, slack, step-limit Interrupts, latent limit (F = 4),
     resets, dangling steps."""
@@ -481,7 +484,7 @@ def test_set_weights_async_from_pinned_memory(ctx):
 
 
 def test_warp_specialized_rollout_against_the_oracle(ctx):
-    """K2z (200 envs) directly against the CPU oracle under production noise: (i) replaying its actions through the oracle, which
+    """K2q (200 envs: one policy warp per CTA) directly against the CPU oracle under production noise: (i) replaying its actions through the oracle, which
     regenerates the Philox reset draws itself, reproduces the trajectory (Terminate / Interrupt codes, lane lengths and
     summary exactly, CartPole observations to 1e-6: sin/cos differ from glibc by <= 1 ulp); (ii) every action is the
     inverse-CDF choice of the oracle's softmax for the recorded observation and the step's Philox uniform."""
@@ -497,7 +500,7 @@ def test_warp_specialized_rollout_against_the_oracle(ctx):
     host = traj.to_host()
     ref = P.oracle_rollout(CARTPOLE, E, T, slack, actor_kind=O.ACTOR_REPLAY, actions=host["action"].copy(), philox_seed=seed,
                            lane_offset=off, t0=t0)
-    P.compare_traj(host, ref, obs_rtol=1e-6, obs_atol=1e-7, what="K2z vs oracle")
+    P.compare_traj(host, ref, obs_rtol=1e-6, obs_atol=1e-7, what="K2q vs oracle")
     P.compare_summary(summ, ref["summary"])
     lib = L.lib()
     awords = np.array([[lib.rl_philox_slot(seed, off + e, t0 + i, 2, 0) & 0xFFFFFFFF for i in range(T + slack)] for e in range(E)],

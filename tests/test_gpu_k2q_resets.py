@@ -1,4 +1,4 @@
-"""K2q (the warp-specialised CartPole rollout past 16 envs per SM) against K2c with 8 threads per env where episodes
+"""K2q (the warp-specialised CartPole rollout) against K2c with 8 threads per env where episodes
 end all the time: a reset after the very first step, episodes ending on consecutive steps, step-limit Interrupts on
 every step or every other step, terminations of the bare env under a saturated policy.  K2q steps the state on a
 dynamics warp from a reset state the aux warp drew ahead into a ring and hands it to the policy warps through named
@@ -14,6 +14,8 @@ pytestmark = pytest.mark.gpu
 
 @pytest.mark.parametrize("E,T,slack,limit,visible,gain", [
     (2400, 24, 0, 1, True, 2.0),     # every step ends its episode: a reset after step 0 and after every step
+    (37, 24, 0, 1, True, 2.0),       # the same with one policy warp per CTA (4-env CTAs, ragged last one)
+    (1501, 30, 4, 2, True, 2.0),     # three policy warps, each on a sub-partition of its own; ragged last CTA, slack
     (2405, 30, 4, 2, True, 2.0),     # ragged last CTA, slack, episodes of two steps
     (4096, 48, 3, 0, False, 6.0),    # the bench size, bare env: episodes end by Terminate only (a saturated policy)
     (4096, 40, 0, 3, False, 6.0),    # latent limit (F = 4), Interrupts and Terminates mixed

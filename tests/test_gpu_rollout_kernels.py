@@ -2,7 +2,7 @@
 
 `rl_rollout` picks a kernel from the env, the module's shape and activation, `lanes_per_env`, the actor, the noise mode
 and the env count (rollout.cu: K2a thread per env, K2g GL threads per env, K2b / K2c CartPole with L threads per env, K2t
-tensor cores, K2z / K2q warp-specialised).  Each case below names the kernel its inputs select, runs one or two
+tensor cores, K2q warp-specialised).  Each case below names the kernel its inputs select, runs one or two
 collection periods and checks them against the oracle, never against a sibling kernel:
 
 * replaying the kernel's own actions through the oracle reproduces the trajectory: lane lengths, successor codes (RL_PAD
@@ -157,8 +157,8 @@ def _build_cases():
                  philox=True, lanes=8, T=40, slack=5),
             Case(f"limit{limit}-K2t", f"rollout_cartpole_tc_kernel<false, {CAT}, true>", cfg, 1000, (128,), "relu", CAT,
                  philox=True, lanes=TC, T=40, slack=5),
-            Case(f"limit{limit}-K2z", "rollout_cartpole_ws5_kernel", cfg, 1000, (128,), "relu", CAT, philox=True, lanes=WS,
-                 T=40, slack=5),
+            Case(f"limit{limit}-K2q-E1000", "rollout_cartpole_ws6_kernel", cfg, 1000, (128,), "relu", CAT, philox=True,
+                 lanes=WS, T=40, slack=5),
             Case(f"limit{limit}-K2q", "rollout_cartpole_ws6_kernel", cfg, 4096, (128,), "relu", CAT, philox=True, lanes=WS,
                  T=40, slack=5),
         ]
